@@ -12,7 +12,7 @@ is computed once and excluded, as in the reference (src/bin/main.rs:130-139 vs :
 inputs resident in HBM, `e2e` times the same call through the host-buffer C ABI entry point (H2D and D2H inside the
 timed region).  Every run decrypts its outputs and checks them against clear AES.
 
-One JSON line is printed by rank 0.
+One JSON line is printed by rank 0.  `--dump-outputs DIR` also writes what the last timed step returned (see dump_outputs).
 """
 import argparse
 import importlib
@@ -27,6 +27,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                                   # the tree may be read-only: bench.py writes nothing into it
 
 METRIC = "fhe_aes128_ctr_blocks_per_s"
 SEED = 2026
@@ -80,6 +81,26 @@ def _sbox():
 
 def counter_blocks(first_ctr, n):
     return [CLI_IV + (first_ctr + i).to_bytes(8, "big") for i in range(n)]          # reference main.rs:108-115
+
+
+DUMP_CTS = 1024                                                  # sampled output ciphertexts: 1024 x 2049 words = 16.8 MB
+
+
+def dump_outputs(path, ck, out):
+    """Writes what the timed path returned in its last step, so that two builds can be compared output for output (keys and
+    inputs are seeded, hence identical from run to run).  Torus words are stored as signed fractions of the torus, w / 2^64.
+      out_phases.npy       [blocks][16][8] float64  decrypted phase of every output bit ciphertext (secret key of the seed);
+                                                    two correct builds agree on it to within the noise, whatever their f64 order
+      out_ciphertexts.npy  [<=1024][2049] float64   the output LWE ciphertexts of a fixed sample of bits: rows
+                                                    sorted(default_rng(SEED).choice(blocks*128, 1024, replace=False)) of the
+                                                    [blocks*128][2049] output (all of it is 268 MB at 128 blocks)"""
+    os.makedirs(path, exist_ok=True)
+    L1 = ck.params.big_lwe_size
+    flat = out.reshape(-1, L1)
+    phases = ck.decrypt_phases(flat).view(np.int64).reshape(out.shape[:-1])
+    rows = np.sort(np.random.default_rng(SEED).choice(flat.shape[0], min(DUMP_CTS, flat.shape[0]), replace=False))
+    np.save(os.path.join(path, "out_phases.npy"), phases.astype(np.float64) * 2.0**-64)
+    np.save(os.path.join(path, "out_ciphertexts.npy"), flat[rows].view(np.int64).astype(np.float64) * 2.0**-64)
 
 
 class ClockSampler:
@@ -334,6 +355,8 @@ def run_gpu(args):
     # decrypt-verify this rank's outputs against clear AES (every block)
     got = out_dev.cpu().numpy().view(np.uint64)
     ok = all(ck.decrypt_bytes(got[i]) == clear_aes(CLI_KEY, blocks_clear[i]) for i in range(nb))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ck, got)
 
     # ---- end-to-end timing through the host-buffer entry point (pinned host memory, H2D + D2H inside)
     e2e_steps = max(1, args.steps)
@@ -464,7 +487,12 @@ def main():
     ap.add_argument("--blocks", type=int, default=int(os.environ.get("TAC_BENCH_BLOCKS", "128")), help="AES blocks per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-key-expansion", action="store_true", help="skip the FHE key-schedule timer")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0's blocks) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     if args.impl == "reference":
         run_reference(args)
     else:
