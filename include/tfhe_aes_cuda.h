@@ -150,6 +150,21 @@ int tac_aes_key_schedule_buffer(tac_ctx* ctx, void** dev_ptr, size_t* bytes);   
  * (1 for fresh).  Returns TAC_ERR_NOISE where the reference would panic with NoiseTooBig. */
 int tac_aes_encrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host);
 int tac_aes_encrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_dev, uint64_t* out_dev);
+/* Aes128Encrypt::encrypt_block_for_rounds over PUBLIC 16-byte blocks (e.g. AES-CTR counter blocks iv ‖ BE64(ctr),
+ * main.rs:108-115) under the device key schedule: state0 = k0 ⊕ trivial(block), no input ciphertexts.  Circuit bootstraps
+ * whose inputs are equal across blocks run once: byte j of two blocks shares the round-r S-box when the blocks agree on the
+ * input bytes that byte depends on (D(1, j) = {j}, then ShiftRows + MixColumns spread it: a diagonal in round 2, all 16
+ * bytes from round 3 on).  Same round structure as tac_aes_encrypt_blocks, including rk10 in the final round.
+ *   blocks_host: [n_blocks][16] bytes.  xor_host: NULL, or [n_blocks][16] public bytes XORed into the output — AES-CTR
+ *   transciphering: pass the AES-CTR ciphertext and the output encrypts the plaintext.  Both are HOST memory in both
+ *   variants.  out: [n_blocks][16][8][kN+1].
+ * Output bits carry squared noise level 8 + 1 = 9, as on the encrypted-block path; identical public blocks give
+ * word-identical outputs, and the output equals tac_aes_encrypt_blocks on trivial encryptions of the same blocks. */
+int tac_aes_encrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host);
+int tac_aes_encrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev);
+/* circuit-bootstrapped S-box boxes per round that tac_aes_encrypt_public_blocks runs for these blocks: boxes[r-1],
+ * r = 1..rounds (16·n_blocks each without sharing).  Host only, needs no context or GPU. */
+int tac_aes_public_plan(int n_blocks, int rounds, const uint8_t* blocks_host /*[n][16]*/, int64_t* boxes);
 
 /* ------------------------------------------------------------------ single stages (parity tests, profiling) */
 /* [U] keyswitch_lwe_ciphertext: [n_cts][kN+1] → [n_cts][n+1] */

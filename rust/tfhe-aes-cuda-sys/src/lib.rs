@@ -99,6 +99,9 @@ extern "C" {
     pub fn tac_aes_key_schedule_buffer(ctx: *mut tac_ctx, dev_ptr: *mut *mut c_void, bytes: *mut usize) -> c_int;
     pub fn tac_aes_encrypt_blocks(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, in_noise_sq: c_int, in_host: *const u64, out_host: *mut u64) -> c_int;
     pub fn tac_aes_encrypt_blocks_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, in_noise_sq: c_int, in_dev: *const u64, out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_encrypt_public_blocks(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, blocks_host: *const u8, xor_host: *const u8, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_encrypt_public_blocks_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, blocks_host: *const u8, xor_host: *const u8, out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_public_plan(n_blocks: c_int, rounds: c_int, blocks_host: *const u8, boxes: *mut i64) -> c_int;
 
     // single stages, profiling
     pub fn tac_stage_keyswitch(ctx: *mut tac_ctx, n_cts: c_int, in_host: *const u64, out_host: *mut u64) -> c_int;

@@ -99,6 +99,9 @@ _SIGNATURES = {
     "tac_aes_key_schedule_buffer": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]),
     "tac_aes_encrypt_blocks": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "tac_aes_encrypt_blocks_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "tac_aes_encrypt_public_blocks": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_encrypt_public_blocks_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_public_plan": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "tac_stage_keyswitch": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
     "tac_extract_bits": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _u64p, _u64p]),
     "tac_stage_pbs": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
@@ -207,6 +210,39 @@ def key_file_info(path):
     if load_library().tac_keys_load_params(os.fsencode(path), C.byref(p), C.byref(mask)) != 0:
         raise OSError(f"{path}: not a key file")
     return p, {i for i in range(32) if mask.value >> i & 1}
+
+
+def _public_blocks(blocks):
+    """[n][16] uint8 from an array, a list of 16-byte strings or one byte string of 16·n bytes"""
+    if isinstance(blocks, (bytes, bytearray, memoryview)):
+        blocks = np.frombuffer(bytes(blocks), dtype=np.uint8)
+    elif not isinstance(blocks, np.ndarray):
+        blocks = np.frombuffer(b"".join(bytes(b) for b in blocks), dtype=np.uint8)
+    b = np.ascontiguousarray(blocks, dtype=np.uint8)
+    if b.size % 16:
+        raise ValueError("public blocks must be whole 16-byte blocks")
+    return b.reshape(-1, 16)
+
+
+def ctr_blocks(iv, first_ctr, n):
+    """AES-CTR counter blocks iv ‖ BE64(first_ctr + i), i < n (reference main.rs:108-115): [n][16] uint8"""
+    iv = bytes(iv)
+    if len(iv) != 8:
+        raise ValueError("iv must be 8 bytes")
+    if n < 0 or first_ctr < 0 or first_ctr + n > 1 << 64:
+        raise ValueError("counter range must lie in [0, 2^64)")
+    return _public_blocks(b"".join(iv + (first_ctr + i).to_bytes(8, "big") for i in range(n)))
+
+
+def aes_public_plan(blocks, rounds=10):
+    """circuit bootstraps per round that FheContext.aes_encrypt_public_blocks runs for these public blocks (rounds 1..rounds);
+    16 per block and round without sharing.  Host only."""
+    b = _public_blocks(blocks)
+    out = np.zeros(max(rounds, 0), dtype=np.int64)
+    rc = load_library().tac_aes_public_plan(b.shape[0], rounds, b.ctypes.data, out.ctypes.data)
+    if rc != 0:
+        raise ValueError(f"aes_public_plan: rounds must be in 1..10 (error {rc})")
+    return [int(v) for v in out]
 
 
 class LookupTable:
@@ -584,6 +620,44 @@ class FheContext(NoiseContext):
 
     def aes_encrypt_blocks_dev(self, n_blocks, in_ptr, out_ptr, rounds=10, in_noise_sq=1):
         self._check(self.L.tac_aes_encrypt_blocks_dev(self.h, n_blocks, rounds, in_noise_sq, C.c_void_p(in_ptr), C.c_void_p(out_ptr)))
+
+    # -- AES over public blocks: AES-CTR keystream and transciphering
+    def _public_args(self, blocks, xor):
+        b = _public_blocks(blocks)
+        x = None
+        if xor is not None:
+            x = _public_blocks(xor)
+            if x.shape != b.shape:
+                raise ValueError("xor must hold one 16-byte row per block")
+        return b, x
+
+    def aes_encrypt_public_blocks(self, blocks, rounds=10, xor=None):
+        """AES of public 16-byte blocks under the device key schedule; xor: optional public bytes [n][16] XORed into the
+        output.  Returns [n][16][8][big+1] bit ciphertexts (squared noise level 9)."""
+        b, x = self._public_args(blocks, xor)
+        out = np.empty((b.shape[0], 16, 8, self.params.big_lwe_size), dtype=np.uint64)
+        self._check(self.L.tac_aes_encrypt_public_blocks(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
+                                                         out.ctypes.data))
+        return out
+
+    def aes_encrypt_public_blocks_dev(self, blocks, out_ptr, rounds=10, xor=None):
+        """the same into device memory out_ptr ([n][16][8][big+1] words), enqueued on the context's stream"""
+        b, x = self._public_args(blocks, xor)
+        self._check(self.L.tac_aes_encrypt_public_blocks_dev(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
+                                                             C.c_void_p(out_ptr)))
+
+    def aes_ctr_keystream(self, iv, first_ctr, n_blocks):
+        """FHE encryptions of the AES-CTR keystream blocks AES(k, iv ‖ BE64(first_ctr + i)): [n_blocks][16][8][big+1]"""
+        return self.aes_encrypt_public_blocks(ctr_blocks(iv, first_ctr, n_blocks))
+
+    def aes_ctr_transcipher(self, iv, first_ctr, data):
+        """Transciphering: `data` is an AES-CTR ciphertext under the FHE-encrypted key (nonce iv ‖ BE64(first_ctr)); returns
+        FHE encryptions of its plaintext bits, [len(data)][8][big+1]."""
+        data = bytes(data)
+        n = (len(data) + 15) // 16
+        padded = data + bytes(16 * n - len(data))
+        out = self.aes_encrypt_public_blocks(ctr_blocks(iv, first_ctr, n), xor=padded)
+        return out.reshape(16 * n, 8, self.params.big_lwe_size)[:len(data)]
 
     def aes_key_schedule_buffer(self):
         ptr, nbytes = C.c_void_p(), C.c_size_t()

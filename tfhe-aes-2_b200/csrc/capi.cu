@@ -3,6 +3,7 @@
 // no usable CUDA device.
 #include "../../include/tfhe_aes_cuda.h"
 #include "kernels_common.cuh"
+#include "aes_plan.h"
 #include "kernels_gemm_umma.cuh"
 #include "ep_step.cuh"
 #include "shape_launch.h"
@@ -88,6 +89,7 @@ struct tac_ctx {
     uint64_t* rc_rows = nullptr;     // trivial(RC[1..10]) as byte ciphertexts [10][8][kN+1], uploaded once
     // workspace
     DevBuf ws_in, ws_out, ws_small, ws_ksdig, ws_pbs, ws_pfdig, ws_ggsw, ws_ggswf, ws_tree_a, ws_tree_b, ws_state, ws_muls, ws_misc;
+    DevBuf ws_plan, ws_rep;          // public-block AES: uploaded plan tables / public bytes, compact S-box inputs
     size_t max_cts = 16384;
     uint32_t fix_cap = kFixCap;      // capacity of the PFKS tie list in use (TAC_FIX_CAP lowers it: exercises the overflow path)
     // profiling: one event tuple per pipeline pass, recorded without synchronising; read back by tac_ctx_stage_times
@@ -374,6 +376,15 @@ int ensure_aes_luts(tac_ctx* ctx) {
     return TAC_OK;
 }
 
+// static squared-noise bookkeeping of the AES circuit (NoiseLevelWithComponents::add_assign, shortint_woppbs_1bit.rs:63-77):
+// round keys are fresh or bootstrapped (level 1); SBOX outputs carry 8·NOMINAL (:325)
+int aes_noise_check(tac_ctx* ctx, int in_noise_sq, int rounds) {
+    const int maxn = ctx->p.max_noise_sq;
+    if (in_noise_sq + 1 > maxn || (rounds > 1 && 4 * 8 + 1 > maxn) || 8 + 1 > maxn)
+        return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: the AES circuit needs max_noise_level_squared >= 33");
+    return TAC_OK;
+}
+
 }  // namespace
 
 // =================================================================================================== C ABI
@@ -422,7 +433,7 @@ void tac_ctx_destroy(tac_ctx* ctx) {
         if (p) cudaFree(p);
     for (auto& l : ctx->luts) cudaFree(l.dev);
     for (DevBuf* b : {&ctx->ws_in, &ctx->ws_out, &ctx->ws_small, &ctx->ws_ksdig, &ctx->ws_pbs, &ctx->ws_pfdig, &ctx->ws_ggsw, &ctx->ws_ggswf,
-                      &ctx->ws_tree_a, &ctx->ws_tree_b, &ctx->ws_state, &ctx->ws_muls, &ctx->ws_misc})
+                      &ctx->ws_tree_a, &ctx->ws_tree_b, &ctx->ws_state, &ctx->ws_muls, &ctx->ws_misc, &ctx->ws_plan, &ctx->ws_rep})
         if (b->p) cudaFree(b->p);
     for (auto& r : ctx->prof_pool) for (auto& ev : r.ev) cudaEventDestroy(ev);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -754,11 +765,7 @@ int tac_aes_encrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_no
     if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
     if (n_blocks < 0 || rounds < 1 || rounds > 10) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range");
     if (n_blocks == 0) return TAC_OK;
-    // static squared-noise bookkeeping (NoiseLevelWithComponents::add_assign, shortint_woppbs_1bit.rs:63-77): round keys
-    // are fresh or bootstrapped (level 1); SBOX outputs carry 8·NOMINAL (:325)
-    const int maxn = ctx->p.max_noise_sq;
-    if (in_noise_sq + 1 > maxn || (rounds > 1 && 4 * 8 + 1 > maxn) || 8 + 1 > maxn)
-        return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: the AES circuit needs max_noise_level_squared >= 33");
+    TRY(aes_noise_check(ctx, in_noise_sq, rounds));
     TRY(ensure_aes_luts(ctx));
     const size_t L = (size_t)ctx->big() + 1, blk = 16 * 8 * L;
     const size_t total = (size_t)n_blocks * blk;
@@ -771,11 +778,11 @@ int tac_aes_encrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_no
     TRY(post_launch(ctx, "aes_add_round_key_kernel"));
     for (int rd = 1; rd < rounds; rd++) {
         TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut24], n_blocks * 16, state, muls));                          // sub_bytes_with_gal_mul :27-48
-        aes_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)rd * blk, (int)L, total, state);
+        aes_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)rd * blk, (int)L, total, state, nullptr);
         TRY(post_launch(ctx, "aes_mix_columns_kernel"));
     }
     TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut8], n_blocks * 16, state, muls));                               // sub_bytes :51-58
-    aes_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)10 * blk, (int)L, total, out_dev);
+    aes_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)10 * blk, (int)L, total, out_dev, nullptr, nullptr);
     return post_launch(ctx, "aes_final_round_kernel");
 }
 int tac_aes_encrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host) {
@@ -787,6 +794,94 @@ int tac_aes_encrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_
     TRY(ensure(ctx, ctx->ws_out, bytes));
     CU(cudaMemcpyAsync(ctx->ws_in.p, in_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
     TRY(tac_aes_encrypt_blocks_dev(ctx, n_blocks, rounds, in_noise_sq, ctx->ws_in.as<uint64_t>(), ctx->ws_out.as<uint64_t>()));
+    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return TAC_OK;
+}
+
+// AES over PUBLIC blocks (aes_plan.h): the round structure of tac_aes_encrypt_blocks_dev with state0 = k0 + trivial(block).
+// Each round bootstraps only the plan's representatives, in one compact batch, and MixColumns / the final round read every
+// position's S-box row through the plan's index table.  Rounds whose plan is the identity (all blocks distinct from
+// round 3 on) run on the full state in place, as the encrypted-block path does.
+int tac_aes_encrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
+    std::vector<AesRoundPlan> plan;
+    if (aes_public_plan_build(n_blocks, rounds, blocks_host, plan)) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range, or NULL blocks");
+    if (n_blocks == 0) return TAC_OK;
+    TRY(aes_noise_check(ctx, 0, rounds));                  // trivial input: no noise of its own
+    TRY(ensure_aes_luts(ctx));
+    const size_t L = (size_t)ctx->big() + 1, byte_words = 8 * L, blk = 16 * byte_words;
+    const size_t npos = (size_t)n_blocks * 16, total = (size_t)n_blocks * blk;
+    // one upload: public blocks, XOR bytes, then rep_pos / idx of every round that shares
+    std::vector<size_t> off_rep(rounds, 0), off_idx(rounds, 0);
+    size_t bytes = 2 * npos, max_rep = plan[0].identity ? 0 : (size_t)plan[0].boxes;
+    for (int r = 0; r < rounds; r++) {
+        if (plan[r].identity) continue;
+        off_rep[r] = bytes; bytes += (size_t)plan[r].boxes * 4;
+        off_idx[r] = bytes; bytes += npos * 4;
+        max_rep = std::max(max_rep, (size_t)plan[r].boxes);
+    }
+    std::vector<uint8_t> host(bytes, 0);
+    std::memcpy(host.data(), blocks_host, npos);
+    if (xor_host) std::memcpy(host.data() + npos, xor_host, npos);
+    for (int r = 0; r < rounds; r++) {
+        if (plan[r].identity) continue;
+        std::memcpy(host.data() + off_rep[r], plan[r].rep_pos.data(), (size_t)plan[r].boxes * 4);
+        std::memcpy(host.data() + off_idx[r], plan[r].idx.data(), npos * 4);
+    }
+    TRY(ensure(ctx, ctx->ws_plan, bytes));
+    TRY(ensure(ctx, ctx->ws_state, total * 8));
+    TRY(ensure(ctx, ctx->ws_muls, total * 3 * 8));
+    TRY(ensure(ctx, ctx->ws_rep, std::max<size_t>(1, max_rep) * byte_words * 8));
+    // pageable source: the call returns once the bytes are staged, so `host` may go out of scope before the copy lands
+    CU(cudaMemcpyAsync(ctx->ws_plan.p, host.data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
+    const uint8_t* d_plan = ctx->ws_plan.as<uint8_t>();
+    auto rep_pos = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_rep[r]); };
+    auto idx = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_idx[r]); };
+    uint64_t* state = ctx->ws_state.as<uint64_t>();
+    uint64_t* muls = ctx->ws_muls.as<uint64_t>();
+    uint64_t* rep = ctx->ws_rep.as<uint64_t>();
+    const int g = grid1d(total, 256, ctx->sm_count);
+    // S-box inputs of round rd (1-based) for its representatives → `in`
+    auto sbox_inputs = [&](int rd, const uint64_t** in) -> int {
+        const int r = rd - 1;
+        const size_t n_words = (size_t)plan[r].boxes * byte_words;
+        if (rd == 1) {
+            uint64_t* dst = plan[r].identity ? state : rep;
+            aes_public_round1_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->key_sched, d_plan, rep_pos(r), (int)L, n_words, dst);
+            TRY(post_launch(ctx, "aes_public_round1_kernel"));
+            *in = dst;
+        } else if (plan[r].identity) {
+            *in = state;
+        } else {
+            aes_gather_bytes_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(state, rep_pos(r), (int)L, n_words, rep);
+            TRY(post_launch(ctx, "aes_gather_bytes_kernel"));
+            *in = rep;
+        }
+        return TAC_OK;
+    };
+    const uint64_t* in = nullptr;
+    for (int rd = 1; rd < rounds; rd++) {
+        TRY(sbox_inputs(rd, &in));
+        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut24], (int)plan[rd - 1].boxes, in, muls));
+        aes_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)rd * blk, (int)L, total, state, idx(rd - 1));
+        TRY(post_launch(ctx, "aes_mix_columns_kernel"));
+    }
+    TRY(sbox_inputs(rounds, &in));
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut8], (int)plan[rounds - 1].boxes, in, muls));
+    aes_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)10 * blk, (int)L, total, out_dev, idx(rounds - 1),
+                                                      xor_host ? d_plan + npos : nullptr);
+    return post_launch(ctx, "aes_final_round_kernel");
+}
+int tac_aes_encrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
+    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
+    TRY(ensure(ctx, ctx->ws_out, bytes));
+    TRY(tac_aes_encrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, ctx->ws_out.as<uint64_t>()));
     CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return TAC_OK;

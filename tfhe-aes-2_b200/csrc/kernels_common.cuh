@@ -4,7 +4,8 @@
 //   pfks_digits_kernel     digits of the private functional packing keyswitch for the integer-pipe GEMM (base_log > 16)
 //   lwe_gemm_kernel        exact integer GEMM mod 2^64 on the integer pipe: out[ct][col] = corr[col] − Σ_k digit'[ct][k]·key[k][col]
 //                          (PFKS of params_sqrd_lvl_1, and the correction rows of both keyswitches at key upload)
-//   aes_*_kernel           AddRoundKey / ShiftRows+MixColumns+AddRoundKey / final round as gather-adds on the flat state
+//   aes_*_kernel           AddRoundKey / ShiftRows+MixColumns+AddRoundKey / final round as gather-adds on the flat state;
+//                          round-1 inputs and representative gathers of the public-block path
 //   lwe_add_kernel         leveled XOR (lwe_ciphertext_add_assign) over a batch; lwe_shl_kernel / lwe_sub_kernel: glue of extract_bits
 //   negate_kernel, dfma_peak_kernel   key-upload helper, FP64 peak microbenchmark (roofline denominator)
 #pragma once
@@ -95,32 +96,66 @@ __global__ void aes_add_round_key_kernel(const uint64_t* __restrict__ in, const 
 }
 // ShiftRows on the three SBOX·{1,2,3} states + MixColumns + AddRoundKey (fhe_sbox_gal_mul_pbs.rs:61-82, :106-117)
 //   new[r][c] = mul2[r] ^ mul1[r-1] ^ mul1[r-2] ^ mul3[r-3]  (rows mod 4, within shifted column c)
-// muls: [block][byte][24 = (S, 2S, 3S) × 8 bits][L]
+// muls: [row][24 = (S, 2S, 3S) × 8 bits][L], row = block·16 + byte, or idx[block·16 + byte] when idx is given (a compact
+// batch of S-box outputs shared by several positions: tac_aes_encrypt_public_blocks)
 __global__ void aes_mix_columns_kernel(const uint64_t* __restrict__ muls, const uint64_t* __restrict__ rk, int L, size_t total,
-                                       uint64_t* __restrict__ state) {
+                                       uint64_t* __restrict__ state, const int32_t* __restrict__ idx) {
     const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
         const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;   // bit·L + e
         const int c = byte >> 2, r = byte & 3;
-        const uint64_t* mb = muls + blk * 16 * 24 * (size_t)L;
         auto src = [&](int which, int row) -> uint64_t {
             const int old_byte = 4 * ((c + row) & 3) + row;        // ShiftRows: new[row][c] = old[row][(c+row)%4]
-            return mb[((size_t)old_byte * 24 + (size_t)which * 8) * L + w];
+            const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
+            return muls[(src_row * 24 + (size_t)which * 8) * L + w];
         };
         state[i] = src(1, r) + src(0, (r + 3) & 3) + src(0, (r + 2) & 3) + src(2, (r + 1) & 3) + rk[rem];
     }
 }
-// last round (fhe_sbox_gal_mul_pbs.rs:119-129): ShiftRows(sub) + rk[40..44]
+// last round (fhe_sbox_gal_mul_pbs.rs:119-129): ShiftRows(sub) + rk[40..44].  sub rows as in aes_mix_columns_kernel
+// ([row][8 bits][L], idx optional).  xr: NULL, or [block][16] public bytes XORed into the output (a trivial ciphertext
+// added: encode_bit(1) = 2^63 on the body of every set bit).
 __global__ void aes_final_round_kernel(const uint64_t* __restrict__ sub, const uint64_t* __restrict__ rk, int L, size_t total,
-                                       uint64_t* __restrict__ out) {
+                                       uint64_t* __restrict__ out, const int32_t* __restrict__ idx,
+                                       const uint8_t* __restrict__ xr) {
     const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
         const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;
         const int c = byte >> 2, r = byte & 3;
         const int old_byte = 4 * ((c + r) & 3) + r;
-        out[i] = sub[blk * blk_words + (size_t)old_byte * byte_words + w] + rk[rem];
+        const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
+        uint64_t v = sub[src_row * byte_words + w] + rk[rem];
+        if (xr) {
+            const int bit = (int)(w / L);
+            if (w - (size_t)bit * L == (size_t)L - 1 && (xr[blk * 16 + byte] & (0x80 >> bit))) v += 1ull << 63;
+        }
+        out[i] = v;
+    }
+}
+// S-box inputs of round 1 over public blocks, one per representative k: k0[byte] + trivial(value), i.e. the key-schedule
+// byte with encode_bit(1) = 2^63 added to the body of every set bit of the public byte (Byte::trivial, data_model.rs:35-43).
+// rep_pos[k] = block·16 + byte (NULL: k itself); out [k][8 bits][L]
+__global__ void aes_public_round1_kernel(const uint64_t* __restrict__ k0, const uint8_t* __restrict__ blocks, const int32_t* __restrict__ rep_pos,
+                                         int L, size_t total, uint64_t* __restrict__ out) {
+    const size_t byte_words = (size_t)8 * L;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t k = i / byte_words; const size_t w = i - k * byte_words;
+        const int pos = rep_pos ? rep_pos[k] : (int)k;
+        const int bit = (int)(w / L);
+        uint64_t v = k0[(size_t)(pos & 15) * byte_words + w];
+        if (w - (size_t)bit * L == (size_t)L - 1 && (blocks[pos] & (0x80 >> bit))) v += 1ull << 63;
+        out[i] = v;
+    }
+}
+// the representatives' S-box inputs out of the full state: out[k] = state[rep_pos[k]], 8·L words each
+__global__ void aes_gather_bytes_kernel(const uint64_t* __restrict__ state, const int32_t* __restrict__ rep_pos, int L, size_t total,
+                                        uint64_t* __restrict__ out) {
+    const size_t byte_words = (size_t)8 * L;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t k = i / byte_words; const size_t w = i - k * byte_words;
+        out[i] = state[(size_t)rep_pos[k] * byte_words + w];
     }
 }
 // leveled XOR (BitXorAssign, shortint_woppbs_1bit.rs:134-142 → lwe_ciphertext_add_assign): a += b, element-wise

@@ -392,6 +392,20 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
             res[q][b][i] = BitCt::with_noise_level(std::vector<uint64_t>(out.begin() + ((q * 16 + b) * 8 + i) * L, out.begin() + ((q * 16 + b) * 8 + i + 1) * L), 8 + 1, c);
         return res;
     }
+    // AES over public blocks (AES-CTR counter blocks) under the device key schedule, no input ciphertexts; `xor` (empty or
+    // one 16-byte row per block) is XORed into the output — the AES-CTR ciphertext for transciphering
+    static std::vector<data_model::BlockT<Bit>> encrypt_public_blocks(const Ctx& c, const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
+                                                                       const std::vector<std::array<uint8_t, 16>>& xor_bytes = {}) {
+        if (!xor_bytes.empty() && xor_bytes.size() != blocks.size()) throw std::invalid_argument("xor_bytes: one row per block");
+        const size_t L = c.lwe_size();
+        std::vector<uint64_t> out(blocks.size() * 128 * L);
+        c.check(tac_aes_encrypt_public_blocks(c.raw(), (int)blocks.size(), rounds, blocks.empty() ? nullptr : blocks[0].data(),
+                                              xor_bytes.empty() ? nullptr : xor_bytes[0].data(), out.data()));
+        std::vector<data_model::BlockT<Bit>> res(blocks.size());
+        for (size_t q = 0; q < blocks.size(); q++) for (int b = 0; b < 16; b++) for (int i = 0; i < 8; i++)
+            res[q][b][i] = BitCt::with_noise_level(std::vector<uint64_t>(out.begin() + ((q * 16 + b) * 8 + i) * L, out.begin() + ((q * 16 + b) * 8 + i + 1) * L), 8 + 1, c);
+        return res;
+    }
 };
 }  // namespace cuda_woppbs_1bit
 }  // namespace fhe_impls
