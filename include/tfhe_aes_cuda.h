@@ -166,6 +166,35 @@ int tac_aes_encrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, co
  * r = 1..rounds (16·n_blocks each without sharing).  Host only, needs no context or GPU. */
 int tac_aes_public_plan(int n_blocks, int rounds, const uint8_t* blocks_host /*[n][16]*/, int64_t* boxes);
 
+/* ------------------------------------------------------------------ AES decryption (no counterpart in the reference) */
+/* Inverse key schedule dk of the equivalent inverse cipher (FIPS-197 §5.3.5), derived on the device from the resident
+ * encryption schedule w: dk[0..3] = w[0..3], dk[40..43] = w[40..43], dk[4rd..4rd+3] = InvMixColumns(w[4rd..4rd+3]) for
+ * rd = 1..9.  Layout as the key schedule, [44 words][4][8][kN+1]; out_host may be NULL.  Runs 144 circuit bootstraps
+ * 8 → 32 and 1152 of 1 bit; its bits carry squared noise level 1.  TAC_ERR_NOISE below max_noise_level_squared 32.
+ * dk stays valid until the encryption schedule changes: tac_aes_set_key_schedule (and so tac_aes_key_schedule and
+ * tac_aes_key_schedule_buffer) marks it stale, and decryption then fails with TAC_ERR_STATE.  No call derives it
+ * implicitly. */
+int tac_aes_inv_key_schedule(tac_ctx* ctx, uint64_t* inv_key_sched_host);
+/* make a given dk resident (e.g. client-encrypted from a clear InvMixColumns schedule); decryption reads every round key,
+ * dk[0..3] and dk[40..43] included, from dk only */
+int tac_aes_set_inv_key_schedule(tac_ctx* ctx, const uint64_t* inv_key_sched_host);
+/* AES decryption of n_blocks blocks with the equivalent inverse cipher: the exact inverse of tac_aes_encrypt_blocks for the
+ * same `rounds` (which adds w[40..43] in its final round for every `rounds`):
+ *   s = in ⊕ dk[40..43];  rd = rounds−1 … 1: s = InvMixColumns(InvShiftRows(InvS(s))) ⊕ dk[rd];  out = InvShiftRows(InvS(s)) ⊕ dk[0..3]
+ * InvS·{14, 11, 13, 9} comes from one 8 → 32 circuit bootstrap per byte.  Noise as in encryption (33 in a middle round,
+ * output 9); TAC_ERR_STATE without a valid dk. */
+int tac_aes_decrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host);
+int tac_aes_decrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_dev, uint64_t* out_dev);
+/* decryption of PUBLIC 16-byte ciphertext blocks: state0 = dk[40..43] ⊕ trivial(block).  AES-ECB / AES-CBC transciphering:
+ * xor_host NULL (ECB) or the previous ciphertext blocks C_{i-1}, C_{-1} = IV (CBC), and the output encrypts the plaintext.
+ * Bootstraps equal across blocks run once, as in tac_aes_encrypt_public_blocks, along the inverse dependence rule
+ * D(r+1, (row, c)) = ∪_{r'} D(r, 4·((c − r') mod 4) + r').  Blocks and XOR bytes are HOST memory in both variants; the
+ * output equals tac_aes_decrypt_blocks on trivial encryptions of the same blocks. */
+int tac_aes_decrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host);
+int tac_aes_decrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev);
+/* boxes per round that tac_aes_decrypt_public_blocks runs for these blocks (as tac_aes_public_plan).  Host only. */
+int tac_aes_public_plan_inv(int n_blocks, int rounds, const uint8_t* blocks_host /*[n][16]*/, int64_t* boxes);
+
 /* ------------------------------------------------------------------ single stages (parity tests, profiling) */
 /* [U] keyswitch_lwe_ciphertext: [n_cts][kN+1] → [n_cts][n+1] */
 int tac_stage_keyswitch(tac_ctx* ctx, int n_cts, const uint64_t* in_host, uint64_t* out_host);

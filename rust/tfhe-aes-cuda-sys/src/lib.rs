@@ -102,6 +102,13 @@ extern "C" {
     pub fn tac_aes_encrypt_public_blocks(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, blocks_host: *const u8, xor_host: *const u8, out_host: *mut u64) -> c_int;
     pub fn tac_aes_encrypt_public_blocks_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, blocks_host: *const u8, xor_host: *const u8, out_dev: *mut u64) -> c_int;
     pub fn tac_aes_public_plan(n_blocks: c_int, rounds: c_int, blocks_host: *const u8, boxes: *mut i64) -> c_int;
+    pub fn tac_aes_inv_key_schedule(ctx: *mut tac_ctx, inv_key_sched_host: *mut u64) -> c_int;
+    pub fn tac_aes_set_inv_key_schedule(ctx: *mut tac_ctx, inv_key_sched_host: *const u64) -> c_int;
+    pub fn tac_aes_decrypt_blocks(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, in_noise_sq: c_int, in_host: *const u64, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_decrypt_blocks_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, in_noise_sq: c_int, in_dev: *const u64, out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_decrypt_public_blocks(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, blocks_host: *const u8, xor_host: *const u8, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_decrypt_public_blocks_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, blocks_host: *const u8, xor_host: *const u8, out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_public_plan_inv(n_blocks: c_int, rounds: c_int, blocks_host: *const u8, boxes: *mut i64) -> c_int;
 
     // single stages, profiling
     pub fn tac_stage_keyswitch(ctx: *mut tac_ctx, n_cts: c_int, in_host: *const u64, out_host: *mut u64) -> c_int;

@@ -102,6 +102,13 @@ _SIGNATURES = {
     "tac_aes_encrypt_public_blocks": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_aes_encrypt_public_blocks_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_aes_public_plan": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "tac_aes_inv_key_schedule": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tac_aes_set_inv_key_schedule": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tac_aes_decrypt_blocks": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "tac_aes_decrypt_blocks_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "tac_aes_decrypt_public_blocks": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_decrypt_public_blocks_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_public_plan_inv": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "tac_stage_keyswitch": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
     "tac_extract_bits": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _u64p, _u64p]),
     "tac_stage_pbs": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
@@ -234,12 +241,14 @@ def ctr_blocks(iv, first_ctr, n):
     return _public_blocks(b"".join(iv + (first_ctr + i).to_bytes(8, "big") for i in range(n)))
 
 
-def aes_public_plan(blocks, rounds=10):
-    """circuit bootstraps per round that FheContext.aes_encrypt_public_blocks runs for these public blocks (rounds 1..rounds);
-    16 per block and round without sharing.  Host only."""
+def aes_public_plan(blocks, rounds=10, decrypt=False):
+    """circuit bootstraps per round that FheContext.aes_encrypt_public_blocks (decrypt=True: aes_decrypt_public_blocks) runs
+    for these public blocks (rounds 1..rounds); 16 per block and round without sharing.  Host only."""
     b = _public_blocks(blocks)
     out = np.zeros(max(rounds, 0), dtype=np.int64)
-    rc = load_library().tac_aes_public_plan(b.shape[0], rounds, b.ctypes.data, out.ctypes.data)
+    L = load_library()
+    plan = L.tac_aes_public_plan_inv if decrypt else L.tac_aes_public_plan
+    rc = plan(b.shape[0], rounds, b.ctypes.data, out.ctypes.data)
     if rc != 0:
         raise ValueError(f"aes_public_plan: rounds must be in 1..10 (error {rc})")
     return [int(v) for v in out]
@@ -658,6 +667,66 @@ class FheContext(NoiseContext):
         padded = data + bytes(16 * n - len(data))
         out = self.aes_encrypt_public_blocks(ctr_blocks(iv, first_ctr, n), xor=padded)
         return out.reshape(16 * n, 8, self.params.big_lwe_size)[:len(data)]
+
+    # -- AES decryption (equivalent inverse cipher) and AES-ECB / AES-CBC transciphering
+    def aes_inv_key_schedule(self):
+        """derive the inverse key schedule dk on the device from the resident key schedule; returns it, [44][4][8][big+1].
+        It stays in use until the key schedule changes (aes_set_key_schedule / aes_key_schedule make it stale)."""
+        out = np.empty((44, 4, 8, self.params.big_lwe_size), dtype=np.uint64)
+        self._check(self.L.tac_aes_inv_key_schedule(self.h, out.ctypes.data))
+        return out
+
+    def aes_set_inv_key_schedule(self, inv_key_sched):
+        dk = np.ascontiguousarray(inv_key_sched, dtype=np.uint64)
+        assert dk.size == 44 * 32 * self.params.big_lwe_size
+        self._check(self.L.tac_aes_set_inv_key_schedule(self.h, dk.ctypes.data))
+
+    def aes_decrypt_blocks(self, blocks, rounds=10, in_noise_sq=1):
+        """AES decryption of FHE-encrypted blocks [n][16][8][big+1] under the resident inverse key schedule"""
+        b = np.ascontiguousarray(blocks, dtype=np.uint64).reshape(-1, 16, 8, self.params.big_lwe_size)
+        out = np.empty_like(b)
+        self._check(self.L.tac_aes_decrypt_blocks(self.h, b.shape[0], rounds, in_noise_sq, b.ctypes.data, out.ctypes.data))
+        return out
+
+    def aes_decrypt_blocks_dev(self, n_blocks, in_ptr, out_ptr, rounds=10, in_noise_sq=1):
+        self._check(self.L.tac_aes_decrypt_blocks_dev(self.h, n_blocks, rounds, in_noise_sq, C.c_void_p(in_ptr), C.c_void_p(out_ptr)))
+
+    def aes_decrypt_public_blocks(self, blocks, rounds=10, xor=None):
+        """AES decryption of public 16-byte ciphertext blocks; xor: optional public bytes [n][16] XORed into the output.
+        Returns [n][16][8][big+1] bit ciphertexts (squared noise level 9)."""
+        b, x = self._public_args(blocks, xor)
+        out = np.empty((b.shape[0], 16, 8, self.params.big_lwe_size), dtype=np.uint64)
+        self._check(self.L.tac_aes_decrypt_public_blocks(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
+                                                         out.ctypes.data))
+        return out
+
+    def aes_decrypt_public_blocks_dev(self, blocks, out_ptr, rounds=10, xor=None):
+        """the same into device memory out_ptr ([n][16][8][big+1] words), enqueued on the context's stream"""
+        b, x = self._public_args(blocks, xor)
+        self._check(self.L.tac_aes_decrypt_public_blocks_dev(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
+                                                             C.c_void_p(out_ptr)))
+
+    @staticmethod
+    def _whole_blocks(data):
+        data = bytes(data)
+        if len(data) % 16:
+            raise ValueError("AES-ECB / AES-CBC ciphertexts are whole 16-byte blocks")
+        return data
+
+    def aes_ecb_transcipher(self, data):
+        """Transciphering: `data` is an AES-ECB ciphertext under the FHE-encrypted key; returns FHE encryptions of its
+        (padded) plaintext bits, [len(data)][8][big+1].  Removing padding is the caller's business."""
+        data = self._whole_blocks(data)
+        return self.aes_decrypt_public_blocks(data).reshape(len(data), 8, self.params.big_lwe_size)
+
+    def aes_cbc_transcipher(self, iv, data):
+        """Transciphering: `data` is an AES-CBC ciphertext under the FHE-encrypted key with the 16-byte `iv`;
+        P_i = AES^-1(C_i) xor C_{i-1}, C_{-1} = iv.  Returns FHE encryptions of the (padded) plaintext bits, [len(data)][8][big+1]."""
+        iv, data = bytes(iv), self._whole_blocks(data)
+        if len(iv) != 16:
+            raise ValueError("iv must be 16 bytes")
+        out = self.aes_decrypt_public_blocks(data, xor=(iv + data[:-16]) if data else None)
+        return out.reshape(len(data), 8, self.params.big_lwe_size)
 
     def aes_key_schedule_buffer(self):
         ptr, nbytes = C.c_void_p(), C.c_size_t()

@@ -1,5 +1,5 @@
-// aes_plan.cpp — the sharing plan of AES over public blocks (aes_plan.h) and its C export tac_aes_public_plan.
-// Host only, pure integer: the CPU tests pin it down, and tac_aes_encrypt_public_blocks[_dev] runs exactly this plan.
+// aes_plan.cpp — the sharing plan of AES over public blocks (aes_plan.h) and its C exports tac_aes_public_plan[_inv].
+// Host only, pure integer: the CPU tests pin it down, and tac_aes_{en,de}crypt_public_blocks[_dev] run exactly this plan.
 #include "aes_plan.h"
 #include "../../include/tfhe_aes_cuda.h"
 
@@ -9,10 +9,11 @@
 
 namespace tac {
 
-int aes_public_plan_build(int n_blocks, int rounds, const uint8_t* blocks, std::vector<AesRoundPlan>& plan) {
+int aes_public_plan_build(int n_blocks, int rounds, const uint8_t* blocks, AesDir dir, std::vector<AesRoundPlan>& plan) {
     if (n_blocks < 0 || rounds < 1 || rounds > 10 || (n_blocks > 0 && !blocks)) return TAC_ERR_ARG;
     plan.assign(rounds, AesRoundPlan{});
     const size_t npos = (size_t)n_blocks * 16;
+    const int sgn = dir == AesDir::Forward ? 1 : -1;        // (c ± r') mod 4: ShiftRows or InvShiftRows
     uint16_t dep[16];                                       // D(r, j) as a bit mask over the 16 input bytes
     for (int j = 0; j < 16; j++) dep[j] = (uint16_t)(1u << j);
     for (int r = 1; r <= rounds; r++) {
@@ -21,7 +22,7 @@ int aes_public_plan_build(int n_blocks, int rounds, const uint8_t* blocks, std::
             for (int j = 0; j < 16; j++) {
                 const int c = j >> 2;
                 next[j] = 0;
-                for (int rr = 0; rr < 4; rr++) next[j] |= dep[4 * ((c + rr) & 3) + rr];
+                for (int rr = 0; rr < 4; rr++) next[j] |= dep[4 * ((c + sgn * rr) & 3) + rr];
             }
             std::copy(next, next + 16, dep);
         }
@@ -48,10 +49,16 @@ int aes_public_plan_build(int n_blocks, int rounds, const uint8_t* blocks, std::
 
 }  // namespace tac
 
-extern "C" int tac_aes_public_plan(int n_blocks, int rounds, const uint8_t* blocks_host, int64_t* boxes) {
+static int export_plan(int n_blocks, int rounds, const uint8_t* blocks_host, tac::AesDir dir, int64_t* boxes) {
     std::vector<tac::AesRoundPlan> plan;
-    if (int rc = tac::aes_public_plan_build(n_blocks, rounds, blocks_host, plan)) return rc;
+    if (int rc = tac::aes_public_plan_build(n_blocks, rounds, blocks_host, dir, plan)) return rc;
     if (!boxes) return TAC_ERR_ARG;
     for (int r = 0; r < rounds; r++) boxes[r] = plan[r].boxes;
     return TAC_OK;
+}
+extern "C" int tac_aes_public_plan(int n_blocks, int rounds, const uint8_t* blocks_host, int64_t* boxes) {
+    return export_plan(n_blocks, rounds, blocks_host, tac::AesDir::Forward, boxes);
+}
+extern "C" int tac_aes_public_plan_inv(int n_blocks, int rounds, const uint8_t* blocks_host, int64_t* boxes) {
+    return export_plan(n_blocks, rounds, blocks_host, tac::AesDir::Inverse, boxes);
 }

@@ -84,8 +84,11 @@ struct tac_ctx {
     // LUTs
     std::vector<Lut> luts;
     int aes_lut24 = -1, aes_lut8 = -1, aes_lut1 = -1;
+    int aes_lut_inv32 = -1, aes_lut_inv8 = -1, aes_lut_key32 = -1;   // decryption: InvS·{14,11,13,9}, InvS, b·{14,11,13,9}
     // AES key schedule
     uint64_t* key_sched = nullptr;
+    uint64_t* inv_key_sched = nullptr;   // equivalent inverse cipher's schedule dk, same layout [44 words][4][8][kN+1]
+    bool inv_key_sched_valid = false;    // dk belongs to the resident key_sched (cleared by tac_aes_set_key_schedule)
     uint64_t* rc_rows = nullptr;     // trivial(RC[1..10]) as byte ciphertexts [10][8][kN+1], uploaded once
     // workspace
     DevBuf ws_in, ws_out, ws_small, ws_ksdig, ws_pbs, ws_pfdig, ws_ggsw, ws_ggswf, ws_tree_a, ws_tree_b, ws_state, ws_muls, ws_misc;
@@ -375,6 +378,28 @@ int ensure_aes_luts(tac_ctx* ctx) {
     id = tac_lut_register(ctx, 1, 1, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut1 = id;
     return TAC_OK;
 }
+// LUTs of the equivalent inverse cipher (FIPS-197 §5.3.5), registered on the first decryption call only.  Outputs in the
+// order of aes_inv_mix_columns_kernel: the byte times {14, 11, 13, 9}, 8 bits each, MSB first.
+int ensure_aes_inv_luts(tac_ctx* ctx) {
+    if (ctx->aes_lut_inv32 >= 0) return TAC_OK;
+    uint8_t S[256], IS[256]; sbox_table(S);
+    for (int b = 0; b < 256; b++) IS[S[b]] = (uint8_t)b;
+    const int N = ctx->p.N;
+    auto inv_mix = [](uint8_t b) {
+        return ((uint64_t)gf_mul(b, 14) << 24) | ((uint64_t)gf_mul(b, 11) << 16) | ((uint64_t)gf_mul(b, 13) << 8) | (uint64_t)gf_mul(b, 9);
+    };
+    std::vector<uint64_t> f(256), t;
+    for (int b = 0; b < 256; b++) f[b] = inv_mix(IS[b]);
+    t.resize(tac_lut_len(8, N) * 32); tac_generate_lut(8, 32, N, f.data(), t.data());
+    int id = tac_lut_register(ctx, 8, 32, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut_inv32 = id;
+    for (int b = 0; b < 256; b++) f[b] = IS[b];
+    t.resize(tac_lut_len(8, N) * 8); tac_generate_lut(8, 8, N, f.data(), t.data());
+    id = tac_lut_register(ctx, 8, 8, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut_inv8 = id;
+    for (int b = 0; b < 256; b++) f[b] = inv_mix((uint8_t)b);
+    t.resize(tac_lut_len(8, N) * 32); tac_generate_lut(8, 32, N, f.data(), t.data());
+    id = tac_lut_register(ctx, 8, 32, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut_key32 = id;
+    return TAC_OK;
+}
 
 // static squared-noise bookkeeping of the AES circuit (NoiseLevelWithComponents::add_assign, shortint_woppbs_1bit.rs:63-77):
 // round keys are fresh or bootstrapped (level 1); SBOX outputs carry 8·NOMINAL (:325)
@@ -382,6 +407,103 @@ int aes_noise_check(tac_ctx* ctx, int in_noise_sq, int rounds) {
     const int maxn = ctx->p.max_noise_sq;
     if (in_noise_sq + 1 > maxn || (rounds > 1 && 4 * 8 + 1 > maxn) || 8 + 1 > maxn)
         return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: the AES circuit needs max_noise_level_squared >= 33");
+    return TAC_OK;
+}
+
+// AES over PUBLIC blocks (aes_plan.h): the round structure of tac_aes_{en,de}crypt_blocks_dev with state0 = k_first +
+// trivial(block).  Each round bootstraps only the plan's representatives, in one compact batch, and (Inv)MixColumns / the
+// final round read every position's S-box row through the plan's index table.  Rounds whose plan is the identity (all
+// blocks distinct from round 3 on) run on the full state in place, as the encrypted-block path does.
+//   Forward: keys w[0], w[rd], w[40..43] from key_sched; S-box LUTs ·{1,2,3} / S; ShiftRows kernels.
+//   Inverse: keys dk[40..43], dk[rounds−rd], dk[0..3] from inv_key_sched; LUTs InvS·{14,11,13,9} / InvS; InvShiftRows kernels.
+int aes_public_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
+    const bool fwd = dir == AesDir::Forward;
+    std::vector<AesRoundPlan> plan;
+    if (aes_public_plan_build(n_blocks, rounds, blocks_host, dir, plan)) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range, or NULL blocks");
+    if (n_blocks == 0) return TAC_OK;
+    TRY(aes_noise_check(ctx, 0, rounds));                  // trivial input: no noise of its own
+    TRY(fwd ? ensure_aes_luts(ctx) : ensure_aes_inv_luts(ctx));
+    const size_t L = (size_t)ctx->big() + 1, byte_words = 8 * L, blk = 16 * byte_words;
+    const size_t npos = (size_t)n_blocks * 16, total = (size_t)n_blocks * blk;
+    const uint64_t* keys = fwd ? ctx->key_sched : ctx->inv_key_sched;
+    const Lut& lut_mid = ctx->luts[fwd ? ctx->aes_lut24 : ctx->aes_lut_inv32];
+    const Lut& lut_last = ctx->luts[fwd ? ctx->aes_lut8 : ctx->aes_lut_inv8];
+    // one upload: public blocks, XOR bytes, then rep_pos / idx of every round that shares
+    std::vector<size_t> off_rep(rounds, 0), off_idx(rounds, 0);
+    size_t bytes = 2 * npos, max_rep = plan[0].identity ? 0 : (size_t)plan[0].boxes;
+    for (int r = 0; r < rounds; r++) {
+        if (plan[r].identity) continue;
+        off_rep[r] = bytes; bytes += (size_t)plan[r].boxes * 4;
+        off_idx[r] = bytes; bytes += npos * 4;
+        max_rep = std::max(max_rep, (size_t)plan[r].boxes);
+    }
+    std::vector<uint8_t> host(bytes, 0);
+    std::memcpy(host.data(), blocks_host, npos);
+    if (xor_host) std::memcpy(host.data() + npos, xor_host, npos);
+    for (int r = 0; r < rounds; r++) {
+        if (plan[r].identity) continue;
+        std::memcpy(host.data() + off_rep[r], plan[r].rep_pos.data(), (size_t)plan[r].boxes * 4);
+        std::memcpy(host.data() + off_idx[r], plan[r].idx.data(), npos * 4);
+    }
+    TRY(ensure(ctx, ctx->ws_plan, bytes));
+    TRY(ensure(ctx, ctx->ws_state, total * 8));
+    TRY(ensure(ctx, ctx->ws_muls, total * (fwd ? 3 : 4) * 8));
+    TRY(ensure(ctx, ctx->ws_rep, std::max<size_t>(1, max_rep) * byte_words * 8));
+    // pageable source: the call returns once the bytes are staged, so `host` may go out of scope before the copy lands
+    CU(cudaMemcpyAsync(ctx->ws_plan.p, host.data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
+    const uint8_t* d_plan = ctx->ws_plan.as<uint8_t>();
+    auto rep_pos = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_rep[r]); };
+    auto idx = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_idx[r]); };
+    uint64_t* state = ctx->ws_state.as<uint64_t>();
+    uint64_t* muls = ctx->ws_muls.as<uint64_t>();
+    uint64_t* rep = ctx->ws_rep.as<uint64_t>();
+    const int g = grid1d(total, 256, ctx->sm_count);
+    // S-box inputs of round rd (1-based) for its representatives → `in`
+    auto sbox_inputs = [&](int rd, const uint64_t** in) -> int {
+        const int r = rd - 1;
+        const size_t n_words = (size_t)plan[r].boxes * byte_words;
+        if (rd == 1) {
+            uint64_t* dst = plan[r].identity ? state : rep;
+            const uint64_t* k_first = fwd ? keys : keys + (size_t)10 * blk;
+            aes_public_round1_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(k_first, d_plan, rep_pos(r), (int)L, n_words, dst);
+            TRY(post_launch(ctx, "aes_public_round1_kernel"));
+            *in = dst;
+        } else if (plan[r].identity) {
+            *in = state;
+        } else {
+            aes_gather_bytes_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(state, rep_pos(r), (int)L, n_words, rep);
+            TRY(post_launch(ctx, "aes_gather_bytes_kernel"));
+            *in = rep;
+        }
+        return TAC_OK;
+    };
+    const uint64_t* in = nullptr;
+    for (int rd = 1; rd < rounds; rd++) {
+        TRY(sbox_inputs(rd, &in));
+        TRY(wopbs_dev(ctx, lut_mid, (int)plan[rd - 1].boxes, in, muls));
+        if (fwd) {
+            aes_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)rd * blk, (int)L, total, state, idx(rd - 1));
+            TRY(post_launch(ctx, "aes_mix_columns_kernel"));
+        } else {
+            aes_inv_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)(rounds - rd) * blk, (int)L, total, state, idx(rd - 1));
+            TRY(post_launch(ctx, "aes_inv_mix_columns_kernel"));
+        }
+    }
+    TRY(sbox_inputs(rounds, &in));
+    TRY(wopbs_dev(ctx, lut_last, (int)plan[rounds - 1].boxes, in, muls));
+    const uint8_t* xr = xor_host ? d_plan + npos : nullptr;
+    if (!fwd) {
+        aes_inv_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, keys, (int)L, total, out_dev, idx(rounds - 1), xr);
+        return post_launch(ctx, "aes_inv_final_round_kernel");
+    }
+    aes_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)10 * blk, (int)L, total, out_dev, idx(rounds - 1), xr);
+    return post_launch(ctx, "aes_final_round_kernel");
+}
+
+// dk present and made from (or uploaded for) the resident encryption schedule
+int inv_key_sched_check(tac_ctx* ctx) {
+    if (!ctx->inv_key_sched || !ctx->inv_key_sched_valid)
+        return fail(ctx, TAC_ERR_STATE, "no inverse key schedule for the resident key schedule (tac_aes_inv_key_schedule or tac_aes_set_inv_key_schedule)");
     return TAC_OK;
 }
 
@@ -429,7 +551,7 @@ void tac_ctx_destroy(tac_ctx* ctx) {
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
     for (void* p : {(void*)ctx->bsk_f, (void*)ctx->ksk, (void*)ctx->pfpksk, (void*)ctx->ks_corr, (void*)ctx->pfks_corr, (void*)ctx->pfks_planes, (void*)ctx->ks_planes, (void*)ctx->pfks_fix, (void*)ctx->wT,
-                    (void*)ctx->key_sched, (void*)ctx->rc_rows})
+                    (void*)ctx->key_sched, (void*)ctx->inv_key_sched, (void*)ctx->rc_rows})
         if (p) cudaFree(p);
     for (auto& l : ctx->luts) cudaFree(l.dev);
     for (DevBuf* b : {&ctx->ws_in, &ctx->ws_out, &ctx->ws_small, &ctx->ws_ksdig, &ctx->ws_pbs, &ctx->ws_pfdig, &ctx->ws_ggsw, &ctx->ws_ggswf,
@@ -746,6 +868,7 @@ int tac_aes_set_key_schedule(tac_ctx* ctx, const uint64_t* ks_host) {
     CU(cudaSetDevice(ctx->device));
     const size_t bytes = (size_t)44 * 32 * (ctx->big() + 1) * 8;
     if (!ctx->key_sched) CU(cudaMalloc(&ctx->key_sched, bytes));
+    ctx->inv_key_sched_valid = false;        // an inverse schedule belongs to the encryption schedule it was made from
     if (ks_host) {
         CU(cudaMemcpyAsync(ctx->key_sched, ks_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
@@ -799,81 +922,12 @@ int tac_aes_encrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_
     return TAC_OK;
 }
 
-// AES over PUBLIC blocks (aes_plan.h): the round structure of tac_aes_encrypt_blocks_dev with state0 = k0 + trivial(block).
-// Each round bootstraps only the plan's representatives, in one compact batch, and MixColumns / the final round read every
-// position's S-box row through the plan's index table.  Rounds whose plan is the identity (all blocks distinct from
-// round 3 on) run on the full state in place, as the encrypted-block path does.
+
 int tac_aes_encrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    std::vector<AesRoundPlan> plan;
-    if (aes_public_plan_build(n_blocks, rounds, blocks_host, plan)) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range, or NULL blocks");
-    if (n_blocks == 0) return TAC_OK;
-    TRY(aes_noise_check(ctx, 0, rounds));                  // trivial input: no noise of its own
-    TRY(ensure_aes_luts(ctx));
-    const size_t L = (size_t)ctx->big() + 1, byte_words = 8 * L, blk = 16 * byte_words;
-    const size_t npos = (size_t)n_blocks * 16, total = (size_t)n_blocks * blk;
-    // one upload: public blocks, XOR bytes, then rep_pos / idx of every round that shares
-    std::vector<size_t> off_rep(rounds, 0), off_idx(rounds, 0);
-    size_t bytes = 2 * npos, max_rep = plan[0].identity ? 0 : (size_t)plan[0].boxes;
-    for (int r = 0; r < rounds; r++) {
-        if (plan[r].identity) continue;
-        off_rep[r] = bytes; bytes += (size_t)plan[r].boxes * 4;
-        off_idx[r] = bytes; bytes += npos * 4;
-        max_rep = std::max(max_rep, (size_t)plan[r].boxes);
-    }
-    std::vector<uint8_t> host(bytes, 0);
-    std::memcpy(host.data(), blocks_host, npos);
-    if (xor_host) std::memcpy(host.data() + npos, xor_host, npos);
-    for (int r = 0; r < rounds; r++) {
-        if (plan[r].identity) continue;
-        std::memcpy(host.data() + off_rep[r], plan[r].rep_pos.data(), (size_t)plan[r].boxes * 4);
-        std::memcpy(host.data() + off_idx[r], plan[r].idx.data(), npos * 4);
-    }
-    TRY(ensure(ctx, ctx->ws_plan, bytes));
-    TRY(ensure(ctx, ctx->ws_state, total * 8));
-    TRY(ensure(ctx, ctx->ws_muls, total * 3 * 8));
-    TRY(ensure(ctx, ctx->ws_rep, std::max<size_t>(1, max_rep) * byte_words * 8));
-    // pageable source: the call returns once the bytes are staged, so `host` may go out of scope before the copy lands
-    CU(cudaMemcpyAsync(ctx->ws_plan.p, host.data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
-    const uint8_t* d_plan = ctx->ws_plan.as<uint8_t>();
-    auto rep_pos = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_rep[r]); };
-    auto idx = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_idx[r]); };
-    uint64_t* state = ctx->ws_state.as<uint64_t>();
-    uint64_t* muls = ctx->ws_muls.as<uint64_t>();
-    uint64_t* rep = ctx->ws_rep.as<uint64_t>();
-    const int g = grid1d(total, 256, ctx->sm_count);
-    // S-box inputs of round rd (1-based) for its representatives → `in`
-    auto sbox_inputs = [&](int rd, const uint64_t** in) -> int {
-        const int r = rd - 1;
-        const size_t n_words = (size_t)plan[r].boxes * byte_words;
-        if (rd == 1) {
-            uint64_t* dst = plan[r].identity ? state : rep;
-            aes_public_round1_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->key_sched, d_plan, rep_pos(r), (int)L, n_words, dst);
-            TRY(post_launch(ctx, "aes_public_round1_kernel"));
-            *in = dst;
-        } else if (plan[r].identity) {
-            *in = state;
-        } else {
-            aes_gather_bytes_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(state, rep_pos(r), (int)L, n_words, rep);
-            TRY(post_launch(ctx, "aes_gather_bytes_kernel"));
-            *in = rep;
-        }
-        return TAC_OK;
-    };
-    const uint64_t* in = nullptr;
-    for (int rd = 1; rd < rounds; rd++) {
-        TRY(sbox_inputs(rd, &in));
-        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut24], (int)plan[rd - 1].boxes, in, muls));
-        aes_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)rd * blk, (int)L, total, state, idx(rd - 1));
-        TRY(post_launch(ctx, "aes_mix_columns_kernel"));
-    }
-    TRY(sbox_inputs(rounds, &in));
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut8], (int)plan[rounds - 1].boxes, in, muls));
-    aes_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)10 * blk, (int)L, total, out_dev, idx(rounds - 1),
-                                                      xor_host ? d_plan + npos : nullptr);
-    return post_launch(ctx, "aes_final_round_kernel");
+    return aes_public_blocks_dev(ctx, AesDir::Forward, n_blocks, rounds, blocks_host, xor_host, out_dev);
 }
 int tac_aes_encrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
     LOCK(ctx);
@@ -884,6 +938,119 @@ int tac_aes_encrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const 
     TRY(tac_aes_encrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, ctx->ws_out.as<uint64_t>()));
     CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
+    return TAC_OK;
+}
+
+// ------------------------------------------------------------------------------------ AES decryption (FIPS-197 §5.3.5)
+// Equivalent inverse cipher, the exact inverse of tac_aes_encrypt_blocks_dev for the same `rounds` (whose final round adds
+// w[40..43] for every `rounds`):
+//   s = in + dk[40..43];  for rd = rounds−1 … 1: s = InvMixColumns(InvShiftRows(InvS(s))) + dk[rd];  out = InvShiftRows(InvS(s)) + dk[0..3]
+// InvS·{14, 11, 13, 9} comes out of one 8 → 32 circuit bootstrap per byte, so a middle round sums 4 outputs of squared noise 8
+// and one round key of level 1: 33, as in the forward direction.  Round keys are read from dk only.
+int tac_aes_decrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_dev, uint64_t* out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    TRY(inv_key_sched_check(ctx));
+    if (n_blocks < 0 || rounds < 1 || rounds > 10) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range");
+    if (n_blocks == 0) return TAC_OK;
+    TRY(aes_noise_check(ctx, in_noise_sq, rounds));
+    TRY(ensure_aes_inv_luts(ctx));
+    const size_t L = (size_t)ctx->big() + 1, blk = 16 * 8 * L;
+    const size_t total = (size_t)n_blocks * blk;
+    TRY(ensure(ctx, ctx->ws_state, total * 8));
+    TRY(ensure(ctx, ctx->ws_muls, total * 4 * 8));
+    uint64_t* state = ctx->ws_state.as<uint64_t>();
+    uint64_t* muls = ctx->ws_muls.as<uint64_t>();
+    const uint64_t* dk = ctx->inv_key_sched;
+    const int g = grid1d(total, 256, ctx->sm_count);
+    aes_add_round_key_kernel<<<g, 256, 0, ctx->stream>>>(in_dev, dk + (size_t)10 * blk, blk, total, state);
+    TRY(post_launch(ctx, "aes_add_round_key_kernel"));
+    for (int rd = rounds - 1; rd >= 1; rd--) {
+        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut_inv32], n_blocks * 16, state, muls));
+        aes_inv_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, dk + (size_t)rd * blk, (int)L, total, state, nullptr);
+        TRY(post_launch(ctx, "aes_inv_mix_columns_kernel"));
+    }
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut_inv8], n_blocks * 16, state, muls));
+    aes_inv_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, dk, (int)L, total, out_dev, nullptr, nullptr);
+    return post_launch(ctx, "aes_inv_final_round_kernel");
+}
+int tac_aes_decrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
+    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
+    TRY(ensure(ctx, ctx->ws_in, bytes));
+    TRY(ensure(ctx, ctx->ws_out, bytes));
+    CU(cudaMemcpyAsync(ctx->ws_in.p, in_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    TRY(tac_aes_decrypt_blocks_dev(ctx, n_blocks, rounds, in_noise_sq, ctx->ws_in.as<uint64_t>(), ctx->ws_out.as<uint64_t>()));
+    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return TAC_OK;
+}
+
+// decryption of PUBLIC ciphertext blocks (AES-ECB / AES-CBC transciphering): state0 = dk[40..43] + trivial(block), the
+// plan runs along the inverse dependence rule, xor_host (the previous ciphertext blocks for CBC) joins the final round
+int tac_aes_decrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    TRY(inv_key_sched_check(ctx));
+    return aes_public_blocks_dev(ctx, AesDir::Inverse, n_blocks, rounds, blocks_host, xor_host, out_dev);
+}
+int tac_aes_decrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
+    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
+    TRY(ensure(ctx, ctx->ws_out, bytes));
+    TRY(tac_aes_decrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, ctx->ws_out.as<uint64_t>()));
+    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return TAC_OK;
+}
+
+// inverse key schedule on the device from the resident encryption schedule: dk[0..3] = w[0..3], dk[40..43] = w[40..43],
+// dk[4rd..4rd+3] = InvMixColumns(w[4rd..4rd+3]) for rd = 1..9.  One 8 → 32 circuit bootstrap (b·{14, 11, 13, 9}) of the
+// 144 key bytes, the InvMixColumns sums (squared noise 32), then one 1-bit bootstrap per sum bit back to level 1 (as
+// boot_word does in the forward key schedule).
+int tac_aes_inv_key_schedule(tac_ctx* ctx, uint64_t* out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
+    if (4 * 8 > ctx->p.max_noise_sq) return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: the inverse key schedule needs max_noise_level_squared >= 32");
+    TRY(ensure_aes_luts(ctx));
+    TRY(ensure_aes_inv_luts(ctx));
+    const size_t L = (size_t)ctx->big() + 1, byte = 8 * L, word = 4 * byte, bytes = 44 * word * 8;
+    const int n_key_bytes = 9 * 16;                          // round keys 1..9
+    if (!ctx->inv_key_sched) CU(cudaMalloc(&ctx->inv_key_sched, bytes));
+    ctx->inv_key_sched_valid = false;
+    uint64_t* dk = ctx->inv_key_sched;
+    const uint64_t* w = ctx->key_sched;
+    TRY(ensure(ctx, ctx->ws_muls, (size_t)n_key_bytes * 32 * L * 8));
+    TRY(ensure(ctx, ctx->ws_state, (size_t)n_key_bytes * byte * 8));
+    CU(cudaMemcpyAsync(dk, w, 4 * word * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(dk + 40 * word, w + 40 * word, 4 * word * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+    uint64_t* muls = ctx->ws_muls.as<uint64_t>();
+    uint64_t* sums = ctx->ws_state.as<uint64_t>();
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut_key32], n_key_bytes, w + 4 * word, muls));
+    const size_t total = (size_t)n_key_bytes * byte;
+    aes_inv_mix_key_kernel<<<grid1d(total, 256, ctx->sm_count), 256, 0, ctx->stream>>>(muls, (int)L, total, sums);
+    TRY(post_launch(ctx, "aes_inv_mix_key_kernel"));
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut1], n_key_bytes * 8, sums, dk + 4 * word));
+    if (out_host) CU(cudaMemcpyAsync(out_host, dk, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ctx->inv_key_sched_valid = true;
+    return TAC_OK;
+}
+int tac_aes_set_inv_key_schedule(tac_ctx* ctx, const uint64_t* dk_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (!dk_host) return fail(ctx, TAC_ERR_ARG, "NULL inverse key schedule");
+    const size_t bytes = (size_t)44 * 32 * (ctx->big() + 1) * 8;
+    if (!ctx->inv_key_sched) CU(cudaMalloc(&ctx->inv_key_sched, bytes));
+    ctx->inv_key_sched_valid = false;
+    CU(cudaMemcpyAsync(ctx->inv_key_sched, dk_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ctx->inv_key_sched_valid = true;
     return TAC_OK;
 }
 

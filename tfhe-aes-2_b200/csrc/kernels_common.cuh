@@ -5,7 +5,8 @@
 //   lwe_gemm_kernel        exact integer GEMM mod 2^64 on the integer pipe: out[ct][col] = corr[col] − Σ_k digit'[ct][k]·key[k][col]
 //                          (PFKS of params_sqrd_lvl_1, and the correction rows of both keyswitches at key upload)
 //   aes_*_kernel           AddRoundKey / ShiftRows+MixColumns+AddRoundKey / final round as gather-adds on the flat state;
-//                          round-1 inputs and representative gathers of the public-block path
+//                          round-1 inputs and representative gathers of the public-block path;
+//   aes_inv_*_kernel       the same glue for the equivalent inverse cipher, and InvMixColumns of the inverse key schedule
 //   lwe_add_kernel         leveled XOR (lwe_ciphertext_add_assign) over a batch; lwe_shl_kernel / lwe_sub_kernel: glue of extract_bits
 //   negate_kernel, dfma_peak_kernel   key-upload helper, FP64 peak microbenchmark (roofline denominator)
 #pragma once
@@ -146,6 +147,63 @@ __global__ void aes_public_round1_kernel(const uint64_t* __restrict__ k0, const 
         const int bit = (int)(w / L);
         uint64_t v = k0[(size_t)(pos & 15) * byte_words + w];
         if (w - (size_t)bit * L == (size_t)L - 1 && (blocks[pos] & (0x80 >> bit))) v += 1ull << 63;
+        out[i] = v;
+    }
+}
+// ---- equivalent inverse cipher (FIPS-197 §5.3.5): the decryption glue, kept apart from the forward kernels above
+// InvShiftRows on the InvS·{14, 11, 13, 9} states + InvMixColumns + AddRoundKey (inverse key schedule dk):
+//   new[row][c] = Σ_{r'} coef[(r' − row) mod 4] · InvS(old[r'][(c − r') mod 4]),   coef = {14, 11, 13, 9}
+// muls: [row][32 = (14, 11, 13, 9)·InvS × 8 bits][L], row = block·16 + byte, or idx[block·16 + byte] (compact batch of the
+// public-block path: tac_aes_decrypt_public_blocks)
+__global__ void aes_inv_mix_columns_kernel(const uint64_t* __restrict__ muls, const uint64_t* __restrict__ rk, int L, size_t total,
+                                           uint64_t* __restrict__ state, const int32_t* __restrict__ idx) {
+    const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
+        const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;   // bit·L + e
+        const int c = byte >> 2, r = byte & 3;
+        uint64_t v = rk[rem];
+#pragma unroll
+        for (int rr = 0; rr < 4; rr++) {
+            const int old_byte = 4 * ((c - rr) & 3) + rr;          // InvShiftRows: new[rr][c] = old[rr][(c−rr)%4]
+            const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
+            v += muls[(src_row * 32 + (size_t)((rr - r) & 3) * 8) * L + w];
+        }
+        state[i] = v;
+    }
+}
+// last inverse round: InvShiftRows(InvS) + dk[0..3].  sub rows [row][8 bits][L] (idx optional); xr: NULL, or [block][16]
+// public bytes XORed into the output (the previous ciphertext block of AES-CBC), as in aes_final_round_kernel
+__global__ void aes_inv_final_round_kernel(const uint64_t* __restrict__ sub, const uint64_t* __restrict__ rk, int L, size_t total,
+                                           uint64_t* __restrict__ out, const int32_t* __restrict__ idx,
+                                           const uint8_t* __restrict__ xr) {
+    const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
+        const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;
+        const int c = byte >> 2, r = byte & 3;
+        const int old_byte = 4 * ((c - r) & 3) + r;
+        const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
+        uint64_t v = sub[src_row * byte_words + w] + rk[rem];
+        if (xr) {
+            const int bit = (int)(w / L);
+            if (w - (size_t)bit * L == (size_t)L - 1 && (xr[blk * 16 + byte] & (0x80 >> bit))) v += 1ull << 63;
+        }
+        out[i] = v;
+    }
+}
+// inverse key schedule, dk[4rd..4rd+3] = InvMixColumns(w[4rd..4rd+3]): InvMixColumns without the shift over round keys.
+// muls: [key byte][32 = (14, 11, 13, 9)·b × 8 bits][L] for consecutive round keys of 16 bytes; out [key byte][8 bits][L]
+// (squared noise 4·8 = 32, bootstrapped back to level 1 by the caller)
+__global__ void aes_inv_mix_key_kernel(const uint64_t* __restrict__ muls, int L, size_t total, uint64_t* __restrict__ out) {
+    const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
+        const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;
+        const int c = byte >> 2, r = byte & 3;
+        uint64_t v = 0;
+#pragma unroll
+        for (int rr = 0; rr < 4; rr++) v += muls[((blk * 16 + 4 * c + rr) * 32 + (size_t)((rr - r) & 3) * 8) * L + w];
         out[i] = v;
     }
 }

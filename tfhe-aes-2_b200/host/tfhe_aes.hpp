@@ -406,6 +406,23 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
             res[q][b][i] = BitCt::with_noise_level(std::vector<uint64_t>(out.begin() + ((q * 16 + b) * 8 + i) * L, out.begin() + ((q * 16 + b) * 8 + i + 1) * L), 8 + 1, c);
         return res;
     }
+    // AES decryption (equivalent inverse cipher, FIPS-197 §5.3.5; the reference has none): derive the inverse key schedule
+    // from the device key schedule, once per key schedule.  Decryption fails (TAC_ERR_STATE) until this has run.
+    static void inv_key_schedule(const Ctx& c) { c.check(tac_aes_inv_key_schedule(c.raw(), nullptr)); }
+    // decryption of public ciphertext blocks under the inverse key schedule; `xor` (empty or one 16-byte row per block) is
+    // XORed into the output — the previous ciphertext blocks (IV first) for AES-CBC transciphering, empty for AES-ECB
+    static std::vector<data_model::BlockT<Bit>> decrypt_public_blocks(const Ctx& c, const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
+                                                                       const std::vector<std::array<uint8_t, 16>>& xor_bytes = {}) {
+        if (!xor_bytes.empty() && xor_bytes.size() != blocks.size()) throw std::invalid_argument("xor_bytes: one row per block");
+        const size_t L = c.lwe_size();
+        std::vector<uint64_t> out(blocks.size() * 128 * L);
+        c.check(tac_aes_decrypt_public_blocks(c.raw(), (int)blocks.size(), rounds, blocks.empty() ? nullptr : blocks[0].data(),
+                                              xor_bytes.empty() ? nullptr : xor_bytes[0].data(), out.data()));
+        std::vector<data_model::BlockT<Bit>> res(blocks.size());
+        for (size_t q = 0; q < blocks.size(); q++) for (int b = 0; b < 16; b++) for (int i = 0; i < 8; i++)
+            res[q][b][i] = BitCt::with_noise_level(std::vector<uint64_t>(out.begin() + ((q * 16 + b) * 8 + i) * L, out.begin() + ((q * 16 + b) * 8 + i + 1) * L), 8 + 1, c);
+        return res;
+    }
 };
 }  // namespace cuda_woppbs_1bit
 }  // namespace fhe_impls
