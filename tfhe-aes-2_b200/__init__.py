@@ -621,39 +621,41 @@ class FheContext(NoiseContext):
         self._check(self.L.tac_aes_key_schedule(self.h, kb.ctypes.data, out.ctypes.data))
         return out
 
-    def aes_encrypt_blocks(self, blocks, rounds=10, in_noise_sq=1):
+    def _aes_blocks(self, fn, blocks, rounds, in_noise_sq):
         b = np.ascontiguousarray(blocks, dtype=np.uint64).reshape(-1, 16, 8, self.params.big_lwe_size)
         out = np.empty_like(b)
-        self._check(self.L.tac_aes_encrypt_blocks(self.h, b.shape[0], rounds, in_noise_sq, b.ctypes.data, out.ctypes.data))
+        self._check(fn(self.h, b.shape[0], rounds, in_noise_sq, b.ctypes.data, out.ctypes.data))
         return out
+
+    def aes_encrypt_blocks(self, blocks, rounds=10, in_noise_sq=1):
+        return self._aes_blocks(self.L.tac_aes_encrypt_blocks, blocks, rounds, in_noise_sq)
 
     def aes_encrypt_blocks_dev(self, n_blocks, in_ptr, out_ptr, rounds=10, in_noise_sq=1):
         self._check(self.L.tac_aes_encrypt_blocks_dev(self.h, n_blocks, rounds, in_noise_sq, C.c_void_p(in_ptr), C.c_void_p(out_ptr)))
 
     # -- AES over public blocks: AES-CTR keystream and transciphering
-    def _public_args(self, blocks, xor):
+    def _aes_public_blocks(self, fn, blocks, rounds, xor, dev=False, out_ptr=None):
+        """fn on public blocks [n][16] with optional XOR bytes [n][16]: into device memory out_ptr (dev), else into the
+        returned host array"""
         b = _public_blocks(blocks)
         x = None
         if xor is not None:
             x = _public_blocks(xor)
             if x.shape != b.shape:
                 raise ValueError("xor must hold one 16-byte row per block")
-        return b, x
+        out = None if dev else np.empty((b.shape[0], 16, 8, self.params.big_lwe_size), dtype=np.uint64)
+        self._check(fn(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
+                       C.c_void_p(out_ptr) if dev else out.ctypes.data))
+        return out
 
     def aes_encrypt_public_blocks(self, blocks, rounds=10, xor=None):
         """AES of public 16-byte blocks under the device key schedule; xor: optional public bytes [n][16] XORed into the
         output.  Returns [n][16][8][big+1] bit ciphertexts (squared noise level 9)."""
-        b, x = self._public_args(blocks, xor)
-        out = np.empty((b.shape[0], 16, 8, self.params.big_lwe_size), dtype=np.uint64)
-        self._check(self.L.tac_aes_encrypt_public_blocks(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
-                                                         out.ctypes.data))
-        return out
+        return self._aes_public_blocks(self.L.tac_aes_encrypt_public_blocks, blocks, rounds, xor)
 
     def aes_encrypt_public_blocks_dev(self, blocks, out_ptr, rounds=10, xor=None):
         """the same into device memory out_ptr ([n][16][8][big+1] words), enqueued on the context's stream"""
-        b, x = self._public_args(blocks, xor)
-        self._check(self.L.tac_aes_encrypt_public_blocks_dev(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
-                                                             C.c_void_p(out_ptr)))
+        self._aes_public_blocks(self.L.tac_aes_encrypt_public_blocks_dev, blocks, rounds, xor, dev=True, out_ptr=out_ptr)
 
     def aes_ctr_keystream(self, iv, first_ctr, n_blocks):
         """FHE encryptions of the AES-CTR keystream blocks AES(k, iv ‖ BE64(first_ctr + i)): [n_blocks][16][8][big+1]"""
@@ -683,10 +685,7 @@ class FheContext(NoiseContext):
 
     def aes_decrypt_blocks(self, blocks, rounds=10, in_noise_sq=1):
         """AES decryption of FHE-encrypted blocks [n][16][8][big+1] under the resident inverse key schedule"""
-        b = np.ascontiguousarray(blocks, dtype=np.uint64).reshape(-1, 16, 8, self.params.big_lwe_size)
-        out = np.empty_like(b)
-        self._check(self.L.tac_aes_decrypt_blocks(self.h, b.shape[0], rounds, in_noise_sq, b.ctypes.data, out.ctypes.data))
-        return out
+        return self._aes_blocks(self.L.tac_aes_decrypt_blocks, blocks, rounds, in_noise_sq)
 
     def aes_decrypt_blocks_dev(self, n_blocks, in_ptr, out_ptr, rounds=10, in_noise_sq=1):
         self._check(self.L.tac_aes_decrypt_blocks_dev(self.h, n_blocks, rounds, in_noise_sq, C.c_void_p(in_ptr), C.c_void_p(out_ptr)))
@@ -694,17 +693,11 @@ class FheContext(NoiseContext):
     def aes_decrypt_public_blocks(self, blocks, rounds=10, xor=None):
         """AES decryption of public 16-byte ciphertext blocks; xor: optional public bytes [n][16] XORed into the output.
         Returns [n][16][8][big+1] bit ciphertexts (squared noise level 9)."""
-        b, x = self._public_args(blocks, xor)
-        out = np.empty((b.shape[0], 16, 8, self.params.big_lwe_size), dtype=np.uint64)
-        self._check(self.L.tac_aes_decrypt_public_blocks(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
-                                                         out.ctypes.data))
-        return out
+        return self._aes_public_blocks(self.L.tac_aes_decrypt_public_blocks, blocks, rounds, xor)
 
     def aes_decrypt_public_blocks_dev(self, blocks, out_ptr, rounds=10, xor=None):
         """the same into device memory out_ptr ([n][16][8][big+1] words), enqueued on the context's stream"""
-        b, x = self._public_args(blocks, xor)
-        self._check(self.L.tac_aes_decrypt_public_blocks_dev(self.h, b.shape[0], rounds, b.ctypes.data, None if x is None else x.ctypes.data,
-                                                             C.c_void_p(out_ptr)))
+        self._aes_public_blocks(self.L.tac_aes_decrypt_public_blocks_dev, blocks, rounds, xor, dev=True, out_ptr=out_ptr)
 
     @staticmethod
     def _whole_blocks(data):

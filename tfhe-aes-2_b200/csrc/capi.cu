@@ -362,43 +362,42 @@ void sbox_table(uint8_t s[256]) {
     } while (p != 1);
     s[0] = 0x63;
 }
+// the n_in → n_out LUT of f (tac_generate_lut), registered on the context; its id into *id
+int register_aes_lut(tac_ctx* ctx, int n_in, int n_out, const uint64_t* f, int* id) {
+    std::vector<uint64_t> t(tac_lut_len(n_in, ctx->p.N) * n_out);
+    tac_generate_lut(n_in, n_out, ctx->p.N, f, t.data());
+    const int r = tac_lut_register(ctx, n_in, n_out, t.data(), t.size());
+    if (r < 0) return r;
+    *id = r;
+    return TAC_OK;
+}
 int ensure_aes_luts(tac_ctx* ctx) {
     if (ctx->aes_lut24 >= 0) return TAC_OK;
     uint8_t S[256]; sbox_table(S);
-    const int N = ctx->p.N;
-    std::vector<uint64_t> f(256), t;
+    std::vector<uint64_t> f(256);
     for (int b = 0; b < 256; b++) f[b] = ((uint64_t)gf_mul(S[b], 1) << 16) | ((uint64_t)gf_mul(S[b], 2) << 8) | (uint64_t)gf_mul(S[b], 3);
-    t.resize(tac_lut_len(8, N) * 24); tac_generate_lut(8, 24, N, f.data(), t.data());
-    int id = tac_lut_register(ctx, 8, 24, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut24 = id;
+    TRY(register_aes_lut(ctx, 8, 24, f.data(), &ctx->aes_lut24));
     for (int b = 0; b < 256; b++) f[b] = S[b];
-    t.resize(tac_lut_len(8, N) * 8); tac_generate_lut(8, 8, N, f.data(), t.data());
-    id = tac_lut_register(ctx, 8, 8, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut8 = id;
+    TRY(register_aes_lut(ctx, 8, 8, f.data(), &ctx->aes_lut8));
     const uint64_t ident[2] = {0, 1};
-    t.resize(tac_lut_len(1, N)); tac_generate_lut(1, 1, N, ident, t.data());
-    id = tac_lut_register(ctx, 1, 1, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut1 = id;
-    return TAC_OK;
+    return register_aes_lut(ctx, 1, 1, ident, &ctx->aes_lut1);
 }
 // LUTs of the equivalent inverse cipher (FIPS-197 §5.3.5), registered on the first decryption call only.  Outputs in the
-// order of aes_inv_mix_columns_kernel: the byte times {14, 11, 13, 9}, 8 bits each, MSB first.
+// order of aes_mix_columns_kernel<false>: the byte times {14, 11, 13, 9}, 8 bits each, MSB first.
 int ensure_aes_inv_luts(tac_ctx* ctx) {
     if (ctx->aes_lut_inv32 >= 0) return TAC_OK;
     uint8_t S[256], IS[256]; sbox_table(S);
     for (int b = 0; b < 256; b++) IS[S[b]] = (uint8_t)b;
-    const int N = ctx->p.N;
     auto inv_mix = [](uint8_t b) {
         return ((uint64_t)gf_mul(b, 14) << 24) | ((uint64_t)gf_mul(b, 11) << 16) | ((uint64_t)gf_mul(b, 13) << 8) | (uint64_t)gf_mul(b, 9);
     };
-    std::vector<uint64_t> f(256), t;
+    std::vector<uint64_t> f(256);
     for (int b = 0; b < 256; b++) f[b] = inv_mix(IS[b]);
-    t.resize(tac_lut_len(8, N) * 32); tac_generate_lut(8, 32, N, f.data(), t.data());
-    int id = tac_lut_register(ctx, 8, 32, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut_inv32 = id;
+    TRY(register_aes_lut(ctx, 8, 32, f.data(), &ctx->aes_lut_inv32));
     for (int b = 0; b < 256; b++) f[b] = IS[b];
-    t.resize(tac_lut_len(8, N) * 8); tac_generate_lut(8, 8, N, f.data(), t.data());
-    id = tac_lut_register(ctx, 8, 8, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut_inv8 = id;
+    TRY(register_aes_lut(ctx, 8, 8, f.data(), &ctx->aes_lut_inv8));
     for (int b = 0; b < 256; b++) f[b] = inv_mix((uint8_t)b);
-    t.resize(tac_lut_len(8, N) * 32); tac_generate_lut(8, 32, N, f.data(), t.data());
-    id = tac_lut_register(ctx, 8, 32, t.data(), t.size()); if (id < 0) return id; ctx->aes_lut_key32 = id;
-    return TAC_OK;
+    return register_aes_lut(ctx, 8, 32, f.data(), &ctx->aes_lut_key32);
 }
 
 // static squared-noise bookkeeping of the AES circuit (NoiseLevelWithComponents::add_assign, shortint_woppbs_1bit.rs:63-77):
@@ -410,47 +409,67 @@ int aes_noise_check(tac_ctx* ctx, int in_noise_sq, int rounds) {
     return TAC_OK;
 }
 
-// AES over PUBLIC blocks (aes_plan.h): the round structure of tac_aes_{en,de}crypt_blocks_dev with state0 = k_first +
-// trivial(block).  Each round bootstraps only the plan's representatives, in one compact batch, and (Inv)MixColumns / the
-// final round read every position's S-box row through the plan's index table.  Rounds whose plan is the identity (all
-// blocks distinct from round 3 on) run on the full state in place, as the encrypted-block path does.
-//   Forward: keys w[0], w[rd], w[40..43] from key_sched; S-box LUTs ·{1,2,3} / S; ShiftRows kernels.
-//   Inverse: keys dk[40..43], dk[rounds−rd], dk[0..3] from inv_key_sched; LUTs InvS·{14,11,13,9} / InvS; InvShiftRows kernels.
-int aes_public_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
-    const bool fwd = dir == AesDir::Forward;
+// The AES rounds of tac_aes_{en,de}crypt{,_public}_blocks_dev, forward cipher or equivalent inverse cipher (FIPS-197 §5.3.5):
+//   Forward  s = in + w[0];        s = MixColumns(ShiftRows(S(s))) + w[rd]                for rd = 1 … rounds−1;  out = ShiftRows(S(s)) + w[40..43]
+//   Inverse  s = in + dk[40..43];  s = InvMixColumns(InvShiftRows(InvS(s))) + dk[rounds−rd];                      out = InvShiftRows(InvS(s)) + dk[0..3]
+// The final round adds w[40..43] (dk[0..3]) for every `rounds`, so decryption inverts encryption for the same `rounds`.
+// Input: ciphertexts in device memory (in_dev), or, with in_dev NULL, PUBLIC blocks on the host (blocks_host, aes_plan.h):
+// state0 = k_first + trivial(block), each round bootstraps only the plan's representatives, in one compact batch, and the
+// mix-columns / final-round kernels read every position's S-box row through the plan's index table.  Rounds whose plan is
+// the identity (every round of ciphertext input; from round 3 on when all blocks differ) run on the full state in place.
+// xor_host (public input only; NULL: none) is XORed into the output.
+int aes_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_dev, const uint8_t* blocks_host,
+                   const uint8_t* xor_host, uint64_t* out_dev) {
+    const bool fwd = dir == AesDir::Forward, pub = in_dev == nullptr;
     std::vector<AesRoundPlan> plan;
-    if (aes_public_plan_build(n_blocks, rounds, blocks_host, dir, plan)) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range, or NULL blocks");
+    if (pub) {
+        if (aes_public_plan_build(n_blocks, rounds, blocks_host, dir, plan)) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range, or NULL blocks");
+    } else {
+        if (n_blocks < 0 || rounds < 1 || rounds > 10) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range");
+        plan.assign(rounds, AesRoundPlan{16 * (int64_t)n_blocks, true});
+    }
     if (n_blocks == 0) return TAC_OK;
-    TRY(aes_noise_check(ctx, 0, rounds));                  // trivial input: no noise of its own
+    TRY(aes_noise_check(ctx, in_noise_sq, rounds));
     TRY(fwd ? ensure_aes_luts(ctx) : ensure_aes_inv_luts(ctx));
     const size_t L = (size_t)ctx->big() + 1, byte_words = 8 * L, blk = 16 * byte_words;
     const size_t npos = (size_t)n_blocks * 16, total = (size_t)n_blocks * blk;
+    // per direction: S-box LUTs S·{1,2,3} / S or InvS·{14,11,13,9} / InvS, round keys, (Inv)ShiftRows kernels
     const uint64_t* keys = fwd ? ctx->key_sched : ctx->inv_key_sched;
     const Lut& lut_mid = ctx->luts[fwd ? ctx->aes_lut24 : ctx->aes_lut_inv32];
     const Lut& lut_last = ctx->luts[fwd ? ctx->aes_lut8 : ctx->aes_lut_inv8];
-    // one upload: public blocks, XOR bytes, then rep_pos / idx of every round that shares
+    const uint64_t* k_first = fwd ? keys : keys + (size_t)10 * blk;
+    const uint64_t* k_last = fwd ? keys + (size_t)10 * blk : keys;
+    const auto mix_columns = fwd ? aes_mix_columns_kernel<true> : aes_mix_columns_kernel<false>;
+    const auto final_round = fwd ? aes_final_round_kernel<true> : aes_final_round_kernel<false>;
+    // public input: one upload of the blocks, the XOR bytes, then rep_pos / idx of every round that shares
     std::vector<size_t> off_rep(rounds, 0), off_idx(rounds, 0);
-    size_t bytes = 2 * npos, max_rep = plan[0].identity ? 0 : (size_t)plan[0].boxes;
-    for (int r = 0; r < rounds; r++) {
-        if (plan[r].identity) continue;
-        off_rep[r] = bytes; bytes += (size_t)plan[r].boxes * 4;
-        off_idx[r] = bytes; bytes += npos * 4;
-        max_rep = std::max(max_rep, (size_t)plan[r].boxes);
+    std::vector<uint8_t> host;
+    size_t max_rep = 0;
+    if (pub) {
+        size_t bytes = 2 * npos;
+        for (int r = 0; r < rounds; r++) {
+            if (plan[r].identity) continue;
+            off_rep[r] = bytes; bytes += (size_t)plan[r].boxes * 4;
+            off_idx[r] = bytes; bytes += npos * 4;
+            max_rep = std::max(max_rep, (size_t)plan[r].boxes);
+        }
+        host.assign(bytes, 0);
+        std::memcpy(host.data(), blocks_host, npos);
+        if (xor_host) std::memcpy(host.data() + npos, xor_host, npos);
+        for (int r = 0; r < rounds; r++) {
+            if (plan[r].identity) continue;
+            std::memcpy(host.data() + off_rep[r], plan[r].rep_pos.data(), (size_t)plan[r].boxes * 4);
+            std::memcpy(host.data() + off_idx[r], plan[r].idx.data(), npos * 4);
+        }
+        TRY(ensure(ctx, ctx->ws_plan, bytes));
     }
-    std::vector<uint8_t> host(bytes, 0);
-    std::memcpy(host.data(), blocks_host, npos);
-    if (xor_host) std::memcpy(host.data() + npos, xor_host, npos);
-    for (int r = 0; r < rounds; r++) {
-        if (plan[r].identity) continue;
-        std::memcpy(host.data() + off_rep[r], plan[r].rep_pos.data(), (size_t)plan[r].boxes * 4);
-        std::memcpy(host.data() + off_idx[r], plan[r].idx.data(), npos * 4);
-    }
-    TRY(ensure(ctx, ctx->ws_plan, bytes));
     TRY(ensure(ctx, ctx->ws_state, total * 8));
     TRY(ensure(ctx, ctx->ws_muls, total * (fwd ? 3 : 4) * 8));
-    TRY(ensure(ctx, ctx->ws_rep, std::max<size_t>(1, max_rep) * byte_words * 8));
-    // pageable source: the call returns once the bytes are staged, so `host` may go out of scope before the copy lands
-    CU(cudaMemcpyAsync(ctx->ws_plan.p, host.data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (pub) {
+        TRY(ensure(ctx, ctx->ws_rep, std::max<size_t>(1, max_rep) * byte_words * 8));
+        // pageable source: the call returns once the bytes are staged, so `host` may go out of scope before the copy lands
+        CU(cudaMemcpyAsync(ctx->ws_plan.p, host.data(), host.size(), cudaMemcpyHostToDevice, ctx->stream));
+    }
     const uint8_t* d_plan = ctx->ws_plan.as<uint8_t>();
     auto rep_pos = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_rep[r]); };
     auto idx = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_idx[r]); };
@@ -462,9 +481,12 @@ int aes_public_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, co
     auto sbox_inputs = [&](int rd, const uint64_t** in) -> int {
         const int r = rd - 1;
         const size_t n_words = (size_t)plan[r].boxes * byte_words;
-        if (rd == 1) {
+        if (rd == 1 && !pub) {
+            aes_add_round_key_kernel<<<g, 256, 0, ctx->stream>>>(in_dev, k_first, blk, total, state);          // :96-99
+            TRY(post_launch(ctx, "aes_add_round_key_kernel"));
+            *in = state;
+        } else if (rd == 1) {
             uint64_t* dst = plan[r].identity ? state : rep;
-            const uint64_t* k_first = fwd ? keys : keys + (size_t)10 * blk;
             aes_public_round1_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(k_first, d_plan, rep_pos(r), (int)L, n_words, dst);
             TRY(post_launch(ctx, "aes_public_round1_kernel"));
             *in = dst;
@@ -480,24 +502,31 @@ int aes_public_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, co
     const uint64_t* in = nullptr;
     for (int rd = 1; rd < rounds; rd++) {
         TRY(sbox_inputs(rd, &in));
-        TRY(wopbs_dev(ctx, lut_mid, (int)plan[rd - 1].boxes, in, muls));
-        if (fwd) {
-            aes_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)rd * blk, (int)L, total, state, idx(rd - 1));
-            TRY(post_launch(ctx, "aes_mix_columns_kernel"));
-        } else {
-            aes_inv_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)(rounds - rd) * blk, (int)L, total, state, idx(rd - 1));
-            TRY(post_launch(ctx, "aes_inv_mix_columns_kernel"));
-        }
+        TRY(wopbs_dev(ctx, lut_mid, (int)plan[rd - 1].boxes, in, muls));                                      // sub_bytes_with_gal_mul :27-48
+        mix_columns<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)(fwd ? rd : rounds - rd) * blk, (int)L, total, state, idx(rd - 1));
+        TRY(post_launch(ctx, "aes_mix_columns_kernel"));
     }
     TRY(sbox_inputs(rounds, &in));
-    TRY(wopbs_dev(ctx, lut_last, (int)plan[rounds - 1].boxes, in, muls));
-    const uint8_t* xr = xor_host ? d_plan + npos : nullptr;
-    if (!fwd) {
-        aes_inv_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, keys, (int)L, total, out_dev, idx(rounds - 1), xr);
-        return post_launch(ctx, "aes_inv_final_round_kernel");
-    }
-    aes_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)10 * blk, (int)L, total, out_dev, idx(rounds - 1), xr);
+    TRY(wopbs_dev(ctx, lut_last, (int)plan[rounds - 1].boxes, in, muls));                                     // sub_bytes :51-58
+    final_round<<<g, 256, 0, ctx->stream>>>(muls, k_last, (int)L, total, out_dev, idx(rounds - 1), xor_host ? d_plan + npos : nullptr);
     return post_launch(ctx, "aes_final_round_kernel");
+}
+
+// host-buffer form of an AES _dev entry point: ciphertext input (ct_in) through ws_in, the output through ws_out;
+// dev_call(in_dev, out_dev) runs the _dev entry point
+template <class DevCall>
+int aes_blocks_host(tac_ctx* ctx, int n_blocks, bool ct_in, const uint64_t* in_host, uint64_t* out_host, DevCall dev_call) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
+    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
+    if (ct_in) TRY(ensure(ctx, ctx->ws_in, bytes));
+    TRY(ensure(ctx, ctx->ws_out, bytes));
+    if (ct_in) CU(cudaMemcpyAsync(ctx->ws_in.p, in_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    TRY(dev_call(ctx->ws_in.as<const uint64_t>(), ctx->ws_out.as<uint64_t>()));
+    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return TAC_OK;
 }
 
 // dk present and made from (or uploaded for) the resident encryption schedule
@@ -886,106 +915,40 @@ int tac_aes_encrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_no
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    if (n_blocks < 0 || rounds < 1 || rounds > 10) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range");
-    if (n_blocks == 0) return TAC_OK;
-    TRY(aes_noise_check(ctx, in_noise_sq, rounds));
-    TRY(ensure_aes_luts(ctx));
-    const size_t L = (size_t)ctx->big() + 1, blk = 16 * 8 * L;
-    const size_t total = (size_t)n_blocks * blk;
-    TRY(ensure(ctx, ctx->ws_state, total * 8));
-    TRY(ensure(ctx, ctx->ws_muls, total * 3 * 8));
-    uint64_t* state = ctx->ws_state.as<uint64_t>();
-    uint64_t* muls = ctx->ws_muls.as<uint64_t>();
-    const int g = grid1d(total, 256, ctx->sm_count);
-    aes_add_round_key_kernel<<<g, 256, 0, ctx->stream>>>(in_dev, ctx->key_sched, blk, total, state);          // :96-99
-    TRY(post_launch(ctx, "aes_add_round_key_kernel"));
-    for (int rd = 1; rd < rounds; rd++) {
-        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut24], n_blocks * 16, state, muls));                          // sub_bytes_with_gal_mul :27-48
-        aes_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)rd * blk, (int)L, total, state, nullptr);
-        TRY(post_launch(ctx, "aes_mix_columns_kernel"));
-    }
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut8], n_blocks * 16, state, muls));                               // sub_bytes :51-58
-    aes_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, ctx->key_sched + (size_t)10 * blk, (int)L, total, out_dev, nullptr, nullptr);
-    return post_launch(ctx, "aes_final_round_kernel");
+    return aes_blocks_dev(ctx, AesDir::Forward, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
 }
 int tac_aes_encrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
-    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
-    TRY(ensure(ctx, ctx->ws_in, bytes));
-    TRY(ensure(ctx, ctx->ws_out, bytes));
-    CU(cudaMemcpyAsync(ctx->ws_in.p, in_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    TRY(tac_aes_encrypt_blocks_dev(ctx, n_blocks, rounds, in_noise_sq, ctx->ws_in.as<uint64_t>(), ctx->ws_out.as<uint64_t>()));
-    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return TAC_OK;
+    return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
+        return tac_aes_encrypt_blocks_dev(ctx, n_blocks, rounds, in_noise_sq, in, out);
+    });
 }
-
 
 int tac_aes_encrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    return aes_public_blocks_dev(ctx, AesDir::Forward, n_blocks, rounds, blocks_host, xor_host, out_dev);
+    return aes_blocks_dev(ctx, AesDir::Forward, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);   // trivial input: no noise of its own
 }
 int tac_aes_encrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
-    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
-    TRY(ensure(ctx, ctx->ws_out, bytes));
-    TRY(tac_aes_encrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, ctx->ws_out.as<uint64_t>()));
-    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return TAC_OK;
+    return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
+        return tac_aes_encrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, out);
+    });
 }
 
 // ------------------------------------------------------------------------------------ AES decryption (FIPS-197 §5.3.5)
-// Equivalent inverse cipher, the exact inverse of tac_aes_encrypt_blocks_dev for the same `rounds` (whose final round adds
-// w[40..43] for every `rounds`):
-//   s = in + dk[40..43];  for rd = rounds−1 … 1: s = InvMixColumns(InvShiftRows(InvS(s))) + dk[rd];  out = InvShiftRows(InvS(s)) + dk[0..3]
-// InvS·{14, 11, 13, 9} comes out of one 8 → 32 circuit bootstrap per byte, so a middle round sums 4 outputs of squared noise 8
-// and one round key of level 1: 33, as in the forward direction.  Round keys are read from dk only.
+// Equivalent inverse cipher (aes_blocks_dev, AesDir::Inverse).  InvS·{14, 11, 13, 9} comes out of one 8 → 32 circuit
+// bootstrap per byte, so a middle round sums 4 outputs of squared noise 8 and one round key of level 1: 33, as in the
+// forward direction.  Round keys are read from dk only.
 int tac_aes_decrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_dev, uint64_t* out_dev) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     TRY(inv_key_sched_check(ctx));
-    if (n_blocks < 0 || rounds < 1 || rounds > 10) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range");
-    if (n_blocks == 0) return TAC_OK;
-    TRY(aes_noise_check(ctx, in_noise_sq, rounds));
-    TRY(ensure_aes_inv_luts(ctx));
-    const size_t L = (size_t)ctx->big() + 1, blk = 16 * 8 * L;
-    const size_t total = (size_t)n_blocks * blk;
-    TRY(ensure(ctx, ctx->ws_state, total * 8));
-    TRY(ensure(ctx, ctx->ws_muls, total * 4 * 8));
-    uint64_t* state = ctx->ws_state.as<uint64_t>();
-    uint64_t* muls = ctx->ws_muls.as<uint64_t>();
-    const uint64_t* dk = ctx->inv_key_sched;
-    const int g = grid1d(total, 256, ctx->sm_count);
-    aes_add_round_key_kernel<<<g, 256, 0, ctx->stream>>>(in_dev, dk + (size_t)10 * blk, blk, total, state);
-    TRY(post_launch(ctx, "aes_add_round_key_kernel"));
-    for (int rd = rounds - 1; rd >= 1; rd--) {
-        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut_inv32], n_blocks * 16, state, muls));
-        aes_inv_mix_columns_kernel<<<g, 256, 0, ctx->stream>>>(muls, dk + (size_t)rd * blk, (int)L, total, state, nullptr);
-        TRY(post_launch(ctx, "aes_inv_mix_columns_kernel"));
-    }
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut_inv8], n_blocks * 16, state, muls));
-    aes_inv_final_round_kernel<<<g, 256, 0, ctx->stream>>>(muls, dk, (int)L, total, out_dev, nullptr, nullptr);
-    return post_launch(ctx, "aes_inv_final_round_kernel");
+    return aes_blocks_dev(ctx, AesDir::Inverse, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
 }
 int tac_aes_decrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
-    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
-    TRY(ensure(ctx, ctx->ws_in, bytes));
-    TRY(ensure(ctx, ctx->ws_out, bytes));
-    CU(cudaMemcpyAsync(ctx->ws_in.p, in_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    TRY(tac_aes_decrypt_blocks_dev(ctx, n_blocks, rounds, in_noise_sq, ctx->ws_in.as<uint64_t>(), ctx->ws_out.as<uint64_t>()));
-    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return TAC_OK;
+    return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
+        return tac_aes_decrypt_blocks_dev(ctx, n_blocks, rounds, in_noise_sq, in, out);
+    });
 }
 
 // decryption of PUBLIC ciphertext blocks (AES-ECB / AES-CBC transciphering): state0 = dk[40..43] + trivial(block), the
@@ -994,18 +957,12 @@ int tac_aes_decrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, co
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     TRY(inv_key_sched_check(ctx));
-    return aes_public_blocks_dev(ctx, AesDir::Inverse, n_blocks, rounds, blocks_host, xor_host, out_dev);
+    return aes_blocks_dev(ctx, AesDir::Inverse, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);   // trivial input: no noise of its own
 }
 int tac_aes_decrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
-    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
-    TRY(ensure(ctx, ctx->ws_out, bytes));
-    TRY(tac_aes_decrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, ctx->ws_out.as<uint64_t>()));
-    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return TAC_OK;
+    return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
+        return tac_aes_decrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, out);
+    });
 }
 
 // inverse key schedule on the device from the resident encryption schedule: dk[0..3] = w[0..3], dk[40..43] = w[40..43],

@@ -4,9 +4,10 @@
 //   pfks_digits_kernel     digits of the private functional packing keyswitch for the integer-pipe GEMM (base_log > 16)
 //   lwe_gemm_kernel        exact integer GEMM mod 2^64 on the integer pipe: out[ct][col] = corr[col] − Σ_k digit'[ct][k]·key[k][col]
 //                          (PFKS of params_sqrd_lvl_1, and the correction rows of both keyswitches at key upload)
-//   aes_*_kernel           AddRoundKey / ShiftRows+MixColumns+AddRoundKey / final round as gather-adds on the flat state;
-//                          round-1 inputs and representative gathers of the public-block path;
-//   aes_inv_*_kernel       the same glue for the equivalent inverse cipher, and InvMixColumns of the inverse key schedule
+//   aes_*_kernel           AddRoundKey / (Inv)ShiftRows+(Inv)MixColumns+AddRoundKey / final round as gather-adds on the flat
+//                          state (aes_mix_columns_kernel and aes_final_round_kernel templated on the direction); round-1
+//                          inputs and representative gathers of the public-block path; InvMixColumns of the inverse key
+//                          schedule (aes_inv_mix_key_kernel)
 //   lwe_add_kernel         leveled XOR (lwe_ciphertext_add_assign) over a batch; lwe_shl_kernel / lwe_sub_kernel: glue of extract_bits
 //   negate_kernel, dfma_peak_kernel   key-upload helper, FP64 peak microbenchmark (roofline denominator)
 #pragma once
@@ -95,28 +96,38 @@ __global__ void aes_add_round_key_kernel(const uint64_t* __restrict__ in, const 
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x)
         out[i] = in[i] + rk[i % blk_words];
 }
-// ShiftRows on the three SBOX·{1,2,3} states + MixColumns + AddRoundKey (fhe_sbox_gal_mul_pbs.rs:61-82, :106-117)
-//   new[r][c] = mul2[r] ^ mul1[r-1] ^ mul1[r-2] ^ mul3[r-3]  (rows mod 4, within shifted column c)
-// muls: [row][24 = (S, 2S, 3S) × 8 bits][L], row = block·16 + byte, or idx[block·16 + byte] when idx is given (a compact
-// batch of S-box outputs shared by several positions: tac_aes_encrypt_public_blocks)
+// ShiftRows + MixColumns + AddRoundKey of a middle round as one gather-add over the S-box rows; Fwd = false is InvShiftRows +
+// InvMixColumns of the equivalent inverse cipher (FIPS-197 §5.3.5, round keys from dk):
+//   new[row][c] = Σ_rr coef[(rr − row) mod 4] · S(old[rr][(c ± rr) mod 4])       (+ for ShiftRows, − for InvShiftRows)
+//   forward  coef = {2, 3, 1, 1}      muls rows [24 = (S, 2S, 3S) × 8 bits][L]               (fhe_sbox_gal_mul_pbs.rs:61-82, :106-117)
+//   inverse  coef = {14, 11, 13, 9}   muls rows [32 = (14, 11, 13, 9)·InvS × 8 bits][L]
+// row = block·16 + byte, or idx[block·16 + byte] when idx is given (a compact batch of S-box outputs shared by several
+// positions: AES over public blocks)
+template <bool Fwd>
 __global__ void aes_mix_columns_kernel(const uint64_t* __restrict__ muls, const uint64_t* __restrict__ rk, int L, size_t total,
                                        uint64_t* __restrict__ state, const int32_t* __restrict__ idx) {
+    constexpr int W = Fwd ? 24 : 32;
     const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
         const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;   // bit·L + e
         const int c = byte >> 2, r = byte & 3;
-        auto src = [&](int which, int row) -> uint64_t {
-            const int old_byte = 4 * ((c + row) & 3) + row;        // ShiftRows: new[row][c] = old[row][(c+row)%4]
+        uint64_t v = rk[rem];
+#pragma unroll
+        for (int rr = 0; rr < 4; rr++) {
+            const int d = (rr - r) & 3;
+            const int slot = Fwd ? (d < 2 ? d + 1 : 0) : d;                  // muls slot of coef[d]
+            const int old_byte = 4 * ((Fwd ? c + rr : c - rr) & 3) + rr;
             const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
-            return muls[(src_row * 24 + (size_t)which * 8) * L + w];
-        };
-        state[i] = src(1, r) + src(0, (r + 3) & 3) + src(0, (r + 2) & 3) + src(2, (r + 1) & 3) + rk[rem];
+            v += muls[(src_row * W + (size_t)slot * 8) * L + w];
+        }
+        state[i] = v;
     }
 }
-// last round (fhe_sbox_gal_mul_pbs.rs:119-129): ShiftRows(sub) + rk[40..44].  sub rows as in aes_mix_columns_kernel
-// ([row][8 bits][L], idx optional).  xr: NULL, or [block][16] public bytes XORed into the output (a trivial ciphertext
-// added: encode_bit(1) = 2^63 on the body of every set bit).
+// last round (fhe_sbox_gal_mul_pbs.rs:119-129): ShiftRows(S) + w[40..43], or InvShiftRows(InvS) + dk[0..3].  sub rows
+// [row][8 bits][L] (idx optional, as in aes_mix_columns_kernel).  xr: NULL, or [block][16] public bytes XORed into the
+// output (a trivial ciphertext added: encode_bit(1) = 2^63 on the body of every set bit).
+template <bool Fwd>
 __global__ void aes_final_round_kernel(const uint64_t* __restrict__ sub, const uint64_t* __restrict__ rk, int L, size_t total,
                                        uint64_t* __restrict__ out, const int32_t* __restrict__ idx,
                                        const uint8_t* __restrict__ xr) {
@@ -125,7 +136,7 @@ __global__ void aes_final_round_kernel(const uint64_t* __restrict__ sub, const u
         const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
         const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;
         const int c = byte >> 2, r = byte & 3;
-        const int old_byte = 4 * ((c + r) & 3) + r;
+        const int old_byte = 4 * ((Fwd ? c + r : c - r) & 3) + r;
         const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
         uint64_t v = sub[src_row * byte_words + w] + rk[rem];
         if (xr) {
@@ -147,48 +158,6 @@ __global__ void aes_public_round1_kernel(const uint64_t* __restrict__ k0, const 
         const int bit = (int)(w / L);
         uint64_t v = k0[(size_t)(pos & 15) * byte_words + w];
         if (w - (size_t)bit * L == (size_t)L - 1 && (blocks[pos] & (0x80 >> bit))) v += 1ull << 63;
-        out[i] = v;
-    }
-}
-// ---- equivalent inverse cipher (FIPS-197 §5.3.5): the decryption glue, kept apart from the forward kernels above
-// InvShiftRows on the InvS·{14, 11, 13, 9} states + InvMixColumns + AddRoundKey (inverse key schedule dk):
-//   new[row][c] = Σ_{r'} coef[(r' − row) mod 4] · InvS(old[r'][(c − r') mod 4]),   coef = {14, 11, 13, 9}
-// muls: [row][32 = (14, 11, 13, 9)·InvS × 8 bits][L], row = block·16 + byte, or idx[block·16 + byte] (compact batch of the
-// public-block path: tac_aes_decrypt_public_blocks)
-__global__ void aes_inv_mix_columns_kernel(const uint64_t* __restrict__ muls, const uint64_t* __restrict__ rk, int L, size_t total,
-                                           uint64_t* __restrict__ state, const int32_t* __restrict__ idx) {
-    const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-        const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
-        const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;   // bit·L + e
-        const int c = byte >> 2, r = byte & 3;
-        uint64_t v = rk[rem];
-#pragma unroll
-        for (int rr = 0; rr < 4; rr++) {
-            const int old_byte = 4 * ((c - rr) & 3) + rr;          // InvShiftRows: new[rr][c] = old[rr][(c−rr)%4]
-            const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
-            v += muls[(src_row * 32 + (size_t)((rr - r) & 3) * 8) * L + w];
-        }
-        state[i] = v;
-    }
-}
-// last inverse round: InvShiftRows(InvS) + dk[0..3].  sub rows [row][8 bits][L] (idx optional); xr: NULL, or [block][16]
-// public bytes XORed into the output (the previous ciphertext block of AES-CBC), as in aes_final_round_kernel
-__global__ void aes_inv_final_round_kernel(const uint64_t* __restrict__ sub, const uint64_t* __restrict__ rk, int L, size_t total,
-                                           uint64_t* __restrict__ out, const int32_t* __restrict__ idx,
-                                           const uint8_t* __restrict__ xr) {
-    const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-        const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
-        const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;
-        const int c = byte >> 2, r = byte & 3;
-        const int old_byte = 4 * ((c - r) & 3) + r;
-        const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
-        uint64_t v = sub[src_row * byte_words + w] + rk[rem];
-        if (xr) {
-            const int bit = (int)(w / L);
-            if (w - (size_t)bit * L == (size_t)L - 1 && (xr[blk * 16 + byte] & (0x80 >> bit))) v += 1ull << 63;
-        }
         out[i] = v;
     }
 }

@@ -396,15 +396,7 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
     // one 16-byte row per block) is XORed into the output — the AES-CTR ciphertext for transciphering
     static std::vector<data_model::BlockT<Bit>> encrypt_public_blocks(const Ctx& c, const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
                                                                        const std::vector<std::array<uint8_t, 16>>& xor_bytes = {}) {
-        if (!xor_bytes.empty() && xor_bytes.size() != blocks.size()) throw std::invalid_argument("xor_bytes: one row per block");
-        const size_t L = c.lwe_size();
-        std::vector<uint64_t> out(blocks.size() * 128 * L);
-        c.check(tac_aes_encrypt_public_blocks(c.raw(), (int)blocks.size(), rounds, blocks.empty() ? nullptr : blocks[0].data(),
-                                              xor_bytes.empty() ? nullptr : xor_bytes[0].data(), out.data()));
-        std::vector<data_model::BlockT<Bit>> res(blocks.size());
-        for (size_t q = 0; q < blocks.size(); q++) for (int b = 0; b < 16; b++) for (int i = 0; i < 8; i++)
-            res[q][b][i] = BitCt::with_noise_level(std::vector<uint64_t>(out.begin() + ((q * 16 + b) * 8 + i) * L, out.begin() + ((q * 16 + b) * 8 + i + 1) * L), 8 + 1, c);
-        return res;
+        return public_blocks(tac_aes_encrypt_public_blocks, c, blocks, rounds, xor_bytes);
     }
     // AES decryption (equivalent inverse cipher, FIPS-197 §5.3.5; the reference has none): derive the inverse key schedule
     // from the device key schedule, once per key schedule.  Decryption fails (TAC_ERR_STATE) until this has run.
@@ -413,11 +405,19 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
     // XORed into the output — the previous ciphertext blocks (IV first) for AES-CBC transciphering, empty for AES-ECB
     static std::vector<data_model::BlockT<Bit>> decrypt_public_blocks(const Ctx& c, const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
                                                                        const std::vector<std::array<uint8_t, 16>>& xor_bytes = {}) {
+        return public_blocks(tac_aes_decrypt_public_blocks, c, blocks, rounds, xor_bytes);
+    }
+
+private:
+    // fn (tac_aes_{en,de}crypt_public_blocks) over the blocks; outputs are bit ciphertexts of squared noise level 9
+    static std::vector<data_model::BlockT<Bit>> public_blocks(int (*fn)(tac_ctx*, int, int, const uint8_t*, const uint8_t*, uint64_t*), const Ctx& c,
+                                                              const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
+                                                              const std::vector<std::array<uint8_t, 16>>& xor_bytes) {
         if (!xor_bytes.empty() && xor_bytes.size() != blocks.size()) throw std::invalid_argument("xor_bytes: one row per block");
         const size_t L = c.lwe_size();
         std::vector<uint64_t> out(blocks.size() * 128 * L);
-        c.check(tac_aes_decrypt_public_blocks(c.raw(), (int)blocks.size(), rounds, blocks.empty() ? nullptr : blocks[0].data(),
-                                              xor_bytes.empty() ? nullptr : xor_bytes[0].data(), out.data()));
+        c.check(fn(c.raw(), (int)blocks.size(), rounds, blocks.empty() ? nullptr : blocks[0].data(), xor_bytes.empty() ? nullptr : xor_bytes[0].data(),
+                   out.data()));
         std::vector<data_model::BlockT<Bit>> res(blocks.size());
         for (size_t q = 0; q < blocks.size(); q++) for (int b = 0; b < 16; b++) for (int i = 0; i < 8; i++)
             res[q][b][i] = BitCt::with_noise_level(std::vector<uint64_t>(out.begin() + ((q * 16 + b) * 8 + i) * L, out.begin() + ((q * 16 + b) * 8 + i + 1) * L), 8 + 1, c);
