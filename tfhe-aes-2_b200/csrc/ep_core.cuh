@@ -32,8 +32,8 @@ struct alignas(16) cplx { double x, y; };
 TAC_HD cplx mk(double x, double y) { cplx r; r.x = x; r.y = y; return r; }
 TAC_HD cplx cmul(cplx a, cplx b) { return mk(fma(-a.y, b.y, a.x * b.x), fma(a.y, b.x, a.x * b.y)); }
 TAC_HD cplx cmul_conj(cplx a, cplx b) { return mk(fma(a.y, b.y, a.x * b.x), fma(-a.x, b.y, a.y * b.x)); }   // a * conj(b)
-// o += a·b.  The order of the four FMAs is part of the contract: every MAC variant (one thread per slot, or the real /
-// imaginary split over a lane pair) accumulates in exactly this order, so all of them produce the same words.
+// o += a·b.  The order of the four FMAs is part of the contract: every MAC (ph_mac, mg_mac, the MAC of pbs_wide_kernel)
+// accumulates in exactly this order, so all of them produce the same words.
 TAC_HD void cfma(cplx& o, cplx a, cplx b) {
     o.x = fma(a.x, b.x, o.x); o.x = fma(-a.y, b.y, o.x);
     o.y = fma(a.y, b.x, o.y); o.y = fma(a.x, b.y, o.y);
@@ -171,30 +171,9 @@ TAC_HD constexpr int slot_of(int q, int i) { return q * 16 + (i ^ (q & 15)); }
 // form "load – compute – store" is executed strictly one element at a time and exposes the shared-memory latency every
 // time (measured: 16 serialised twiddle loads ≈ 400 cycles of a 1550-cycle pass, tools/fft_lat.cu; PBS kernel 119.4 → 113.4 ms).  The passes below are
 // therefore written in CHUNKS: all loads of a chunk first, then the arithmetic and the stores of the chunk.
-#ifndef TAC_CHUNK
-#define TAC_CHUNK 8
-#endif
-#ifndef TAC_LOAD_CHUNK
-#define TAC_LOAD_CHUNK 4
-#endif
-constexpr int kChunk = TAC_CHUNK;             // twiddles per chunk (32 registers in flight); measured on B200: 8 → 113.4 ms, 4 or 16 → 116.5 ms
-constexpr int kLoadChunk = TAC_LOAD_CHUNK;    // operand pairs per chunk of the decomposing pass (2, 4, 8, 16 measure the same)
+constexpr int kLoadChunk = 4;                 // operand pairs per chunk of the decomposing pass (2, 4, 8, 16 measure the same)
 TAC_HD constexpr int tab_len(int N) { return N; }    // entries of wT
 
-// S[slot] = v[i] · conj(wT[slot]) for the P registers of thread t, chunked
-template <int P, class SlotFn>
-TAC_HD void twiddle_store_conj(const cplx* v, SlotFn slot, const cplx* __restrict__ wT, cplx* __restrict__ S) {
-    constexpr int CH = P < kChunk ? P : kChunk;
-    static_for<0, P, CH>([&](auto cc) {
-        constexpr int c0 = decltype(cc)::value;
-        cplx w[CH];
-        static_for<0, CH>([&](auto kc) { constexpr int k = decltype(kc)::value; w[k] = wT[slot(c0 + k)]; });
-        static_for<0, CH>([&](auto kc) {
-            constexpr int k = decltype(kc)::value;
-            if constexpr (c0 + k == 0) S[slot(0)] = v[0]; else S[slot(c0 + k)] = cmul_conj(v[c0 + k], w[k]);
-        });
-    });
-}
 // the pass-1 DFT of the forward transform on v[bitrev(m)] = z_{t+16m}: twist c^m folded (see above)
 template <int N>
 TAC_HD void dft_fwd_twisted(cplx* v) {
@@ -258,35 +237,6 @@ TAC_HD void fft_fwd_pass1_m(int t, Src src, cplx* __restrict__ S) {
     static_for<0, P>([&](auto qc) { constexpr int q = decltype(qc)::value; S[slot_of(q, t)] = v[q]; });
 }
 // ------------------------------------------------------------------------------------------------ forward, pass 2 (in place)
-// The 15 butterfly twiddles of lane q do not depend on the data: a caller can fetch them into registers BEFORE pass 1
-// (fft_fwd_twiddles), so that those shared-memory reads overlap the FP64 work of pass 1 instead of lengthening the load
-// burst at the start of pass 2 — every group of a CTA runs the same pass at the same time, so a pass is a burst of loads,
-// then arithmetic, then a burst of stores, and the load/store unit idles exactly while the FP64 pipe is busy.
-// (Only when a thread runs one DFT-16 in pass 2, i.e. N = 512; larger N load them inside the pass.)
-#ifndef TAC_FWD_TW_PREFETCH
-#define TAC_FWD_TW_PREFETCH 0
-#endif
-#ifndef TAC_INV_TW_EARLY
-#define TAC_INV_TW_EARLY 0
-#endif
-template <int N> struct FwdTw { static constexpr bool PRE = TAC_FWD_TW_PREFETCH && (N / 32 == 16); static constexpr int LEN = PRE ? 15 : 1; };
-template <int N>
-TAC_HD void fft_fwd_twiddles(int t, const cplx* __restrict__ wT, cplx (&tw)[FwdTw<N>::LEN]) {
-    if constexpr (FwdTw<N>::PRE) {
-        constexpr int M = N / 2, P = M / 16;
-        static_for<0, 15>([&](auto ec) { constexpr int e = decltype(ec)::value; tw[e] = wT[M + e * P + t]; });
-    }
-}
-template <int N, class TwFn>
-TAC_HD void fft_fwd_pass2_core(int q, TwFn&& twf, cplx* __restrict__ S) {
-    cplx v[16];
-    static_for<0, 16>([&](auto tc) { constexpr int tt = decltype(tc)::value; v[bitrev<16>(tt)] = S[slot_of(q, tt)]; });
-    dit_stages<16, 2>(v, [&](auto lc, auto kc, cplx& u, cplx& w) {
-        constexpr int LEN = decltype(lc)::value, k = decltype(kc)::value;
-        bfly_r(u, w, twf(std::integral_constant<int, LEN / 2 - 1 + k>{}));
-    });
-    static_for<0, 16>([&](auto rc) { constexpr int r = decltype(rc)::value; S[slot_of(q, r)] = v[r]; });
-}
 // multiply by exp(2πi·A/128), A a compile-time angle (free for multiples of a quarter turn)
 template <int A>
 TAC_HD cplx rot128(cplx d) {
@@ -297,13 +247,10 @@ TAC_HD cplx rot128(cplx d) {
     else if constexpr (a == 96) return mk(d.y, -d.x);
     else { const double c = cosq<a>(), sn = sinq<a>(); return mk(fma(-d.y, sn, d.x * c), fma(d.y, c, d.x * sn)); }
 }
-#ifndef TAC_TW_DERIVE
-#define TAC_TW_DERIVE 1
-#endif
-// TAC_TW_DERIVE: the 15 twiddles of pass 2 are  ρ_q^{16/LEN} · e^{-2πi k/LEN}.  Only the four powers ρ_q^{8,4,2,1} (the
-// k = 0 entries) are read from the table; the others are formed with a compile-time rotation — 8 complex multiplies per
-// pass instead of 11 more 16-byte shared-memory loads per thread.  The kernel's load/store unit is its busiest resource
-// (63 % of the data-pipe wavefronts) while the FP64 pipe has slack (46 %), so arithmetic is the cheaper currency.
+// The 15 twiddles of pass 2 are  ρ_q^{16/LEN} · e^{-2πi k/LEN}.  Only the four powers ρ_q^{8,4,2,1} (the k = 0 entries)
+// are read from the table; the others are formed with a compile-time rotation — 8 complex multiplies per pass instead of
+// 11 more 16-byte shared-memory loads per thread.  The kernel's load/store unit is its busiest resource (63 % of the
+// data-pipe wavefronts) while the FP64 pipe has slack (46 %), so arithmetic is the cheaper currency.
 template <int N>
 TAC_HD void fft_fwd_pass2(int t, const cplx* __restrict__ wT, cplx* __restrict__ S) {
     constexpr int M = N / 2, P = M / 16;
@@ -311,28 +258,22 @@ TAC_HD void fft_fwd_pass2(int t, const cplx* __restrict__ wT, cplx* __restrict__
 #pragma unroll
     for (int c2 = 0; c2 < P / 16; c2++) {
         const int q = t + 16 * c2;
-#if TAC_TW_DERIVE
         cplx base[4];                      // LEN = 2, 4, 8, 16 at k = 0: table entries 0, 1, 3, 7
         static_for<0, 4>([&](auto ic) { constexpr int i = decltype(ic)::value; base[i] = wF[((1 << i) - 1) * P + q]; });
-        fft_fwd_pass2_core<N>(q, [&](auto ec) {
-            constexpr int e = decltype(ec)::value;
-            constexpr int lg = (e >= 7) ? 3 : (e >= 3) ? 2 : (e >= 1) ? 1 : 0, LEN = 2 << lg, k = e - (LEN / 2 - 1);
-            return rot128<-128 * k / LEN>(base[lg]);
-        }, S);
-#else
-        fft_fwd_pass2_core<N>(q, [&](auto ec) { return wF[decltype(ec)::value * P + q]; }, S);
-#endif
+        cplx v[16];
+        static_for<0, 16>([&](auto tc) { constexpr int tt = decltype(tc)::value; v[bitrev<16>(tt)] = S[slot_of(q, tt)]; });
+        dit_stages<16, 2>(v, [&](auto lc, auto kc, cplx& u, cplx& w) {
+            constexpr int LEN = decltype(lc)::value, k = decltype(kc)::value;
+            constexpr int lg = (LEN == 16) ? 3 : (LEN == 8) ? 2 : (LEN == 4) ? 1 : 0;
+            bfly_r(u, w, rot128<-128 * k / LEN>(base[lg]));
+        });
+        static_for<0, 16>([&](auto rc) { constexpr int r = decltype(rc)::value; S[slot_of(q, r)] = v[r]; });
     }
 }
-// pass 2 with the twiddles already in registers (fft_fwd_twiddles)
-template <int N>
-TAC_HD void fft_fwd_pass2(int t, const cplx* __restrict__ wT, const cplx (&tw)[FwdTw<N>::LEN], cplx* __restrict__ S) {
-    if constexpr (FwdTw<N>::PRE) fft_fwd_pass2_core<N>(t, [&](auto ec) { return tw[decltype(ec)::value]; }, S);
-    else fft_fwd_pass2<N>(t, wT, S);
-}
 // ------------------------------------------------------------------------------------------------ inverse, pass A (in place)
-// the 16 twiddles are requested together with the data, ahead of the arithmetic (same reasoning as above)
-template <int N, int MODE = (TAC_TW_DERIVE ? 2 : TAC_INV_TW_EARLY ? 1 : 0)>
+// ρ_q^t for t = 1, 2, 4, 8 are requested together with the data, ahead of the arithmetic (see "Memory-operation order");
+// the other powers are formed as products (at most three multiplications deep)
+template <int N>
 TAC_HD void fft_inv_passA(int t, const cplx* __restrict__ wT, cplx* __restrict__ S) {
     constexpr int M = N / 2, P = M / 16;
 #pragma unroll
@@ -340,8 +281,6 @@ TAC_HD void fft_inv_passA(int t, const cplx* __restrict__ wT, cplx* __restrict__
         const int q = t + 16 * c2;
         cplx v[16];
         static_for<0, 16>([&](auto rc) { constexpr int r = decltype(rc)::value; v[bitrev<16>(r)] = S[slot_of(q, r)]; });
-        if constexpr (MODE == 2) {
-        // ρ_q^t for t = 1, 2, 4, 8 from the table, the other powers as products (at most three multiplications deep)
         cplx w[16];
         w[1] = wT[slot_of(q, 1)]; w[2] = wT[slot_of(q, 2)]; w[4] = wT[slot_of(q, 4)]; w[8] = wT[slot_of(q, 8)];
         dft_inv<16>(v);
@@ -349,16 +288,6 @@ TAC_HD void fft_inv_passA(int t, const cplx* __restrict__ wT, cplx* __restrict__
         static_for<9, 16>([&](auto tc) { constexpr int tt = decltype(tc)::value; w[tt] = cmul(w[8], w[tt - 8]); });
         S[slot_of(q, 0)] = v[0];
         static_for<1, 16>([&](auto tc) { constexpr int tt = decltype(tc)::value; S[slot_of(q, tt)] = cmul_conj(v[tt], w[tt]); });
-        } else if constexpr (MODE == 1) {
-        cplx w[16];
-        static_for<1, 16>([&](auto tc) { constexpr int tt = decltype(tc)::value; w[tt] = wT[slot_of(q, tt)]; });
-        dft_inv<16>(v);
-        S[slot_of(q, 0)] = v[0];
-        static_for<1, 16>([&](auto tc) { constexpr int tt = decltype(tc)::value; S[slot_of(q, tt)] = cmul_conj(v[tt], w[tt]); });
-        } else {
-        dft_inv<16>(v);
-        twiddle_store_conj<16>(v, [&](int tt) { return slot_of(q, tt); }, wT, S);
-        }
     }
 }
 // ------------------------------------------------------------------------------------------------ inverse, pass B

@@ -27,31 +27,14 @@
 
 namespace tac {
 
-// Key loads: read-only path; TAC_LDG_MODE picks the cache hint (0: ld.global.nc, 1: + L1::no_allocate, 2: + L1::evict_first,
-// 3: ld.global.cg-style L2-only via .L1::no_allocate.L2::128B prefetch size) — measured with tools/pbs_bench.cu.
-#ifndef TAC_LDG_MODE
-#define TAC_LDG_MODE 0
-#endif
+// Key loads take the read-only path (ld.global.nc); cache hints on top of it measured no different (DESIGN.md §4).
+TAC_HD cplx ldg_key(const cplx* p) {
 #if defined(__CUDA_ARCH__)
-__device__ __forceinline__ cplx tac_ldg_key(const cplx* p) {
-    cplx r;
-#if TAC_LDG_MODE == 1
-    asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0, %1}, [%2];" : "=d"(r.x), "=d"(r.y) : "l"(p));
-#elif TAC_LDG_MODE == 2
-    asm volatile("ld.global.nc.L1::evict_first.v2.f64 {%0, %1}, [%2];" : "=d"(r.x), "=d"(r.y) : "l"(p));
-#elif TAC_LDG_MODE == 3
-    asm volatile("ld.global.nc.L1::no_allocate.L2::128B.v2.f64 {%0, %1}, [%2];" : "=d"(r.x), "=d"(r.y) : "l"(p));
-#elif TAC_LDG_MODE == 4
-    asm volatile("ld.global.nc.L1::no_allocate.L2::256B.v2.f64 {%0, %1}, [%2];" : "=d"(r.x), "=d"(r.y) : "l"(p));
+    return __ldg(p);
 #else
-    r = __ldg(p);
+    return *p;
 #endif
-    return r;
 }
-#define TAC_LDG(p) tac_ldg_key(p)
-#else
-#define TAC_LDG(p) (*(p))
-#endif
 
 template <int N_, int K_, int L_, int B_>
 struct EpCfg {
@@ -90,31 +73,19 @@ TAC_HD void grp_fwd1(int t, int job, int lev, const DecompFast& dc, const uint32
 }
 template <class C>
 TAC_HD void grp_fwd2(int t, int job, const cplx* __restrict__ wT, cplx* __restrict__ S) { fft_fwd_pass2<C::N>(t, wT, S + (size_t)job * C::M); }
-template <class C>
-TAC_HD void grp_fwd2(int t, int job, const cplx* __restrict__ wT, const cplx (&tw)[FwdTw<C::N>::LEN], cplx* __restrict__ S) {
-    fft_fwd_pass2<C::N>(t, wT, tw, S + (size_t)job * C::M);
-}
 // out[b][c] += Σ_p fft(digits_{lev,p} of ct b) · GGSW[lev-1][p][c]   at the slots owned by this thread.
 // ggsw: Fourier GGSW of this step, [L][G][G][M] slot-ordered (already scaled by 2^-64 / M).
 // Key prefetch ring of the MAC: rows 0..MAC_DEPTH-1 of this thread's first slot are requested BEFORE the barrier that
 // precedes the MAC (the L2 latency hides behind the barrier wait), row p+MAC_DEPTH is requested while row p is multiplied.
 // MAC_DEPTH is a kernel template parameter (register budget: each ring entry is G complex values).
-// TAC_DBG_KEY_ONE_ROW (development only, tools/pbs_bench.cu): every key load hits the same 20 KB row, which stays in L1 —
-// times the kernel WITHOUT its L2 → SM key stream (results are then meaningless).
 template <class C, int NT_MAC>
 TAC_HD void mac_load_row(const cplx* __restrict__ gl, int p, int tau, cplx (&dst)[C::G]) {
-#ifdef TAC_DBG_KEY_ONE_ROW
-    p = 0;
-#endif
 #pragma unroll
-    for (int c = 0; c < C::G; c++) dst[c] = TAC_LDG(gl + (size_t)(p * C::G + c) * C::M + tau);
+    for (int c = 0; c < C::G; c++) dst[c] = ldg_key(gl + (size_t)(p * C::G + c) * C::M + tau);
 }
 template <class C, int NT_MAC, int MAC_DEPTH>
 TAC_HD void ph_mac_prefetch(int tid, int lev, const cplx* __restrict__ ggsw, cplx (&g)[MAC_DEPTH][C::G]) {
     if (tid >= NT_MAC) return;
-#ifdef TAC_DBG_KEY_ONE_ROW
-    lev = 1;
-#endif
     const cplx* gl = ggsw + (size_t)(lev - 1) * C::G * C::G * C::M;
 #pragma unroll
     for (int p = 0; p < MAC_DEPTH && p < C::G; p++) mac_load_row<C, NT_MAC>(gl, p, tid, g[p]);
@@ -123,9 +94,6 @@ template <class C, int NT_MAC, int SPT, int MAC_DEPTH>
 TAC_HD void ph_mac(int tid, int lev, const cplx* __restrict__ ggsw, const cplx* __restrict__ S, cplx (&out)[SPT][C::B][C::G],
                    cplx (&g)[MAC_DEPTH][C::G]) {
     if (tid >= NT_MAC) return;
-#ifdef TAC_DBG_KEY_ONE_ROW
-    lev = 1;
-#endif
     const cplx* gl = ggsw + (size_t)(lev - 1) * C::G * C::G * C::M;
 #pragma unroll
     for (int it = 0; it < SPT; it++) {
@@ -143,35 +111,6 @@ TAC_HD void ph_mac(int tid, int lev, const cplx* __restrict__ ggsw, const cplx* 
                 for (int c = 0; c < C::G; c++) cfma(out[it][b][c], x, g[p % MAC_DEPTH][c]);
             }
             if (p + MAC_DEPTH < C::G) mac_load_row<C, NT_MAC>(gl, p + MAC_DEPTH, tau, g[p % MAC_DEPTH]);
-        }
-    }
-}
-// MAC with the first NS key rows of the level STAGED in shared memory (kst: [NS][G][M], filled by a bulk asynchronous copy
-// while the forward transforms ran) and the remaining rows in the register ring, all of them requested before the barrier:
-// nothing is fetched from L2 while the MAC runs.  Rows are still consumed in the order 0 … G-1, so the sums are the same words.
-template <class C, int NT_MAC, int MAC_DEPTH, int NS>
-TAC_HD void ph_mac_prefetch_staged(int tid, int lev, const cplx* __restrict__ ggsw, cplx (&g)[MAC_DEPTH][C::G]) {
-    static_assert(NS + MAC_DEPTH >= C::G, "every row that is not staged must fit the ring");
-    if (tid >= NT_MAC) return;
-    const cplx* gl = ggsw + (size_t)(lev - 1) * C::G * C::G * C::M;
-#pragma unroll
-    for (int p = NS; p < C::G; p++) mac_load_row<C, NT_MAC>(gl, p, tid, g[p - NS]);
-}
-template <class C, int NT_MAC, int MAC_DEPTH, int NS>
-TAC_HD void ph_mac_staged(int tid, const cplx* __restrict__ kst, const cplx* __restrict__ S, cplx (&out)[1][C::B][C::G], cplx (&g)[MAC_DEPTH][C::G]) {
-    if (tid >= NT_MAC) return;
-#pragma unroll
-    for (int p = 0; p < C::G; p++) {
-        cplx row[C::G];
-        if (p < NS) {
-#pragma unroll
-            for (int c = 0; c < C::G; c++) row[c] = kst[(size_t)(p * C::G + c) * C::M + tid];
-        }
-#pragma unroll
-        for (int b = 0; b < C::B; b++) {
-            const cplx x = S[(size_t)(b * C::G + p) * C::M + tid];
-#pragma unroll
-            for (int c = 0; c < C::G; c++) cfma(out[0][b][c], x, p < NS ? row[c] : g[p < NS ? 0 : p - NS][c]);
         }
     }
 }
@@ -225,11 +164,8 @@ constexpr int kL2PrefetchSteps = 2;          // how many steps ahead
 // coefficients t + 16m and t + 16m + M of the group's polynomial) and the rotation copy `Rj` in the rows of FFT buffer 0.
 //
 // digits of all L levels of (Rj · X^rot − own): dg[s][m] packs the level-(s+1) digits of samples t + 16m (low half-word) and
-// t + 16m + M (high half-word); the rotated loads of a chunk are issued first (cf. rot_diff_pair)
-// TAC_MG_TIE_CHUNK = 0: one tie test per coefficient pair (decompose_pair), the form the other kernels use — 1.7 % slower here
-#ifndef TAC_MG_TIE_CHUNK
-#define TAC_MG_TIE_CHUNK 1
-#endif
+// t + 16m + M (high half-word); the rotated loads of a chunk are issued first (cf. rot_diff_pair).  One tie test per chunk:
+// a test per coefficient pair (decompose_pair, the form the other kernels use) measured 1.7 % slower here.
 template <class C>
 TAC_HD void mg_digits(int t, const uint64_t* __restrict__ Rj, int rot, const uint64_t (&own0)[C::M / 16], const uint64_t (&own1)[C::M / 16],
                       const DecompFast& dc, uint32_t (&dg)[C::L][C::M / 16]) {
@@ -247,7 +183,6 @@ TAC_HD void mg_digits(int t, const uint64_t* __restrict__ Rj, int rot, const uin
             g0[k] = s0 >> LOGN; g1[k] = g0[k] ^ (i0 >> (LOGN - 1));
             v0[k] = Rj[i0]; v1[k] = Rj[i1];
         });
-#if TAC_MG_TIE_CHUNK
         // closed-form digits of the whole chunk, ONE tie test per chunk (a branch per pair exposes the latency of the
         // pair's dependent chain every time: in-order issue waits for the predicate)
         uint64_t x0[CH], x1[CH];
@@ -281,17 +216,6 @@ TAC_HD void mg_digits(int t, const uint64_t* __restrict__ Rj, int rot, const uin
                 }
             });
         }
-#else
-        static_for<0, CH>([&](auto kc) {
-            constexpr int k = decltype(kc)::value, m = c0 + k;
-            const uint32_t m0 = 0u - g0[k], m1 = 0u - g1[k];
-            const uint64_t w0 = ((uint64_t)((uint32_t)(v0[k] >> 32) ^ m0) << 32) | ((uint32_t)v0[k] ^ m0);
-            const uint64_t w1 = ((uint64_t)((uint32_t)(v1[k] >> 32) ^ m1) << 32) | ((uint32_t)v1[k] ^ m1);
-            uint32_t w[C::L];
-            decompose_pair<C::L>((w0 + g0[k]) - own0[m], (w1 + g1[k]) - own1[m], dc, w);
-            static_for<0, C::L>([&](auto sc) { constexpr int s = decltype(sc)::value; dg[s][m] = w[s]; });
-        });
-#endif
     });
 }
 // key row r of a step's Fourier GGSW in MAC order: level L first, polynomial p inside

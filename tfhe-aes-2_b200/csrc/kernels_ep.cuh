@@ -49,66 +49,11 @@ struct EpSmem {
 // accumulators receive  acc += GGSW ⊡ operand.
 // Ends with a __syncwarp(): the accumulator rows of a job are only touched by the job's own 16-thread group, so the next
 // step's decomposition may follow without a CTA barrier.  (Readers of acc from other groups must __syncthreads() first.)
-// TAC_EP_DBG (development only, tools/pbs_bench.cu): bit 0 skips the Fourier MAC, bit 1 the forward FFT passes, bit 2 the
-// inverse passes, bit 3 the decomposition — timing attribution of the phases in situ; the results are then meaningless.
-#ifndef TAC_EP_DBG
-#define TAC_EP_DBG 0
-#endif
-// TAC_EP_TIMING (development only): thread 0 of CTA 0 accumulates clock64() deltas per phase of the step into tac_ep_times
-#ifdef TAC_EP_TIMING
-__device__ long long tac_ep_times[32];
-#define TAC_EP_T(k) do { if (tid == 0 && blockIdx.x == 0) { const long long now_ = clock64(); tac_ep_times[k] += now_ - tac_tprev; tac_tprev = now_; } } while (0)
-#else
-#define TAC_EP_T(k) do { } while (0)
-#endif
-// ---- key staging: the first NS rows of a level's Fourier GGSW travel into shared memory by one bulk asynchronous copy
-// (cp.async.bulk, completion on an mbarrier) issued a whole FFT phase ahead of the MAC that consumes them
-namespace kstage {
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count)); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-}  // namespace kstage
-template <class C, int NS>
-struct KeyStage {
-    cplx* buf;                   // [NS][G][M]
-    uint32_t bar;                // shared-memory address of the mbarrier
-    uint32_t uses;               // completed waits (parity of the next one)
-    static constexpr uint32_t row_bytes = (uint32_t)(C::G * C::M * sizeof(cplx));
-    static constexpr size_t bytes = (size_t)NS * row_bytes;
-    // one thread: request rows 0 … NS-1 of level `lev` of `ggsw`
-    __device__ __forceinline__ void request(const cplx* __restrict__ ggsw, int lev) const {
-        const cplx* gl = ggsw + (size_t)(lev - 1) * C::G * C::G * C::M;
-        kstage::mbar_expect_tx(bar, NS * row_bytes);
-#pragma unroll
-        for (int r = 0; r < NS; r++) kstage::bulk_g2s(kstage::smem_u32(buf) + r * row_bytes, gl + (size_t)r * C::G * C::M, row_bytes, bar);
-    }
-    __device__ __forceinline__ void wait() { kstage::mbar_wait(bar, uses & 1u); uses++; }
-};
-template <class C> struct KeyStage<C, 0> { static constexpr size_t bytes = 0; };
-// dynamic shared memory of pbs_kernel: the EP buffers, 64 bytes for the rotation degrees and the mbarrier, the staged rows
-template <class C, int NS> struct PbsSmem { static constexpr size_t bytes = EpSmem<C>::bytes + 64 + KeyStage<C, NS>::bytes; };
-
-template <class C, int NT, int MAC_DEPTH = 5, int NS = 0, class CoefFn>
+template <class C, int NT, int MAC_DEPTH = 5, class CoefFn>
 __device__ __forceinline__ void ep_step_device(int tid, const EpSmem<C>& sm, const cplx* __restrict__ ggsw, CoefFn coef, int base_log,
-                                               cplx (&out)[MacCfg<C, NT>::SPT][C::B][C::G], KeyStage<C, NS>* stage = nullptr,
-                                               const cplx* __restrict__ ggsw_next = nullptr) {
+                                               cplx (&out)[MacCfg<C, NT>::SPT][C::B][C::G]) {
     typedef MacCfg<C, NT> MC;
     static_assert(NT / 16 >= C::JOBS, "one 16-thread group per operand polynomial");
-    constexpr bool DO_MAC = !(TAC_EP_DBG & 1), DO_FWD = !(TAC_EP_DBG & 2), DO_INV = !(TAC_EP_DBG & 4), DO_DEC = !(TAC_EP_DBG & 8);
     const int job = tid >> 4, t = tid & 15;
     const bool active = job < C::JOBS;
     cplx g[MAC_DEPTH][C::G];            // key prefetch ring (ep_step.cuh)
@@ -116,86 +61,32 @@ __device__ __forceinline__ void ep_step_device(int tid, const EpSmem<C>& sm, con
     // (A variant that ping-pongs between two FFT buffers, so that mac(l) and the transforms of level l-1 share one barrier
     // interval — L+1 barriers instead of 2L — measured 3 % SLOWER on B200 (tools/pbs_bench.cu, 123.2 vs 119.4 ms for 6144
     // ciphertexts) and costs 61 KB more shared memory; the single-buffer schedule below is the one that ships.)
-#ifdef TAC_EP_TIMING
-    long long tac_tprev = clock64();
-#endif
-    cplx tw[FwdTw<C::N>::LEN];          // pass-2 twiddles of this lane, fetched ahead of pass 1 (ep_core.cuh)
-    if (active && DO_FWD) fft_fwd_twiddles<C::N>(t, sm.wT, tw);
-    if (active && DO_FWD && DO_DEC) grp_decomp_fwd1<C>(t, job, [&](int jj, uint64_t& x0, uint64_t& x1) { coef(job, jj, x0, x1); }, dc, sm.dig, sm.S);
-    if (active && !DO_FWD && DO_DEC) {          // decomposition alone
-        for (int m = 0; m < C::M / 16; m++) {
-            uint32_t w[C::L];
-            uint64_t x0, x1;
-            coef(job, t + 16 * m, x0, x1);
-            decompose_pair<C::L>(x0, x1, dc, w);
-#pragma unroll
-            for (int s2 = 0; s2 + 1 < C::L; s2++) sm.dig[((size_t)job * (C::L - 1) + s2) * C::M + t + 16 * m] = w[s2];
-            sm.S[(size_t)job * C::M + t + 16 * m].x = (double)w[C::L - 1];
-        }
-    }
-    if (active && DO_FWD && !DO_DEC) grp_fwd1<C>(t, job, 1, dc, sm.dig, sm.S);
-    TAC_EP_T(0);
+    if (active) grp_decomp_fwd1<C>(t, job, [&](int jj, uint64_t& x0, uint64_t& x1) { coef(job, jj, x0, x1); }, dc, sm.dig, sm.S);
     // The first key rows are requested AFTER pass 2 (in flight during the barrier only): pass 2 holds 16 values and 15
     // twiddles, and a ring that is live across it costs registers the FFT needs (measured with the FMA-fused passes:
-    // 112.4 ms late vs 121.8 ms early for 6144 ciphertexts).  TAC_PREFETCH_EARLY restores the old order (tools/pbs_bench.cu).
-#ifdef TAC_PREFETCH_EARLY
-    if (DO_MAC) ph_mac_prefetch<C, MC::NT_MAC, MAC_DEPTH>(tid, C::L, ggsw, g);
-#endif
+    // 112.4 ms late vs 121.8 ms early for 6144 ciphertexts).
     __syncwarp();
-    if (active && DO_FWD) grp_fwd2<C>(t, job, sm.wT, tw, sm.S);
-#ifndef TAC_PREFETCH_EARLY
-    if constexpr (NS > 0) { if (DO_MAC) ph_mac_prefetch_staged<C, MC::NT_MAC, MAC_DEPTH, NS>(tid, C::L, ggsw, g); }
-    else if (DO_MAC) ph_mac_prefetch<C, MC::NT_MAC, MAC_DEPTH>(tid, C::L, ggsw, g);
-#endif
-    TAC_EP_T(1);
+    if (active) grp_fwd2<C>(t, job, sm.wT, sm.S);
+    ph_mac_prefetch<C, MC::NT_MAC, MAC_DEPTH>(tid, C::L, ggsw, g);
     __syncthreads();
-    TAC_EP_T(2);
-    if constexpr (NS > 0) {
-        stage->wait();
-        if (DO_MAC) ph_mac_staged<C, MC::NT_MAC, MAC_DEPTH, NS>(tid, stage->buf, sm.S, out, g);
-    } else if (DO_MAC) ph_mac<C, MC::NT_MAC, MC::SPT, MAC_DEPTH>(tid, C::L, ggsw, sm.S, out, g);
+    ph_mac<C, MC::NT_MAC, MC::SPT, MAC_DEPTH>(tid, C::L, ggsw, sm.S, out, g);
     if (C::L == 1) ph_outw<C, MC::NT_MAC, MC::SPT>(tid, sm.S, out);         // own slots only: no barrier needed in between
-    TAC_EP_T(3);
     __syncthreads();
-    if constexpr (NS > 0) {                 // the staging buffer is free again: rows of the next level (or of the next step)
-        if (tid == 0) { if (C::L > 1) stage->request(ggsw, C::L - 1); else if (ggsw_next) stage->request(ggsw_next, C::L); }
-    }
-    TAC_EP_T(4);
 #pragma unroll
     for (int lev = C::L - 1; lev >= 1; lev--) {
-        if (active && DO_FWD) fft_fwd_twiddles<C::N>(t, sm.wT, tw);
-        if (active && DO_FWD) grp_fwd1<C>(t, job, lev, dc, sm.dig, sm.S);
-        TAC_EP_T(5);
-#ifdef TAC_PREFETCH_EARLY
-        if (DO_MAC) ph_mac_prefetch<C, MC::NT_MAC, MAC_DEPTH>(tid, lev, ggsw, g);
-#endif
+        if (active) grp_fwd1<C>(t, job, lev, dc, sm.dig, sm.S);
         __syncwarp();
-        if (active && DO_FWD) grp_fwd2<C>(t, job, sm.wT, tw, sm.S);
-#ifndef TAC_PREFETCH_EARLY
-        if constexpr (NS > 0) { if (DO_MAC) ph_mac_prefetch_staged<C, MC::NT_MAC, MAC_DEPTH, NS>(tid, lev, ggsw, g); }
-        else if (DO_MAC) ph_mac_prefetch<C, MC::NT_MAC, MAC_DEPTH>(tid, lev, ggsw, g);
-#endif
-        TAC_EP_T(6);
+        if (active) grp_fwd2<C>(t, job, sm.wT, sm.S);
+        ph_mac_prefetch<C, MC::NT_MAC, MAC_DEPTH>(tid, lev, ggsw, g);
         __syncthreads();
-        TAC_EP_T(7);
-        if constexpr (NS > 0) {
-            stage->wait();
-            if (DO_MAC) ph_mac_staged<C, MC::NT_MAC, MAC_DEPTH, NS>(tid, stage->buf, sm.S, out, g);
-        } else if (DO_MAC) ph_mac<C, MC::NT_MAC, MC::SPT, MAC_DEPTH>(tid, lev, ggsw, sm.S, out, g);
+        ph_mac<C, MC::NT_MAC, MC::SPT, MAC_DEPTH>(tid, lev, ggsw, sm.S, out, g);
         if (lev == 1) ph_outw<C, MC::NT_MAC, MC::SPT>(tid, sm.S, out);
-        TAC_EP_T(8);
         __syncthreads();
-        if constexpr (NS > 0) {
-            if (tid == 0) { if (lev > 1) stage->request(ggsw, lev - 1); else if (ggsw_next) stage->request(ggsw_next, C::L); }
-        }
-        TAC_EP_T(9);
     }
-    if (active && DO_INV) grp_inv1<C>(t, job, sm.wT, sm.S);
+    if (active) grp_inv1<C>(t, job, sm.wT, sm.S);
     __syncwarp();
-    TAC_EP_T(10);
-    if (active && DO_INV) grp_inv2<C>(t, job, sm.S, sm.acc);
+    if (active) grp_inv2<C>(t, job, sm.S, sm.acc);
     __syncwarp();
-    TAC_EP_T(11);
 }
 
 // [U] glwe_sample_extraction.rs::extract_lwe_sample_from_glwe_ciphertext(.., MonomialDegree(0)); element e of the LWE
@@ -221,10 +112,13 @@ __global__ void sample_extract_kernel(const uint64_t* __restrict__ glwe, size_t 
 // ================================================================================================ PBS (homomorphic_shift_boolean)
 // in: small LWE [nct][n+1]; out: big LWE [nct][kN+1] encrypting bit·2·alpha.
 // [U] wop_pbs.rs::homomorphic_shift_boolean + bootstrap.rs::{blind_rotate_assign, bootstrap}
-// NS > 0: the first NS key rows of every level are staged in shared memory by bulk asynchronous copies (KeyStage); the
-// register ring then holds the remaining G - NS rows, so MAC_DEPTH must be >= G - NS.
-template <int N, int K, int L, int B, int NT, int MINB, int MAC_DEPTH = 5, int NS = 0>
-__global__ void __launch_bounds__(NT, MINB)
+// The level-by-level schedule: the PBS path for N = 1024, and at N = 512 the bit-identity reference of pbs_merged_kernel and
+// pbs_wide_kernel in tools/pbs_bench.cu.
+// rot_sm: the monomial degrees of the current and the next step, [2][B] ints, in a 64-byte area after the EP buffers
+template <class C> struct PbsSmem { static constexpr size_t bytes = EpSmem<C>::bytes + 64; };
+
+template <int N, int K, int L, int B, int NT, int MAC_DEPTH = 5>
+__global__ void __launch_bounds__(NT, 1)
 pbs_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cplx* __restrict__ bsk, int base_log, uint64_t alpha,
            const cplx* __restrict__ g_wT, uint64_t* __restrict__ out_big) {
     typedef EpCfg<N, K, L, B> C;
@@ -234,17 +128,6 @@ pbs_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cplx* _
     int* rot_sm = reinterpret_cast<int*>(sm.extra);               // [2][B] monomial degree of the current / next step
     const int tid = threadIdx.x;
     const int ct0 = blockIdx.x * B;
-    KeyStage<C, NS> stage;
-    if constexpr (NS > 0) {
-        unsigned char* base = sm.extra + 64;                       // rot_sm (<= 32 B), the mbarrier at +32, the rows 16-byte aligned
-        stage.buf = reinterpret_cast<cplx*>(base);
-        stage.bar = kstage::smem_u32(sm.extra + 32);
-        stage.uses = 0;
-        if (tid == 0) {
-            kstage::mbar_init(stage.bar, 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-    }
     const int n1 = n + 1;
     // modulus-switched element i of ciphertext b (0 for the padding ciphertexts of the last CTA)
     auto switched = [&](int b, int i) -> int {
@@ -276,18 +159,12 @@ pbs_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cplx* _
 #pragma unroll
             for (int c = 0; c < C::G; c++) out[a][b][c] = mk(0.0, 0.0);
     const size_t ggsw_sz = (size_t)L * C::G * C::G * C::M;
-    if constexpr (NS > 0) { if (tid == 0 && n > 0) stage.request(bsk, L); }                    // (after the barrier that published the mbarrier)
     for (int i = 0; i < n; i++) {
         const int* rot = rot_sm + (i & 1) * B;
         if (tid < B && i + 1 < n) rot_sm[((i + 1) & 1) * B + tid] = switched(tid, i + 1);      // consumed after >= 1 barrier
-#ifdef TAC_DBG_KEY_ONE_ROW
-        const cplx* ggsw_i = bsk;
-#else
-        const cplx* ggsw_i = bsk + ggsw_sz * i;
-#endif
-        ep_step_device<C, NT, MAC_DEPTH, NS>(tid, sm, ggsw_i,
+        ep_step_device<C, NT, MAC_DEPTH>(tid, sm, bsk + ggsw_sz * i,
                               [&](int job, int jj, uint64_t& x0, uint64_t& x1) { rot_diff_pair<N>(sm.acc + (size_t)job * N, jj, rot[job / C::G], x0, x1); },
-                              base_log, out, &stage, i + 1 < n ? ggsw_i + ggsw_sz : nullptr);
+                              base_log, out);
     }
     __syncthreads();
     constexpr int LW = K * N + 1;
@@ -310,10 +187,7 @@ pbs_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cplx* _
 //   P1  group (level, job): forward FFT of that level from the cached digits                 ── barrier ──
 //   P2  256 slot threads: out = Σ_{level, p} fft(digits) · BSK row, written to the level-1 buffer   ── barrier ──
 //   P3  group (0, job): inverse FFT + torus accumulate                                        ── barrier ──
-// NS > 0: the LAST NS key rows of every step are staged in shared memory by bulk asynchronous copies issued at the top of the
-// step — a lone ciphertext per SM spends its MAC waiting for the 307 KB GGSW to stream in from L2 (the same kernel with every key
-// load served from L1 runs 19 % faster), and the digit / FFT phases leave that path idle.
-template <int N, int K, int L, int B, int NT, int MAC_DEPTH = 5, int NS = 0>
+template <int N, int K, int L, int B, int NT, int MAC_DEPTH = 5>
 __global__ void __launch_bounds__(NT, 1)
 pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cplx* __restrict__ bsk, int base_log, uint64_t alpha,
                 const cplx* __restrict__ g_wT, uint64_t* __restrict__ out_big) {
@@ -328,15 +202,6 @@ pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cp
     cplx* wT = reinterpret_cast<cplx*>(dig + (size_t)JOBS * L * C::M);
     int* rot_sm = reinterpret_cast<int*>(wT + tab_len(C::N));                  // [2][B]
     const int tid = threadIdx.x;
-    cplx* kst = reinterpret_cast<cplx*>(reinterpret_cast<unsigned char*>(rot_sm) + 64);      // [NS][G][M] staged rows (16-byte aligned)
-    const uint32_t kbar = kstage::smem_u32(reinterpret_cast<unsigned char*>(rot_sm) + 32);
-    uint32_t kuses = 0;
-    constexpr uint32_t ROW_BYTES = (uint32_t)(C::G * C::M * sizeof(cplx));
-    static_assert(NS <= ROWS - MAC_DEPTH && 2 * B * sizeof(int) <= 32, "staged rows come after the rows of the register ring");
-    if (NS > 0 && tid == 0) {
-        kstage::mbar_init(kbar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
     const int grp = tid >> 4, t = tid & 15;
     const int part = grp / JOBS, job = grp - part * JOBS;                      // part: share of the pairs in P0, level index in P1
     const bool active = grp < L * JOBS;
@@ -367,27 +232,12 @@ pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cp
     constexpr int P = C::M / 16;
     const int m0 = part * P / L, m1 = (part + 1) * P / L;                     // this group's share of the P register rows
     // key row r (MAC order: level L first, then L-1, …; polynomial p inside) of the step's GGSW
-#ifdef TAC_DBG_KEY_ONE_ROW
-    auto row_ptr = [&](const cplx* ggsw, int) { return ggsw; };
-#else
     auto row_ptr = [&](const cplx* ggsw, int r) { return ggsw + (size_t)((L - 1 - r / C::G) * C::G + (r % C::G)) * C::G * C::M; };
-#endif
     for (int i = 0; i < n; i++) {
         const int* rot = rot_sm + (i & 1) * B;
-#ifdef TAC_DBG_KEY_ONE_ROW
-        const cplx* ggsw = bsk;
-#else
         const cplx* ggsw = bsk + ggsw_sz * i;
-#endif
         if (tid < B && i + 1 < n) rot_sm[((i + 1) & 1) * B + tid] = switched(tid, i + 1);      // consumed after >= 1 barrier
-#ifndef TAC_DBG_KEY_ONE_ROW
         if (i + kL2PrefetchSteps < n) ggsw_l2_prefetch<C>(ggsw + ggsw_sz * kL2PrefetchSteps, tid, NT);
-#endif
-        if (NS > 0 && tid == 0) {              // rows ROWS-NS … ROWS-1 of this step: in flight during P0 and P1
-            kstage::mbar_expect_tx(kbar, NS * ROW_BYTES);
-#pragma unroll
-            for (int r = 0; r < NS; r++) kstage::bulk_g2s(kstage::smem_u32(kst) + r * ROW_BYTES, row_ptr(ggsw, ROWS - NS + r), ROW_BYTES, kbar);
-        }
         // ---- P0: digits
         if (active) {
             const uint64_t* poly = acc + (size_t)job * N;
@@ -407,27 +257,17 @@ pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cp
         __syncthreads();
         // ---- P1: forward FFT of level part+1 of polynomial job; the MAC threads request their first key rows
         cplx g[MAC_DEPTH][C::G];
-#ifndef TAC_WIDE_PREFETCH_LATE
         if (tid < NMAC) {
 #pragma unroll
             for (int r = 0; r < MAC_DEPTH; r++) mac_load_row<C, NMAC>(row_ptr(ggsw, r), 0, tid, g[r]);
         }
-#endif
         {
             const uint32_t* d = dig + ((size_t)job * L + part) * C::M;
             cplx* Sj = S + ((size_t)part * JOBS + job) * C::M;
-            cplx tw[FwdTw<N>::LEN];
-            if (active) fft_fwd_twiddles<N>(t, wT, tw);
             if (active) fft_fwd_pass1<N>(t, [&](int jj, double& a, double& b) { unpack_digits(d[jj], dc, a, b); }, Sj);
             __syncwarp();                          // outside the predicate: a warp may hold one active and one idle group
-            if (active) fft_fwd_pass2<N>(t, wT, tw, Sj);
+            if (active) fft_fwd_pass2<N>(t, wT, Sj);
         }
-#ifdef TAC_WIDE_PREFETCH_LATE
-        if (tid < NMAC) {
-#pragma unroll
-            for (int r = 0; r < MAC_DEPTH; r++) mac_load_row<C, NMAC>(row_ptr(ggsw, r), 0, tid, g[r]);
-        }
-#endif
         __syncthreads();
         // ---- P2: Fourier MAC over all L·G key rows
         if (tid < NMAC) {
@@ -437,7 +277,7 @@ pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cp
 #pragma unroll
                 for (int c = 0; c < C::G; c++) out[b][c] = mk(0.0, 0.0);
 #pragma unroll
-            for (int r = 0; r < ROWS - NS; r++) {
+            for (int r = 0; r < ROWS; r++) {
                 const int s = L - 1 - r / C::G, p = r % C::G;                  // storage index of the level, polynomial
 #pragma unroll
                 for (int b = 0; b < B; b++) {
@@ -445,23 +285,7 @@ pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cp
 #pragma unroll
                     for (int c = 0; c < C::G; c++) cfma(out[b][c], x, g[r % MAC_DEPTH][c]);
                 }
-                if (r + MAC_DEPTH < ROWS - NS) mac_load_row<C, NMAC>(row_ptr(ggsw, r + MAC_DEPTH), 0, tid, g[r % MAC_DEPTH]);
-            }
-            if constexpr (NS > 0) {            // the staged rows arrived while the digits and the transforms were computed
-                kstage::mbar_wait(kbar, kuses & 1u);
-#pragma unroll
-                for (int r = ROWS - NS; r < ROWS; r++) {
-                    const int s = L - 1 - r / C::G, p = r % C::G;
-                    cplx row[C::G];
-#pragma unroll
-                    for (int c = 0; c < C::G; c++) row[c] = kst[(size_t)((r - (ROWS - NS)) * C::G + c) * C::M + tid];
-#pragma unroll
-                    for (int b = 0; b < B; b++) {
-                        const cplx x = S[((size_t)s * JOBS + b * C::G + p) * C::M + tid];
-#pragma unroll
-                        for (int c = 0; c < C::G; c++) cfma(out[b][c], x, row[c]);
-                    }
-                }
+                if (r + MAC_DEPTH < ROWS) mac_load_row<C, NMAC>(row_ptr(ggsw, r + MAC_DEPTH), 0, tid, g[r % MAC_DEPTH]);
             }
             // every thread has finished READING its slot of all buffers only after the barrier; the result goes to rows
             // of buffer 0 at this thread's own slot, which no other thread reads in P2
@@ -470,7 +294,6 @@ pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cp
 #pragma unroll
                 for (int c = 0; c < C::G; c++) S[(size_t)(b * C::G + c) * C::M + tid] = out[b][c];
         }
-        if (NS > 0) kuses++;
         __syncthreads();
         // ---- P3: inverse FFT and accumulate (the groups of part 0)
         if (active && part == 0) grp_inv1<C>(t, job, wT, S);
@@ -487,8 +310,9 @@ pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cp
         out_big[(size_t)ct * LW + e] = v;
     }
 }
-template <class C, int NS = 0> struct WideSmem {
-    static constexpr size_t bytes = 64 + (size_t)NS * C::G * C::M * sizeof(cplx) + C::acc_words * 8 + (size_t)C::L * C::s_cplx * 16 + (size_t)C::JOBS * C::L * C::M * 4 + (size_t)tab_len(C::N) * 16 + 2 * C::B * sizeof(int) + 16;
+// acc, S, dig, wT, then rot_sm ([2][B] ints) with 80 bytes of slack
+template <class C> struct WideSmem {
+    static constexpr size_t bytes = C::acc_words * 8 + (size_t)C::L * C::s_cplx * 16 + (size_t)C::JOBS * C::L * C::M * 4 + (size_t)tab_len(C::N) * 16 + 2 * C::B * sizeof(int) + 16 + 64;
 };
 
 // ================================================================================================ PBS, levels merged (throughput path)

@@ -16,11 +16,11 @@ __global__ void __launch_bounds__(NT) fft_loop(const cplx* g_wT, int reps, uint6
     constexpr bool HAS_S = MODE <= 2, HAS_DIG = MODE != 1, HAS_ACC = MODE >= 1;
     extern __shared__ __align__(16) unsigned char raw[];
     cplx* wT = reinterpret_cast<cplx*>(raw);
-    cplx* S = wT + M;                                                            // [NG][M]
+    cplx* S = wT + tab_len(N);                                                   // [NG][M]
     uint32_t* dig = reinterpret_cast<uint32_t*>(S + (HAS_S ? NG * M : 0));       // [NG][M]
     uint64_t* acc = reinterpret_cast<uint64_t*>(dig + (HAS_DIG ? NG * M : 0));   // [NG][N]
     const int tid = threadIdx.x, grp = tid >> 4, t = tid & 15;
-    for (int i = tid; i < M; i += NT) wT[i] = g_wT[i];
+    for (int i = tid; i < tab_len(N); i += NT) wT[i] = g_wT[i];
     if (HAS_DIG) for (int i = tid; i < NG * M; i += NT) dig[i] = (i * 2654435761u) & 0x0FFF0FFFu;
     if (HAS_ACC) for (int i = tid; i < NG * N; i += NT) acc[i] = i * 0x9E3779B97F4A7C15ull;
     if (HAS_S) for (int i = tid; i < NG * M; i += NT) S[i] = mk(1e-3 * i, -2e-3 * i);
@@ -31,9 +31,9 @@ __global__ void __launch_bounds__(NT) fft_loop(const cplx* g_wT, int reps, uint6
     for (int r = 0; r < reps; r++) {
         if (SYNC) __syncthreads();
         if (MODE == 0 || MODE == 2) {
-            if (active) fft_fwd_pass1<N>(t, [&](int jj, double& a, double& b) { unpack_digits(dg[jj], dc, a, b); }, wT, Sg);
+            if (active) fft_fwd_pass1<N>(t, [&](int jj, double& a, double& b) { unpack_digits(dg[jj], dc, a, b); }, Sg);
             __syncwarp();
-            if (active) fft_fwd_pass2<N>(t, Sg);
+            if (active) fft_fwd_pass2<N>(t, wT, Sg);
             __syncwarp();
         }
         if (MODE == 1 || MODE == 2) {
@@ -63,7 +63,7 @@ __global__ void __launch_bounds__(NT) fft_loop(const cplx* g_wT, int reps, uint6
 template <int MODE, int NT, int SYNC = 0>
 void run(const char* name, const cplx* wT, uint64_t* sink, int reps, double peak) {
     constexpr int NG = NT / 16;
-    const size_t need = 4096 + (size_t)NG * ((MODE <= 2 ? 4096 : 0) + (MODE != 1 ? 1024 : 0) + (MODE >= 1 ? 4096 : 0));
+    const size_t need = (size_t)tab_len(512) * 16 + (size_t)NG * ((MODE <= 2 ? 4096 : 0) + (MODE != 1 ? 1024 : 0) + (MODE >= 1 ? 4096 : 0));
     for (int want = 1; want <= 8; want++) {
         size_t smem = (227 * 1024 / want) & ~(size_t)1023;
         if (smem > 1024) smem -= 1024;
@@ -84,8 +84,8 @@ void run(const char* name, const cplx* wT, uint64_t* sink, int reps, double peak
 }
 int main(int argc, char** argv) {
     const int reps = argc > 1 ? atoi(argv[1]) : 2000;
-    std::vector<cplx> wT(256); build_wT(512, wT.data());
-    cplx* d_wT; CK(cudaMalloc(&d_wT, 256 * 16)); CK(cudaMemcpy(d_wT, wT.data(), 256 * 16, cudaMemcpyHostToDevice));
+    std::vector<cplx> wT(tab_len(512)); build_wT(512, wT.data());
+    cplx* d_wT; CK(cudaMalloc(&d_wT, wT.size() * 16)); CK(cudaMemcpy(d_wT, wT.data(), wT.size() * 16, cudaMemcpyHostToDevice));
     uint64_t* sink; CK(cudaMalloc(&sink, 148 * 8 * 8));
     run<0, 256, 0>("forward", d_wT, sink, reps, 36.8);
     run<0, 256, 1>("forward", d_wT, sink, reps, 36.8);

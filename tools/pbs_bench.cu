@@ -1,21 +1,21 @@
-// tools/pbs_bench.cu — stand-alone timing harness for pbs_kernel variants (development tool, not part of the product path).
+// tools/pbs_bench.cu — stand-alone timing of the blind-rotation kernels (development tool, not part of the product path).
 //
 //   nvcc -O3 -std=c++17 -lineinfo -gencode arch=compute_100a,code=sm_100a -I../tfhe-aes-2_b200/csrc -o pbs_bench pbs_bench.cu
-//   ./pbs_bench [n_cts=6144] [reps=3] [variant mask]
+//   ./pbs_bench [n_cts=6144] [reps=3] [mask]
 //
-// Random Fourier-domain BSK and random small LWEs (timing does not depend on the values; all variants get the same
-// inputs, and because the per-ciphertext arithmetic does not depend on how many ciphertexts share a CTA, every variant
-// must print the same output checksum).  Reports ms per launch and the fraction of the measured DFMA peak.
+// Random Fourier-domain BSK and random small LWEs (timing does not depend on the values).  Three configurations run on the
+// same inputs; bit i of the optional mask selects configuration i:
+//   0  pbs_merged_kernel, the shipped throughput kernel
+//   1  pbs_wide_kernel, the shipped latency kernel for small batches
+//   2  pbs_kernel, the level-by-level schedule, kept as the bit-identity reference
+// The arithmetic of a ciphertext does not depend on the kernel or on how many ciphertexts share a CTA, so all three must
+// print the same output checksum.  Reports ms per launch and the fraction of the measured DFMA peak.
 #include <cuda_runtime.h>
 #include <cstdio>
 #include <cstdlib>
 #include <vector>
 #include <random>
 #include "kernels_ep.cuh"
-#include "experiments/kernels_park.cuh"
-#include "experiments/kernels_wide512.cuh"
-#include "experiments/kernels_merged.cuh"
-#include "experiments/kernels_wide_tma.cuh"
 
 using namespace tac;
 
@@ -44,64 +44,21 @@ constexpr int N = 512, K = 4, L = 3, n_lwe = 677, BASE_LOG = 12;
 
 struct Bufs { uint64_t* small; cplx* bsk; cplx* wT; uint64_t* out; unsigned long long* sum; int nct; int reps; double peak; };
 
-template <int B, int NT, int MINB, int DEPTH, int NS = 0>
-void run(const char* name, const Bufs& b) {
-    typedef EpCfg<N, K, L, B> C;
-    const size_t smem = PbsSmem<C, NS>::bytes;
-    auto kern = pbs_kernel<N, K, L, B, NT, MINB, DEPTH, NS>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaFuncAttributes fa; CK(cudaFuncGetAttributes(&fa, kern));
-    int occ = 0; CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
-    const unsigned grid = (b.nct + B - 1) / B;
-    cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-    CK(cudaMemset(b.out, 0, (size_t)b.nct * (K * N + 1) * 8));
-    kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);     // warm-up
-    CK(cudaDeviceSynchronize());
-    float best = 1e30f, tot = 0;
-    for (int r = 0; r < b.reps; r++) {
-        CK(cudaEventRecord(e0));
-        kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-        CK(cudaEventRecord(e1));
-        CK(cudaEventSynchronize(e1));
-        float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
-        best = ms < best ? ms : best; tot += ms;
-    }
-    CK(cudaMemset(b.sum, 0, 8));
-    checksum_kernel<<<256, 256>>>(b.out, (size_t)b.nct * (K * N + 1), b.sum);
-    unsigned long long h; CK(cudaMemcpy(&h, b.sum, 8, cudaMemcpyDeviceToHost));
-    const double flop = (double)b.nct * n_lwe * 389120.0;
-    printf("%-28s regs=%3d lmem=%4zu smem=%6zu occ=%d  best %8.3f ms  avg %8.3f ms  %6.2f TF/s  frac %.3f  %7.1f PBS/ms  sum=%016llx\n", name, fa.numRegs,
-           (size_t)fa.localSizeBytes, smem, occ, best, tot / b.reps, flop / (best * 1e-3) / 1e12, flop / (best * 1e-3) / 1e12 / b.peak, b.nct / best, h);
-#ifdef TAC_EP_TIMING
-    {   // per-phase clock attribution (thread 0 of CTA 0; build with -DTAC_EP_TIMING)
-        long long tt[32]; CK(cudaMemcpyFromSymbol(tt, tac_ep_times, sizeof(tt)));
-        const double steps = (double)n_lwe * (b.reps + 1);                       // CTA 0 runs once per launch
-        const char* nm[12] = {"decomp+fwd1(L)", "fwd2(L)", "barrier", "mac(L)", "barrier", "fwd1(l<L)", "fwd2(l<L)", "barrier", "mac(l<L)", "barrier", "inv1", "inv2+acc"};
-        double tot2 = 0; for (int i = 0; i < 12; i++) tot2 += tt[i] / steps;
-        printf("   thread 0 cycles/step (%.0f):", tot2); for (int i = 0; i < 12; i++) printf(" %s=%.0f", nm[i], tt[i] / steps); printf("\n");
-        long long z[32] = {0}; CK(cudaMemcpyToSymbol(tac_ep_times, z, sizeof(z)));
-    }
-#endif
-    fflush(stdout);
-}
+// the signature shared by the three PBS kernels
+typedef void (*PbsKernel)(const uint64_t*, int, int, const cplx*, int, uint64_t, const cplx*, uint64_t*);
 
-template <int B, int NT, int DEPTH, int NS = 0>
-void run_wide(const char* name, const Bufs& b) {
-    typedef EpCfg<N, K, L, B> C;
-    const size_t smem = WideSmem<C, NS>::bytes;
-    auto kern = pbs_wide_kernel<N, K, L, B, NT, DEPTH, NS>;
+void run(const char* name, PbsKernel kern, unsigned grid, int nt, size_t smem, const Bufs& b) {
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaFuncAttributes fa; CK(cudaFuncGetAttributes(&fa, kern));
-    int occ = 0; CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
-    const unsigned grid = (b.nct + B - 1) / B;
+    int occ = 0; CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, nt, smem));
     cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
     CK(cudaMemset(b.out, 0, (size_t)b.nct * (K * N + 1) * 8));
-    kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
+    kern<<<grid, nt, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);     // warm-up
     CK(cudaDeviceSynchronize());
     float best = 1e30f, tot = 0;
     for (int r = 0; r < b.reps; r++) {
         CK(cudaEventRecord(e0));
-        kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
+        kern<<<grid, nt, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
         CK(cudaEventRecord(e1));
         CK(cudaEventSynchronize(e1));
         float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
@@ -113,170 +70,7 @@ void run_wide(const char* name, const Bufs& b) {
     const double flop = (double)b.nct * n_lwe * 389120.0;
     printf("%-28s regs=%3d lmem=%4zu smem=%6zu occ=%d  best %8.3f ms  avg %8.3f ms  %6.2f TF/s  frac %.3f  %7.1f PBS/ms  sum=%016llx\n", name, fa.numRegs,
            (size_t)fa.localSizeBytes, smem, occ, best, tot / b.reps, flop / (best * 1e-3) / 1e12, flop / (best * 1e-3) / 1e12 / b.peak, b.nct / best, h);
-    fflush(stdout);
-}
-
-template <int B, int NT, int DEPTH, bool SPLIT>
-void run_park(const char* name, const Bufs& b) {
-    typedef EpCfg<N, K, L, B> C;
-    const size_t smem = ParkSmem<C>::bytes;
-    auto kern = pbs_park_kernel<N, K, L, B, NT, DEPTH, SPLIT>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaFuncAttributes fa; CK(cudaFuncGetAttributes(&fa, kern));
-    int occ = 0; CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
-    const unsigned grid = (b.nct + B - 1) / B;
-    cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-    CK(cudaMemset(b.out, 0, (size_t)b.nct * (K * N + 1) * 8));
-    kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-    CK(cudaDeviceSynchronize());
-    float best = 1e30f, tot = 0;
-    for (int r = 0; r < b.reps; r++) {
-        CK(cudaEventRecord(e0));
-        kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-        CK(cudaEventRecord(e1));
-        CK(cudaEventSynchronize(e1));
-        float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
-        best = ms < best ? ms : best; tot += ms;
-    }
-    CK(cudaMemset(b.sum, 0, 8));
-    checksum_kernel<<<256, 256>>>(b.out, (size_t)b.nct * (K * N + 1), b.sum);
-    unsigned long long h; CK(cudaMemcpy(&h, b.sum, 8, cudaMemcpyDeviceToHost));
-    const double flop = (double)b.nct * n_lwe * 389120.0;
-    printf("%-28s regs=%3d lmem=%4zu smem=%6zu occ=%d  best %8.3f ms  avg %8.3f ms  %6.2f TF/s  frac %.3f  %7.1f PBS/ms  sum=%016llx\n", name, fa.numRegs,
-           (size_t)fa.localSizeBytes, smem, occ, best, tot / b.reps, flop / (best * 1e-3) / 1e12, flop / (best * 1e-3) / 1e12 / b.peak, b.nct / best, h);
-    fflush(stdout);
-}
-
-template <int DEPTH>
-void run_wide512(const char* name, const Bufs& b) {
-    typedef EpCfg<N, K, L, 1> C;
-    const size_t smem = WideSmem<C>::bytes;
-    auto kern = pbs_wide512_kernel<N, K, L, DEPTH>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaFuncAttributes fa; CK(cudaFuncGetAttributes(&fa, kern));
-    int occ = 0; CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 512, smem));
-    cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-    CK(cudaMemset(b.out, 0, (size_t)b.nct * (K * N + 1) * 8));
-    kern<<<b.nct, 512, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-    CK(cudaDeviceSynchronize());
-    float best = 1e30f, tot = 0;
-    for (int r = 0; r < b.reps; r++) {
-        CK(cudaEventRecord(e0));
-        kern<<<b.nct, 512, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-        CK(cudaEventRecord(e1));
-        CK(cudaEventSynchronize(e1));
-        float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
-        best = ms < best ? ms : best; tot += ms;
-    }
-    CK(cudaMemset(b.sum, 0, 8));
-    checksum_kernel<<<256, 256>>>(b.out, (size_t)b.nct * (K * N + 1), b.sum);
-    unsigned long long h; CK(cudaMemcpy(&h, b.sum, 8, cudaMemcpyDeviceToHost));
-    const double flop = (double)b.nct * n_lwe * 389120.0;
-    printf("%-28s regs=%3d lmem=%4zu smem=%6zu occ=%d  best %8.3f ms  avg %8.3f ms  %6.2f TF/s  frac %.3f  %7.1f PBS/ms  sum=%016llx\n", name, fa.numRegs,
-           (size_t)fa.localSizeBytes, smem, occ, best, tot / b.reps, flop / (best * 1e-3) / 1e12, flop / (best * 1e-3) / 1e12 / b.peak, b.nct / best, h);
-    fflush(stdout);
-}
-
-template <int B, int NT, int DEPTH, int NS = 0>
-void run_merged(const char* name, const Bufs& b) {
-    typedef EpCfg<N, K, L, B> C;
-    const size_t smem = MergedXSmem<C, NS>::bytes;
-    auto kern = pbs_mergedx_kernel<N, K, L, B, NT, DEPTH, NS>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaFuncAttributes fa; CK(cudaFuncGetAttributes(&fa, kern));
-    int occ = 0; CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
-    const unsigned grid = (b.nct + B - 1) / B;
-    cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-    CK(cudaMemset(b.out, 0, (size_t)b.nct * (K * N + 1) * 8));
-    kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-    CK(cudaDeviceSynchronize());
-    float best = 1e30f, tot = 0;
-    for (int r = 0; r < b.reps; r++) {
-        CK(cudaEventRecord(e0));
-        kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-        CK(cudaEventRecord(e1));
-        CK(cudaEventSynchronize(e1));
-        float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
-        best = ms < best ? ms : best; tot += ms;
-    }
-    CK(cudaMemset(b.sum, 0, 8));
-    checksum_kernel<<<256, 256>>>(b.out, (size_t)b.nct * (K * N + 1), b.sum);
-    unsigned long long h; CK(cudaMemcpy(&h, b.sum, 8, cudaMemcpyDeviceToHost));
-    const double flop = (double)b.nct * n_lwe * 389120.0;
-    printf("%-28s regs=%3d lmem=%4zu smem=%6zu occ=%d  best %8.3f ms  avg %8.3f ms  %6.2f TF/s  frac %.3f  %7.1f PBS/ms  sum=%016llx\n", name, fa.numRegs,
-           (size_t)fa.localSizeBytes, smem, occ, best, tot / b.reps, flop / (best * 1e-3) / 1e12, flop / (best * 1e-3) / 1e12 / b.peak, b.nct / best, h);
-#ifdef TAC_MG_TIMING
-    {
-        long long tt[16]; CK(cudaMemcpyFromSymbol(tt, tac_mg_times, sizeof(tt)));
-        const double steps = (double)n_lwe * (b.reps + 1);
-        const char* nm[8] = {"digits", "pass1", "pass2+ring", "barrier", "mac", "barrier", "invA", "invB+acc"};
-        double tot2 = 0; for (int i = 0; i < 8; i++) tot2 += tt[i] / steps;
-        printf("   thread 0 cycles/step (%.0f):", tot2); for (int i = 0; i < 8; i++) printf(" %s=%.0f", nm[i], tt[i] / steps); printf("\n");
-        long long z[16] = {0}; CK(cudaMemcpyToSymbol(tac_mg_times, z, sizeof(z)));
-    }
-#endif
-    fflush(stdout);
-}
-
-// the shipped pbs_merged_kernel (kernels_ep.cuh)
-template <int B, int NT, int DEPTH, int BLOG>
-void run_merged_prod(const char* name, const Bufs& b) {
-    typedef EpCfg<N, K, L, B> C;
-    const size_t smem = MergedSmem<C>::bytes;
-    auto kern = pbs_merged_kernel<N, K, L, B, NT, DEPTH, BLOG>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaFuncAttributes fa; CK(cudaFuncGetAttributes(&fa, kern));
-    int occ = 0; CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
-    const unsigned grid = (b.nct + B - 1) / B;
-    cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-    CK(cudaMemset(b.out, 0, (size_t)b.nct * (K * N + 1) * 8));
-    kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-    CK(cudaDeviceSynchronize());
-    float best = 1e30f, tot = 0;
-    for (int r = 0; r < b.reps; r++) {
-        CK(cudaEventRecord(e0));
-        kern<<<grid, NT, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-        CK(cudaEventRecord(e1));
-        CK(cudaEventSynchronize(e1));
-        float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
-        best = ms < best ? ms : best; tot += ms;
-    }
-    CK(cudaMemset(b.sum, 0, 8));
-    checksum_kernel<<<256, 256>>>(b.out, (size_t)b.nct * (K * N + 1), b.sum);
-    unsigned long long h; CK(cudaMemcpy(&h, b.sum, 8, cudaMemcpyDeviceToHost));
-    const double flop = (double)b.nct * n_lwe * 389120.0;
-    printf("%-28s regs=%3d lmem=%4zu smem=%6zu occ=%d  best %8.3f ms  avg %8.3f ms  %6.2f TF/s  frac %.3f  %7.1f PBS/ms  sum=%016llx\n", name, fa.numRegs,
-           (size_t)fa.localSizeBytes, smem, occ, best, tot / b.reps, flop / (best * 1e-3) / 1e12, flop / (best * 1e-3) / 1e12 / b.peak, b.nct / best, h);
-    fflush(stdout);
-}
-
-template <int R, int NT_>
-void run_wide_tma(const char* name, const Bufs& b) {
-    typedef EpCfg<N, K, L, 1> C;
-    const size_t smem = WideTmaSmem<C, R>::bytes;
-    auto kern = pbs_wide_tma_kernel<N, K, L, NT_, R>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaFuncAttributes fa; CK(cudaFuncGetAttributes(&fa, kern));
-    int occ = 0; CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT_, smem));
-    cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-    CK(cudaMemset(b.out, 0, (size_t)b.nct * (K * N + 1) * 8));
-    kern<<<b.nct, NT_, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-    CK(cudaDeviceSynchronize());
-    float best = 1e30f, tot = 0;
-    for (int r = 0; r < b.reps; r++) {
-        CK(cudaEventRecord(e0));
-        kern<<<b.nct, NT_, smem>>>(b.small, b.nct, n_lwe, b.bsk, BASE_LOG, 1ull << 50, b.wT, b.out);
-        CK(cudaEventRecord(e1));
-        CK(cudaEventSynchronize(e1));
-        float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
-        best = ms < best ? ms : best; tot += ms;
-    }
-    CK(cudaMemset(b.sum, 0, 8));
-    checksum_kernel<<<256, 256>>>(b.out, (size_t)b.nct * (K * N + 1), b.sum);
-    unsigned long long h; CK(cudaMemcpy(&h, b.sum, 8, cudaMemcpyDeviceToHost));
-    const double flop = (double)b.nct * n_lwe * 389120.0;
-    printf("%-28s regs=%3d lmem=%4zu smem=%6zu occ=%d  best %8.3f ms  avg %8.3f ms  %6.2f TF/s  frac %.3f  %7.1f PBS/ms  sum=%016llx\n", name, fa.numRegs,
-           (size_t)fa.localSizeBytes, smem, occ, best, tot / b.reps, flop / (best * 1e-3) / 1e12, flop / (best * 1e-3) / 1e12 / b.peak, b.nct / best, h);
+    CK(cudaEventDestroy(e0)); CK(cudaEventDestroy(e1));
     fflush(stdout);
 }
 
@@ -312,30 +106,9 @@ int main(int argc, char** argv) {
         b.peak = best;
         printf("DFMA peak %.2f TFLOP/s; n_cts %d\n", best, b.nct);
     }
-    int v = 0;
-#define V(B_, NT_, MINB_, D_) if (mask & (1u << v)) run<B_, NT_, MINB_, D_>("B=" #B_ " NT=" #NT_ " minb=" #MINB_ " depth=" #D_, b); v++;
-#define VN(B_, NT_, MINB_, D_, NS_) if (mask & (1u << v)) run<B_, NT_, MINB_, D_, NS_>("B=" #B_ " NT=" #NT_ " depth=" #D_ " staged=" #NS_, b); v++;
-#define VW(B_, NT_, D_) if (mask & (1u << v)) run_wide<B_, NT_, D_>("wide B=" #B_ " NT=" #NT_ " depth=" #D_, b); v++;
-#define VWN(B_, NT_, D_, NS_) if (mask & (1u << v)) run_wide<B_, NT_, D_, NS_>("wide B=" #B_ " depth=" #D_ " staged=" #NS_, b); v++;
-#define VP(B_, NT_, D_) if (mask & (1u << v)) run_park<B_, NT_, D_, false>("park B=" #B_ " NT=" #NT_ " depth=" #D_, b); v++;
-#define VM(B_, NT_, D_, NS_) if (mask & (1u << v)) run_merged<B_, NT_, D_, NS_>("merged B=" #B_ " depth=" #D_ " staged=" #NS_, b); v++;
-#define VMP(B_, NT_, D_, BL_) if (mask & (1u << v)) run_merged_prod<B_, NT_, D_, BL_>("merged(prod) B=" #B_ " depth=" #D_ " blog=" #BL_, b); v++;
-#define VWT(R_, NT_) if (mask & (1u << v)) run_wide_tma<R_, NT_>("wide/tma ring=" #R_ " NT=" #NT_, b); v++;
-#define VW5(D_) if (mask & (1u << v)) run_wide512<D_>("wide512 depth=" #D_, b); v++;
-#define VS(B_, NT_, D_) if (mask & (1u << v)) run_park<B_, NT_, D_, true>("park/split B=" #B_ " NT=" #NT_ " depth=" #D_, b); v++;
-#ifndef TAC_VARIANTS
-#define TAC_VARIANTS "pbs_bench_variants.inc"
-#endif
-#include TAC_VARIANTS
-#undef V
-#undef VN
-#undef VW
-#undef VWN
-#undef VP
-#undef VS
-#undef VW5
-#undef VWT
-#undef VMP
-#undef VM
+    const unsigned grid3 = (unsigned)((b.nct + 2) / 3), grid1 = (unsigned)b.nct;
+    if (mask & 1) run("merged B=3 depth=4 blog=12", pbs_merged_kernel<N, K, L, 3, 256, 4, 12>, grid3, 256, MergedSmem<EpCfg<N, K, L, 3>>::bytes, b);
+    if (mask & 2) run("wide B=1 NT=256 depth=3", pbs_wide_kernel<N, K, L, 1, 256, 3>, grid1, 256, WideSmem<EpCfg<N, K, L, 1>>::bytes, b);
+    if (mask & 4) run("B=3 NT=256 depth=5", pbs_kernel<N, K, L, 3, 256, 5>, grid3, 256, PbsSmem<EpCfg<N, K, L, 3>>::bytes, b);
     return 0;
 }

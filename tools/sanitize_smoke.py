@@ -3,7 +3,7 @@
 is available (it is closed on the B200 pool used for this round, so only the plain run was done here):
    compute-sanitizer --tool memcheck  python tools/sanitize_smoke.py
    compute-sanitizer --tool racecheck python tools/sanitize_smoke.py
-One 8->24 SBOX circuit bootstrap (level-parallel PBS kernel), a batch of 50 (throughput PBS kernel with the staged key row),
+One 8->24 SBOX circuit bootstrap (level-parallel PBS kernel), a batch of 50 (throughput PBS kernel),
 a PFKS batch that overflows the tie list (scan fallback), one AES block for 2 rounds; everything decrypt-checked."""
 import importlib
 import os
