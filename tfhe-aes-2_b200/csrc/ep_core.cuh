@@ -32,8 +32,8 @@ struct alignas(16) cplx { double x, y; };
 TAC_HD cplx mk(double x, double y) { cplx r; r.x = x; r.y = y; return r; }
 TAC_HD cplx cmul(cplx a, cplx b) { return mk(fma(-a.y, b.y, a.x * b.x), fma(a.y, b.x, a.x * b.y)); }
 TAC_HD cplx cmul_conj(cplx a, cplx b) { return mk(fma(a.y, b.y, a.x * b.x), fma(-a.x, b.y, a.y * b.x)); }   // a * conj(b)
-// o += a·b.  The order of the four FMAs is part of the contract: every MAC (ph_mac, mg_mac, the MAC of pbs_wide_kernel)
-// accumulates in exactly this order, so all of them produce the same words.
+// o += a·b.  The order of the four FMAs is part of the contract: every MAC (ph_mac, and mg_mac, which pbs_merged_kernel and
+// pbs_wide_kernel share) accumulates in exactly this order, so all of them produce the same words.
 TAC_HD void cfma(cplx& o, cplx a, cplx b) {
     o.x = fma(a.x, b.x, o.x); o.x = fma(-a.y, b.y, o.x);
     o.y = fma(a.y, b.x, o.y); o.y = fma(a.x, b.y, o.y);

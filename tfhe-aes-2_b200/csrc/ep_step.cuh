@@ -19,6 +19,7 @@
 //   group:  inv1 | inv2 |                                                                     ( | = __syncwarp )
 // Both the CUDA kernels (kernels_ep.cuh) and the CPU emulation (tests/cpu/ep_emul.cpp) follow this order.
 // pbs_merged_kernel runs the L levels of a step in ONE barrier interval (accumulators in registers): see the mg_* functions.
+// pbs_wide_kernel shares their one-pass MAC over all L·G key rows (mg_mac_prefetch, mg_mac).
 #pragma once
 #include "ep_core.cuh"
 
@@ -218,6 +219,7 @@ TAC_HD void mg_digits(int t, const uint64_t* __restrict__ Rj, int rot, const uin
         }
     });
 }
+// The one-pass MAC over all L·G key rows, used by pbs_merged_kernel and pbs_wide_kernel.
 // key row r of a step's Fourier GGSW in MAC order: level L first, polynomial p inside
 template <class C>
 TAC_HD const cplx* mg_row(const cplx* __restrict__ ggsw, int r) { return ggsw + (size_t)((C::L - 1 - r / C::G) * C::G + (r % C::G)) * C::G * C::M; }

@@ -45,6 +45,17 @@ struct EpSmem {
     static constexpr size_t bytes = C::acc_words * 8 + C::s_cplx * 16 + C::dig_words * 4 + (size_t)tab_len(C::N) * 16;
 };
 
+// the Fourier-domain accumulators of ep_step_device start at zero (ph_outw clears them again after each step)
+template <int SPT, int B, int G>
+__device__ __forceinline__ void zero_fourier_acc(cplx (&out)[SPT][B][G]) {
+#pragma unroll
+    for (int a = 0; a < SPT; a++)
+#pragma unroll
+        for (int b = 0; b < B; b++)
+#pragma unroll
+            for (int c = 0; c < G; c++) out[a][b][c] = mk(0.0, 0.0);
+}
+
 // one step on the operand whose coefficients jj and jj + N/2 of polynomial `job` are given by coef(job, jj, x0, x1); the
 // accumulators receive  acc += GGSW ⊡ operand.
 // Ends with a __syncwarp(): the accumulator rows of a job are only touched by the job's own 16-thread group, so the next
@@ -112,10 +123,69 @@ __global__ void sample_extract_kernel(const uint64_t* __restrict__ glwe, size_t 
 // ================================================================================================ PBS (homomorphic_shift_boolean)
 // in: small LWE [nct][n+1]; out: big LWE [nct][kN+1] encrypting bit·2·alpha.
 // [U] wop_pbs.rs::homomorphic_shift_boolean + bootstrap.rs::{blind_rotate_assign, bootstrap}
+// pbs_kernel, pbs_wide_kernel and pbs_merged_kernel differ only in the step.  They share the mod switch, the prologue
+// (twiddles, monomial degrees, trivial accumulators), the epilogue (sample extraction) and rot_sm, the monomial degrees of the
+// current and the next step, [2][B] ints after the buffers of each shared-memory layout.  Each layout struct places its
+// buffers and counts its bytes; the count sets the dynamic shared memory and with it the L1 left for the in-flight key
+// loads, which moves the PBS time (DESIGN.md §4).
+constexpr size_t kRotSmBytes = 64;          // the rot_sm area of PbsSmem and MergedSmem
+
+// modulus-switched element i of ciphertext ct0 + b (0 for the padding ciphertexts of the last CTA); n1 = n + 1 is the stride
+template <int N>
+struct PbsModSwitch {
+    const uint64_t* lwe_small;
+    int nct, n, n1, ct0;
+    __device__ __forceinline__ int operator()(int b, int i) const {
+        const int ct = ct0 + b;
+        if (ct >= nct) return 0;
+        uint64_t a = __ldg(lwe_small + (size_t)ct * n1 + i);
+        if (i == n) a += (1ull << 62);                             // centre the error for the negacyclic LUT
+        return modswitch(a, LogN<N>::v);
+    }
+};
+
+// twiddle table; rot_sm = (degree of step 0, degree of the body b~); accumulator = trivial GLWE(-alpha in every coefficient) · X^{-b~}
+template <class C, int NT, class Smem>
+__device__ __forceinline__ void pbs_prologue(int tid, const Smem& sm, const PbsModSwitch<C::N>& switched, uint64_t alpha,
+                                             const cplx* __restrict__ g_wT) {
+    constexpr int N = C::N, B = C::B;
+    for (int i = tid; i < tab_len(N); i += NT) sm.wT[i] = g_wT[i];
+    if (tid < B) { sm.rot_sm[tid] = switched(tid, 0); sm.rot_sm[B + tid] = switched(tid, switched.n); }
+    __syncthreads();
+    for (int idx = tid; idx < (int)C::acc_words; idx += NT) {
+        const int b = idx / (C::G * N), rem = idx - b * C::G * N, p = rem / N, j = rem - p * N;
+        uint64_t v = 0;
+        if (p == C::K) {
+            const int s = (j + sm.rot_sm[B + b]) & (2 * N - 1);
+            v = (s < N) ? (0ull - alpha) : alpha;
+        }
+        sm.acc[idx] = v;
+    }
+    __syncthreads();
+}
+
+// sample extraction of the B accumulators into out[set][first + b] (out: [][count][kN+1]) for first + b < count, alpha added to
+// the body.  The caller orders the accumulator writes before it.
+template <class C, int NT>
+__device__ __forceinline__ void pbs_epilogue(int tid, const uint64_t* acc, uint64_t* out, int set, int first, int count, uint64_t alpha) {
+    constexpr int LW = C::K * C::N + 1;
+    for (int idx = tid; idx < C::B * LW; idx += NT) {
+        const int b = idx / LW, e = idx - b * LW, ct = first + b;
+        if (ct >= count) continue;
+        uint64_t v = sample_extract_elem<C>(acc + (size_t)b * C::G * C::N, e);
+        if (e == C::K * C::N) v += alpha;
+        out[((size_t)set * count + ct) * LW + e] = v;
+    }
+}
+
 // The level-by-level schedule: the PBS path for N = 1024, and at N = 512 the bit-identity reference of pbs_merged_kernel and
-// pbs_wide_kernel in tools/pbs_bench.cu.
-// rot_sm: the monomial degrees of the current and the next step, [2][B] ints, in a 64-byte area after the EP buffers
-template <class C> struct PbsSmem { static constexpr size_t bytes = EpSmem<C>::bytes + 64; };
+// pbs_wide_kernel in tools/pbs_bench.cu.  Layout: EpSmem, then rot_sm.
+template <class C> struct PbsSmem : EpSmem<C> {
+    int* rot_sm;
+    __device__ explicit PbsSmem(unsigned char* raw) : EpSmem<C>(raw), rot_sm(reinterpret_cast<int*>(this->extra)) {}
+    static constexpr size_t bytes = EpSmem<C>::bytes + kRotSmBytes;
+    static_assert(2 * C::B * sizeof(int) <= kRotSmBytes, "rot_sm");
+};
 
 template <int N, int K, int L, int B, int NT, int MAC_DEPTH = 5>
 __global__ void __launch_bounds__(NT, 1)
@@ -124,57 +194,23 @@ pbs_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cplx* _
     typedef EpCfg<N, K, L, B> C;
     typedef MacCfg<C, NT> MC;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    EpSmem<C> sm(smem_raw);
-    int* rot_sm = reinterpret_cast<int*>(sm.extra);               // [2][B] monomial degree of the current / next step
+    const PbsSmem<C> sm(smem_raw);
     const int tid = threadIdx.x;
     const int ct0 = blockIdx.x * B;
-    const int n1 = n + 1;
-    // modulus-switched element i of ciphertext b (0 for the padding ciphertexts of the last CTA)
-    auto switched = [&](int b, int i) -> int {
-        const int ct = ct0 + b;
-        if (ct >= nct) return 0;
-        uint64_t a = __ldg(lwe_small + (size_t)ct * n1 + i);
-        if (i == n) a += (1ull << 62);                             // centre the error for the negacyclic LUT
-        return modswitch(a, LogN<N>::v);
-    };
-    for (int i = tid; i < tab_len(C::N); i += NT) sm.wT[i] = g_wT[i];
-    if (tid < B) { rot_sm[tid] = switched(tid, 0); rot_sm[B + tid] = switched(tid, n); }
-    __syncthreads();
-    // accumulator = trivial GLWE(-alpha in every coefficient) · X^{-b~}
-    for (int idx = tid; idx < (int)C::acc_words; idx += NT) {
-        const int b = idx / (C::G * N), rem = idx - b * C::G * N, p = rem / N, j = rem - p * N;
-        uint64_t v = 0;
-        if (p == K) {
-            const int s = (j + rot_sm[B + b]) & (2 * N - 1);
-            v = (s < N) ? (0ull - alpha) : alpha;
-        }
-        sm.acc[idx] = v;
-    }
-    __syncthreads();
+    const PbsModSwitch<N> switched{lwe_small, nct, n, n + 1, ct0};
+    pbs_prologue<C, NT>(tid, sm, switched, alpha, g_wT);
     cplx out[MC::SPT][B][C::G];
-#pragma unroll
-    for (int a = 0; a < MC::SPT; a++)
-#pragma unroll
-        for (int b = 0; b < B; b++)
-#pragma unroll
-            for (int c = 0; c < C::G; c++) out[a][b][c] = mk(0.0, 0.0);
+    zero_fourier_acc(out);
     const size_t ggsw_sz = (size_t)L * C::G * C::G * C::M;
     for (int i = 0; i < n; i++) {
-        const int* rot = rot_sm + (i & 1) * B;
-        if (tid < B && i + 1 < n) rot_sm[((i + 1) & 1) * B + tid] = switched(tid, i + 1);      // consumed after >= 1 barrier
+        const int* rot = sm.rot_sm + (i & 1) * B;
+        if (tid < B && i + 1 < n) sm.rot_sm[((i + 1) & 1) * B + tid] = switched(tid, i + 1);      // consumed after >= 1 barrier
         ep_step_device<C, NT, MAC_DEPTH>(tid, sm, bsk + ggsw_sz * i,
                               [&](int job, int jj, uint64_t& x0, uint64_t& x1) { rot_diff_pair<N>(sm.acc + (size_t)job * N, jj, rot[job / C::G], x0, x1); },
                               base_log, out);
     }
     __syncthreads();
-    constexpr int LW = K * N + 1;
-    for (int idx = tid; idx < B * LW; idx += NT) {
-        const int b = idx / LW, e = idx - b * LW, ct = ct0 + b;
-        if (ct >= nct) continue;
-        uint64_t v = sample_extract_elem<C>(sm.acc + (size_t)b * C::G * N, e);
-        if (e == K * N) v += alpha;
-        out_big[(size_t)ct * LW + e] = v;
-    }
+    pbs_epilogue<C, NT>(tid, sm.acc, out_big, 0, ct0, nct, alpha);
 }
 
 // ================================================================================================ PBS, level-parallel variant
@@ -187,62 +223,54 @@ pbs_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cplx* _
 //   P1  group (level, job): forward FFT of that level from the cached digits                 ── barrier ──
 //   P2  256 slot threads: out = Σ_{level, p} fft(digits) · BSK row, written to the level-1 buffer   ── barrier ──
 //   P3  group (0, job): inverse FFT + torus accumulate                                        ── barrier ──
+// Layout: acc [B][G][N], S [L][JOBS][M] (storage index s ↔ level s+1), dig [JOBS][L][M], wT, rot_sm [2][B], then 80 bytes that
+// nothing uses: the mbarrier area and alignment pad of the key staging this kernel had before commit 0336db3.  They stay so
+// that the kernel keeps the shared-memory size (and so the L1 size) it was measured with.
+template <class C> struct WideSmem {
+    uint64_t* acc; cplx* S; uint32_t* dig; cplx* wT; int* rot_sm;
+    __device__ explicit WideSmem(unsigned char* raw) {
+        acc = reinterpret_cast<uint64_t*>(raw);
+        S = reinterpret_cast<cplx*>(acc + C::acc_words);
+        dig = reinterpret_cast<uint32_t*>(S + (size_t)C::L * C::s_cplx);
+        wT = reinterpret_cast<cplx*>(dig + (size_t)C::JOBS * C::L * C::M);
+        rot_sm = reinterpret_cast<int*>(wT + tab_len(C::N));
+    }
+    static constexpr size_t kUnused = 80;
+    static constexpr size_t bytes = C::acc_words * 8 + (size_t)C::L * C::s_cplx * 16 + (size_t)C::JOBS * C::L * C::M * 4 +
+                                    (size_t)tab_len(C::N) * 16 + 2 * C::B * sizeof(int) + kUnused;
+};
+
 template <int N, int K, int L, int B, int NT, int MAC_DEPTH = 5>
 __global__ void __launch_bounds__(NT, 1)
 pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cplx* __restrict__ bsk, int base_log, uint64_t alpha,
                 const cplx* __restrict__ g_wT, uint64_t* __restrict__ out_big) {
     typedef EpCfg<N, K, L, B> C;
-    constexpr int JOBS = C::JOBS, ROWS = L * C::G, NMAC = C::M;
+    constexpr int JOBS = C::JOBS, NMAC = C::M;
     static_assert(NT / 16 >= L * JOBS, "one 16-thread group per (level, polynomial)");
-    static_assert(NT >= NMAC && MAC_DEPTH <= ROWS, "one MAC thread per frequency slot");
+    static_assert(NT >= NMAC && MAC_DEPTH <= L * C::G, "one MAC thread per frequency slot");
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    uint64_t* acc = reinterpret_cast<uint64_t*>(smem_raw);                    // [B][G][N]
-    cplx* S = reinterpret_cast<cplx*>(acc + C::acc_words);                     // [L][JOBS][M]   (storage index s ↔ level s+1)
-    uint32_t* dig = reinterpret_cast<uint32_t*>(S + (size_t)L * C::s_cplx);    // [JOBS][L][M]
-    cplx* wT = reinterpret_cast<cplx*>(dig + (size_t)JOBS * L * C::M);
-    int* rot_sm = reinterpret_cast<int*>(wT + tab_len(C::N));                  // [2][B]
+    const WideSmem<C> sm(smem_raw);
     const int tid = threadIdx.x;
     const int grp = tid >> 4, t = tid & 15;
     const int part = grp / JOBS, job = grp - part * JOBS;                      // part: share of the pairs in P0, level index in P1
     const bool active = grp < L * JOBS;
     const int ct0 = blockIdx.x * B;
-    const int n1 = n + 1;
-    auto switched = [&](int b, int i) -> int {
-        const int ct = ct0 + b;
-        if (ct >= nct) return 0;
-        uint64_t a = __ldg(lwe_small + (size_t)ct * n1 + i);
-        if (i == n) a += (1ull << 62);
-        return modswitch(a, LogN<N>::v);
-    };
-    for (int i = tid; i < tab_len(C::N); i += NT) wT[i] = g_wT[i];
-    if (tid < B) { rot_sm[tid] = switched(tid, 0); rot_sm[B + tid] = switched(tid, n); }
-    __syncthreads();
-    for (int idx = tid; idx < (int)C::acc_words; idx += NT) {
-        const int b = idx / (C::G * N), rem = idx - b * C::G * N, p = rem / N, j = rem - p * N;
-        uint64_t v = 0;
-        if (p == K) {
-            const int s = (j + rot_sm[B + b]) & (2 * N - 1);
-            v = (s < N) ? (0ull - alpha) : alpha;
-        }
-        acc[idx] = v;
-    }
-    __syncthreads();
+    const PbsModSwitch<N> switched{lwe_small, nct, n, n + 1, ct0};
+    pbs_prologue<C, NT>(tid, sm, switched, alpha, g_wT);
     const DecompFast dc = make_decomp_fast(base_log, L);
     const size_t ggsw_sz = (size_t)L * C::G * C::G * C::M;
     constexpr int P = C::M / 16;
     const int m0 = part * P / L, m1 = (part + 1) * P / L;                     // this group's share of the P register rows
-    // key row r (MAC order: level L first, then L-1, …; polynomial p inside) of the step's GGSW
-    auto row_ptr = [&](const cplx* ggsw, int r) { return ggsw + (size_t)((L - 1 - r / C::G) * C::G + (r % C::G)) * C::G * C::M; };
     for (int i = 0; i < n; i++) {
-        const int* rot = rot_sm + (i & 1) * B;
+        const int* rot = sm.rot_sm + (i & 1) * B;
         const cplx* ggsw = bsk + ggsw_sz * i;
-        if (tid < B && i + 1 < n) rot_sm[((i + 1) & 1) * B + tid] = switched(tid, i + 1);      // consumed after >= 1 barrier
+        if (tid < B && i + 1 < n) sm.rot_sm[((i + 1) & 1) * B + tid] = switched(tid, i + 1);      // consumed after >= 1 barrier
         if (i + kL2PrefetchSteps < n) ggsw_l2_prefetch<C>(ggsw + ggsw_sz * kL2PrefetchSteps, tid, NT);
         // ---- P0: digits
         if (active) {
-            const uint64_t* poly = acc + (size_t)job * N;
+            const uint64_t* poly = sm.acc + (size_t)job * N;
             const int r = rot[job / C::G];
-            uint32_t* dj = dig + (size_t)job * L * C::M;
+            uint32_t* dj = sm.dig + (size_t)job * L * C::M;
 #pragma unroll 2
             for (int m = m0; m < m1; m++) {
                 const int jj = t + 16 * m;
@@ -257,63 +285,26 @@ pbs_wide_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const cp
         __syncthreads();
         // ---- P1: forward FFT of level part+1 of polynomial job; the MAC threads request their first key rows
         cplx g[MAC_DEPTH][C::G];
-        if (tid < NMAC) {
-#pragma unroll
-            for (int r = 0; r < MAC_DEPTH; r++) mac_load_row<C, NMAC>(row_ptr(ggsw, r), 0, tid, g[r]);
-        }
+        if (tid < NMAC) mg_mac_prefetch<C, MAC_DEPTH>(tid, ggsw, g);
         {
-            const uint32_t* d = dig + ((size_t)job * L + part) * C::M;
-            cplx* Sj = S + ((size_t)part * JOBS + job) * C::M;
+            const uint32_t* d = sm.dig + ((size_t)job * L + part) * C::M;
+            cplx* Sj = sm.S + ((size_t)part * JOBS + job) * C::M;
             if (active) fft_fwd_pass1<N>(t, [&](int jj, double& a, double& b) { unpack_digits(d[jj], dc, a, b); }, Sj);
             __syncwarp();                          // outside the predicate: a warp may hold one active and one idle group
-            if (active) fft_fwd_pass2<N>(t, wT, Sj);
+            if (active) fft_fwd_pass2<N>(t, sm.wT, Sj);
         }
         __syncthreads();
-        // ---- P2: Fourier MAC over all L·G key rows
-        if (tid < NMAC) {
-            cplx out[B][C::G];
-#pragma unroll
-            for (int b = 0; b < B; b++)
-#pragma unroll
-                for (int c = 0; c < C::G; c++) out[b][c] = mk(0.0, 0.0);
-#pragma unroll
-            for (int r = 0; r < ROWS; r++) {
-                const int s = L - 1 - r / C::G, p = r % C::G;                  // storage index of the level, polynomial
-#pragma unroll
-                for (int b = 0; b < B; b++) {
-                    const cplx x = S[((size_t)s * JOBS + b * C::G + p) * C::M + tid];
-#pragma unroll
-                    for (int c = 0; c < C::G; c++) cfma(out[b][c], x, g[r % MAC_DEPTH][c]);
-                }
-                if (r + MAC_DEPTH < ROWS) mac_load_row<C, NMAC>(row_ptr(ggsw, r + MAC_DEPTH), 0, tid, g[r % MAC_DEPTH]);
-            }
-            // every thread has finished READING its slot of all buffers only after the barrier; the result goes to rows
-            // of buffer 0 at this thread's own slot, which no other thread reads in P2
-#pragma unroll
-            for (int b = 0; b < B; b++)
-#pragma unroll
-                for (int c = 0; c < C::G; c++) S[(size_t)(b * C::G + c) * C::M + tid] = out[b][c];
-        }
+        // ---- P2: Fourier MAC over all L·G key rows; the sums go to the thread's own slot of buffer 0
+        if (tid < NMAC) mg_mac<C, MAC_DEPTH, 0>(tid, ggsw, sm.S, g);
         __syncthreads();
         // ---- P3: inverse FFT and accumulate (the groups of part 0)
-        if (active && part == 0) grp_inv1<C>(t, job, wT, S);
+        if (active && part == 0) grp_inv1<C>(t, job, sm.wT, sm.S);
         __syncwarp();
-        if (active && part == 0) grp_inv2<C>(t, job, S, acc);
+        if (active && part == 0) grp_inv2<C>(t, job, sm.S, sm.acc);
         __syncthreads();
     }
-    constexpr int LW = K * N + 1;
-    for (int idx = tid; idx < B * LW; idx += NT) {
-        const int b = idx / LW, e = idx - b * LW, ct = ct0 + b;
-        if (ct >= nct) continue;
-        uint64_t v = sample_extract_elem<C>(acc + (size_t)b * C::G * N, e);
-        if (e == K * N) v += alpha;
-        out_big[(size_t)ct * LW + e] = v;
-    }
+    pbs_epilogue<C, NT>(tid, sm.acc, out_big, 0, ct0, nct, alpha);
 }
-// acc, S, dig, wT, then rot_sm ([2][B] ints) with 80 bytes of slack
-template <class C> struct WideSmem {
-    static constexpr size_t bytes = C::acc_words * 8 + (size_t)C::L * C::s_cplx * 16 + (size_t)C::JOBS * C::L * C::M * 4 + (size_t)tab_len(C::N) * 16 + 2 * C::B * sizeof(int) + 16 + 64;
-};
 
 // ================================================================================================ PBS, levels merged (throughput path)
 // pbs_kernel runs a step as L × (forward FFT → barrier → MAC → barrier) because one FFT buffer per (ciphertext, polynomial)
@@ -333,7 +324,18 @@ template <class C> struct WideSmem {
 // another; the MAC is one contiguous key stream instead of L ramps.  Same arithmetic in the same order as pbs_kernel —
 // bit-identical results (tools/pbs_bench.cu prints the same checksum): 98.3 ms against 111.9 ms for 6144 ciphertexts.
 // BLOG > 0: the decomposition base log as a compile-time constant (shifts and masks fold; 0.6 %).
-template <class C> struct MergedSmem { static constexpr size_t bytes = (size_t)C::L * C::s_cplx * 16 + (size_t)tab_len(C::N) * 16 + 64; };
+// Layout: S [L][JOBS][M] (buffer s ↔ level s+1) with acc [B][G][N], the rotation copy, on buffer 0; wT, rot_sm.
+template <class C> struct MergedSmem {
+    cplx* S; uint64_t* acc; cplx* wT; int* rot_sm;
+    __device__ explicit MergedSmem(unsigned char* raw) {
+        S = reinterpret_cast<cplx*>(raw);
+        acc = reinterpret_cast<uint64_t*>(raw);
+        wT = S + (size_t)C::L * C::s_cplx;
+        rot_sm = reinterpret_cast<int*>(wT + tab_len(C::N));
+    }
+    static constexpr size_t bytes = (size_t)C::L * C::s_cplx * 16 + (size_t)tab_len(C::N) * 16 + kRotSmBytes;
+    static_assert(C::acc_words * 8 == C::s_cplx * 16 && 2 * C::B * sizeof(int) <= kRotSmBytes, "layout");
+};
 
 template <int N, int K, int L, int B, int NT, int MAC_DEPTH = 4, int BLOG = 0>
 __global__ void __launch_bounds__(NT, 1)
@@ -345,45 +347,23 @@ pbs_merged_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const 
     static_assert(L >= 2, "the sums use buffer 1, the rotation copy buffer 0");
     static_assert(NT / 16 >= JOBS && NT >= NMAC && MAC_DEPTH <= L * C::G, "thread layout");
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    cplx* S = reinterpret_cast<cplx*>(smem_raw);                               // [L][JOBS][M]   (buffer s ↔ level s+1)
-    uint64_t* acc = reinterpret_cast<uint64_t*>(smem_raw);                     // [B][G][N]      rotation copy = buffer 0
-    cplx* wT = S + (size_t)L * C::s_cplx;
-    int* rot_sm = reinterpret_cast<int*>(wT + tab_len(N));                     // [2][B]
+    const MergedSmem<C> sm(smem_raw);
     const int tid = threadIdx.x;
     const int job = tid >> 4, t = tid & 15;
     const bool active = job < JOBS;
     const int ct0 = blockIdx.x * B;
-    const int n1 = n + 1;
-    auto switched = [&](int b, int i) -> int {
-        const int ct = ct0 + b;
-        if (ct >= nct) return 0;
-        uint64_t a = __ldg(lwe_small + (size_t)ct * n1 + i);
-        if (i == n) a += (1ull << 62);
-        return modswitch(a, LogN<N>::v);
-    };
-    for (int i = tid; i < tab_len(N); i += NT) wT[i] = g_wT[i];
-    if (tid < B) { rot_sm[tid] = switched(tid, 0); rot_sm[B + tid] = switched(tid, n); }
-    __syncthreads();
-    for (int idx = tid; idx < (int)C::acc_words; idx += NT) {
-        const int b = idx / (C::G * N), rem = idx - b * C::G * N, p = rem / N, j = rem - p * N;
-        uint64_t v = 0;
-        if (p == K) {
-            const int s = (j + rot_sm[B + b]) & (2 * N - 1);
-            v = (s < N) ? (0ull - alpha) : alpha;
-        }
-        acc[idx] = v;
-    }
-    __syncthreads();
-    uint64_t* Rj = acc + (size_t)(active ? job : 0) * N;                       // this group's polynomial (rotation copy)
-    cplx* Sjob = S + (size_t)(active ? job : 0) * M;                           // + s·JOBS·M for buffer s
+    const PbsModSwitch<N> switched{lwe_small, nct, n, n + 1, ct0};
+    pbs_prologue<C, NT>(tid, sm, switched, alpha, g_wT);
+    uint64_t* Rj = sm.acc + (size_t)(active ? job : 0) * N;                    // this group's polynomial (rotation copy)
+    cplx* Sjob = sm.S + (size_t)(active ? job : 0) * M;                        // + s·JOBS·M for buffer s
     uint64_t own0[P], own1[P];                                                 // coefficients t + 16m and t + 16m + M
     static_for<0, P>([&](auto mc) { constexpr int m = decltype(mc)::value; own0[m] = Rj[t + 16 * m]; own1[m] = Rj[t + 16 * m + M]; });
     const DecompFast dc = make_decomp_fast(BLOG ? BLOG : base_log, L);
     const size_t ggsw_sz = (size_t)L * C::G * C::G * C::M;
     for (int i = 0; i < n; i++) {
-        const int rot = rot_sm[(i & 1) * B + (active ? job / C::G : 0)];
+        const int rot = sm.rot_sm[(i & 1) * B + (active ? job / C::G : 0)];
         const cplx* ggsw = bsk + ggsw_sz * i;
-        if (tid < B && i + 1 < n) rot_sm[((i + 1) & 1) * B + tid] = switched(tid, i + 1);      // consumed after >= 1 barrier
+        if (tid < B && i + 1 < n) sm.rot_sm[((i + 1) & 1) * B + tid] = switched(tid, i + 1);      // consumed after >= 1 barrier
         if (i + kL2PrefetchSteps < n) ggsw_l2_prefetch<C>(ggsw + ggsw_sz * kL2PrefetchSteps, tid, NT);
         // ---- digits of all levels, in registers
         uint32_t dg[L][P];
@@ -400,29 +380,22 @@ pbs_merged_kernel(const uint64_t* __restrict__ lwe_small, int nct, int n, const 
         // ---- forward pass 2 of every level; then the first key rows are requested (in flight during the barrier)
         static_for<0, L>([&](auto ic) {
             constexpr int s = L - 1 - decltype(ic)::value;
-            if (active) fft_fwd_pass2<N>(t, wT, Sjob + (size_t)s * JOBS * M);
+            if (active) fft_fwd_pass2<N>(t, sm.wT, Sjob + (size_t)s * JOBS * M);
         });
         cplx g[MAC_DEPTH][C::G];
         if (tid < NMAC) mg_mac_prefetch<C, MAC_DEPTH>(tid, ggsw, g);
         __syncthreads();
         // ---- Fourier MAC over all L·G key rows; a thread reads and writes only its own slot of every buffer
-        if (tid < NMAC) mg_mac<C, MAC_DEPTH, SUMS>(tid, ggsw, S, g);
+        if (tid < NMAC) mg_mac<C, MAC_DEPTH, SUMS>(tid, ggsw, sm.S, g);
         __syncthreads();
         // ---- inverse transform of the sums; accumulate in registers; refresh the rotation copy
-        if (active) fft_inv_passA<N>(t, wT, Sjob + (size_t)SUMS * JOBS * M);
+        if (active) fft_inv_passA<N>(t, sm.wT, Sjob + (size_t)SUMS * JOBS * M);
         __syncwarp();
         if (active) mg_inv2<C>(t, Sjob + (size_t)SUMS * JOBS * M, Rj, own0, own1);
         __syncwarp();
     }
     __syncthreads();
-    constexpr int LW = K * N + 1;
-    for (int idx = tid; idx < B * LW; idx += NT) {
-        const int b = idx / LW, e = idx - b * LW, ct = ct0 + b;
-        if (ct >= nct) continue;
-        uint64_t v = sample_extract_elem<C>(acc + (size_t)b * C::G * N, e);
-        if (e == K * N) v += alpha;
-        out_big[(size_t)ct * LW + e] = v;
-    }
+    pbs_epilogue<C, NT>(tid, sm.acc, out_big, 0, ct0, nct, alpha);
 }
 
 // ================================================================================================ vertical packing
@@ -452,12 +425,7 @@ vp_kernel(const cplx* __restrict__ ggsw_f, int n_in, int first_ggsw, const uint6
     }
     __syncthreads();
     cplx outr[MC::SPT][B][C::G];
-#pragma unroll
-    for (int a = 0; a < MC::SPT; a++)
-#pragma unroll
-        for (int b = 0; b < B; b++)
-#pragma unroll
-            for (int c = 0; c < C::G; c++) outr[a][b][c] = mk(0.0, 0.0);
+    zero_fourier_acc(outr);
     const size_t ggsw_sz = (size_t)L * C::G * C::G * C::M;
     const cplx* gbox = ggsw_f + (size_t)box * n_in * ggsw_sz;
     int deg = 1;
@@ -468,12 +436,7 @@ vp_kernel(const cplx* __restrict__ ggsw_f, int n_in, int first_ggsw, const uint6
         deg <<= 1;
     }
     __syncthreads();
-    constexpr int LW = K * N + 1;
-    for (int idx = tid; idx < B * LW; idx += NT) {
-        const int b = idx / LW, e = idx - b * LW, o = o0 + b;
-        if (o >= n_out) continue;
-        out[((size_t)box * n_out + o) * LW + e] = sample_extract_elem<C>(sm.acc + (size_t)b * C::G * N, e);
-    }
+    pbs_epilogue<C, NT>(tid, sm.acc, out, box, o0, n_out, 0);
 }
 
 // One CMux-tree layer ([U] wop_pbs.rs::cmux_tree_memory_optimized, evaluated level by level): for every (box, output,
@@ -508,10 +471,7 @@ cmux_tree_kernel(const cplx* __restrict__ ggsw_f, int n_in, int ggsw_idx, const 
     }
     __syncthreads();
     cplx outr[MC::SPT][1][C::G];
-#pragma unroll
-    for (int a = 0; a < MC::SPT; a++)
-#pragma unroll
-        for (int c = 0; c < C::G; c++) outr[a][0][c] = mk(0.0, 0.0);
+    zero_fourier_acc(outr);
     const size_t ggsw_sz = (size_t)L * C::G * C::G * C::M;
     const cplx* ggsw = ggsw_f + ((size_t)box * n_in + ggsw_idx) * ggsw_sz;
     ep_step_device<C, NT>(tid, sm, ggsw, [&](int job, int jj, uint64_t& x0, uint64_t& x1) { x0 = diff[(size_t)job * N + jj]; x1 = diff[(size_t)job * N + jj + N / 2]; },
