@@ -195,6 +195,54 @@ int tac_aes_decrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, co
 /* boxes per round that tac_aes_decrypt_public_blocks runs for these blocks (as tac_aes_public_plan).  Host only. */
 int tac_aes_public_plan_inv(int n_blocks, int rounds, const uint8_t* blocks_host /*[n][16]*/, int64_t* boxes);
 
+/* ------------------------------------------------------------------ AES under many keys (no counterpart in the reference) */
+/* A context holds, beside the single key schedule above, a KEY TABLE of n_keys AES-128 key schedules and optionally the
+ * matching table of inverse schedules dk.  Neither replaces the other: loading a table leaves the single schedule (and its
+ * dk) as it is, and tac_aes_set_key_schedule leaves the table as it is.  Keyed entry points take a host array
+ * key_idx[n_blocks] with values in [0, n_keys); block b runs under table entry key_idx[b], blocks of different keys mix
+ * freely in one call.  The output for block b equals, word for word, what the single-key entry point gives for that block
+ * with entry key_idx[b]'s schedule resident; noise as there (33 in a middle round, 9 at the output).
+ * Errors: TAC_ERR_STATE without a key table, or, decrypting, without a valid inverse table (none is derived implicitly);
+ * TAC_ERR_ARG for n_keys < 1, a NULL key_idx with n_blocks > 0 or an index outside [0, n_keys), checked before anything is
+ * enqueued; TAC_ERR_CUDA when a table does not fit in device memory (one schedule is 44·32·(kN+1)·8 bytes, 23 MB at
+ * kN+1 = 2049; the inverse table as much again). */
+/* Batched key expansion (no counterpart in the reference): n_keys FHE-encrypted keys [n_keys][128][kN+1] expanded together —
+ * each of the 40 steps bootstraps the bytes and bits of all keys in one pass — into the resident key table
+ * [n_keys][44][4][8][kN+1]; key_scheds_host may be NULL.  Entry k equals tac_aes_key_schedule of key k.  Marks the
+ * inverse table stale. */
+int tac_aes_key_table(tac_ctx* ctx, int n_keys, const uint64_t* key_bits_host, uint64_t* key_scheds_host);
+/* make n_keys expanded keys [n_keys][44][4][8][kN+1] the resident key table (no counterpart in the reference); marks the
+ * inverse table stale */
+int tac_aes_set_key_table(tac_ctx* ctx, int n_keys, const uint64_t* key_scheds_host);
+/* dk of every entry of the resident key table, as tac_aes_inv_key_schedule (no counterpart in the reference); out may be NULL */
+int tac_aes_inv_key_table(tac_ctx* ctx, uint64_t* inv_key_scheds_host);
+/* make given inverse schedules resident, n_keys of the resident table (no counterpart in the reference) */
+int tac_aes_set_inv_key_table(tac_ctx* ctx, const uint64_t* inv_key_scheds_host);
+/* tac_aes_encrypt_blocks / tac_aes_decrypt_blocks with block b under table entry key_idx[b] (no counterpart in the reference) */
+int tac_aes_encrypt_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_host,
+                                 uint64_t* out_host);
+int tac_aes_encrypt_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_dev,
+                                     uint64_t* out_dev);
+int tac_aes_decrypt_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_host,
+                                 uint64_t* out_host);
+int tac_aes_decrypt_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_dev,
+                                     uint64_t* out_dev);
+/* tac_aes_encrypt_public_blocks / tac_aes_decrypt_public_blocks with block b under table entry key_idx[b] (no counterpart
+ * in the reference): AES-CTR / AES-ECB / AES-CBC transciphering for many senders in one call.  A bootstrap is shared only
+ * between blocks of the same key, so identical counter blocks under two keys share nothing. */
+int tac_aes_encrypt_public_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
+                                        const uint8_t* xor_host, uint64_t* out_host);
+int tac_aes_encrypt_public_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
+                                            const uint8_t* xor_host, uint64_t* out_dev);
+int tac_aes_decrypt_public_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
+                                        const uint8_t* xor_host, uint64_t* out_host);
+int tac_aes_decrypt_public_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
+                                            const uint8_t* xor_host, uint64_t* out_dev);
+/* boxes per round of the keyed public paths (decrypt 0: encryption, else decryption; no counterpart in the reference);
+ * key_idx NULL = one key, and then the result equals tac_aes_public_plan / tac_aes_public_plan_inv.  TAC_ERR_ARG for a
+ * negative index.  Host only. */
+int tac_aes_public_plan_keyed(int n_blocks, int rounds, int decrypt, const int32_t* key_idx, const uint8_t* blocks_host /*[n][16]*/, int64_t* boxes);
+
 /* ------------------------------------------------------------------ single stages (parity tests, profiling) */
 /* [U] keyswitch_lwe_ciphertext: [n_cts][kN+1] → [n_cts][n+1] */
 int tac_stage_keyswitch(tac_ctx* ctx, int n_cts, const uint64_t* in_host, uint64_t* out_host);

@@ -109,6 +109,20 @@ extern "C" {
     pub fn tac_aes_decrypt_public_blocks(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, blocks_host: *const u8, xor_host: *const u8, out_host: *mut u64) -> c_int;
     pub fn tac_aes_decrypt_public_blocks_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, blocks_host: *const u8, xor_host: *const u8, out_dev: *mut u64) -> c_int;
     pub fn tac_aes_public_plan_inv(n_blocks: c_int, rounds: c_int, blocks_host: *const u8, boxes: *mut i64) -> c_int;
+    // AES under many keys (no counterpart in the reference)
+    pub fn tac_aes_key_table(ctx: *mut tac_ctx, n_keys: c_int, key_bits_host: *const u64, key_scheds_host: *mut u64) -> c_int;
+    pub fn tac_aes_set_key_table(ctx: *mut tac_ctx, n_keys: c_int, key_scheds_host: *const u64) -> c_int;
+    pub fn tac_aes_inv_key_table(ctx: *mut tac_ctx, inv_key_scheds_host: *mut u64) -> c_int;
+    pub fn tac_aes_set_inv_key_table(ctx: *mut tac_ctx, inv_key_scheds_host: *const u64) -> c_int;
+    pub fn tac_aes_encrypt_blocks_keyed(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, in_noise_sq: c_int, key_idx_host: *const i32, in_host: *const u64, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_encrypt_blocks_keyed_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, in_noise_sq: c_int, key_idx_host: *const i32, in_dev: *const u64, out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_decrypt_blocks_keyed(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, in_noise_sq: c_int, key_idx_host: *const i32, in_host: *const u64, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_decrypt_blocks_keyed_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, in_noise_sq: c_int, key_idx_host: *const i32, in_dev: *const u64, out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_encrypt_public_blocks_keyed(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, key_idx_host: *const i32, blocks_host: *const u8, xor_host: *const u8, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_encrypt_public_blocks_keyed_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, key_idx_host: *const i32, blocks_host: *const u8, xor_host: *const u8, out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_decrypt_public_blocks_keyed(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, key_idx_host: *const i32, blocks_host: *const u8, xor_host: *const u8, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_decrypt_public_blocks_keyed_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, key_idx_host: *const i32, blocks_host: *const u8, xor_host: *const u8, out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_public_plan_keyed(n_blocks: c_int, rounds: c_int, decrypt: c_int, key_idx: *const i32, blocks_host: *const u8, boxes: *mut i64) -> c_int;
 
     // single stages, profiling
     pub fn tac_stage_keyswitch(ctx: *mut tac_ctx, n_cts: c_int, in_host: *const u64, out_host: *mut u64) -> c_int;

@@ -109,6 +109,19 @@ _SIGNATURES = {
     "tac_aes_decrypt_public_blocks": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_aes_decrypt_public_blocks_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_aes_public_plan_inv": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "tac_aes_key_table": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "tac_aes_set_key_table": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "tac_aes_inv_key_table": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tac_aes_set_inv_key_table": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tac_aes_encrypt_blocks_keyed": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_encrypt_blocks_keyed_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_decrypt_blocks_keyed": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_decrypt_blocks_keyed_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_encrypt_public_blocks_keyed": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_encrypt_public_blocks_keyed_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_decrypt_public_blocks_keyed": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_decrypt_public_blocks_keyed_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_public_plan_keyed": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_stage_keyswitch": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
     "tac_extract_bits": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _u64p, _u64p]),
     "tac_stage_pbs": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
@@ -241,16 +254,38 @@ def ctr_blocks(iv, first_ctr, n):
     return _public_blocks(b"".join(iv + (first_ctr + i).to_bytes(8, "big") for i in range(n)))
 
 
-def aes_public_plan(blocks, rounds=10, decrypt=False):
+def _key_index(key_index, n_blocks, n_keys=None):
+    """int32 [n_blocks] from a sequence of key indices; with n_keys, every index must lie in [0, n_keys)"""
+    if key_index is None:
+        raise ValueError("a key index per block is required")
+    k = np.asarray(key_index)
+    if k.size and not np.issubdtype(k.dtype, np.integer):
+        raise ValueError("key indices must be integers")
+    k = np.ascontiguousarray(k, dtype=np.int64).ravel()
+    if k.size != n_blocks:
+        raise ValueError(f"{k.size} key indices for {n_blocks} blocks")
+    if k.size and (k.min() < 0 or (n_keys is not None and k.max() >= n_keys)):
+        raise ValueError(f"key index outside [0, {n_keys})")
+    return k.astype(np.int32)
+
+
+def aes_public_plan(blocks, rounds=10, decrypt=False, key_index=None):
     """circuit bootstraps per round that FheContext.aes_encrypt_public_blocks (decrypt=True: aes_decrypt_public_blocks) runs
-    for these public blocks (rounds 1..rounds); 16 per block and round without sharing.  Host only."""
+    for these public blocks (rounds 1..rounds); 16 per block and round without sharing.  key_index: the keyed paths' plan
+    (aes_encrypt_public_blocks_keyed / aes_decrypt_public_blocks_keyed), where only blocks of the same key share.  Host only."""
     b = _public_blocks(blocks)
     out = np.zeros(max(rounds, 0), dtype=np.int64)
     L = load_library()
-    plan = L.tac_aes_public_plan_inv if decrypt else L.tac_aes_public_plan
-    rc = plan(b.shape[0], rounds, b.ctypes.data, out.ctypes.data)
+    if key_index is None:
+        plan = L.tac_aes_public_plan_inv if decrypt else L.tac_aes_public_plan
+        rc = plan(b.shape[0], rounds, b.ctypes.data, out.ctypes.data)
+    else:
+        k = np.ascontiguousarray(np.asarray(key_index, dtype=np.int64).ravel(), dtype=np.int32)
+        if k.size != b.shape[0]:
+            raise ValueError(f"{k.size} key indices for {b.shape[0]} blocks")
+        rc = L.tac_aes_public_plan_keyed(b.shape[0], rounds, int(decrypt), k.ctypes.data, b.ctypes.data, out.ctypes.data)
     if rc != 0:
-        raise ValueError(f"aes_public_plan: rounds must be in 1..10 (error {rc})")
+        raise ValueError(f"aes_public_plan: rounds must be in 1..10 and key indices non-negative (error {rc})")
     return [int(v) for v in out]
 
 
@@ -720,6 +755,138 @@ class FheContext(NoiseContext):
             raise ValueError("iv must be 16 bytes")
         out = self.aes_decrypt_public_blocks(data, xor=(iv + data[:-16]) if data else None)
         return out.reshape(len(data), 8, self.params.big_lwe_size)
+
+    # -- AES under many keys: a resident table of key schedules, one call over blocks of many keys
+    def aes_key_table(self, keys_bits):
+        """batched key expansion of K FHE-encrypted keys [K][128][big+1] (K >= 1); the result becomes the resident key
+        table and is returned, [K][44][4][8][big+1].  Entry k equals aes_key_schedule of key k.  The single key schedule
+        is left as it is; the inverse table becomes stale."""
+        kb = np.ascontiguousarray(keys_bits, dtype=np.uint64)
+        L1 = self.params.big_lwe_size
+        if kb.size == 0 or kb.size % (128 * L1):
+            raise ValueError("keys_bits must hold [K][128][big+1] words, K >= 1")
+        K = kb.size // (128 * L1)
+        out = np.empty((K, 44, 4, 8, L1), dtype=np.uint64)
+        self._n_keys = 0
+        self._check(self.L.tac_aes_key_table(self.h, K, kb.ctypes.data, out.ctypes.data))
+        self._n_keys = K
+        return out
+
+    def aes_set_key_table(self, key_scheds):
+        """make K expanded keys [K][44][4][8][big+1] the resident key table; the inverse table becomes stale"""
+        ks = np.ascontiguousarray(key_scheds, dtype=np.uint64)
+        per = 44 * 32 * self.params.big_lwe_size
+        if ks.size == 0 or ks.size % per:
+            raise ValueError("key_scheds must hold [K][44][4][8][big+1] words, K >= 1")
+        self._n_keys = 0
+        self._check(self.L.tac_aes_set_key_table(self.h, ks.size // per, ks.ctypes.data))
+        self._n_keys = ks.size // per
+
+    def aes_inv_key_table(self):
+        """derive the inverse key schedule of every entry of the resident key table; returns them, [K][44][4][8][big+1]"""
+        out = np.empty((max(self.n_keys, 1), 44, 4, 8, self.params.big_lwe_size), dtype=np.uint64)
+        self._check(self.L.tac_aes_inv_key_table(self.h, out.ctypes.data))
+        return out
+
+    def aes_set_inv_key_table(self, inv_key_scheds):
+        """make given inverse schedules [K][44][4][8][big+1] resident, K of the resident key table"""
+        dk = np.ascontiguousarray(inv_key_scheds, dtype=np.uint64)
+        if dk.size != self.n_keys * 44 * 32 * self.params.big_lwe_size:
+            raise ValueError(f"inverse key schedules must match the resident key table of {self.n_keys} keys")
+        self._check(self.L.tac_aes_set_inv_key_table(self.h, dk.ctypes.data))
+
+    @property
+    def n_keys(self):
+        """entries of the resident key table (0: none)"""
+        return getattr(self, "_n_keys", 0)
+
+    def _aes_blocks_keyed(self, fn, blocks, key_index, rounds, in_noise_sq):
+        b = np.ascontiguousarray(blocks, dtype=np.uint64).reshape(-1, 16, 8, self.params.big_lwe_size)
+        k = _key_index(key_index, b.shape[0], self.n_keys)
+        out = np.empty_like(b)
+        self._check(fn(self.h, b.shape[0], rounds, in_noise_sq, k.ctypes.data, b.ctypes.data, out.ctypes.data))
+        return out
+
+    def _aes_blocks_keyed_dev(self, fn, n_blocks, key_index, in_ptr, out_ptr, rounds, in_noise_sq):
+        k = _key_index(key_index, n_blocks, self.n_keys)
+        self._check(fn(self.h, n_blocks, rounds, in_noise_sq, k.ctypes.data, C.c_void_p(in_ptr), C.c_void_p(out_ptr)))
+
+    def aes_encrypt_blocks_keyed(self, blocks, key_index, rounds=10, in_noise_sq=1):
+        """aes_encrypt_blocks with block b under key table entry key_index[b]"""
+        return self._aes_blocks_keyed(self.L.tac_aes_encrypt_blocks_keyed, blocks, key_index, rounds, in_noise_sq)
+
+    def aes_encrypt_blocks_keyed_dev(self, n_blocks, key_index, in_ptr, out_ptr, rounds=10, in_noise_sq=1):
+        self._aes_blocks_keyed_dev(self.L.tac_aes_encrypt_blocks_keyed_dev, n_blocks, key_index, in_ptr, out_ptr, rounds, in_noise_sq)
+
+    def aes_decrypt_blocks_keyed(self, blocks, key_index, rounds=10, in_noise_sq=1):
+        """aes_decrypt_blocks with block b under inverse table entry key_index[b]"""
+        return self._aes_blocks_keyed(self.L.tac_aes_decrypt_blocks_keyed, blocks, key_index, rounds, in_noise_sq)
+
+    def aes_decrypt_blocks_keyed_dev(self, n_blocks, key_index, in_ptr, out_ptr, rounds=10, in_noise_sq=1):
+        self._aes_blocks_keyed_dev(self.L.tac_aes_decrypt_blocks_keyed_dev, n_blocks, key_index, in_ptr, out_ptr, rounds, in_noise_sq)
+
+    def _aes_public_blocks_keyed(self, fn, blocks, key_index, rounds, xor, dev=False, out_ptr=None):
+        b = _public_blocks(blocks)
+        k = _key_index(key_index, b.shape[0], self.n_keys)
+        return self._aes_public_blocks(lambda h, n, r, bp, xp, op: fn(h, n, r, k.ctypes.data, bp, xp, op), b, rounds, xor, dev, out_ptr)
+
+    def aes_encrypt_public_blocks_keyed(self, blocks, key_index, rounds=10, xor=None):
+        """aes_encrypt_public_blocks with block b under key table entry key_index[b]"""
+        return self._aes_public_blocks_keyed(self.L.tac_aes_encrypt_public_blocks_keyed, blocks, key_index, rounds, xor)
+
+    def aes_encrypt_public_blocks_keyed_dev(self, blocks, key_index, out_ptr, rounds=10, xor=None):
+        self._aes_public_blocks_keyed(self.L.tac_aes_encrypt_public_blocks_keyed_dev, blocks, key_index, rounds, xor, dev=True, out_ptr=out_ptr)
+
+    def aes_decrypt_public_blocks_keyed(self, blocks, key_index, rounds=10, xor=None):
+        """aes_decrypt_public_blocks with block b under inverse table entry key_index[b]"""
+        return self._aes_public_blocks_keyed(self.L.tac_aes_decrypt_public_blocks_keyed, blocks, key_index, rounds, xor)
+
+    def aes_decrypt_public_blocks_keyed_dev(self, blocks, key_index, out_ptr, rounds=10, xor=None):
+        self._aes_public_blocks_keyed(self.L.tac_aes_decrypt_public_blocks_keyed_dev, blocks, key_index, rounds, xor, dev=True, out_ptr=out_ptr)
+
+    def aes_ctr_transcipher_many(self, messages):
+        """aes_ctr_transcipher for many senders in one call: messages = [(key_index, iv, first_ctr, data)], each an AES-CTR
+        ciphertext under key table entry key_index.  Returns one array per message, [len(data)][8][big+1]."""
+        blocks, xor, kidx, sizes = [], [], [], []
+        for key_index, iv, first_ctr, data in messages:
+            data = bytes(data)
+            n = (len(data) + 15) // 16
+            blocks.append(ctr_blocks(iv, first_ctr, n))
+            xor.append(data + bytes(16 * n - len(data)))
+            kidx += [key_index] * n
+            sizes.append(len(data))
+        k = _key_index(kidx, len(kidx), self.n_keys)
+        if not sizes:
+            return []
+        out = self.aes_encrypt_public_blocks_keyed(np.concatenate(blocks), k, xor=b"".join(xor))
+        return self._split_messages(out, sizes)
+
+    def aes_cbc_transcipher_many(self, messages):
+        """aes_cbc_transcipher for many senders in one call: messages = [(key_index, iv, data)], each an AES-CBC ciphertext
+        under key table entry key_index.  Returns one array per message, [len(data)][8][big+1]."""
+        blocks, xor, kidx, sizes = [], [], [], []
+        for key_index, iv, data in messages:
+            iv, data = bytes(iv), self._whole_blocks(data)
+            if len(iv) != 16:
+                raise ValueError("iv must be 16 bytes")
+            blocks.append(data)
+            xor.append((iv + data[:-16]) if data else b"")
+            kidx += [key_index] * (len(data) // 16)
+            sizes.append(len(data))
+        k = _key_index(kidx, len(kidx), self.n_keys)
+        if not sizes:
+            return []
+        out = self.aes_decrypt_public_blocks_keyed(b"".join(blocks), k, xor=b"".join(xor))
+        return self._split_messages(out, sizes)
+
+    def _split_messages(self, out, sizes):
+        """[n][16][8][big+1] of whole blocks → one [size][8][big+1] array per message (each padded to whole blocks)"""
+        flat = out.reshape(-1, 8, self.params.big_lwe_size)
+        res, off = [], 0
+        for n in sizes:
+            res.append(flat[off:off + n])
+            off += 16 * ((n + 15) // 16)
+        return res
 
     def aes_key_schedule_buffer(self):
         ptr, nbytes = C.c_void_p(), C.c_size_t()

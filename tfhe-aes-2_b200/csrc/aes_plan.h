@@ -8,6 +8,9 @@
 //
 // The equivalent inverse cipher (tac_aes_decrypt_public_blocks) spreads dependence along the other diagonal:
 //   D(r+1, (row, c)) = ∪_{r'=0..3} D(r, 4·((c − r') mod 4) + r')                             (InvShiftRows + InvMixColumns)
+//
+// Under many keys (a per-block key index into a table of key schedules) the key schedule is shared only among blocks of
+// the same key: two positions share a bootstrap when their blocks have the same key index AND agree on D(r, j).
 #pragma once
 #include <cstdint>
 #include <vector>
@@ -23,8 +26,9 @@ struct AesRoundPlan {
 
 enum class AesDir { Forward, Inverse };
 
-// plan[r-1] for r = 1..rounds of the cipher in direction `dir`; returns TAC_OK or TAC_ERR_ARG (n_blocks < 0, rounds outside
-// 1..10, NULL blocks with n_blocks > 0)
-int aes_public_plan_build(int n_blocks, int rounds, const uint8_t* blocks /*[n][16]*/, AesDir dir, std::vector<AesRoundPlan>& plan);
+// plan[r-1] for r = 1..rounds of the cipher in direction `dir`; key_idx: NULL (one key) or the key index of every block.
+// Returns TAC_OK or TAC_ERR_ARG (n_blocks < 0, rounds outside 1..10, NULL blocks with n_blocks > 0, a negative key index)
+int aes_public_plan_build(int n_blocks, int rounds, const uint8_t* blocks /*[n][16]*/, AesDir dir, std::vector<AesRoundPlan>& plan,
+                          const int32_t* key_idx = nullptr /*[n]*/);
 
 }  // namespace tac

@@ -90,6 +90,11 @@ struct tac_ctx {
     uint64_t* inv_key_sched = nullptr;   // equivalent inverse cipher's schedule dk, same layout [44 words][4][8][kN+1]
     bool inv_key_sched_valid = false;    // dk belongs to the resident key_sched (cleared by tac_aes_set_key_schedule)
     uint64_t* rc_rows = nullptr;     // trivial(RC[1..10]) as byte ciphertexts [10][8][kN+1], uploaded once
+    // AES under many keys: a table of n_keys schedules [n_keys][44 words][4][8][kN+1] and their inverse schedules, apart
+    // from the single schedule above (neither replaces the other)
+    DevBuf key_table, inv_key_table;
+    int n_keys = 0;                      // 0: no key table
+    bool inv_key_table_valid = false;    // inv_key_table belongs to the resident key_table
     // workspace
     DevBuf ws_in, ws_out, ws_small, ws_ksdig, ws_pbs, ws_pfdig, ws_ggsw, ws_ggswf, ws_tree_a, ws_tree_b, ws_state, ws_muls, ws_misc;
     DevBuf ws_plan, ws_rep;          // public-block AES: uploaded plan tables / public bytes, compact S-box inputs
@@ -418,12 +423,15 @@ int aes_noise_check(tac_ctx* ctx, int in_noise_sq, int rounds) {
 // mix-columns / final-round kernels read every position's S-box row through the plan's index table.  Rounds whose plan is
 // the identity (every round of ciphertext input; from round 3 on when all blocks differ) run on the full state in place.
 // xor_host (public input only; NULL: none) is XORed into the output.
-int aes_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_dev, const uint8_t* blocks_host,
-                   const uint8_t* xor_host, uint64_t* out_dev) {
+// keys: the schedule (w or dk) of the direction.  key_idx_host: NULL, or (AES under many keys) the index of every block's
+// schedule in the table at `keys`; it travels to the device with the plan, every round kernel offsets block b's round
+// keys by key_idx[b] schedules, and the plan shares a bootstrap only among blocks of the same key.  Callers validate it.
+int aes_blocks_dev(tac_ctx* ctx, AesDir dir, const uint64_t* keys, const int32_t* key_idx_host, int n_blocks, int rounds, int in_noise_sq,
+                   const uint64_t* in_dev, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
     const bool fwd = dir == AesDir::Forward, pub = in_dev == nullptr;
     std::vector<AesRoundPlan> plan;
     if (pub) {
-        if (aes_public_plan_build(n_blocks, rounds, blocks_host, dir, plan)) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range, or NULL blocks");
+        if (aes_public_plan_build(n_blocks, rounds, blocks_host, dir, plan, key_idx_host)) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range, or NULL blocks");
     } else {
         if (n_blocks < 0 || rounds < 1 || rounds > 10) return fail(ctx, TAC_ERR_ARG, "n_blocks / rounds out of range");
         plan.assign(rounds, AesRoundPlan{16 * (int64_t)n_blocks, true});
@@ -433,44 +441,49 @@ int aes_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, int in_no
     TRY(fwd ? ensure_aes_luts(ctx) : ensure_aes_inv_luts(ctx));
     const size_t L = (size_t)ctx->big() + 1, byte_words = 8 * L, blk = 16 * byte_words;
     const size_t npos = (size_t)n_blocks * 16, total = (size_t)n_blocks * blk;
+    const size_t key_words = key_idx_host ? 11 * blk : 0;        // one schedule: 44 words = 11 round keys of a block's size
     // per direction: S-box LUTs S·{1,2,3} / S or InvS·{14,11,13,9} / InvS, round keys, (Inv)ShiftRows kernels
-    const uint64_t* keys = fwd ? ctx->key_sched : ctx->inv_key_sched;
     const Lut& lut_mid = ctx->luts[fwd ? ctx->aes_lut24 : ctx->aes_lut_inv32];
     const Lut& lut_last = ctx->luts[fwd ? ctx->aes_lut8 : ctx->aes_lut_inv8];
     const uint64_t* k_first = fwd ? keys : keys + (size_t)10 * blk;
     const uint64_t* k_last = fwd ? keys + (size_t)10 * blk : keys;
     const auto mix_columns = fwd ? aes_mix_columns_kernel<true> : aes_mix_columns_kernel<false>;
     const auto final_round = fwd ? aes_final_round_kernel<true> : aes_final_round_kernel<false>;
-    // public input: one upload of the blocks, the XOR bytes, then rep_pos / idx of every round that shares
+    // one upload: public input's blocks and XOR bytes, the key index, then rep_pos / idx of every round that shares
     std::vector<size_t> off_rep(rounds, 0), off_idx(rounds, 0);
     std::vector<uint8_t> host;
-    size_t max_rep = 0;
+    size_t max_rep = 0, bytes = pub ? 2 * npos : 0;
+    const size_t off_kidx = bytes;
+    if (key_idx_host) bytes += (size_t)n_blocks * 4;
     if (pub) {
-        size_t bytes = 2 * npos;
         for (int r = 0; r < rounds; r++) {
             if (plan[r].identity) continue;
             off_rep[r] = bytes; bytes += (size_t)plan[r].boxes * 4;
             off_idx[r] = bytes; bytes += npos * 4;
             max_rep = std::max(max_rep, (size_t)plan[r].boxes);
         }
+    }
+    if (bytes) {
         host.assign(bytes, 0);
-        std::memcpy(host.data(), blocks_host, npos);
-        if (xor_host) std::memcpy(host.data() + npos, xor_host, npos);
-        for (int r = 0; r < rounds; r++) {
-            if (plan[r].identity) continue;
-            std::memcpy(host.data() + off_rep[r], plan[r].rep_pos.data(), (size_t)plan[r].boxes * 4);
-            std::memcpy(host.data() + off_idx[r], plan[r].idx.data(), npos * 4);
+        if (pub) {
+            std::memcpy(host.data(), blocks_host, npos);
+            if (xor_host) std::memcpy(host.data() + npos, xor_host, npos);
+            for (int r = 0; r < rounds; r++) {
+                if (plan[r].identity) continue;
+                std::memcpy(host.data() + off_rep[r], plan[r].rep_pos.data(), (size_t)plan[r].boxes * 4);
+                std::memcpy(host.data() + off_idx[r], plan[r].idx.data(), npos * 4);
+            }
         }
+        if (key_idx_host) std::memcpy(host.data() + off_kidx, key_idx_host, (size_t)n_blocks * 4);
         TRY(ensure(ctx, ctx->ws_plan, bytes));
     }
     TRY(ensure(ctx, ctx->ws_state, total * 8));
     TRY(ensure(ctx, ctx->ws_muls, total * (fwd ? 3 : 4) * 8));
-    if (pub) {
-        TRY(ensure(ctx, ctx->ws_rep, std::max<size_t>(1, max_rep) * byte_words * 8));
-        // pageable source: the call returns once the bytes are staged, so `host` may go out of scope before the copy lands
-        CU(cudaMemcpyAsync(ctx->ws_plan.p, host.data(), host.size(), cudaMemcpyHostToDevice, ctx->stream));
-    }
+    if (pub) TRY(ensure(ctx, ctx->ws_rep, std::max<size_t>(1, max_rep) * byte_words * 8));
+    // pageable source: the call returns once the bytes are staged, so `host` may go out of scope before the copy lands
+    if (bytes) CU(cudaMemcpyAsync(ctx->ws_plan.p, host.data(), host.size(), cudaMemcpyHostToDevice, ctx->stream));
     const uint8_t* d_plan = ctx->ws_plan.as<uint8_t>();
+    const int32_t* kidx = key_idx_host ? reinterpret_cast<const int32_t*>(d_plan + off_kidx) : nullptr;
     auto rep_pos = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_rep[r]); };
     auto idx = [&](int r) { return plan[r].identity ? nullptr : reinterpret_cast<const int32_t*>(d_plan + off_idx[r]); };
     uint64_t* state = ctx->ws_state.as<uint64_t>();
@@ -482,12 +495,12 @@ int aes_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, int in_no
         const int r = rd - 1;
         const size_t n_words = (size_t)plan[r].boxes * byte_words;
         if (rd == 1 && !pub) {
-            aes_add_round_key_kernel<<<g, 256, 0, ctx->stream>>>(in_dev, k_first, blk, total, state);          // :96-99
+            aes_add_round_key_kernel<<<g, 256, 0, ctx->stream>>>(in_dev, k_first, blk, total, state, kidx, key_words);          // :96-99
             TRY(post_launch(ctx, "aes_add_round_key_kernel"));
             *in = state;
         } else if (rd == 1) {
             uint64_t* dst = plan[r].identity ? state : rep;
-            aes_public_round1_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(k_first, d_plan, rep_pos(r), (int)L, n_words, dst);
+            aes_public_round1_kernel<<<grid1d(n_words, 256, ctx->sm_count), 256, 0, ctx->stream>>>(k_first, d_plan, rep_pos(r), (int)L, n_words, dst, kidx, key_words);
             TRY(post_launch(ctx, "aes_public_round1_kernel"));
             *in = dst;
         } else if (plan[r].identity) {
@@ -503,12 +516,12 @@ int aes_blocks_dev(tac_ctx* ctx, AesDir dir, int n_blocks, int rounds, int in_no
     for (int rd = 1; rd < rounds; rd++) {
         TRY(sbox_inputs(rd, &in));
         TRY(wopbs_dev(ctx, lut_mid, (int)plan[rd - 1].boxes, in, muls));                                      // sub_bytes_with_gal_mul :27-48
-        mix_columns<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)(fwd ? rd : rounds - rd) * blk, (int)L, total, state, idx(rd - 1));
+        mix_columns<<<g, 256, 0, ctx->stream>>>(muls, keys + (size_t)(fwd ? rd : rounds - rd) * blk, (int)L, total, state, idx(rd - 1), kidx, key_words);
         TRY(post_launch(ctx, "aes_mix_columns_kernel"));
     }
     TRY(sbox_inputs(rounds, &in));
     TRY(wopbs_dev(ctx, lut_last, (int)plan[rounds - 1].boxes, in, muls));                                     // sub_bytes :51-58
-    final_round<<<g, 256, 0, ctx->stream>>>(muls, k_last, (int)L, total, out_dev, idx(rounds - 1), xor_host ? d_plan + npos : nullptr);
+    final_round<<<g, 256, 0, ctx->stream>>>(muls, k_last, (int)L, total, out_dev, idx(rounds - 1), xor_host ? d_plan + npos : nullptr, kidx, key_words);
     return post_launch(ctx, "aes_final_round_kernel");
 }
 
@@ -533,6 +546,118 @@ int aes_blocks_host(tac_ctx* ctx, int n_blocks, bool ct_in, const uint64_t* in_h
 int inv_key_sched_check(tac_ctx* ctx) {
     if (!ctx->inv_key_sched || !ctx->inv_key_sched_valid)
         return fail(ctx, TAC_ERR_STATE, "no inverse key schedule for the resident key schedule (tac_aes_inv_key_schedule or tac_aes_set_inv_key_schedule)");
+    return TAC_OK;
+}
+
+size_t key_sched_bytes(const tac_ctx* ctx) { return (size_t)44 * 32 * (ctx->big() + 1) * 8; }
+
+// room for n_keys schedules in a key table (contents not kept when it grows)
+int alloc_key_table(tac_ctx* ctx, DevBuf& b, int n_keys) {
+    const size_t bytes = (size_t)n_keys * key_sched_bytes(ctx);
+    if (b.cap >= bytes) return TAC_OK;
+    if (b.p) CU(cudaFree(b.p));
+    b.p = nullptr; b.cap = 0;
+    if (cudaMalloc(&b.p, bytes) != cudaSuccess) {
+        cudaGetLastError();          // clear the allocation error so that the next launch check does not report it
+        b.p = nullptr;
+        return fail(ctx, TAC_ERR_CUDA, "a key table of " + std::to_string(n_keys) + " schedules (" + std::to_string(bytes >> 20) +
+                                           " MiB) does not fit in device memory");
+    }
+    b.cap = bytes;
+    return TAC_OK;
+}
+
+// the resident key table (and, decrypting, its inverse table) and a key index in [0, n_keys) for every block, checked on
+// the host before anything is enqueued
+int key_table_check(tac_ctx* ctx, AesDir dir, int n_blocks, const int32_t* key_idx) {
+    if (ctx->n_keys < 1) return fail(ctx, TAC_ERR_STATE, "no key table on the device (tac_aes_key_table or tac_aes_set_key_table)");
+    if (dir == AesDir::Inverse && !ctx->inv_key_table_valid)
+        return fail(ctx, TAC_ERR_STATE, "no inverse key table for the resident key table (tac_aes_inv_key_table or tac_aes_set_inv_key_table)");
+    if (n_blocks > 0 && !key_idx) return fail(ctx, TAC_ERR_ARG, "NULL key index");
+    for (int b = 0; b < n_blocks; b++)
+        if (key_idx[b] < 0 || key_idx[b] >= ctx->n_keys)
+            return fail(ctx, TAC_ERR_ARG, "key index " + std::to_string(key_idx[b]) + " of block " + std::to_string(b) + " outside [0, " +
+                                              std::to_string(ctx->n_keys) + ")");
+    return TAC_OK;
+}
+
+int key_schedule_noise_check(tac_ctx* ctx) {
+    if (8 + 1 > ctx->p.max_noise_sq) return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: key schedule needs max_noise_level_squared >= 9");
+    return TAC_OK;
+}
+int inv_key_schedule_noise_check(tac_ctx* ctx) {
+    if (4 * 8 > ctx->p.max_noise_sq) return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: the inverse key schedule needs max_noise_level_squared >= 32");
+    return TAC_OK;
+}
+
+// fhe_sbox_gal_mul_pbs::key_schedule (:134-164) with boot_word (:166-180) and sub_word (:182-191) on the device, for K keys
+// at once: key_bits_host [K][128][kN+1] → ek [K][44 words][4][8][kN+1].  Each of the 40 steps bootstraps all K keys
+// together: sub_word is one pass over 4K bytes, boot_word one over 32K bits, and aes_key_step_kernel forms the sums of all
+// keys.  sub_word bootstraps w[i−1] as it is (the bootstrap of a byte does not depend on its neighbours in the batch) and
+// the step kernel reads it rotated, so w[i−1] of every key is used where the previous boot_word left it, contiguous.
+int key_expand(tac_ctx* ctx, int K, const uint64_t* key_bits_host, uint64_t* ek) {
+    TRY(ensure_aes_luts(ctx));
+    const size_t L = (size_t)ctx->big() + 1, byte = 8 * L, word = 4 * byte, sched = 44 * word;
+    TRY(ensure(ctx, ctx->ws_state, (size_t)K * 3 * word * 8));
+    uint64_t* prev = ctx->ws_state.as<uint64_t>();      // [K][word]: w[i−1] of every key
+    uint64_t* sub = prev + (size_t)K * word;             // [K][word]: SubWord(w[i−1])
+    uint64_t* acc = sub + (size_t)K * word;              // [K][word]: the sums boot_word bootstraps
+    CU(cudaMemcpy2DAsync(ek, sched * 8, key_bits_host, 4 * word * 8, 4 * word * 8, (size_t)K, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpy2DAsync(prev, word * 8, key_bits_host + 3 * word, 4 * word * 8, word * 8, (size_t)K, cudaMemcpyHostToDevice, ctx->stream));
+    // trivial(RC) constants: body += encode_bit(1) on the set bits of RC[i/4], byte 0 (:154; Byte::trivial data_model.rs:35-43).
+    // All ten rows are uploaded once per context, so the 40 steps below enqueue without a host synchronisation.
+    if (!ctx->rc_rows) {
+        static const uint8_t RC[11] = {0x00, 0x01, 0x02, 0x04, 0x08, 0x10, 0x20, 0x40, 0x80, 0x1B, 0x36};
+        std::vector<uint64_t> rows((size_t)10 * byte, 0ull);
+        for (int r = 1; r <= 10; r++)
+            for (int bit = 0; bit < 8; bit++)
+                if (RC[r] & (0x80 >> bit)) rows[(size_t)(r - 1) * byte + (size_t)bit * L + (L - 1)] = tac_encode_bit(1);
+        CU(cudaMalloc(&ctx->rc_rows, rows.size() * 8));
+        CU(cudaMemcpy(ctx->rc_rows, rows.data(), rows.size() * 8, cudaMemcpyHostToDevice));
+    }
+    const size_t total = (size_t)K * word;
+    for (int i = 4; i < 44; i++) {
+        const bool rot = i % 4 == 0;
+        if (rot) TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut8], 4 * K, prev, sub));                                  // sub_word
+        aes_key_step_kernel<<<grid1d(total, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ek, sched, i, rot ? sub : nullptr,
+                                                                                        ctx->rc_rows + (size_t)(i / 4 - 1) * byte, (int)L, total, acc);
+        TRY(post_launch(ctx, "aes_key_step_kernel"));
+        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut1], 32 * K, acc, prev));                                          // boot_word → bootstrap_assign
+        CU(cudaMemcpy2DAsync(ek + (size_t)i * word, sched * 8, prev, word * 8, word * 8, (size_t)K, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    return TAC_OK;
+}
+
+// inverse key schedules of K schedules w [K][44 words] → dk, same layout: dk[0..3] = w[0..3], dk[40..43] = w[40..43],
+// dk[4rd..4rd+3] = InvMixColumns(w[4rd..4rd+3]) for rd = 1..9.  One 8 → 32 circuit bootstrap (b·{14, 11, 13, 9}) of the
+// 144K key bytes, the InvMixColumns sums (squared noise 32), then one 1-bit bootstrap per sum bit back to level 1 (as
+// boot_word does in the forward key schedule).  Keys go in groups that fill one pipeline pass, which bounds the workspace.
+int inv_key_expand(tac_ctx* ctx, int K, const uint64_t* w, uint64_t* dk) {
+    TRY(ensure_aes_luts(ctx));
+    TRY(ensure_aes_inv_luts(ctx));
+    const size_t L = (size_t)ctx->big() + 1, byte = 8 * L, word = 4 * byte, sched = 44 * word, mid = 36 * word;
+    const int n_key_bytes = 9 * 16;                          // round keys 1..9
+    CU(cudaMemcpy2DAsync(dk, sched * 8, w, sched * 8, 4 * word * 8, (size_t)K, cudaMemcpyDeviceToDevice, ctx->stream));
+    CU(cudaMemcpy2DAsync(dk + 40 * word, sched * 8, w + 40 * word, sched * 8, 4 * word * 8, (size_t)K, cudaMemcpyDeviceToDevice, ctx->stream));
+    const int group = (int)std::max<size_t>(1, ctx->max_cts / (8 * (size_t)n_key_bytes));
+    for (int k0 = 0; k0 < K; k0 += group) {
+        const int nk = std::min(group, K - k0);
+        TRY(ensure(ctx, ctx->ws_in, (size_t)nk * mid * 8));
+        TRY(ensure(ctx, ctx->ws_muls, (size_t)nk * n_key_bytes * 32 * L * 8));
+        TRY(ensure(ctx, ctx->ws_state, (size_t)nk * n_key_bytes * byte * 8));
+        TRY(ensure(ctx, ctx->ws_out, (size_t)nk * mid * 8));
+        uint64_t* keys = ctx->ws_in.as<uint64_t>();          // [nk][36 words]: w[4..39] of the group
+        uint64_t* muls = ctx->ws_muls.as<uint64_t>();
+        uint64_t* sums = ctx->ws_state.as<uint64_t>();
+        uint64_t* bits = ctx->ws_out.as<uint64_t>();         // [nk][36 words]: dk[4..39] of the group
+        CU(cudaMemcpy2DAsync(keys, mid * 8, w + (size_t)k0 * sched + 4 * word, sched * 8, mid * 8, (size_t)nk, cudaMemcpyDeviceToDevice, ctx->stream));
+        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut_key32], nk * n_key_bytes, keys, muls));
+        const size_t total = (size_t)nk * n_key_bytes * byte;
+        aes_inv_mix_key_kernel<<<grid1d(total, 256, ctx->sm_count), 256, 0, ctx->stream>>>(muls, (int)L, total, sums);
+        TRY(post_launch(ctx, "aes_inv_mix_key_kernel"));
+        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut1], nk * n_key_bytes * 8, sums, bits));
+        CU(cudaMemcpy2DAsync(dk + (size_t)k0 * sched + 4 * word, sched * 8, bits, mid * 8, mid * 8, (size_t)nk, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
     return TAC_OK;
 }
 
@@ -584,7 +709,8 @@ void tac_ctx_destroy(tac_ctx* ctx) {
         if (p) cudaFree(p);
     for (auto& l : ctx->luts) cudaFree(l.dev);
     for (DevBuf* b : {&ctx->ws_in, &ctx->ws_out, &ctx->ws_small, &ctx->ws_ksdig, &ctx->ws_pbs, &ctx->ws_pfdig, &ctx->ws_ggsw, &ctx->ws_ggswf,
-                      &ctx->ws_tree_a, &ctx->ws_tree_b, &ctx->ws_state, &ctx->ws_muls, &ctx->ws_misc, &ctx->ws_plan, &ctx->ws_rep})
+                      &ctx->ws_tree_a, &ctx->ws_tree_b, &ctx->ws_state, &ctx->ws_muls, &ctx->ws_misc, &ctx->ws_plan, &ctx->ws_rep,
+                      &ctx->key_table, &ctx->inv_key_table})
         if (b->p) cudaFree(b->p);
     for (auto& r : ctx->prof_pool) for (auto& ev : r.ev) cudaEventDestroy(ev);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -915,7 +1041,7 @@ int tac_aes_encrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_no
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    return aes_blocks_dev(ctx, AesDir::Forward, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
+    return aes_blocks_dev(ctx, AesDir::Forward, ctx->key_sched, nullptr, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
 }
 int tac_aes_encrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host) {
     return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
@@ -927,7 +1053,7 @@ int tac_aes_encrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, co
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    return aes_blocks_dev(ctx, AesDir::Forward, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);   // trivial input: no noise of its own
+    return aes_blocks_dev(ctx, AesDir::Forward, ctx->key_sched, nullptr, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);   // trivial input: no noise of its own
 }
 int tac_aes_encrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
     return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
@@ -943,7 +1069,7 @@ int tac_aes_decrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_no
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     TRY(inv_key_sched_check(ctx));
-    return aes_blocks_dev(ctx, AesDir::Inverse, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
+    return aes_blocks_dev(ctx, AesDir::Inverse, ctx->inv_key_sched, nullptr, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
 }
 int tac_aes_decrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host) {
     return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
@@ -957,7 +1083,7 @@ int tac_aes_decrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, co
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     TRY(inv_key_sched_check(ctx));
-    return aes_blocks_dev(ctx, AesDir::Inverse, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);   // trivial input: no noise of its own
+    return aes_blocks_dev(ctx, AesDir::Inverse, ctx->inv_key_sched, nullptr, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);   // trivial input: no noise of its own
 }
 int tac_aes_decrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
     return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
@@ -965,35 +1091,16 @@ int tac_aes_decrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const 
     });
 }
 
-// inverse key schedule on the device from the resident encryption schedule: dk[0..3] = w[0..3], dk[40..43] = w[40..43],
-// dk[4rd..4rd+3] = InvMixColumns(w[4rd..4rd+3]) for rd = 1..9.  One 8 → 32 circuit bootstrap (b·{14, 11, 13, 9}) of the
-// 144 key bytes, the InvMixColumns sums (squared noise 32), then one 1-bit bootstrap per sum bit back to level 1 (as
-// boot_word does in the forward key schedule).
+// inverse key schedule on the device from the resident encryption schedule (inv_key_expand with one key)
 int tac_aes_inv_key_schedule(tac_ctx* ctx, uint64_t* out_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    if (4 * 8 > ctx->p.max_noise_sq) return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: the inverse key schedule needs max_noise_level_squared >= 32");
-    TRY(ensure_aes_luts(ctx));
-    TRY(ensure_aes_inv_luts(ctx));
-    const size_t L = (size_t)ctx->big() + 1, byte = 8 * L, word = 4 * byte, bytes = 44 * word * 8;
-    const int n_key_bytes = 9 * 16;                          // round keys 1..9
-    if (!ctx->inv_key_sched) CU(cudaMalloc(&ctx->inv_key_sched, bytes));
+    TRY(inv_key_schedule_noise_check(ctx));
+    if (!ctx->inv_key_sched) CU(cudaMalloc(&ctx->inv_key_sched, key_sched_bytes(ctx)));
     ctx->inv_key_sched_valid = false;
-    uint64_t* dk = ctx->inv_key_sched;
-    const uint64_t* w = ctx->key_sched;
-    TRY(ensure(ctx, ctx->ws_muls, (size_t)n_key_bytes * 32 * L * 8));
-    TRY(ensure(ctx, ctx->ws_state, (size_t)n_key_bytes * byte * 8));
-    CU(cudaMemcpyAsync(dk, w, 4 * word * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(dk + 40 * word, w + 40 * word, 4 * word * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-    uint64_t* muls = ctx->ws_muls.as<uint64_t>();
-    uint64_t* sums = ctx->ws_state.as<uint64_t>();
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut_key32], n_key_bytes, w + 4 * word, muls));
-    const size_t total = (size_t)n_key_bytes * byte;
-    aes_inv_mix_key_kernel<<<grid1d(total, 256, ctx->sm_count), 256, 0, ctx->stream>>>(muls, (int)L, total, sums);
-    TRY(post_launch(ctx, "aes_inv_mix_key_kernel"));
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut1], n_key_bytes * 8, sums, dk + 4 * word));
-    if (out_host) CU(cudaMemcpyAsync(out_host, dk, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    TRY(inv_key_expand(ctx, 1, ctx->key_sched, ctx->inv_key_sched));
+    if (out_host) CU(cudaMemcpyAsync(out_host, ctx->inv_key_sched, key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     ctx->inv_key_sched_valid = true;
     return TAC_OK;
@@ -1011,50 +1118,135 @@ int tac_aes_set_inv_key_schedule(tac_ctx* ctx, const uint64_t* dk_host) {
     return TAC_OK;
 }
 
-// fhe_sbox_gal_mul_pbs::key_schedule (:134-164) with boot_word (:166-180) and sub_word (:182-191) on the device
+// fhe_sbox_gal_mul_pbs::key_schedule (:134-164): key_expand with one key, into the single schedule
 int tac_aes_key_schedule(tac_ctx* ctx, const uint64_t* key_bits_host, uint64_t* out_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
-    if (8 + 1 > ctx->p.max_noise_sq) return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: key schedule needs max_noise_level_squared >= 9");
+    TRY(key_schedule_noise_check(ctx));
     TRY(ensure_aes_luts(ctx));
     TRY(tac_aes_set_key_schedule(ctx, nullptr));
-    const size_t L = (size_t)ctx->big() + 1, byte = 8 * L, word = 4 * byte;
-    uint64_t* ek = ctx->key_sched;
-    TRY(ensure(ctx, ctx->ws_state, 3 * word * 8));
-    uint64_t* rot = ctx->ws_state.as<uint64_t>();       // rotated previous word / its SBOX image
-    uint64_t* sub = rot + word;
-    uint64_t* acc = sub + word;
-    CU(cudaMemcpyAsync(ek, key_bits_host, 4 * word * 8, cudaMemcpyHostToDevice, ctx->stream));
-    // trivial(RC) constants: body += encode_bit(1) on the set bits of RC[i/4], byte 0 (:154; Byte::trivial data_model.rs:35-43).
-    // All ten rows are uploaded once per context, so the 40 steps below enqueue without a host synchronisation.
-    if (!ctx->rc_rows) {
-        static const uint8_t RC[11] = {0x00, 0x01, 0x02, 0x04, 0x08, 0x10, 0x20, 0x40, 0x80, 0x1B, 0x36};
-        std::vector<uint64_t> rows((size_t)10 * byte, 0ull);
-        for (int r = 1; r <= 10; r++)
-            for (int bit = 0; bit < 8; bit++)
-                if (RC[r] & (0x80 >> bit)) rows[(size_t)(r - 1) * byte + (size_t)bit * L + (L - 1)] = tac_encode_bit(1);
-        CU(cudaMalloc(&ctx->rc_rows, rows.size() * 8));
-        CU(cudaMemcpy(ctx->rc_rows, rows.data(), rows.size() * 8, cudaMemcpyHostToDevice));
-    }
-    for (int i = 4; i < 44; i++) {
-        uint64_t* cur = ek + (size_t)i * word;
-        const uint64_t* prev = ek + (size_t)(i - 1) * word;
-        const uint64_t* addend = prev;
-        if (i % 4 == 0) {
-            // rotate_left(1): bytes [1,2,3,0]
-            CU(cudaMemcpyAsync(rot, prev + byte, 3 * byte * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-            CU(cudaMemcpyAsync(rot + 3 * byte, prev, byte * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-            TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut8], 4, rot, sub));                                       // sub_word
-            TRY(tac_lwe_add_batch_dev(ctx, sub, ctx->rc_rows + (size_t)(i / 4 - 1) * byte, 8));
-            addend = sub;
-        }
-        CU(cudaMemcpyAsync(acc, ek + (size_t)(i - 4) * word, word * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-        TRY(tac_lwe_add_batch_dev(ctx, acc, addend, 32));
-        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut1], 32, acc, cur));                                          // boot_word → bootstrap_assign
-    }
-    if (out_host) CU(cudaMemcpyAsync(out_host, ek, 44 * word * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    TRY(key_expand(ctx, 1, key_bits_host, ctx->key_sched));
+    if (out_host) CU(cudaMemcpyAsync(out_host, ctx->key_sched, key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return TAC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ AES under many keys
+// A table of key schedules beside the single one.  Block b of a keyed call runs under entry key_idx[b]; its output equals,
+// word for word, the single-key entry point's for that block with that entry resident (every stage gives the same words
+// whatever the batch).
+int tac_aes_key_table(tac_ctx* ctx, int n_keys, const uint64_t* key_bits_host, uint64_t* key_scheds_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (n_keys < 1 || !key_bits_host) return fail(ctx, TAC_ERR_ARG, "need n_keys >= 1 and key bits");
+    TRY(key_schedule_noise_check(ctx));
+    ctx->n_keys = 0;
+    ctx->inv_key_table_valid = false;
+    TRY(alloc_key_table(ctx, ctx->key_table, n_keys));
+    TRY(key_expand(ctx, n_keys, key_bits_host, ctx->key_table.as<uint64_t>()));
+    if (key_scheds_host) CU(cudaMemcpyAsync(key_scheds_host, ctx->key_table.p, (size_t)n_keys * key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ctx->n_keys = n_keys;
+    return TAC_OK;
+}
+int tac_aes_set_key_table(tac_ctx* ctx, int n_keys, const uint64_t* key_scheds_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (n_keys < 1 || !key_scheds_host) return fail(ctx, TAC_ERR_ARG, "need n_keys >= 1 and key schedules");
+    ctx->n_keys = 0;
+    ctx->inv_key_table_valid = false;
+    TRY(alloc_key_table(ctx, ctx->key_table, n_keys));
+    CU(cudaMemcpyAsync(ctx->key_table.p, key_scheds_host, (size_t)n_keys * key_sched_bytes(ctx), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ctx->n_keys = n_keys;
+    return TAC_OK;
+}
+int tac_aes_inv_key_table(tac_ctx* ctx, uint64_t* inv_key_scheds_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (ctx->n_keys < 1) return fail(ctx, TAC_ERR_STATE, "no key table on the device (tac_aes_key_table or tac_aes_set_key_table)");
+    TRY(inv_key_schedule_noise_check(ctx));
+    ctx->inv_key_table_valid = false;
+    TRY(alloc_key_table(ctx, ctx->inv_key_table, ctx->n_keys));
+    TRY(inv_key_expand(ctx, ctx->n_keys, ctx->key_table.as<uint64_t>(), ctx->inv_key_table.as<uint64_t>()));
+    if (inv_key_scheds_host)
+        CU(cudaMemcpyAsync(inv_key_scheds_host, ctx->inv_key_table.p, (size_t)ctx->n_keys * key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ctx->inv_key_table_valid = true;
+    return TAC_OK;
+}
+int tac_aes_set_inv_key_table(tac_ctx* ctx, const uint64_t* inv_key_scheds_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (ctx->n_keys < 1) return fail(ctx, TAC_ERR_STATE, "no key table on the device (tac_aes_key_table or tac_aes_set_key_table)");
+    if (!inv_key_scheds_host) return fail(ctx, TAC_ERR_ARG, "NULL inverse key schedules");
+    ctx->inv_key_table_valid = false;
+    TRY(alloc_key_table(ctx, ctx->inv_key_table, ctx->n_keys));
+    CU(cudaMemcpyAsync(ctx->inv_key_table.p, inv_key_scheds_host, (size_t)ctx->n_keys * key_sched_bytes(ctx), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ctx->inv_key_table_valid = true;
+    return TAC_OK;
+}
+
+int tac_aes_encrypt_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_dev,
+                                     uint64_t* out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    TRY(key_table_check(ctx, AesDir::Forward, n_blocks, key_idx_host));
+    return aes_blocks_dev(ctx, AesDir::Forward, ctx->key_table.as<uint64_t>(), key_idx_host, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
+}
+int tac_aes_encrypt_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_host,
+                                 uint64_t* out_host) {
+    LOCK(ctx);
+    TRY(key_table_check(ctx, AesDir::Forward, n_blocks, key_idx_host));
+    return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
+        return tac_aes_encrypt_blocks_keyed_dev(ctx, n_blocks, rounds, in_noise_sq, key_idx_host, in, out);
+    });
+}
+int tac_aes_encrypt_public_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
+                                            const uint8_t* xor_host, uint64_t* out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    TRY(key_table_check(ctx, AesDir::Forward, n_blocks, key_idx_host));
+    return aes_blocks_dev(ctx, AesDir::Forward, ctx->key_table.as<uint64_t>(), key_idx_host, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);
+}
+int tac_aes_encrypt_public_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
+                                        const uint8_t* xor_host, uint64_t* out_host) {
+    LOCK(ctx);
+    TRY(key_table_check(ctx, AesDir::Forward, n_blocks, key_idx_host));
+    return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
+        return tac_aes_encrypt_public_blocks_keyed_dev(ctx, n_blocks, rounds, key_idx_host, blocks_host, xor_host, out);
+    });
+}
+int tac_aes_decrypt_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_dev,
+                                     uint64_t* out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    TRY(key_table_check(ctx, AesDir::Inverse, n_blocks, key_idx_host));
+    return aes_blocks_dev(ctx, AesDir::Inverse, ctx->inv_key_table.as<uint64_t>(), key_idx_host, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
+}
+int tac_aes_decrypt_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_host,
+                                 uint64_t* out_host) {
+    LOCK(ctx);
+    TRY(key_table_check(ctx, AesDir::Inverse, n_blocks, key_idx_host));
+    return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
+        return tac_aes_decrypt_blocks_keyed_dev(ctx, n_blocks, rounds, in_noise_sq, key_idx_host, in, out);
+    });
+}
+int tac_aes_decrypt_public_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
+                                            const uint8_t* xor_host, uint64_t* out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    TRY(key_table_check(ctx, AesDir::Inverse, n_blocks, key_idx_host));
+    return aes_blocks_dev(ctx, AesDir::Inverse, ctx->inv_key_table.as<uint64_t>(), key_idx_host, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);
+}
+int tac_aes_decrypt_public_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
+                                        const uint8_t* xor_host, uint64_t* out_host) {
+    LOCK(ctx);
+    TRY(key_table_check(ctx, AesDir::Inverse, n_blocks, key_idx_host));
+    return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
+        return tac_aes_decrypt_public_blocks_keyed_dev(ctx, n_blocks, rounds, key_idx_host, blocks_host, xor_host, out);
+    });
 }
 
 // ------------------------------------------------------------------------------------------------ single stages

@@ -7,7 +7,7 @@
 //   aes_*_kernel           AddRoundKey / (Inv)ShiftRows+(Inv)MixColumns+AddRoundKey / final round as gather-adds on the flat
 //                          state (aes_mix_columns_kernel and aes_final_round_kernel templated on the direction); round-1
 //                          inputs and representative gathers of the public-block path; InvMixColumns of the inverse key
-//                          schedule (aes_inv_mix_key_kernel)
+//                          schedule (aes_inv_mix_key_kernel); the sums of a batched key-expansion step (aes_key_step_kernel)
 //   lwe_add_kernel         leveled XOR (lwe_ciphertext_add_assign) over a batch; lwe_shl_kernel / lwe_sub_kernel: glue of extract_bits
 //   negate_kernel, dfma_peak_kernel   key-upload helper, FP64 peak microbenchmark (roofline denominator)
 #pragma once
@@ -90,11 +90,18 @@ lwe_gemm_kernel(const uint32_t* __restrict__ dig, int nct, int Kd, const uint64_
 
 // ================================================================================================ AES linear layers
 // flat state: [block][byte = 4·col + row][bit, MSB first][L]   (reference data_model.rs:165-188 re-expressed)
+// Round keys of block b: rk, or rk + kidx[b]·key_words when a per-block key index is given (AES under many keys: rk points
+// into entry 0 of a table of key schedules `key_words` apart).
+__device__ __forceinline__ const uint64_t* aes_block_key(const uint64_t* rk, const int32_t* kidx, size_t key_words, size_t blk) {
+    return kidx ? rk + (size_t)kidx[blk] * key_words : rk;
+}
 // AddRoundKey (data_model.rs:270-274): out = in + rk, rk broadcast over blocks
 __global__ void aes_add_round_key_kernel(const uint64_t* __restrict__ in, const uint64_t* __restrict__ rk, size_t blk_words, size_t total,
-                                         uint64_t* __restrict__ out) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x)
-        out[i] = in[i] + rk[i % blk_words];
+                                         uint64_t* __restrict__ out, const int32_t* __restrict__ kidx, size_t key_words) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t blk = i / blk_words;
+        out[i] = in[i] + aes_block_key(rk, kidx, key_words, blk)[i - blk * blk_words];
+    }
 }
 // ShiftRows + MixColumns + AddRoundKey of a middle round as one gather-add over the S-box rows; Fwd = false is InvShiftRows +
 // InvMixColumns of the equivalent inverse cipher (FIPS-197 §5.3.5, round keys from dk):
@@ -102,17 +109,18 @@ __global__ void aes_add_round_key_kernel(const uint64_t* __restrict__ in, const 
 //   forward  coef = {2, 3, 1, 1}      muls rows [24 = (S, 2S, 3S) × 8 bits][L]               (fhe_sbox_gal_mul_pbs.rs:61-82, :106-117)
 //   inverse  coef = {14, 11, 13, 9}   muls rows [32 = (14, 11, 13, 9)·InvS × 8 bits][L]
 // row = block·16 + byte, or idx[block·16 + byte] when idx is given (a compact batch of S-box outputs shared by several
-// positions: AES over public blocks)
+// positions: AES over public blocks); round keys per block as in aes_add_round_key_kernel
 template <bool Fwd>
 __global__ void aes_mix_columns_kernel(const uint64_t* __restrict__ muls, const uint64_t* __restrict__ rk, int L, size_t total,
-                                       uint64_t* __restrict__ state, const int32_t* __restrict__ idx) {
+                                       uint64_t* __restrict__ state, const int32_t* __restrict__ idx, const int32_t* __restrict__ kidx,
+                                       size_t key_words) {
     constexpr int W = Fwd ? 24 : 32;
     const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
         const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;   // bit·L + e
         const int c = byte >> 2, r = byte & 3;
-        uint64_t v = rk[rem];
+        uint64_t v = aes_block_key(rk, kidx, key_words, blk)[rem];
 #pragma unroll
         for (int rr = 0; rr < 4; rr++) {
             const int d = (rr - r) & 3;
@@ -126,11 +134,12 @@ __global__ void aes_mix_columns_kernel(const uint64_t* __restrict__ muls, const 
 }
 // last round (fhe_sbox_gal_mul_pbs.rs:119-129): ShiftRows(S) + w[40..43], or InvShiftRows(InvS) + dk[0..3].  sub rows
 // [row][8 bits][L] (idx optional, as in aes_mix_columns_kernel).  xr: NULL, or [block][16] public bytes XORed into the
-// output (a trivial ciphertext added: encode_bit(1) = 2^63 on the body of every set bit).
+// output (a trivial ciphertext added: encode_bit(1) = 2^63 on the body of every set bit).  Round keys per block as in
+// aes_add_round_key_kernel.
 template <bool Fwd>
 __global__ void aes_final_round_kernel(const uint64_t* __restrict__ sub, const uint64_t* __restrict__ rk, int L, size_t total,
                                        uint64_t* __restrict__ out, const int32_t* __restrict__ idx,
-                                       const uint8_t* __restrict__ xr) {
+                                       const uint8_t* __restrict__ xr, const int32_t* __restrict__ kidx, size_t key_words) {
     const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t blk = i / blk_words; const size_t rem = i - blk * blk_words;
@@ -138,7 +147,7 @@ __global__ void aes_final_round_kernel(const uint64_t* __restrict__ sub, const u
         const int c = byte >> 2, r = byte & 3;
         const int old_byte = 4 * ((Fwd ? c + r : c - r) & 3) + r;
         const size_t src_row = idx ? (size_t)idx[blk * 16 + old_byte] : blk * 16 + old_byte;
-        uint64_t v = sub[src_row * byte_words + w] + rk[rem];
+        uint64_t v = sub[src_row * byte_words + w] + aes_block_key(rk, kidx, key_words, blk)[rem];
         if (xr) {
             const int bit = (int)(w / L);
             if (w - (size_t)bit * L == (size_t)L - 1 && (xr[blk * 16 + byte] & (0x80 >> bit))) v += 1ull << 63;
@@ -148,15 +157,16 @@ __global__ void aes_final_round_kernel(const uint64_t* __restrict__ sub, const u
 }
 // S-box inputs of round 1 over public blocks, one per representative k: k0[byte] + trivial(value), i.e. the key-schedule
 // byte with encode_bit(1) = 2^63 added to the body of every set bit of the public byte (Byte::trivial, data_model.rs:35-43).
-// rep_pos[k] = block·16 + byte (NULL: k itself); out [k][8 bits][L]
+// rep_pos[k] = block·16 + byte (NULL: k itself); out [k][8 bits][L].  The key is the one of the representative's block
+// (kidx as in aes_add_round_key_kernel; positions that share a representative share its key, aes_plan.h).
 __global__ void aes_public_round1_kernel(const uint64_t* __restrict__ k0, const uint8_t* __restrict__ blocks, const int32_t* __restrict__ rep_pos,
-                                         int L, size_t total, uint64_t* __restrict__ out) {
+                                         int L, size_t total, uint64_t* __restrict__ out, const int32_t* __restrict__ kidx, size_t key_words) {
     const size_t byte_words = (size_t)8 * L;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t k = i / byte_words; const size_t w = i - k * byte_words;
         const int pos = rep_pos ? rep_pos[k] : (int)k;
         const int bit = (int)(w / L);
-        uint64_t v = k0[(size_t)(pos & 15) * byte_words + w];
+        uint64_t v = aes_block_key(k0, kidx, key_words, (size_t)(pos >> 4))[(size_t)(pos & 15) * byte_words + w];
         if (w - (size_t)bit * L == (size_t)L - 1 && (blocks[pos] & (0x80 >> bit))) v += 1ull << 63;
         out[i] = v;
     }
@@ -174,6 +184,27 @@ __global__ void aes_inv_mix_key_kernel(const uint64_t* __restrict__ muls, int L,
 #pragma unroll
         for (int rr = 0; rr < 4; rr++) v += muls[((blk * 16 + 4 * c + rr) * 32 + (size_t)((rr - r) & 3) * 8) * L + w];
         out[i] = v;
+    }
+}
+// one step i (4 <= i < 44) of the key expansion over K schedules ek [K][44 words][4 bytes][8 bits][L] (sched_words apart):
+//   acc[k] = w[i−4] + RotWord(sub[k]) + trivial(RC)   when sub is given (i % 4 == 0: sub[k] = SubWord(w[i−1]), unrotated)
+//   acc[k] = w[i−4] + w[i−1]                          otherwise
+// rc: the 8 ciphertexts of trivial(RC[i/4]) added to byte 0; acc [K][4][8][L], bootstrapped back to level 1 by the caller
+__global__ void aes_key_step_kernel(const uint64_t* __restrict__ ek, size_t sched_words, int i, const uint64_t* __restrict__ sub,
+                                    const uint64_t* __restrict__ rc, int L, size_t total, uint64_t* __restrict__ acc) {
+    const size_t byte_words = (size_t)8 * L, word = 4 * byte_words;
+    for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+        const size_t k = t / word; const size_t w = t - k * word;
+        const uint64_t* e = ek + k * sched_words;
+        uint64_t v = e[(size_t)(i - 4) * word + w];
+        if (sub) {
+            const int byte = (int)(w / byte_words);
+            v += sub[k * word + (size_t)((byte + 1) & 3) * byte_words + (w - (size_t)byte * byte_words)];   // rotate_left(1): bytes [1,2,3,0]
+            if (byte == 0) v += rc[w];
+        } else {
+            v += e[(size_t)(i - 1) * word + w];
+        }
+        acc[t] = v;
     }
 }
 // the representatives' S-box inputs out of the full state: out[k] = state[rep_pos[k]], 8·L words each

@@ -407,10 +407,41 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
                                                                        const std::vector<std::array<uint8_t, 16>>& xor_bytes = {}) {
         return public_blocks(tac_aes_decrypt_public_blocks, c, blocks, rounds, xor_bytes);
     }
+    // AES under many keys (the reference has none): batched key expansion of FHE-encrypted keys into the resident key table,
+    // beside the single key schedule above; inv_key_table derives the table's inverse schedules for the keyed decryption
+    static void key_table(const Ctx& c, const std::vector<std::array<Byte, 16>>& keys) {
+        const size_t L = c.lwe_size();
+        std::vector<uint64_t> bits(keys.size() * 128 * L);
+        for (size_t k = 0; k < keys.size(); k++) for (int b = 0; b < 16; b++) for (int i = 0; i < 8; i++)
+            std::copy(keys[k][b][i].ct.begin(), keys[k][b][i].ct.end(), bits.begin() + ((k * 16 + b) * 8 + i) * L);
+        c.check(tac_aes_key_table(c.raw(), (int)keys.size(), bits.data(), nullptr));
+    }
+    static void inv_key_table(const Ctx& c) { c.check(tac_aes_inv_key_table(c.raw(), nullptr)); }
+    // encrypt_public_blocks / decrypt_public_blocks with block q under key table entry key_idx[q] (transciphering for many
+    // senders in one call)
+    static std::vector<data_model::BlockT<Bit>> encrypt_public_blocks_keyed(const Ctx& c, const std::vector<int32_t>& key_idx,
+                                                                             const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
+                                                                             const std::vector<std::array<uint8_t, 16>>& xor_bytes = {}) {
+        return public_blocks_keyed(tac_aes_encrypt_public_blocks_keyed, c, key_idx, blocks, rounds, xor_bytes);
+    }
+    static std::vector<data_model::BlockT<Bit>> decrypt_public_blocks_keyed(const Ctx& c, const std::vector<int32_t>& key_idx,
+                                                                             const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
+                                                                             const std::vector<std::array<uint8_t, 16>>& xor_bytes = {}) {
+        return public_blocks_keyed(tac_aes_decrypt_public_blocks_keyed, c, key_idx, blocks, rounds, xor_bytes);
+    }
 
 private:
-    // fn (tac_aes_{en,de}crypt_public_blocks) over the blocks; outputs are bit ciphertexts of squared noise level 9
-    static std::vector<data_model::BlockT<Bit>> public_blocks(int (*fn)(tac_ctx*, int, int, const uint8_t*, const uint8_t*, uint64_t*), const Ctx& c,
+    static std::vector<data_model::BlockT<Bit>> public_blocks_keyed(int (*fn)(tac_ctx*, int, int, const int32_t*, const uint8_t*, const uint8_t*, uint64_t*),
+                                                                    const Ctx& c, const std::vector<int32_t>& key_idx,
+                                                                    const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
+                                                                    const std::vector<std::array<uint8_t, 16>>& xor_bytes) {
+        if (key_idx.size() != blocks.size()) throw std::invalid_argument("key_idx: one key index per block");
+        return public_blocks([&](tac_ctx* ctx, int n, int r, const uint8_t* b, const uint8_t* x, uint64_t* o) { return fn(ctx, n, r, key_idx.data(), b, x, o); },
+                             c, blocks, rounds, xor_bytes);
+    }
+    // fn (tac_aes_{en,de}crypt_public_blocks[_keyed]) over the blocks; outputs are bit ciphertexts of squared noise level 9
+    template <class Fn>
+    static std::vector<data_model::BlockT<Bit>> public_blocks(Fn fn, const Ctx& c,
                                                               const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
                                                               const std::vector<std::array<uint8_t, 16>>& xor_bytes) {
         if (!xor_bytes.empty() && xor_bytes.size() != blocks.size()) throw std::invalid_argument("xor_bytes: one row per block");
