@@ -243,6 +243,39 @@ int tac_aes_decrypt_public_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int roun
  * negative index.  Host only. */
 int tac_aes_public_plan_keyed(int n_blocks, int rounds, int decrypt, const int32_t* key_idx, const uint8_t* blocks_host /*[n][16]*/, int64_t* boxes);
 
+/* ------------------------------------------------------------------ AES-CCM transciphering (no counterpart in the reference) */
+/* One AES-CCM record (NIST SP 800-38C, RFC 3610; AES-128, 10 rounds): nonce N of 7..13 bytes (q = 15 − |N|), public
+ * associated data A, data = C ‖ U with C the ciphertext of p = data_len − tag_len bytes and U the received tag of tag_len
+ * bytes, tag_len in {4, 6, 8, 10, 12, 14, 16}.  This is what AES-CCM encryption of (N, P, A) returns. */
+typedef struct tac_ccm_msg {
+    const uint8_t* nonce;
+    int32_t nonce_len;
+    int32_t tag_len;
+    const uint8_t* aad;
+    uint64_t aad_len;
+    const uint8_t* data;
+    uint64_t data_len;
+} tac_ccm_msg;
+/* AES-CCM transciphering with the tag checked under FHE.  For every message: the FHE plaintext bits of C (as
+ * tac_aes_encrypt_public_blocks over the counter blocks A_1..A_m with XOR bytes C gives them, squared noise 9) and one
+ * encrypted VALIDITY BIT, 1 exactly when U is the CBC-MAC tag of (N, A, P) under the FHE-encrypted key (squared noise 2).
+ * The CBC-MAC chain runs over the FHE plaintext on the encrypted-block path, batched across messages; the tag is compared
+ * homomorphically.  key_idx NULL: every message under the single resident schedule; else message i under key table entry
+ * key_idx[i].  pt_out [Σ (data_len − tag_len)][8][kN+1] in message order, valid_out [n_msgs][kN+1].
+ * Errors, all before anything is enqueued: TAC_ERR_ARG for n_msgs < 0, a nonce length outside 7..13, a tag length not in
+ * the set, data_len < tag_len, a payload of 2^(8q) bytes or more, a NULL pointer with a non-zero length, a key index
+ * outside [0, n_keys); TAC_ERR_STATE without evaluation keys or without the schedule / key table; TAC_ERR_NOISE below
+ * max_noise_level_squared 33 (lvl_64 and lvl_256 suffice). */
+int tac_aes_ccm_transcipher(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_host,
+                            uint64_t* valid_out_host);
+/* the same with device outputs, enqueued on the context's stream (messages and key indices are host memory) */
+int tac_aes_ccm_transcipher_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_dev,
+                                uint64_t* valid_out_dev);
+/* The public blocks of one message.  ctr_blocks: A_0..A_m (m = ceil(p/16)); mac_blocks: B_0, the AAD blocks (length prefix,
+ * A, zero padding), then m payload blocks of zeros, which stand for the FHE plaintext the chain adds.  counts = {m + 1,
+ * CBC-MAC blocks}; NULL ctr_blocks / mac_blocks query the counts only.  TAC_ERR_ARG as tac_aes_ccm_transcipher.  Host only. */
+int tac_aes_ccm_format(const tac_ccm_msg* msg, uint8_t* ctr_blocks, uint8_t* mac_blocks, int64_t counts[2]);
+
 /* ------------------------------------------------------------------ single stages (parity tests, profiling) */
 /* [U] keyswitch_lwe_ciphertext: [n_cts][kN+1] → [n_cts][n+1] */
 int tac_stage_keyswitch(tac_ctx* ctx, int n_cts, const uint64_t* in_host, uint64_t* out_host);

@@ -41,6 +41,19 @@ pub struct tac_client_key {
     _private: [u8; 0],
 }
 
+/// One AES-CCM record (NIST SP 800-38C): `data` = C ‖ U, the ciphertext and the received tag of `tag_len` bytes
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct tac_ccm_msg {
+    pub nonce: *const u8,
+    pub nonce_len: i32,
+    pub tag_len: i32,
+    pub aad: *const u8,
+    pub aad_len: u64,
+    pub data: *const u8,
+    pub data_len: u64,
+}
+
 extern "C" {
     // parameters, encodings, LUTs
     pub fn tac_params_preset(id: c_int, out: *mut tac_params) -> c_int;
@@ -123,6 +136,12 @@ extern "C" {
     pub fn tac_aes_decrypt_public_blocks_keyed(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, key_idx_host: *const i32, blocks_host: *const u8, xor_host: *const u8, out_host: *mut u64) -> c_int;
     pub fn tac_aes_decrypt_public_blocks_keyed_dev(ctx: *mut tac_ctx, n_blocks: c_int, rounds: c_int, key_idx_host: *const i32, blocks_host: *const u8, xor_host: *const u8, out_dev: *mut u64) -> c_int;
     pub fn tac_aes_public_plan_keyed(n_blocks: c_int, rounds: c_int, decrypt: c_int, key_idx: *const i32, blocks_host: *const u8, boxes: *mut i64) -> c_int;
+    // AES-CCM transciphering with the tag checked under FHE (no counterpart in the reference)
+    pub fn tac_aes_ccm_transcipher(ctx: *mut tac_ctx, n_msgs: c_int, key_idx: *const i32, msgs: *const tac_ccm_msg, pt_out_host: *mut u64,
+                                   valid_out_host: *mut u64) -> c_int;
+    pub fn tac_aes_ccm_transcipher_dev(ctx: *mut tac_ctx, n_msgs: c_int, key_idx: *const i32, msgs: *const tac_ccm_msg, pt_out_dev: *mut u64,
+                                       valid_out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_ccm_format(msg: *const tac_ccm_msg, ctr_blocks: *mut u8, mac_blocks: *mut u8, counts: *mut i64) -> c_int;
 
     // single stages, profiling
     pub fn tac_stage_keyswitch(ctx: *mut tac_ctx, n_cts: c_int, in_host: *const u64, out_host: *mut u64) -> c_int;

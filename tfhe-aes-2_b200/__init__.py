@@ -122,6 +122,9 @@ _SIGNATURES = {
     "tac_aes_decrypt_public_blocks_keyed": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_aes_decrypt_public_blocks_keyed_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_aes_public_plan_keyed": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_ccm_transcipher": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_ccm_transcipher_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_ccm_format": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_stage_keyswitch": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
     "tac_extract_bits": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _u64p, _u64p]),
     "tac_stage_pbs": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
@@ -287,6 +290,57 @@ def aes_public_plan(blocks, rounds=10, decrypt=False, key_index=None):
     if rc != 0:
         raise ValueError(f"aes_public_plan: rounds must be in 1..10 and key indices non-negative (error {rc})")
     return [int(v) for v in out]
+
+
+CCM_TAG_LENGTHS = (4, 6, 8, 10, 12, 14, 16)
+
+
+class CcmMsg(C.Structure):
+    """one AES-CCM record, layout of `tac_ccm_msg`: data = C ‖ U (ciphertext, then the received tag)"""
+    _fields_ = [
+        ("nonce", C.c_void_p), ("nonce_len", C.c_int32), ("tag_len", C.c_int32),
+        ("aad", C.c_void_p), ("aad_len", C.c_uint64),
+        ("data", C.c_void_p), ("data_len", C.c_uint64),
+    ]
+
+
+def _ccm_messages(messages):
+    """(CcmMsg array, the byte strings it points into, payload length of every message) from [(nonce, data, tag_len, aad)];
+    ValueError for every argument the C entry points reject with TAC_ERR_ARG"""
+    msgs = (CcmMsg * max(1, len(messages)))()
+    keep, sizes = [], []
+    for i, (nonce, data, tag_len, aad) in enumerate(messages):
+        nonce, data, aad = bytes(nonce), bytes(data), bytes(aad)
+        if not 7 <= len(nonce) <= 13:
+            raise ValueError(f"AES-CCM message {i}: the nonce must be 7..13 bytes, not {len(nonce)}")
+        if not isinstance(tag_len, (int, np.integer)) or int(tag_len) not in CCM_TAG_LENGTHS:
+            raise ValueError(f"AES-CCM message {i}: tag length {tag_len!r} not in {CCM_TAG_LENGTHS}")
+        tag_len = int(tag_len)
+        if len(data) < tag_len:
+            raise ValueError(f"AES-CCM message {i}: {len(data)} data bytes cannot hold a {tag_len}-byte tag")
+        q, p = 15 - len(nonce), len(data) - tag_len
+        if q < 8 and p >> (8 * q):
+            raise ValueError(f"AES-CCM message {i}: a payload of {p} bytes does not fit the {q}-byte length field of a {len(nonce)}-byte nonce")
+        keep += [nonce, data, aad]
+        ptr = lambda b: C.cast(C.c_char_p(b), C.c_void_p).value
+        msgs[i] = CcmMsg(ptr(nonce), len(nonce), tag_len, ptr(aad), len(aad), ptr(data), len(data))
+        sizes.append(p)
+    return msgs, keep, sizes
+
+
+def aes_ccm_format(nonce, data, tag_len=16, aad=b""):
+    """the public blocks of one AES-CCM record (NIST SP 800-38C): (counter blocks A_0..A_m [m+1][16], CBC-MAC blocks
+    [B_0, AAD blocks, m zero blocks that stand for the plaintext] [n][16]) as uint8 arrays; data = C ‖ U.  Host only."""
+    msgs, keep, _ = _ccm_messages([(nonce, data, tag_len, aad)])
+    L = load_library()
+    counts = np.zeros(2, dtype=np.int64)
+    if L.tac_aes_ccm_format(C.addressof(msgs[0]), None, None, counts.ctypes.data) != 0:
+        raise ValueError("aes_ccm_format: bad arguments")
+    ctr = np.zeros((int(counts[0]), 16), dtype=np.uint8)
+    mac = np.zeros((int(counts[1]), 16), dtype=np.uint8)
+    if L.tac_aes_ccm_format(C.addressof(msgs[0]), ctr.ctypes.data, mac.ctypes.data, counts.ctypes.data) != 0:
+        raise ValueError("aes_ccm_format: bad arguments")
+    return ctr, mac
 
 
 class LookupTable:
@@ -878,6 +932,33 @@ class FheContext(NoiseContext):
             return []
         out = self.aes_decrypt_public_blocks_keyed(b"".join(blocks), k, xor=b"".join(xor))
         return self._split_messages(out, sizes)
+
+    # -- AES-CCM transciphering with the tag checked under FHE
+    def aes_ccm_transcipher(self, nonce, data, tag_len=16, aad=b""):
+        """Transciphering of one AES-CCM record under the resident key schedule: `data` = C ‖ U is what AES-CCM encryption
+        of (nonce, P, aad) returns, with a tag of tag_len bytes.  Returns (FHE encryptions of the plaintext bits
+        [len(data) − tag_len][8][big+1], an encrypted validity bit [big+1]: 1 exactly when the tag is genuine).  The
+        plaintext comes back whatever the tag; acting on the validity bit is the caller's business."""
+        return self._aes_ccm([(nonce, data, tag_len, aad)], None)[0]
+
+    def aes_ccm_transcipher_many(self, messages):
+        """aes_ccm_transcipher for many senders in one call: messages = [(key_index, nonce, data, tag_len, aad)], each
+        under key table entry key_index.  Returns one (plaintext bits, validity bit) pair per message."""
+        messages = list(messages)
+        k = _key_index([m[0] for m in messages], len(messages), self.n_keys)
+        return self._aes_ccm([m[1:] for m in messages], k)
+
+    def _aes_ccm(self, messages, key_index):
+        msgs, keep, sizes = _ccm_messages(messages)
+        if not sizes:
+            return []
+        L1 = self.params.big_lwe_size
+        pt = np.empty((sum(sizes), 8, L1), dtype=np.uint64)
+        valid = np.empty((len(sizes), L1), dtype=np.uint64)
+        self._check(self.L.tac_aes_ccm_transcipher(self.h, len(sizes), None if key_index is None else key_index.ctypes.data, msgs,
+                                                   pt.ctypes.data, valid.ctypes.data))
+        offs = np.cumsum([0] + sizes)
+        return [(pt[offs[i]:offs[i + 1]], valid[i]) for i in range(len(sizes))]
 
     def _split_messages(self, out, sizes):
         """[n][16][8][big+1] of whole blocks → one [size][8][big+1] array per message (each padded to whole blocks)"""

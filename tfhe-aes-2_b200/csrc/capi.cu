@@ -4,6 +4,7 @@
 #include "../../include/tfhe_aes_cuda.h"
 #include "kernels_common.cuh"
 #include "aes_plan.h"
+#include "aes_ccm.h"
 #include "kernels_gemm_umma.cuh"
 #include "ep_step.cuh"
 #include "shape_launch.h"
@@ -85,6 +86,7 @@ struct tac_ctx {
     std::vector<Lut> luts;
     int aes_lut24 = -1, aes_lut8 = -1, aes_lut1 = -1;
     int aes_lut_inv32 = -1, aes_lut_inv8 = -1, aes_lut_key32 = -1;   // decryption: InvS·{14,11,13,9}, InvS, b·{14,11,13,9}
+    int ccm_lut_zero8 = -1, ccm_lut_ones8 = -1, ccm_lut_ones2 = -1;   // AES-CCM tag check: byte == 0, 8 bits all 1, 2 bits all 1
     // AES key schedule
     uint64_t* key_sched = nullptr;
     uint64_t* inv_key_sched = nullptr;   // equivalent inverse cipher's schedule dk, same layout [44 words][4][8][kN+1]
@@ -98,6 +100,9 @@ struct tac_ctx {
     // workspace
     DevBuf ws_in, ws_out, ws_small, ws_ksdig, ws_pbs, ws_pfdig, ws_ggsw, ws_ggswf, ws_tree_a, ws_tree_b, ws_state, ws_muls, ws_misc;
     DevBuf ws_plan, ws_rep;          // public-block AES: uploaded plan tables / public bytes, compact S-box inputs
+    // AES-CCM, apart from the buffers aes_blocks_dev reuses on every call: the public call's output (rows 0..n−1 are the
+    // CBC-MAC chain state), the chain input / tag check, and the descriptors of all steps
+    DevBuf ccm_pub, ccm_work, ccm_desc;
     size_t max_cts = 16384;
     uint32_t fix_cap = kFixCap;      // capacity of the PFKS tie list in use (TAC_FIX_CAP lowers it: exercises the overflow path)
     // profiling: one event tuple per pipeline pass, recorded without synchronising; read back by tac_ctx_stage_times
@@ -661,6 +666,106 @@ int inv_key_expand(tac_ctx* ctx, int K, const uint64_t* w, uint64_t* dk) {
     return TAC_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ AES-CCM
+// LUTs of the tag check, registered on the first AES-CCM call: 8 → 1 "byte is zero", 8 → 1 "all 8 bits set", 2 → 1 "both set"
+int ensure_ccm_luts(tac_ctx* ctx) {
+    if (ctx->ccm_lut_ones2 >= 0) return TAC_OK;
+    std::vector<uint64_t> f(256);
+    for (int v = 0; v < 256; v++) f[v] = v == 0;
+    TRY(register_aes_lut(ctx, 8, 1, f.data(), &ctx->ccm_lut_zero8));
+    for (int v = 0; v < 256; v++) f[v] = v == 255;
+    TRY(register_aes_lut(ctx, 8, 1, f.data(), &ctx->ccm_lut_ones8));
+    const uint64_t both[4] = {0, 0, 0, 1};
+    return register_aes_lut(ctx, 2, 1, both, &ctx->ccm_lut_ones2);
+}
+
+// everything an AES-CCM call checks on the host before it enqueues anything; Σ p into *pt_bytes
+int ccm_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_bytes) {
+    if (n_msgs < 0) return fail(ctx, TAC_ERR_ARG, "negative n_msgs");
+    if (n_msgs > 0 && !msgs) return fail(ctx, TAC_ERR_ARG, "NULL messages");
+    *pt_bytes = 0;
+    for (int c = 0; c < n_msgs; c++) {
+        CcmShape s;
+        if (ccm_shape(msgs[c], s))
+            return fail(ctx, TAC_ERR_ARG, "AES-CCM message " + std::to_string(c) + ": need a nonce of 7..13 bytes, a tag length in {4, 6, …, 16}, "
+                                          "data_len >= tag_len, a payload below 2^(8q) bytes and no NULL pointer with a non-zero length");
+        *pt_bytes += s.p;
+    }
+    TRY(aes_noise_check(ctx, 18, 10));           // a chain input X ⊕ P carries 18; a middle round 33
+    if (key_idx) {
+        TRY(key_table_check(ctx, AesDir::Forward, n_msgs, key_idx));
+    } else if (!ctx->key_sched) {
+        return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
+    }
+    if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
+    return TAC_OK;
+}
+
+// AES-CCM transciphering of n messages (aes_ccm.h): one public-block AES call for B_0, A_0 and A_1..A_m of every message,
+// the CBC-MAC chain in place on the B_0 rows (step s: aes_ccm_chain_input_kernel over the first a_s sorted messages, then
+// one encrypted-block AES call of a_s blocks), then the tag check: aes_ccm_tag_diff_kernel forms D = MSB_t(X) ⊕ E(A_0) ⊕ U
+// per message (caller order, 16 bytes, those >= t trivial zero) and three circuit bootstraps reduce it to one bit:
+// byte == 0 over 16·n bytes, all-8-set over 2·n groups, both-set over n pairs.  Squared noise: chain inputs 18 (9 in a step
+// of AAD blocks only), D 18, the zero tests 8, the 8-bit ANDs 8, the validity bit 2; the plaintext bits 9.  The
+// descriptors of all steps, the ranks and the tag lengths travel to the device in one upload into ccm_desc, since
+// aes_blocks_dev reuses ws_plan on every call.
+int aes_ccm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out, uint64_t* valid_out) {
+    uint64_t pt_bytes = 0;
+    TRY(ccm_check(ctx, n_msgs, key_idx, msgs, &pt_bytes));
+    if ((n_msgs > 0 && !valid_out) || (pt_bytes > 0 && !pt_out)) return fail(ctx, TAC_ERR_ARG, "NULL output");
+    if (n_msgs == 0) return TAC_OK;
+    TRY(ensure_ccm_luts(ctx));
+    CcmPlan plan;
+    ccm_plan_build(n_msgs, msgs, key_idx, plan);
+    const int n = n_msgs;
+    const uint64_t* keys = key_idx ? ctx->key_table.as<uint64_t>() : ctx->key_sched;
+    const size_t L = (size_t)ctx->big() + 1, byte_words = 8 * L, blk = 16 * byte_words;
+    const int64_t rows = (int64_t)(plan.pub_blocks.size() / 16);
+    TRY(ensure(ctx, ctx->ccm_pub, (size_t)rows * blk * 8));
+    TRY(ensure(ctx, ctx->ccm_work, ((size_t)n * blk + (size_t)n * 18 * L) * 8));
+    const size_t desc_bytes = plan.desc.size() * sizeof(CcmChainDesc);
+    std::vector<uint8_t> host(desc_bytes + (size_t)n * 8);
+    if (desc_bytes) std::memcpy(host.data(), plan.desc.data(), desc_bytes);
+    std::memcpy(host.data() + desc_bytes, plan.rank.data(), (size_t)n * 4);
+    std::memcpy(host.data() + desc_bytes + (size_t)n * 4, plan.tag_len.data(), (size_t)n * 4);
+    TRY(ensure(ctx, ctx->ccm_desc, host.size()));
+    // pageable source: the call returns once the bytes are staged
+    CU(cudaMemcpyAsync(ctx->ccm_desc.p, host.data(), host.size(), cudaMemcpyHostToDevice, ctx->stream));
+    const CcmChainDesc* d_desc = ctx->ccm_desc.as<CcmChainDesc>();
+    const int32_t* d_rank = reinterpret_cast<const int32_t*>(ctx->ccm_desc.as<uint8_t>() + desc_bytes);
+    const int32_t* d_tag_len = d_rank + n;
+    uint64_t* pub = ctx->ccm_pub.as<uint64_t>();
+    uint64_t* work = ctx->ccm_work.as<uint64_t>();
+
+    TRY(aes_blocks_dev(ctx, AesDir::Forward, keys, key_idx ? plan.pub_kidx.data() : nullptr, (int)rows, 10, 0, nullptr, plan.pub_blocks.data(),
+                       plan.pub_xor.data(), pub));
+    size_t d0 = 0;
+    for (size_t s = 0; s < plan.active.size(); s++) {
+        const int a = plan.active[s];
+        const size_t total = (size_t)a * blk;
+        aes_ccm_chain_input_kernel<<<grid1d(total, 256, ctx->sm_count), 256, 0, ctx->stream>>>(pub, d_desc + d0, (int)L, total, work);
+        TRY(post_launch(ctx, "aes_ccm_chain_input_kernel"));
+        TRY(aes_blocks_dev(ctx, AesDir::Forward, keys, key_idx ? plan.kidx_sorted.data() : nullptr, a, 10, plan.adds_plaintext[s] ? 18 : 9, work,
+                           nullptr, nullptr, pub));
+        d0 += (size_t)a;
+    }
+
+    uint64_t* diff = work;                                   // [n][16][8][L]
+    uint64_t* zero = diff + (size_t)n * blk;                 // [n][16][L]: byte b of D is zero
+    uint64_t* ones = zero + (size_t)n * 16 * L;              // [n][2][L]: bytes 0..7 / 8..15 all zero
+    aes_ccm_tag_diff_kernel<<<grid1d((size_t)n * blk, 256, ctx->sm_count), 256, 0, ctx->stream>>>(pub, d_rank, d_tag_len, n, (int)L, (size_t)n * blk, diff);
+    TRY(post_launch(ctx, "aes_ccm_tag_diff_kernel"));
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_zero8], 16 * n, diff, zero));
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones8], 2 * n, zero, ones));
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones2], n, ones, valid_out));
+    // plaintext: the first p bytes of a message's A_1..A_m rows, contiguous, into its place in the caller's order
+    for (int c = 0; c < n; c++)
+        if (plan.shape[c].p)
+            CU(cudaMemcpyAsync(pt_out + (size_t)plan.pt_off[c] * byte_words, pub + (size_t)plan.pt_row[c] * blk, plan.shape[c].p * byte_words * 8,
+                               cudaMemcpyDeviceToDevice, ctx->stream));
+    return TAC_OK;
+}
+
 }  // namespace
 
 // =================================================================================================== C ABI
@@ -710,7 +815,7 @@ void tac_ctx_destroy(tac_ctx* ctx) {
     for (auto& l : ctx->luts) cudaFree(l.dev);
     for (DevBuf* b : {&ctx->ws_in, &ctx->ws_out, &ctx->ws_small, &ctx->ws_ksdig, &ctx->ws_pbs, &ctx->ws_pfdig, &ctx->ws_ggsw, &ctx->ws_ggswf,
                       &ctx->ws_tree_a, &ctx->ws_tree_b, &ctx->ws_state, &ctx->ws_muls, &ctx->ws_misc, &ctx->ws_plan, &ctx->ws_rep,
-                      &ctx->key_table, &ctx->inv_key_table})
+                      &ctx->key_table, &ctx->inv_key_table, &ctx->ccm_pub, &ctx->ccm_work, &ctx->ccm_desc})
         if (b->p) cudaFree(b->p);
     for (auto& r : ctx->prof_pool) for (auto& ev : r.ev) cudaEventDestroy(ev);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -1247,6 +1352,32 @@ int tac_aes_decrypt_public_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, 
     return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
         return tac_aes_decrypt_public_blocks_keyed_dev(ctx, n_blocks, rounds, key_idx_host, blocks_host, xor_host, out);
     });
+}
+
+// ------------------------------------------------------------------------------------------------ AES-CCM transciphering
+// aes_ccm_dev under the single resident schedule (key_idx NULL) or the key table; the context lock is taken here only
+int tac_aes_ccm_transcipher_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_dev,
+                                uint64_t* valid_out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    return aes_ccm_dev(ctx, n_msgs, key_idx, msgs, pt_out_dev, valid_out_dev);
+}
+int tac_aes_ccm_transcipher(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_host,
+                            uint64_t* valid_out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    uint64_t pt_bytes = 0;
+    TRY(ccm_check(ctx, n_msgs, key_idx, msgs, &pt_bytes));
+    if ((n_msgs > 0 && !valid_out_host) || (pt_bytes > 0 && !pt_out_host)) return fail(ctx, TAC_ERR_ARG, "NULL output");
+    if (n_msgs == 0) return TAC_OK;
+    const size_t L = (size_t)ctx->big() + 1, pt_words = (size_t)pt_bytes * 8 * L, valid_words = (size_t)n_msgs * L;
+    TRY(ensure(ctx, ctx->ws_out, (pt_words + valid_words) * 8));
+    uint64_t* pt = ctx->ws_out.as<uint64_t>();
+    TRY(aes_ccm_dev(ctx, n_msgs, key_idx, msgs, pt, pt + pt_words));
+    if (pt_words) CU(cudaMemcpyAsync(pt_out_host, pt, pt_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(valid_out_host, pt + pt_words, valid_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return TAC_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ single stages

@@ -8,11 +8,13 @@
 //                          state (aes_mix_columns_kernel and aes_final_round_kernel templated on the direction); round-1
 //                          inputs and representative gathers of the public-block path; InvMixColumns of the inverse key
 //                          schedule (aes_inv_mix_key_kernel); the sums of a batched key-expansion step (aes_key_step_kernel)
+//   aes_ccm_*_kernel       AES-CCM: the CBC-MAC chain input X ⊕ B of one step, and the tag difference the tag check bootstraps
 //   lwe_add_kernel         leveled XOR (lwe_ciphertext_add_assign) over a batch; lwe_shl_kernel / lwe_sub_kernel: glue of extract_bits
 //   negate_kernel, dfma_peak_kernel   key-upload helper, FP64 peak microbenchmark (roofline denominator)
 #pragma once
 #include <cuda_runtime.h>
 #include "tac_common.h"
+#include "aes_ccm.h"
 
 namespace tac {
 
@@ -216,6 +218,43 @@ __global__ void aes_gather_bytes_kernel(const uint64_t* __restrict__ state, cons
         out[i] = state[(size_t)rep_pos[k] * byte_words + w];
     }
 }
+// ================================================================================================ AES-CCM (aes_ccm.h)
+// CBC-MAC chain input of one step over the first a active messages (sorted order): out[j] = X[j] ⊕ B, where X[j] is row j
+// of the public call's output `pub` (the chain state, updated in place by the caller) and B is, by desc[j] (CcmChainDesc),
+// the first len bytes of the FHE plaintext row desc[j].src of `pub` (zero padding: nothing added) or the public AAD bytes
+// as a trivial ciphertext (encode_bit(1) = 2^63 on the body of every set bit, as xr in aes_final_round_kernel).
+// total = a·16·8·L words.
+__global__ void aes_ccm_chain_input_kernel(const uint64_t* __restrict__ pub, const CcmChainDesc* __restrict__ desc, int L, size_t total,
+                                           uint64_t* __restrict__ out) {
+    const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t j = i / blk_words; const size_t rem = i - j * blk_words;
+        const int byte = (int)(rem / byte_words); const size_t w = rem - (size_t)byte * byte_words;
+        const CcmChainDesc& d = desc[j];
+        uint64_t v = pub[i];
+        if (d.src >= 0) {
+            if (byte < d.len) v += pub[(size_t)d.src * blk_words + rem];
+        } else {
+            const int bit = (int)(w / L);
+            if (w - (size_t)bit * L == (size_t)L - 1 && (d.aad[byte] & (0x80 >> bit))) v += 1ull << 63;
+        }
+        out[i] = v;
+    }
+}
+// tag difference, message c in the caller's order: D[c][b] = X[r][b] ⊕ (E(A_0) ⊕ U)[r][b] for bytes b < tag_len[c], trivial
+// zero for the rest, r = rank[c] its sorted row.  X = rows 0..n−1 of `pub`, E(A_0) ⊕ U = rows n..2n−1.  D is zero exactly
+// when the tag is genuine.  out [n][16][8][L]; total = n·16·8·L words.
+__global__ void aes_ccm_tag_diff_kernel(const uint64_t* __restrict__ pub, const int32_t* __restrict__ rank, const int32_t* __restrict__ tag_len,
+                                        int n, int L, size_t total, uint64_t* __restrict__ out) {
+    const size_t byte_words = (size_t)8 * L, blk_words = 16 * byte_words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t c = i / blk_words; const size_t rem = i - c * blk_words;
+        const int byte = (int)(rem / byte_words);
+        const size_t r = (size_t)rank[c];
+        out[i] = byte < tag_len[c] ? pub[r * blk_words + rem] + pub[((size_t)n + r) * blk_words + rem] : 0ull;
+    }
+}
+
 // leveled XOR (BitXorAssign, shortint_woppbs_1bit.rs:134-142 → lwe_ciphertext_add_assign): a += b, element-wise
 __global__ void lwe_add_kernel(uint64_t* __restrict__ a, const uint64_t* __restrict__ b, size_t total) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) a[i] += b[i];
