@@ -276,6 +276,42 @@ int tac_aes_ccm_transcipher_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx
  * CBC-MAC blocks}; NULL ctr_blocks / mac_blocks query the counts only.  TAC_ERR_ARG as tac_aes_ccm_transcipher.  Host only. */
 int tac_aes_ccm_format(const tac_ccm_msg* msg, uint8_t* ctr_blocks, uint8_t* mac_blocks, int64_t counts[2]);
 
+/* ------------------------------------------------------------------ AES-GCM transciphering (no counterpart in the reference) */
+/* GHASH key tables: H = E_K(0^128) and its powers H^1..H^depth, each bit at squared noise 1, resident per key, laid out
+ * [K][depth][128][kN+1] (bit order of the state: coefficient i of a GF(2^128) element is row 8·byte + bit, MSB first).
+ * tac_aes_gcm_hash_key covers the single schedule (K = 1), tac_aes_gcm_hash_key_table every entry of the key table.
+ * depth is a power of two in [1, 1024] (else TAC_ERR_ARG); records of at most depth GHASH blocks need no encrypted
+ * GF(2^128) product.  H comes from one public-block AES call over all keys; pass j computes H^(2^j+1) … H^(2^(j+1)), even
+ * powers as squarings (linear), odd ones as one batched product call.  out_host may be NULL.  A table takes
+ * depth · 128 · (kN+1) · 8 bytes per key (2 MiB per power at kN+1 = 2049); TAC_ERR_CUDA when it does not fit.
+ * tac_aes_set_key_schedule (and every call that sets the schedule) marks the single table stale, tac_aes_key_table and
+ * tac_aes_set_key_table the keyed one; a GCM call then fails with TAC_ERR_STATE.  No call derives a table implicitly.
+ * TAC_ERR_STATE without evaluation keys or the schedule / key table; TAC_ERR_NOISE below max_noise_level_squared 33, or
+ * 64 when depth > 1 (the product sums 8 box outputs of squared noise 8). */
+int tac_aes_gcm_hash_key(tac_ctx* ctx, int depth, uint64_t* out_host);
+int tac_aes_gcm_hash_key_table(tac_ctx* ctx, int depth, uint64_t* out_host);
+/* AES-128-GCM transciphering with the tag checked under FHE (NIST SP 800-38D, 96-bit IVs only).  A record is a
+ * tac_ccm_msg: nonce = the 12-byte IV, tag_len in {4, 8, 12, 13, 14, 15, 16}, AAD, data = C ‖ T.  For every record: the FHE
+ * plaintext bits of C (word for word tac_aes_encrypt_public_blocks over inc32^i(J0), i = 1..m, with XOR bytes C; squared
+ * noise 9) and one encrypted VALIDITY BIT, 1 exactly when T is the GCM tag of (IV, A, C) under the FHE-encrypted key
+ * (squared noise 2).  GHASH runs in Horner form over chunks of `depth` blocks with the resident GHASH key table: a record of
+ * at most depth blocks (AAD, C, the length block) runs only sums and refreshes, a longer one one GF(2^128) product per
+ * further chunk, batched across records.  key_idx NULL: every record under the single schedule; else record i under key
+ * table entry key_idx[i].  pt_out [Σ (data_len − tag_len)][8][kN+1] in record order, valid_out [n_msgs][kN+1].  A record's
+ * outputs do not depend on the batch it is in.  Errors, all before anything is enqueued: TAC_ERR_ARG for n_msgs < 0, an IV
+ * that is not 12 bytes, a tag length not in the set, data_len < tag_len, a payload above 2^36 − 32 bytes, AAD of 2^61
+ * bytes or more, a NULL pointer with a non-zero length, a key index outside [0, n_keys); TAC_ERR_STATE without evaluation
+ * keys, the schedule / key table or a valid GHASH key table; TAC_ERR_NOISE below max_noise_level_squared 33 (64 for records
+ * longer than depth). */
+int tac_aes_gcm_transcipher(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_host,
+                            uint64_t* valid_out_host);
+int tac_aes_gcm_transcipher_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_dev,
+                                uint64_t* valid_out_dev);
+/* The public blocks of one record.  ctr_blocks: J0 = IV ‖ 0^31 ‖ 1, then inc32^i(J0), i = 1..m (m = ceil(p/16));
+ * ghash_blocks: X_1..X_M = the AAD and C, each zero-padded to whole blocks, then [len(A)]_64 ‖ [len(C)]_64 in bits.
+ * counts = {m + 1, M}; NULL block pointers query the counts only.  TAC_ERR_ARG as tac_aes_gcm_transcipher.  Host only. */
+int tac_aes_gcm_format(const tac_ccm_msg* msg, uint8_t* ctr_blocks, uint8_t* ghash_blocks, int64_t counts[2]);
+
 /* ------------------------------------------------------------------ single stages (parity tests, profiling) */
 /* [U] keyswitch_lwe_ciphertext: [n_cts][kN+1] → [n_cts][n+1] */
 int tac_stage_keyswitch(tac_ctx* ctx, int n_cts, const uint64_t* in_host, uint64_t* out_host);
@@ -285,6 +321,11 @@ int tac_stage_keyswitch(tac_ctx* ctx, int n_cts, const uint64_t* in_host, uint64
  * (shortint_woppbs_1bit.rs:339-363) is the (63, 1) case = tac_stage_keyswitch; the 8-bit model uses (56, 8)
  * (shortint_woppbs_8bit.rs:271-275). */
 int tac_extract_bits(tac_ctx* ctx, int delta_log, int n_bits, int n_cts, const uint64_t* in_host, uint64_t* out_host);
+/* n encrypted products a·b in GF(2^128) (GCM's field x^128 + x^7 + x^2 + x + 1 and bit order): a, b, out [n][128][kN+1],
+ * operand bits at squared noise <= max_noise_level_squared, output bits at squared noise 1.  The GGSW stage runs once
+ * over the 256·n operand bits, then 1024·n vertical-packing boxes (4-bit × 4-bit carry-less products, 8 → 7) read their
+ * GGSWs by index, and the sums and the reduction run as refreshed linear layers.  TAC_ERR_NOISE below 64. */
+int tac_gf128_mul(tac_ctx* ctx, int n, const uint64_t* a_host, const uint64_t* b_host, uint64_t* out_host);
 /* [U] homomorphic_shift_boolean: [n_cts][n+1] → [n_cts][kN+1] */
 int tac_stage_pbs(tac_ctx* ctx, int n_cts, const uint64_t* in_host, uint64_t* out_host);
 /* [U] private_functional_keyswitch ×(k+1): [n_cts][kN+1] → [n_cts][k+1][(k+1)N] */

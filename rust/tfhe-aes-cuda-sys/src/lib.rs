@@ -142,6 +142,14 @@ extern "C" {
     pub fn tac_aes_ccm_transcipher_dev(ctx: *mut tac_ctx, n_msgs: c_int, key_idx: *const i32, msgs: *const tac_ccm_msg, pt_out_dev: *mut u64,
                                        valid_out_dev: *mut u64) -> c_int;
     pub fn tac_aes_ccm_format(msg: *const tac_ccm_msg, ctr_blocks: *mut u8, mac_blocks: *mut u8, counts: *mut i64) -> c_int;
+    pub fn tac_aes_gcm_hash_key(ctx: *mut tac_ctx, depth: c_int, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_gcm_hash_key_table(ctx: *mut tac_ctx, depth: c_int, out_host: *mut u64) -> c_int;
+    pub fn tac_aes_gcm_transcipher(ctx: *mut tac_ctx, n_msgs: c_int, key_idx: *const i32, msgs: *const tac_ccm_msg, pt_out_host: *mut u64,
+                                   valid_out_host: *mut u64) -> c_int;
+    pub fn tac_aes_gcm_transcipher_dev(ctx: *mut tac_ctx, n_msgs: c_int, key_idx: *const i32, msgs: *const tac_ccm_msg, pt_out_dev: *mut u64,
+                                       valid_out_dev: *mut u64) -> c_int;
+    pub fn tac_aes_gcm_format(msg: *const tac_ccm_msg, ctr_blocks: *mut u8, ghash_blocks: *mut u8, counts: *mut i64) -> c_int;
+    pub fn tac_gf128_mul(ctx: *mut tac_ctx, n: c_int, a_host: *const u64, b_host: *const u64, out_host: *mut u64) -> c_int;
 
     // single stages, profiling
     pub fn tac_stage_keyswitch(ctx: *mut tac_ctx, n_cts: c_int, in_host: *const u64, out_host: *mut u64) -> c_int;

@@ -125,6 +125,12 @@ _SIGNATURES = {
     "tac_aes_ccm_transcipher": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_aes_ccm_transcipher_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tac_aes_ccm_format": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_gcm_hash_key": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "tac_aes_gcm_hash_key_table": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "tac_aes_gcm_transcipher": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_gcm_transcipher_dev": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_aes_gcm_format": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tac_gf128_mul": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p, _u64p]),
     "tac_stage_keyswitch": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
     "tac_extract_bits": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _u64p, _u64p]),
     "tac_stage_pbs": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
@@ -341,6 +347,55 @@ def aes_ccm_format(nonce, data, tag_len=16, aad=b""):
     if L.tac_aes_ccm_format(C.addressof(msgs[0]), ctr.ctypes.data, mac.ctypes.data, counts.ctypes.data) != 0:
         raise ValueError("aes_ccm_format: bad arguments")
     return ctr, mac
+
+
+GCM_TAG_LENGTHS = (4, 8, 12, 13, 14, 15, 16)
+
+
+def _gcm_messages(messages):
+    """(CcmMsg array, the byte strings it points into, payload length of every record) from [(iv, data, tag_len, aad)];
+    ValueError for every argument the C entry points reject with TAC_ERR_ARG"""
+    msgs = (CcmMsg * max(1, len(messages)))()
+    keep, sizes = [], []
+    for i, (iv, data, tag_len, aad) in enumerate(messages):
+        iv, data, aad = bytes(iv), bytes(data), bytes(aad)
+        if len(iv) != 12:
+            raise ValueError(f"AES-GCM record {i}: the IV must be 12 bytes, not {len(iv)}")
+        if not isinstance(tag_len, (int, np.integer)) or int(tag_len) not in GCM_TAG_LENGTHS:
+            raise ValueError(f"AES-GCM record {i}: tag length {tag_len!r} not in {GCM_TAG_LENGTHS}")
+        tag_len = int(tag_len)
+        if len(data) < tag_len:
+            raise ValueError(f"AES-GCM record {i}: {len(data)} data bytes cannot hold a {tag_len}-byte tag")
+        p = len(data) - tag_len
+        if p > (1 << 36) - 32 or len(aad) >= 1 << 61:
+            raise ValueError(f"AES-GCM record {i}: a payload above 2^36 - 32 bytes or AAD of 2^61 bytes or more")
+        keep += [iv, data, aad]
+        ptr = lambda b: C.cast(C.c_char_p(b), C.c_void_p).value
+        msgs[i] = CcmMsg(ptr(iv), len(iv), tag_len, ptr(aad), len(aad), ptr(data), len(data))
+        sizes.append(p)
+    return msgs, keep, sizes
+
+
+def aes_gcm_format(iv, data, tag_len=16, aad=b""):
+    """the public blocks of one AES-GCM record (NIST SP 800-38D, 96-bit IV): (counter blocks J0, inc32(J0), …
+    [m+1][16], GHASH blocks X_1..X_M [M][16]: AAD and C zero-padded, then the bit lengths) as uint8 arrays; data = C ‖ T.
+    Host only."""
+    msgs, keep, _ = _gcm_messages([(iv, data, tag_len, aad)])
+    L = load_library()
+    counts = np.zeros(2, dtype=np.int64)
+    if L.tac_aes_gcm_format(C.addressof(msgs[0]), None, None, counts.ctypes.data) != 0:
+        raise ValueError("aes_gcm_format: bad arguments")
+    ctr = np.zeros((int(counts[0]), 16), dtype=np.uint8)
+    ghash = np.zeros((int(counts[1]), 16), dtype=np.uint8)
+    if L.tac_aes_gcm_format(C.addressof(msgs[0]), ctr.ctypes.data, ghash.ctypes.data, counts.ctypes.data) != 0:
+        raise ValueError("aes_gcm_format: bad arguments")
+    return ctr, ghash
+
+
+def _gcm_depth(depth):
+    if not isinstance(depth, (int, np.integer)) or not 1 <= int(depth) <= 1024 or int(depth) & (int(depth) - 1):
+        raise ValueError(f"GHASH key depth must be a power of two in [1, 1024], not {depth!r}")
+    return int(depth)
 
 
 class LookupTable:
@@ -959,6 +1014,60 @@ class FheContext(NoiseContext):
                                                    pt.ctypes.data, valid.ctypes.data))
         offs = np.cumsum([0] + sizes)
         return [(pt[offs[i]:offs[i + 1]], valid[i]) for i in range(len(sizes))]
+
+    # -- AES-GCM transciphering with the tag checked under FHE
+    def aes_gcm_hash_key(self, depth=8):
+        """GHASH key table of the resident key schedule: H = E_K(0) and its powers H^1..H^depth, returned as
+        [depth][128][big+1] (bit order of the state).  It stays valid until the key schedule changes."""
+        depth = _gcm_depth(depth)
+        out = np.empty((depth, 128, self.params.big_lwe_size), dtype=np.uint64)
+        self._check(self.L.tac_aes_gcm_hash_key(self.h, depth, out.ctypes.data))
+        return out
+
+    def aes_gcm_hash_key_table(self, depth=8):
+        """GHASH key tables of every entry of the resident key table, [K][depth][128][big+1]; valid until the key table
+        changes"""
+        depth = _gcm_depth(depth)
+        out = np.empty((max(self.n_keys, 1), depth, 128, self.params.big_lwe_size), dtype=np.uint64)
+        self._check(self.L.tac_aes_gcm_hash_key_table(self.h, depth, out.ctypes.data))
+        return out
+
+    def aes_gcm_transcipher(self, iv, data, tag_len=16, aad=b""):
+        """Transciphering of one AES-GCM record under the resident key schedule and its GHASH key table: `data` = C ‖ T is
+        what AES-GCM encryption of (iv, P, aad) returns.  Returns (FHE encryptions of the plaintext bits
+        [len(data) − tag_len][8][big+1], an encrypted validity bit [big+1]: 1 exactly when the tag is genuine)."""
+        return self._aes_gcm([(iv, data, tag_len, aad)], None)[0]
+
+    def aes_gcm_transcipher_many(self, messages):
+        """aes_gcm_transcipher for many senders in one call: messages = [(key_index, iv, data, tag_len, aad)], each under
+        key table entry key_index.  Returns one (plaintext bits, validity bit) pair per record."""
+        messages = list(messages)
+        k = _key_index([m[0] for m in messages], len(messages), self.n_keys)
+        return self._aes_gcm([m[1:] for m in messages], k)
+
+    def _aes_gcm(self, messages, key_index):
+        msgs, keep, sizes = _gcm_messages(messages)
+        if not sizes:
+            return []
+        L1 = self.params.big_lwe_size
+        pt = np.empty((sum(sizes), 8, L1), dtype=np.uint64)
+        valid = np.empty((len(sizes), L1), dtype=np.uint64)
+        self._check(self.L.tac_aes_gcm_transcipher(self.h, len(sizes), None if key_index is None else key_index.ctypes.data, msgs,
+                                                   pt.ctypes.data, valid.ctypes.data))
+        offs = np.cumsum([0] + sizes)
+        return [(pt[offs[i]:offs[i + 1]], valid[i]) for i in range(len(sizes))]
+
+    def gf128_mul(self, a, b):
+        """encrypted products a·b in GF(2^128) (GCM's field and bit order): a, b [n][128][big+1] → [n][128][big+1], output
+        bits at squared noise 1"""
+        L1 = self.params.big_lwe_size
+        x = np.ascontiguousarray(a, dtype=np.uint64).reshape(-1, 128, L1)
+        y = np.ascontiguousarray(b, dtype=np.uint64).reshape(-1, 128, L1)
+        if x.shape != y.shape:
+            raise ValueError("gf128_mul: operands of different counts")
+        out = np.empty_like(x)
+        self._check(self.L.tac_gf128_mul(self.h, x.shape[0], x.reshape(-1), y.reshape(-1), out.reshape(-1)))
+        return out
 
     def _split_messages(self, out, sizes):
         """[n][16][8][big+1] of whole blocks → one [size][8][big+1] array per message (each padded to whole blocks)"""

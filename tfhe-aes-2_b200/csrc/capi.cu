@@ -5,10 +5,12 @@
 #include "kernels_common.cuh"
 #include "aes_plan.h"
 #include "aes_ccm.h"
+#include "aes_gcm.h"
 #include "kernels_gemm_umma.cuh"
 #include "ep_step.cuh"
 #include "shape_launch.h"
 
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <condition_variable>
@@ -87,6 +89,7 @@ struct tac_ctx {
     int aes_lut24 = -1, aes_lut8 = -1, aes_lut1 = -1;
     int aes_lut_inv32 = -1, aes_lut_inv8 = -1, aes_lut_key32 = -1;   // decryption: InvS·{14,11,13,9}, InvS, b·{14,11,13,9}
     int ccm_lut_zero8 = -1, ccm_lut_ones8 = -1, ccm_lut_ones2 = -1;   // AES-CCM tag check: byte == 0, 8 bits all 1, 2 bits all 1
+    int gf_lut_mul = -1;                 // GF(2^128) product: 8 → 7 carry-less product of two 4-bit polynomials
     // AES key schedule
     uint64_t* key_sched = nullptr;
     uint64_t* inv_key_sched = nullptr;   // equivalent inverse cipher's schedule dk, same layout [44 words][4][8][kN+1]
@@ -103,6 +106,13 @@ struct tac_ctx {
     // AES-CCM, apart from the buffers aes_blocks_dev reuses on every call: the public call's output (rows 0..n−1 are the
     // CBC-MAC chain state), the chain input / tag check, and the descriptors of all steps
     DevBuf ccm_pub, ccm_work, ccm_desc;
+    // AES-GCM: the GHASH key tables H^1..H^depth [K][depth][128][kN+1] of the single schedule and of the key table (valid
+    // while the schedule / key table they were made from is resident); the linear layer's descriptors, group sums and
+    // level outputs; the product's GGSW index table, box outputs and operands; a transciphering call's buffers
+    struct GcmTable { DevBuf buf; int depth = 0, n_keys = 0; bool valid = false; };
+    GcmTable gcm_h, gcm_h_keyed;
+    DevBuf lin_desc, lin_sum, lin_lvl, gf_idx, gf_box, gf_ops, gf_prod, gcm_pub, gcm_dy;
+    int gf_idx_np = 0;                   // products per pass gf_idx was built for
     size_t max_cts = 16384;
     uint32_t fix_cap = kFixCap;      // capacity of the PFKS tie list in use (TAC_FIX_CAP lowers it: exercises the overflow path)
     // profiling: one event tuple per pipeline pass, recorded without synchronising; read back by tac_ctx_stage_times
@@ -300,41 +310,49 @@ int stage_pfks(tac_ctx* ctx, const uint64_t* in, int nct, uint64_t* ggsw) {
     return post_launch(ctx, "pfks_fixup_scan_kernel");
 }
 
-// the whole circuit bootstrap for `nbox` boxes resident on the device
+// The GGSW stage of a circuit bootstrap: keyswitch → PBS (one per level) → PFKS → FFT of nct input bits [nct][big+1] into
+// Fourier GGSWs ggsw_f [nct][cbs_l][G][G][M] (room provided by the caller)
+int ggsw_stage(tac_ctx* ctx, const uint64_t* cin, int nct, cplx* ggsw_f) {
+    const TacParams& p = ctx->p;
+    const int big1 = ctx->big() + 1, G = ctx->G(), lc = p.cbs_l;
+    const size_t ggsw_words = (size_t)G * G * p.N;
+    TRY(ensure(ctx, ctx->ws_small, (size_t)nct * (p.n + 1) * 8));
+    TRY(ensure(ctx, ctx->ws_pbs, (size_t)nct * lc * big1 * 8));
+    TRY(ensure(ctx, ctx->ws_ggsw, (size_t)nct * lc * ggsw_words * 8));
+    TRY(stage_event(ctx, 0));
+    TRY(stage_ks(ctx, cin, nct, ctx->ws_small.as<uint64_t>()));                       // extract_dual_bit_from_bit
+    TRY(stage_event(ctx, 1));
+    // circuit_bootstrap_boolean: one homomorphic_shift_boolean per level (all four shipped parameter sets have one level)
+    if (lc == 1) {
+        TRY(pbs(ctx, ctx->ws_small.as<uint64_t>(), nct, ctx->ws_pbs.as<uint64_t>()));
+    } else {
+        TRY(ensure(ctx, ctx->ws_tree_a, (size_t)nct * big1 * 8));
+        for (int lv = 1; lv <= lc; lv++) {          // level lv lands at [ct][lv-1] so that the PFKS rows come out as [ct][level][row]
+            TRY(pbs(ctx, ctx->ws_small.as<uint64_t>(), nct, ctx->ws_tree_a.as<uint64_t>(), 1ull << (63 - p.cbs_b * lv)));
+            CU(cudaMemcpy2DAsync(ctx->ws_pbs.as<uint64_t>() + (size_t)(lv - 1) * big1, (size_t)lc * big1 * 8, ctx->ws_tree_a.p, (size_t)big1 * 8,
+                                 (size_t)big1 * 8, (size_t)nct, cudaMemcpyDeviceToDevice, ctx->stream));
+        }
+    }
+    TRY(stage_event(ctx, 2));
+    TRY(stage_pfks(ctx, ctx->ws_pbs.as<uint64_t>(), nct * lc, ctx->ws_ggsw.as<uint64_t>()));
+    TRY(stage_event(ctx, 3));
+    TRY(poly_fft(ctx, ctx->ws_ggsw.as<uint64_t>(), (size_t)nct * lc * G * G, ggsw_f));   // fill_with_forward_fourier
+    return stage_event(ctx, 4);
+}
+
+// the whole circuit bootstrap for `nbox` boxes resident on the device: the GGSW stage, then vertical packing
 int wopbs_dev(tac_ctx* ctx, const Lut& lut, int nbox, const uint64_t* in, uint64_t* out) {
     const TacParams& p = ctx->p;
     if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
     const int big1 = ctx->big() + 1, G = ctx->G(), M = p.N / 2, lc = p.cbs_l;
-    const size_t ggsw_words = (size_t)G * G * p.N;
     const int max_boxes = (int)std::max<size_t>(1, ctx->max_cts / ((size_t)lut.n_in * lc));
     for (int b0 = 0; b0 < nbox; b0 += max_boxes) {
         const int nb = std::min(max_boxes, nbox - b0);
         const int nct = nb * lut.n_in;
         const uint64_t* cin = in + (size_t)b0 * lut.n_in * big1;
         uint64_t* cout = out + (size_t)b0 * lut.n_out * big1;
-        TRY(ensure(ctx, ctx->ws_small, (size_t)nct * (p.n + 1) * 8));
-        TRY(ensure(ctx, ctx->ws_pbs, (size_t)nct * lc * big1 * 8));
-        TRY(ensure(ctx, ctx->ws_ggsw, (size_t)nct * lc * ggsw_words * 8));
         TRY(ensure(ctx, ctx->ws_ggswf, (size_t)nct * lc * G * G * M * sizeof(cplx)));
-        TRY(stage_event(ctx, 0));
-        TRY(stage_ks(ctx, cin, nct, ctx->ws_small.as<uint64_t>()));                       // extract_dual_bit_from_bit
-        TRY(stage_event(ctx, 1));
-        // circuit_bootstrap_boolean: one homomorphic_shift_boolean per level (all four shipped parameter sets have one level)
-        if (lc == 1) {
-            TRY(pbs(ctx, ctx->ws_small.as<uint64_t>(), nct, ctx->ws_pbs.as<uint64_t>()));
-        } else {
-            TRY(ensure(ctx, ctx->ws_tree_a, (size_t)nct * big1 * 8));
-            for (int lv = 1; lv <= lc; lv++) {          // level lv lands at [ct][lv-1] so that the PFKS rows come out as [ct][level][row]
-                TRY(pbs(ctx, ctx->ws_small.as<uint64_t>(), nct, ctx->ws_tree_a.as<uint64_t>(), 1ull << (63 - p.cbs_b * lv)));
-                CU(cudaMemcpy2DAsync(ctx->ws_pbs.as<uint64_t>() + (size_t)(lv - 1) * big1, (size_t)lc * big1 * 8, ctx->ws_tree_a.p, (size_t)big1 * 8,
-                                     (size_t)big1 * 8, (size_t)nct, cudaMemcpyDeviceToDevice, ctx->stream));
-            }
-        }
-        TRY(stage_event(ctx, 2));
-        TRY(stage_pfks(ctx, ctx->ws_pbs.as<uint64_t>(), nct * lc, ctx->ws_ggsw.as<uint64_t>()));
-        TRY(stage_event(ctx, 3));
-        TRY(poly_fft(ctx, ctx->ws_ggsw.as<uint64_t>(), (size_t)nct * lc * G * G, ctx->ws_ggswf.as<cplx>()));   // fill_with_forward_fourier
-        TRY(stage_event(ctx, 4));
+        TRY(ggsw_stage(ctx, cin, nct, ctx->ws_ggswf.as<cplx>()));
         TRY(vertical_packing(ctx, lut, ctx->ws_ggswf.as<cplx>(), nb, cout));
         TRY(stage_event(ctx, 5));
     }
@@ -766,6 +784,355 @@ int aes_ccm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_
     return TAC_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ AES-GCM (aes_gcm.h)
+// Runs a linear-layer plan: srcs are the plan's input sources 0..first_src−1; level k's group sums go through one 1-bit
+// circuit bootstrap each into source first_src + k; the final gather-add writes row r to out row out_row[r] (or r).  All
+// descriptors travel in one upload into lin_desc.
+int lin_run(tac_ctx* ctx, const LinPlan& plan, const std::vector<const uint64_t*>& srcs, const std::vector<uint32_t>* out_row, uint64_t* out) {
+    if ((int)(srcs.size() + plan.levels.size()) > kLinMaxSrc) return fail(ctx, TAC_ERR_ARG, "linear layer: too many sources");
+    TRY(ensure_aes_luts(ctx));
+    const size_t L = (size_t)ctx->big() + 1;
+    std::vector<uint32_t> host;
+    std::vector<size_t> off;
+    auto put = [&](const std::vector<uint32_t>& v) { off.push_back(host.size()); host.insert(host.end(), v.begin(), v.end()); };
+    size_t lvl_rows = 0, max_rows = 0;
+    for (const LinSums& l : plan.levels) {
+        put(l.row_ptr); put(l.terms);
+        lvl_rows += l.rows(); max_rows = std::max(max_rows, l.rows());
+    }
+    put(plan.final.row_ptr); put(plan.final.terms);
+    if (out_row) put(*out_row);
+    const size_t cbit_off = host.size() * 4;
+    const size_t nrows = plan.final.rows();
+    if (nrows == 0) return TAC_OK;
+    std::vector<uint8_t> bytes(cbit_off + nrows);
+    std::memcpy(bytes.data(), host.data(), cbit_off);
+    std::memcpy(bytes.data() + cbit_off, plan.final.cbit.data(), nrows);
+    TRY(ensure(ctx, ctx->lin_desc, bytes.size()));
+    TRY(ensure(ctx, ctx->lin_sum, std::max<size_t>(1, max_rows) * L * 8));
+    TRY(ensure(ctx, ctx->lin_lvl, std::max<size_t>(1, lvl_rows) * L * 8));
+    // pageable source: the call returns once the bytes are staged
+    CU(cudaMemcpyAsync(ctx->lin_desc.p, bytes.data(), bytes.size(), cudaMemcpyHostToDevice, ctx->stream));
+    const uint32_t* d = ctx->lin_desc.as<uint32_t>();
+    LinSrcs s{};
+    for (size_t i = 0; i < srcs.size(); i++) s.p[i] = srcs[i];
+    uint64_t* lvl = ctx->lin_lvl.as<uint64_t>();
+    size_t k = 0;
+    for (size_t i = 0; i < plan.levels.size(); i++, k += 2) {
+        const size_t rows = plan.levels[i].rows();
+        lwe_gather_add_kernel<<<grid1d(rows * L, 256, ctx->sm_count), 256, 0, ctx->stream>>>(s, d + off[k], d + off[k + 1], nullptr, nullptr, (int)L,
+                                                                                            rows * L, ctx->lin_sum.as<uint64_t>());
+        TRY(post_launch(ctx, "lwe_gather_add_kernel"));
+        TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut1], (int)rows, ctx->lin_sum.as<uint64_t>(), lvl));            // refresh to squared noise 1
+        s.p[srcs.size() + i] = lvl;
+        lvl += rows * L;
+    }
+    lwe_gather_add_kernel<<<grid1d(nrows * L, 256, ctx->sm_count), 256, 0, ctx->stream>>>(
+        s, d + off[k], d + off[k + 1], ctx->lin_desc.as<uint8_t>() + cbit_off, out_row ? d + off[k + 2] : nullptr, (int)L, nrows * L, out);
+    return post_launch(ctx, "lwe_gather_add_kernel");
+}
+
+// copies rows: out row r (or out_row[r]) = row rows[r] of src
+int gather_rows(tac_ctx* ctx, const uint64_t* src, const std::vector<uint32_t>& rows, const std::vector<uint32_t>* out_row, uint64_t* out) {
+    LinPlan plan;
+    for (uint32_t r : rows) {
+        plan.final.terms.push_back(lin_id(0, r));
+        plan.final.row_ptr.push_back((uint32_t)plan.final.terms.size());
+    }
+    plan.final.cbit.assign(rows.size(), 0);
+    return lin_run(ctx, plan, {src}, out_row, out);
+}
+
+int ensure_gf_lut(tac_ctx* ctx) {
+    if (ctx->gf_lut_mul >= 0) return TAC_OK;
+    std::vector<uint64_t> f(256);
+    for (int v = 0; v < 256; v++) f[v] = gf128_box_fn(v);
+    return register_aes_lut(ctx, 8, 7, f.data(), &ctx->gf_lut_mul);
+}
+
+// n encrypted GF(2^128) products out = a · b, operands [n][128][kN+1] at squared noise <= max_noise_level_squared, output
+// bits at squared noise 1 (out row p·128 + j, or out_row[p·128 + j]).  Per pass of np products: the GGSW stage over the
+// 128·np bits of a and of b, 1024·np boxes of vertical packing over GGSWs picked by index (box (i, j) of product p: nibble i
+// of a, nibble j of b), then the linear layer (sums, reduction mod x^128 + x^7 + x^2 + x + 1, refreshes).
+int gf128_mul_dev(tac_ctx* ctx, int n, const uint64_t* a, const uint64_t* b, uint64_t* out, const std::vector<uint32_t>* out_row = nullptr) {
+    if (n <= 0) return TAC_OK;
+    if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
+    TRY(ensure_gf_lut(ctx));
+    const TacParams& p = ctx->p;
+    const size_t L = (size_t)ctx->big() + 1, ggsw_cplx = (size_t)p.cbs_l * ctx->G() * ctx->G() * (p.N / 2);
+    // products per pass: their GGSWs fill one pipeline pass, and their boxes one launch (grid.y <= 65535)
+    const int np_max = (int)std::max<size_t>(1, std::min<size_t>(ctx->max_cts / 256, 65535 / 1024));
+    if (ctx->gf_idx_np != np_max) {
+        // GGSWs of a pass: [a bits of its products][b bits], np_max·128 each
+        std::vector<int32_t> idx((size_t)np_max * 1024 * 8);
+        for (int q = 0; q < np_max; q++)
+            for (int i = 0; i < 32; i++)
+                for (int j = 0; j < 32; j++)
+                    for (int k = 0; k < 4; k++) {
+                        int32_t* e = &idx[(((size_t)q * 1024) + i * 32 + j) * 8];
+                        e[k] = q * 128 + 4 * i + k;
+                        e[4 + k] = np_max * 128 + q * 128 + 4 * j + k;
+                    }
+        TRY(ensure(ctx, ctx->gf_idx, idx.size() * 4));
+        CU(cudaMemcpy(ctx->gf_idx.p, idx.data(), idx.size() * 4, cudaMemcpyHostToDevice));
+        ctx->gf_idx_np = np_max;
+    }
+    const Lut& lut = ctx->luts[ctx->gf_lut_mul];
+    for (int p0 = 0; p0 < n; p0 += np_max) {
+        const int np = std::min(np_max, n - p0);
+        TRY(ensure(ctx, ctx->ws_ggswf, (size_t)2 * np_max * 128 * ggsw_cplx * sizeof(cplx)));
+        TRY(ensure(ctx, ctx->gf_box, (size_t)np * 1024 * 7 * L * 8));
+        cplx* gf = ctx->ws_ggswf.as<cplx>();
+        TRY(ggsw_stage(ctx, a + (size_t)p0 * 128 * L, 128 * np, gf));
+        TRY(stage_event(ctx, 5));
+        TRY(ggsw_stage(ctx, b + (size_t)p0 * 128 * L, 128 * np, gf + (size_t)np_max * 128 * ggsw_cplx));
+        TRY(check_launch(ctx, ctx->ops->vp_gather(klaunch(ctx), p.cbs_l, gf, ctx->gf_idx.as<int32_t>(), 1024 * np, 8, lut.dev, lut.len, 7, p.cbs_b,
+                                                  ctx->gf_box.as<uint64_t>()), "vp_gather_kernel"));
+        TRY(stage_event(ctx, 5));
+        std::vector<LinRow> rows;
+        gf128_rows(np, rows);
+        LinPlan plan;
+        if (lin_plan_build(rows, p.max_noise_sq, 1, 1, plan)) return fail(ctx, TAC_ERR_NOISE, "GF(2^128) product: the sums do not fit max_noise_level_squared");
+        std::vector<uint32_t> orow;
+        if (out_row) orow.assign(out_row->begin() + (size_t)p0 * 128, out_row->begin() + (size_t)(p0 + np) * 128);
+        TRY(lin_run(ctx, plan, {ctx->gf_box.as<uint64_t>()}, out_row ? &orow : nullptr, out_row ? out : out + (size_t)p0 * 128 * L));
+    }
+    return TAC_OK;
+}
+
+int gf_noise_check(tac_ctx* ctx) {
+    // the box outputs of one unreduced coefficient are summed 8 at a time (squared noise 8 each)
+    if (8 * 8 > ctx->p.max_noise_sq) return fail(ctx, TAC_ERR_NOISE, "NoiseTooBig: the GF(2^128) product needs max_noise_level_squared >= 64");
+    return TAC_OK;
+}
+
+// H = E_K(0) of K keys (key_idx NULL: the single schedule) and its powers H^1..H^w into table [K][w][128][L].  H comes
+// out of one public-block call and a refresh.  Pass j computes H^(2^j+1) … H^(2^(j+1)): even powers square an earlier
+// power (a linear map, at most 5 terms per bit, then a refresh), odd ones are the products H^(2^j) · H^(e − 2^j) of all
+// keys in one gf128_mul_dev call.
+int gcm_hash_key_build(tac_ctx* ctx, const uint64_t* keys, const int32_t* key_idx, int K, int w, uint64_t* table) {
+    TRY(ensure_aes_luts(ctx));
+    const size_t L = (size_t)ctx->big() + 1;
+    auto row = [&](int k, int e, int bit) { return (uint32_t)(((size_t)k * w + (e - 1)) * 128 + bit); };
+    TRY(ensure(ctx, ctx->gcm_pub, (size_t)K * 128 * L * 8));
+    std::vector<uint8_t> zero((size_t)K * 16, 0);
+    TRY(aes_blocks_dev(ctx, AesDir::Forward, keys, key_idx, K, 10, 0, nullptr, zero.data(), nullptr, ctx->gcm_pub.as<uint64_t>()));
+    {
+        std::vector<LinRow> rows((size_t)K * 128);
+        std::vector<uint32_t> orow(rows.size());
+        for (int k = 0; k < K; k++)
+            for (int j = 0; j < 128; j++) {
+                rows[(size_t)k * 128 + j].terms.push_back(LinTerm{lin_id(0, (size_t)k * 128 + j), 9, 0});
+                orow[(size_t)k * 128 + j] = row(k, 1, j);
+            }
+        LinPlan plan;
+        TRY(lin_plan_build(rows, ctx->p.max_noise_sq, 1, 1, plan) ? fail(ctx, TAC_ERR_NOISE, "GHASH key: refresh") : TAC_OK);
+        TRY(lin_run(ctx, plan, {ctx->gcm_pub.as<uint64_t>()}, &orow, table));
+    }
+    std::vector<std::vector<int>> sq(128);            // bit r of y^2: XOR of y's bits sq[r]
+    for (int l = 0; l < 128; l++)
+        for (int r : gf128_fold(2 * l)) sq[r].push_back(l);
+    for (int lo = 1; lo < w; lo *= 2) {
+        std::vector<LinRow> rows;
+        std::vector<uint32_t> orow, a_rows, b_rows, prow;
+        for (int k = 0; k < K; k++)
+            for (int e = lo + 1; e <= 2 * lo; e++)
+                for (int j = 0; j < 128; j++) {
+                    if (e % 2 == 0) {
+                        LinRow r;
+                        for (int l : sq[j]) r.terms.push_back(LinTerm{lin_id(0, row(k, e / 2, l)), 1, 0});
+                        rows.push_back(r);
+                        orow.push_back(row(k, e, j));
+                    } else {
+                        a_rows.push_back(row(k, lo, j));
+                        b_rows.push_back(row(k, e - lo, j));
+                        prow.push_back(row(k, e, j));
+                    }
+                }
+        LinPlan plan;
+        TRY(lin_plan_build(rows, ctx->p.max_noise_sq, 1, 1, plan) ? fail(ctx, TAC_ERR_NOISE, "GHASH key: squares") : TAC_OK);
+        TRY(lin_run(ctx, plan, {table}, &orow, table));
+        const int nprod = (int)(a_rows.size() / 128);
+        if (nprod) {
+            TRY(ensure(ctx, ctx->gf_ops, (size_t)2 * nprod * 128 * L * 8));
+            uint64_t* ops = ctx->gf_ops.as<uint64_t>();
+            TRY(gather_rows(ctx, table, a_rows, nullptr, ops));
+            TRY(gather_rows(ctx, table, b_rows, nullptr, ops + (size_t)nprod * 128 * L));
+            TRY(gf128_mul_dev(ctx, nprod, ops, ops + (size_t)nprod * 128 * L, table, &prow));
+        }
+    }
+    return TAC_OK;
+}
+
+// the GHASH key table of the single schedule (keyed false) or of the key table, built for `depth` powers
+int gcm_hash_key(tac_ctx* ctx, bool keyed, int depth, uint64_t* out_host) {
+    if (depth < 1 || depth > 1024 || (depth & (depth - 1))) return fail(ctx, TAC_ERR_ARG, "GHASH key depth must be a power of two in [1, 1024]");
+    if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
+    if (keyed ? ctx->n_keys < 1 : !ctx->key_sched)
+        return fail(ctx, TAC_ERR_STATE, keyed ? "no key table on the device (tac_aes_key_table or tac_aes_set_key_table)"
+                                              : "no key schedule on the device (tac_aes_set_key_schedule)");
+    TRY(aes_noise_check(ctx, 0, 10));
+    if (depth > 1) TRY(gf_noise_check(ctx));
+    tac_ctx::GcmTable& t = keyed ? ctx->gcm_h_keyed : ctx->gcm_h;
+    const int K = keyed ? ctx->n_keys : 1;
+    const size_t L = (size_t)ctx->big() + 1, bytes = (size_t)K * depth * 128 * L * 8;
+    t.valid = false;
+    if (t.buf.cap < bytes) {
+        if (t.buf.p) CU(cudaFree(t.buf.p));
+        t.buf.p = nullptr; t.buf.cap = 0;
+        if (cudaMalloc(&t.buf.p, bytes) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(ctx, TAC_ERR_CUDA, "a GHASH key table of " + std::to_string(K) + " keys × " + std::to_string(depth) + " powers (" +
+                                               std::to_string(bytes >> 20) + " MiB) does not fit in device memory");
+        }
+        t.buf.cap = bytes;
+    }
+    std::vector<int32_t> kidx(K);
+    for (int k = 0; k < K; k++) kidx[k] = k;
+    TRY(gcm_hash_key_build(ctx, keyed ? ctx->key_table.as<uint64_t>() : ctx->key_sched, keyed ? kidx.data() : nullptr, K, depth, t.buf.as<uint64_t>()));
+    if (out_host) CU(cudaMemcpyAsync(out_host, t.buf.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    t.depth = depth; t.n_keys = K; t.valid = true;
+    return TAC_OK;
+}
+
+// everything an AES-GCM call checks on the host before it enqueues anything; Σ p into *pt_bytes
+int gcm_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_bytes) {
+    if (n_msgs < 0) return fail(ctx, TAC_ERR_ARG, "negative n_msgs");
+    if (n_msgs > 0 && !msgs) return fail(ctx, TAC_ERR_ARG, "NULL messages");
+    *pt_bytes = 0;
+    for (int c = 0; c < n_msgs; c++) {
+        GcmShape s;
+        if (gcm_shape(msgs[c], s))
+            return fail(ctx, TAC_ERR_ARG, "AES-GCM record " + std::to_string(c) + ": need a 12-byte IV, a tag length in {4, 8, 12, 13, 14, 15, 16}, "
+                                          "data_len >= tag_len, a payload of at most 2^36 − 32 bytes, AAD below 2^61 bytes and no NULL pointer "
+                                          "with a non-zero length");
+        *pt_bytes += s.p;
+    }
+    TRY(aes_noise_check(ctx, 0, 10));
+    if (key_idx) {
+        TRY(key_table_check(ctx, AesDir::Forward, n_msgs, key_idx));
+    } else if (!ctx->key_sched) {
+        return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
+    }
+    if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
+    const tac_ctx::GcmTable& t = key_idx ? ctx->gcm_h_keyed : ctx->gcm_h;
+    if (!t.valid) return fail(ctx, TAC_ERR_STATE, key_idx ? "no GHASH key table for the resident key table (tac_aes_gcm_hash_key_table)"
+                                                          : "no GHASH key table for the resident key schedule (tac_aes_gcm_hash_key)");
+    return TAC_OK;
+}
+
+// AES-GCM transciphering of n records.  1. One public-block call over J0 of every record (rows 0..n−1, sorted order) and
+// inc32^i(J0), i = 1..m, with XOR bytes C (the plaintext rows).  2. GHASH in Horner form over chunks of w blocks, the first
+// chunk the short one: Y_c = Y_(c−1) · H^w ⊕ Σ_(i in chunk c) X_i · H^(pos); records are sorted by chunk count, descending,
+// so step c runs over a prefix of them: one batched product (from step 1 on), then one linear layer whose rows are Y_c
+// (squared noise <= max) or, in a record's last step, the tag difference D = MSB_t(E(J0) ⊕ S) ⊕ T (bytes >= t trivial
+// zero).  3. CCM's three zero-test passes reduce D to the validity bit.
+int aes_gcm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out, uint64_t* valid_out) {
+    uint64_t pt_bytes = 0;
+    TRY(gcm_check(ctx, n_msgs, key_idx, msgs, &pt_bytes));
+    if ((n_msgs > 0 && !valid_out) || (pt_bytes > 0 && !pt_out)) return fail(ctx, TAC_ERR_ARG, "NULL output");
+    if (n_msgs == 0) return TAC_OK;
+    const tac_ctx::GcmTable& tab = key_idx ? ctx->gcm_h_keyed : ctx->gcm_h;
+    const int n = n_msgs, w = tab.depth, maxn = ctx->p.max_noise_sq;
+    std::vector<GcmShape> sh(n);
+    std::vector<int64_t> chunks(n);
+    for (int c = 0; c < n; c++) {
+        gcm_shape(msgs[c], sh[c]);
+        chunks[c] = (sh[c].M + w - 1) / w;
+    }
+    if (chunks.size() && *std::max_element(chunks.begin(), chunks.end()) > 1) TRY(gf_noise_check(ctx));
+    TRY(ensure_ccm_luts(ctx));
+    std::vector<int32_t> order(n), rank(n);
+    for (int c = 0; c < n; c++) order[c] = c;
+    std::stable_sort(order.begin(), order.end(), [&](int32_t a, int32_t b) { return chunks[a] > chunks[b]; });
+    for (int r = 0; r < n; r++) rank[order[r]] = r;
+    const size_t L = (size_t)ctx->big() + 1, byte_words = 8 * L, blk = 16 * byte_words;
+    // the public call: [J0 rows][counter rows of every record], sorted order
+    int64_t rows = n;
+    std::vector<int64_t> pt_row(n);
+    for (int r = 0; r < n; r++) { pt_row[order[r]] = rows; rows += sh[order[r]].m; }
+    std::vector<uint8_t> blocks((size_t)rows * 16), xr((size_t)rows * 16, 0);
+    std::vector<int32_t> kidx(key_idx ? rows : 0);
+    for (int r = 0; r < n; r++) {
+        const int c = order[r];
+        gcm_ctr_block(msgs[c], 1, &blocks[(size_t)r * 16]);
+        for (int64_t i = 1; i <= sh[c].m; i++) gcm_ctr_block(msgs[c], (uint32_t)(1 + i), &blocks[(size_t)(pt_row[c] + i - 1) * 16]);
+        if (sh[c].p) std::memcpy(&xr[(size_t)pt_row[c] * 16], msgs[c].data, (size_t)sh[c].p);
+        if (key_idx) {
+            kidx[r] = key_idx[c];
+            for (int64_t i = 0; i < sh[c].m; i++) kidx[(size_t)(pt_row[c] + i)] = key_idx[c];
+        }
+    }
+    TRY(ensure(ctx, ctx->gcm_pub, (size_t)rows * blk * 8));
+    TRY(ensure(ctx, ctx->gcm_dy, (size_t)2 * n * blk * 8));
+    TRY(ensure(ctx, ctx->ccm_work, (size_t)n * 18 * L * 8));
+    uint64_t* pub = ctx->gcm_pub.as<uint64_t>();
+    uint64_t* dy = ctx->gcm_dy.as<uint64_t>();             // [n][128]: D in caller order, then [n][128]: Y in sorted order
+    TRY(aes_blocks_dev(ctx, AesDir::Forward, key_idx ? ctx->key_table.as<uint64_t>() : ctx->key_sched, key_idx ? kidx.data() : nullptr, (int)rows, 10, 0,
+                       nullptr, blocks.data(), xr.data(), pub));
+    // GHASH steps
+    std::vector<std::vector<uint8_t>> X(n);
+    for (int c = 0; c < n; c++) {
+        X[c].resize((size_t)sh[c].M * 16);
+        gcm_ghash_blocks(msgs[c], sh[c], X[c].data());
+    }
+    const int64_t steps = chunks[order[0]];
+    for (int64_t s = 0; s < steps; s++) {
+        int a = 0;
+        while (a < n && chunks[order[a]] > s) a++;
+        if (s > 0) {
+            std::vector<uint32_t> hw((size_t)a * 128);
+            for (int r = 0; r < a; r++)
+                for (int j = 0; j < 128; j++)
+                    hw[(size_t)r * 128 + j] = (uint32_t)(((size_t)(key_idx ? key_idx[order[r]] : 0) * w + (w - 1)) * 128 + j);
+            TRY(ensure(ctx, ctx->gf_ops, (size_t)a * 128 * L * 8));
+            TRY(ensure(ctx, ctx->gf_prod, (size_t)a * 128 * L * 8));
+            TRY(gather_rows(ctx, tab.buf.as<uint64_t>(), hw, nullptr, ctx->gf_ops.as<uint64_t>()));
+            TRY(gf128_mul_dev(ctx, a, dy + (size_t)n * 128 * L, ctx->gf_ops.as<uint64_t>(), ctx->gf_prod.as<uint64_t>()));
+        }
+        std::vector<LinRow> lrows((size_t)a * 128);
+        std::vector<uint32_t> orow((size_t)a * 128);
+        for (int r = 0; r < a; r++) {
+            const int c = order[r];
+            const int64_t first = sh[c].M - (chunks[c] - 1) * w;                       // blocks in chunk 0
+            const int64_t b0 = s == 0 ? 0 : first + (s - 1) * w, b1 = s == 0 ? first : first + s * w;
+            std::vector<int> exps;
+            for (int64_t i = b0; i < b1; i++) exps.push_back((int)(b1 - i));
+            const uint64_t base = (uint64_t)(key_idx ? key_idx[c] : 0) * w * 128;
+            LinRow* rr = &lrows[(size_t)r * 128];
+            ghash_terms(&X[c][(size_t)b0 * 16], (int)(b1 - b0), exps.data(), 0, base, (int64_t)r << 20, rr);
+            const int64_t own = ((int64_t)r << 20) | 0xFFFFF;
+            for (int j = 0; j < 128; j++)
+                if (s > 0) rr[j].terms.push_back(LinTerm{lin_id(1, (size_t)r * 128 + j), 1, own});
+            const bool last = s == chunks[c] - 1;
+            for (int j = 0; j < 128; j++) {
+                orow[(size_t)r * 128 + j] = (uint32_t)(last ? (size_t)c * 128 + j : (size_t)(n + r) * 128 + j);
+                if (!last) continue;
+                if (j >= 8 * sh[c].t) { rr[j] = LinRow{}; continue; }
+                rr[j].terms.push_back(LinTerm{lin_id(2, (size_t)r * 128 + j), 9, own - 1});          // E(J0)
+                rr[j].cbit = (msgs[c].data[sh[c].p + j / 8] >> (7 - j % 8)) & 1;                    // T
+            }
+        }
+        LinPlan plan;
+        if (lin_plan_build(lrows, maxn, maxn, 3, plan)) return fail(ctx, TAC_ERR_NOISE, "GHASH: the sums do not fit max_noise_level_squared");
+        TRY(lin_run(ctx, plan, {tab.buf.as<uint64_t>(), ctx->gf_prod.p ? ctx->gf_prod.as<uint64_t>() : pub, pub}, &orow, dy));
+    }
+    uint64_t* zero = ctx->ccm_work.as<uint64_t>();          // [n][16][L]: byte b of D is zero
+    uint64_t* ones = zero + (size_t)n * 16 * L;              // [n][2][L]: bytes 0..7 / 8..15 all zero
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_zero8], 16 * n, dy, zero));
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones8], 2 * n, zero, ones));
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones2], n, ones, valid_out));
+    // plaintext: the first p bytes of a record's counter rows, contiguous, into its place in the caller's order
+    uint64_t off = 0;
+    for (int c = 0; c < n; c++) {
+        if (sh[c].p)
+            CU(cudaMemcpyAsync(pt_out + off * byte_words, pub + (size_t)pt_row[c] * blk, sh[c].p * byte_words * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+        off += sh[c].p;
+    }
+    return TAC_OK;
+}
+
 }  // namespace
 
 // =================================================================================================== C ABI
@@ -815,7 +1182,9 @@ void tac_ctx_destroy(tac_ctx* ctx) {
     for (auto& l : ctx->luts) cudaFree(l.dev);
     for (DevBuf* b : {&ctx->ws_in, &ctx->ws_out, &ctx->ws_small, &ctx->ws_ksdig, &ctx->ws_pbs, &ctx->ws_pfdig, &ctx->ws_ggsw, &ctx->ws_ggswf,
                       &ctx->ws_tree_a, &ctx->ws_tree_b, &ctx->ws_state, &ctx->ws_muls, &ctx->ws_misc, &ctx->ws_plan, &ctx->ws_rep,
-                      &ctx->key_table, &ctx->inv_key_table, &ctx->ccm_pub, &ctx->ccm_work, &ctx->ccm_desc})
+                      &ctx->key_table, &ctx->inv_key_table, &ctx->ccm_pub, &ctx->ccm_work, &ctx->ccm_desc, &ctx->gcm_h.buf,
+                      &ctx->gcm_h_keyed.buf, &ctx->lin_desc, &ctx->lin_sum, &ctx->lin_lvl, &ctx->gf_idx, &ctx->gf_box, &ctx->gf_ops,
+                      &ctx->gf_prod, &ctx->gcm_pub, &ctx->gcm_dy})
         if (b->p) cudaFree(b->p);
     for (auto& r : ctx->prof_pool) for (auto& ev : r.ev) cudaEventDestroy(ev);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -1129,6 +1498,7 @@ int tac_aes_set_key_schedule(tac_ctx* ctx, const uint64_t* ks_host) {
     const size_t bytes = (size_t)44 * 32 * (ctx->big() + 1) * 8;
     if (!ctx->key_sched) CU(cudaMalloc(&ctx->key_sched, bytes));
     ctx->inv_key_sched_valid = false;        // an inverse schedule belongs to the encryption schedule it was made from
+    ctx->gcm_h.valid = false;                // and so does a GHASH key table
     if (ks_host) {
         CU(cudaMemcpyAsync(ctx->key_sched, ks_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
@@ -1247,6 +1617,7 @@ int tac_aes_key_table(tac_ctx* ctx, int n_keys, const uint64_t* key_bits_host, u
     TRY(key_schedule_noise_check(ctx));
     ctx->n_keys = 0;
     ctx->inv_key_table_valid = false;
+    ctx->gcm_h_keyed.valid = false;
     TRY(alloc_key_table(ctx, ctx->key_table, n_keys));
     TRY(key_expand(ctx, n_keys, key_bits_host, ctx->key_table.as<uint64_t>()));
     if (key_scheds_host) CU(cudaMemcpyAsync(key_scheds_host, ctx->key_table.p, (size_t)n_keys * key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1260,6 +1631,7 @@ int tac_aes_set_key_table(tac_ctx* ctx, int n_keys, const uint64_t* key_scheds_h
     if (n_keys < 1 || !key_scheds_host) return fail(ctx, TAC_ERR_ARG, "need n_keys >= 1 and key schedules");
     ctx->n_keys = 0;
     ctx->inv_key_table_valid = false;
+    ctx->gcm_h_keyed.valid = false;
     TRY(alloc_key_table(ctx, ctx->key_table, n_keys));
     CU(cudaMemcpyAsync(ctx->key_table.p, key_scheds_host, (size_t)n_keys * key_sched_bytes(ctx), cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
@@ -1380,6 +1752,41 @@ int tac_aes_ccm_transcipher(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, co
     return TAC_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ AES-GCM transciphering
+int tac_aes_gcm_hash_key(tac_ctx* ctx, int depth, uint64_t* out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    return gcm_hash_key(ctx, false, depth, out_host);
+}
+int tac_aes_gcm_hash_key_table(tac_ctx* ctx, int depth, uint64_t* out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    return gcm_hash_key(ctx, true, depth, out_host);
+}
+int tac_aes_gcm_transcipher_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_dev,
+                                uint64_t* valid_out_dev) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    return aes_gcm_dev(ctx, n_msgs, key_idx, msgs, pt_out_dev, valid_out_dev);
+}
+int tac_aes_gcm_transcipher(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_host,
+                            uint64_t* valid_out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    uint64_t pt_bytes = 0;
+    TRY(gcm_check(ctx, n_msgs, key_idx, msgs, &pt_bytes));
+    if ((n_msgs > 0 && !valid_out_host) || (pt_bytes > 0 && !pt_out_host)) return fail(ctx, TAC_ERR_ARG, "NULL output");
+    if (n_msgs == 0) return TAC_OK;
+    const size_t L = (size_t)ctx->big() + 1, pt_words = (size_t)pt_bytes * 8 * L, valid_words = (size_t)n_msgs * L;
+    TRY(ensure(ctx, ctx->ws_out, (pt_words + valid_words) * 8));
+    uint64_t* pt = ctx->ws_out.as<uint64_t>();
+    TRY(aes_gcm_dev(ctx, n_msgs, key_idx, msgs, pt, pt + pt_words));
+    if (pt_words) CU(cudaMemcpyAsync(pt_out_host, pt, pt_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(valid_out_host, pt + pt_words, valid_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return TAC_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ single stages
 int tac_stage_keyswitch(tac_ctx* ctx, int n, const uint64_t* in_host, uint64_t* out_host) {
     LOCK(ctx);
@@ -1391,6 +1798,24 @@ int tac_stage_keyswitch(tac_ctx* ctx, int n, const uint64_t* in_host, uint64_t* 
     CU(cudaMemcpyAsync(ctx->ws_in.p, in_host, ib, cudaMemcpyHostToDevice, ctx->stream));
     TRY(stage_ks(ctx, ctx->ws_in.as<uint64_t>(), n, ctx->ws_small.as<uint64_t>()));
     CU(cudaMemcpyAsync(out_host, ctx->ws_small.p, ob, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return TAC_OK;
+}
+// n products a·b in GF(2^128) (GCM's field and bit order), a, b, out [n][128][kN+1]; outputs at squared noise 1
+int tac_gf128_mul(tac_ctx* ctx, int n, const uint64_t* a_host, const uint64_t* b_host, uint64_t* out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
+    if (n <= 0) return n == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative count");
+    if (!a_host || !b_host || !out_host) return fail(ctx, TAC_ERR_ARG, "NULL operand or output");
+    TRY(gf_noise_check(ctx));
+    const size_t words = (size_t)n * 128 * (ctx->big() + 1);
+    TRY(ensure(ctx, ctx->ws_in, 2 * words * 8));
+    TRY(ensure(ctx, ctx->ws_out, words * 8));
+    CU(cudaMemcpyAsync(ctx->ws_in.p, a_host, words * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(ctx->ws_in.as<uint64_t>() + words, b_host, words * 8, cudaMemcpyHostToDevice, ctx->stream));
+    TRY(gf128_mul_dev(ctx, n, ctx->ws_in.as<uint64_t>(), ctx->ws_in.as<uint64_t>() + words, ctx->ws_out.as<uint64_t>()));
+    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, words * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return TAC_OK;
 }

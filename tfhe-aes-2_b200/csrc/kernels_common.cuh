@@ -9,6 +9,7 @@
 //                          inputs and representative gathers of the public-block path; InvMixColumns of the inverse key
 //                          schedule (aes_inv_mix_key_kernel); the sums of a batched key-expansion step (aes_key_step_kernel)
 //   aes_ccm_*_kernel       AES-CCM: the CBC-MAC chain input X ⊕ B of one step, and the tag difference the tag check bootstraps
+//   lwe_gather_add_kernel  the linear layer of AES-GCM (aes_gcm.h): rows as sums of rows of several arrays, plus a constant bit
 //   lwe_add_kernel         leveled XOR (lwe_ciphertext_add_assign) over a batch; lwe_shl_kernel / lwe_sub_kernel: glue of extract_bits
 //   negate_kernel, dfma_peak_kernel   key-upload helper, FP64 peak microbenchmark (roofline denominator)
 #pragma once
@@ -252,6 +253,33 @@ __global__ void aes_ccm_tag_diff_kernel(const uint64_t* __restrict__ pub, const 
         const int byte = (int)(rem / byte_words);
         const size_t r = (size_t)rank[c];
         out[i] = byte < tag_len[c] ? pub[r * blk_words + rem] + pub[((size_t)n + r) * blk_words + rem] : 0ull;
+    }
+}
+
+// ================================================================================================ linear layer (aes_gcm.h)
+// the gather-add's inputs: any device ciphertext arrays [rows][L], addressed by a term's source (its top 3 bits).  The
+// output may lie in one of them when no row reads what another writes (out is not __restrict__).
+struct LinSrcs {
+    const uint64_t* p[8];
+};
+// out row r (at out_row[r] when given) = Σ_{t in [row_ptr[r], row_ptr[r+1])} row (terms[t] & 2^29−1) of source terms[t] >> 29,
+// mod 2^64, + 2^63 on the body when cbit[r] (a public constant bit: a trivial ciphertext).  A row without terms is a
+// trivial zero.  total = rows·L words.
+__global__ void lwe_gather_add_kernel(LinSrcs src, const uint32_t* __restrict__ row_ptr, const uint32_t* __restrict__ terms,
+                                      const uint8_t* __restrict__ cbit, const uint32_t* __restrict__ out_row, int L, size_t total,
+                                      uint64_t* out) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t r = i / L; const size_t e = i - r * L;
+        uint64_t v = 0;
+        for (uint32_t t = row_ptr[r], end = row_ptr[r + 1]; t < end; t++) {
+            const uint32_t id = __ldg(terms + t), k = id >> 29;
+            const uint64_t* base = src.p[0];
+#pragma unroll
+            for (uint32_t q = 1; q < 8; q++) base = k == q ? src.p[q] : base;      // selects: an indexed parameter would go to the stack
+            v += base[(size_t)(id & ((1u << 29) - 1)) * L + e];
+        }
+        if (cbit && cbit[r] && e == (size_t)L - 1) v += 1ull << 63;
+        out[(out_row ? (size_t)out_row[r] : r) * L + e] = v;
     }
 }
 

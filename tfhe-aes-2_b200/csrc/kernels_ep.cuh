@@ -1,5 +1,5 @@
 // kernels_ep.cuh — the FFT / external-product kernels (templated on the polynomial size and GLWE dimension):
-// poly_fft_kernel, pbs_kernel, pbs_wide_kernel, pbs_merged_kernel, vp_kernel, cmux_tree_kernel.  Instantiated per shape in kernels_n512.cu / kernels_n1024.cu.
+// poly_fft_kernel, pbs_kernel, pbs_wide_kernel, pbs_merged_kernel, vp_kernel, vp_gather_kernel, cmux_tree_kernel.  Instantiated per shape in kernels_n512.cu / kernels_n1024.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include "ep_step.cuh"
@@ -432,6 +432,41 @@ vp_kernel(const cplx* __restrict__ ggsw_f, int n_in, int first_ggsw, const uint6
     for (int g = n_in - 1; g >= first_ggsw; g--) {
         const int rot = 2 * N - deg;            // multiply by X^{-deg}
         ep_step_device<C, NT>(tid, sm, gbox + (size_t)g * ggsw_sz,
+                              [&](int job, int jj, uint64_t& x0, uint64_t& x1) { rot_diff_pair<N>(sm.acc + (size_t)job * N, jj, rot, x0, x1); }, base_log, outr);
+        deg <<= 1;
+    }
+    __syncthreads();
+    pbs_epilogue<C, NT>(tid, sm.acc, out, box, o0, n_out, 0);
+}
+
+// Vertical packing over GGSWs picked by index: box b's input g is GGSW ggsw_idx[b·n_in + g] of ggsw_f ([][L][G][G][M]), so
+// boxes may share GGSWs (the 4×4-bit boxes of a GF(2^128) product read each operand bit's GGSW 32 times).  No CMux tree
+// (n_in <= log2 N): the accumulator starts from the trivial GLWE of LUT polynomial o, and the steps are vp_kernel's.
+template <int N, int K, int L, int B, int NT>
+__global__ void __launch_bounds__(NT, 1)
+vp_gather_kernel(const cplx* __restrict__ ggsw_f, const int32_t* __restrict__ ggsw_idx, int n_in, const uint64_t* __restrict__ lut,
+                 size_t lut_stride, int n_out, int base_log, const cplx* __restrict__ g_wT, uint64_t* __restrict__ out) {
+    typedef EpCfg<N, K, L, B> C;
+    typedef MacCfg<C, NT> MC;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    EpSmem<C> sm(smem_raw);
+    const int tid = threadIdx.x;
+    const int box = blockIdx.y, o0 = blockIdx.x * B;
+    for (int i = tid; i < tab_len(C::N); i += NT) sm.wT[i] = g_wT[i];
+    for (int idx = tid; idx < (int)C::acc_words; idx += NT) {
+        const int b = idx / (C::G * N), rem = idx - b * C::G * N, p = rem / N, j = rem - p * N;
+        const int o = o0 + b;
+        sm.acc[idx] = (o < n_out && p == K) ? lut[(size_t)o * lut_stride + j] : 0ull;
+    }
+    __syncthreads();
+    cplx outr[MC::SPT][B][C::G];
+    zero_fourier_acc(outr);
+    const size_t ggsw_sz = (size_t)L * C::G * C::G * C::M;
+    const int32_t* gidx = ggsw_idx + (size_t)box * n_in;
+    int deg = 1;
+    for (int g = n_in - 1; g >= 0; g--) {
+        const int rot = 2 * N - deg;            // multiply by X^{-deg}
+        ep_step_device<C, NT>(tid, sm, ggsw_f + (size_t)__ldg(gidx + g) * ggsw_sz,
                               [&](int job, int jj, uint64_t& x0, uint64_t& x1) { rot_diff_pair<N>(sm.acc + (size_t)job * N, jj, rot, x0, x1); }, base_log, outr);
         deg <<= 1;
     }

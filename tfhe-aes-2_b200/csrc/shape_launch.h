@@ -24,6 +24,10 @@ struct ShapeOps {
     // cudaErrorInvalidValue if that level count is not instantiated
     cudaError_t (*vp)(const KLaunch&, int levels, const double2* ggsw_f, int nbox, int n_in, int first, const uint64_t* lut, size_t lut_stride,
                       const uint64_t* init_glwe, int n_out, int base_log, uint64_t* out);
+    // vertical packing with box b's input g read from GGSW ggsw_idx[b·n_in + g] (device array); n_in <= log2 N, else
+    // cudaErrorInvalidValue
+    cudaError_t (*vp_gather)(const KLaunch&, int levels, const double2* ggsw_f, const int32_t* ggsw_idx, int nbox, int n_in, const uint64_t* lut,
+                             size_t lut_stride, int n_out, int base_log, uint64_t* out);
     // one CMux-tree layer
     cudaError_t (*tree)(const KLaunch&, int levels, const double2* ggsw_f, int nbox, int n_in, int ggsw_idx, const uint64_t* lut, size_t lut_stride,
                         const uint64_t* node_in, int n_nodes_in, int n_out, int base_log, uint64_t* node_out);

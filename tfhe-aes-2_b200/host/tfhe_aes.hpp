@@ -461,6 +461,35 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
         }
         return res;
     }
+    // AES-GCM transciphering with the tag checked under FHE (NIST SP 800-38D, 96-bit IVs; the reference has none).  A record
+    // is a CcmRecord with nonce = the 12-byte IV and data = C ‖ T.  Needs the GHASH key table of the schedule in use
+    // (gcm_hash_key / gcm_hash_key_table).  Outputs and noise as ccm_transcipher.
+    static void gcm_hash_key(const Ctx& c, int depth = 8) { c.check(tac_aes_gcm_hash_key(c.raw(), depth, nullptr)); }
+    static void gcm_hash_key_table(const Ctx& c, int depth = 8) { c.check(tac_aes_gcm_hash_key_table(c.raw(), depth, nullptr)); }
+    static std::vector<std::pair<std::vector<Byte>, BitCt>> gcm_transcipher(const Ctx& c, const std::vector<CcmRecord>& records,
+                                                                             const std::vector<int32_t>& key_idx = {}) {
+        if (!key_idx.empty() && key_idx.size() != records.size()) throw std::invalid_argument("key_idx: one key index per record");
+        std::vector<tac_ccm_msg> msgs(records.size());
+        std::vector<size_t> off(records.size() + 1, 0);
+        for (size_t i = 0; i < records.size(); i++) {
+            const CcmRecord& r = records[i];
+            msgs[i] = tac_ccm_msg{r.nonce.data(), (int32_t)r.nonce.size(), r.tag_len, r.aad.data(), r.aad.size(), r.data.data(), r.data.size()};
+            off[i + 1] = off[i] + (r.data.size() >= (size_t)std::max(r.tag_len, 0) ? r.data.size() - r.tag_len : 0);
+        }
+        const size_t L = c.lwe_size();
+        std::vector<uint64_t> pt(off.back() * 8 * L), valid(records.size() * L);
+        c.check(tac_aes_gcm_transcipher(c.raw(), (int)records.size(), key_idx.empty() ? nullptr : key_idx.data(), msgs.data(), pt.data(), valid.data()));
+        auto bit = [&](const std::vector<uint64_t>& v, size_t idx, uint64_t noise) {
+            return BitCt::with_noise_level(std::vector<uint64_t>(v.begin() + idx * L, v.begin() + (idx + 1) * L), noise, c);
+        };
+        std::vector<std::pair<std::vector<Byte>, BitCt>> res;
+        for (size_t i = 0; i < records.size(); i++) {
+            std::vector<Byte> bytes(off[i + 1] - off[i]);
+            for (size_t b = 0; b < bytes.size(); b++) for (int j = 0; j < 8; j++) bytes[b][j] = bit(pt, (off[i] + b) * 8 + j, 8 + 1);
+            res.emplace_back(std::move(bytes), bit(valid, i, 2));
+        }
+        return res;
+    }
 
 private:
     static std::vector<data_model::BlockT<Bit>> public_blocks_keyed(int (*fn)(tac_ctx*, int, int, const int32_t*, const uint8_t*, const uint8_t*, uint64_t*),
