@@ -304,4 +304,6 @@ def test_state_rules(tac, ck64, client, ol):
     assert L.tac_aes_set_key_table(ctx.h, 0, out.ctypes.data) == TAC_ERR_ARG
     assert L.tac_aes_key_table(ctx.h, 0, out.ctypes.data, None) == TAC_ERR_ARG
     assert L.tac_aes_set_inv_key_table(ctx.h, None) == TAC_ERR_ARG
+    assert L.tac_aes_key_schedule(ctx.h, None, None) == TAC_ERR_ARG
     assert ctx.launch_count() == launches
+    assert_words_equal(ctx.aes_encrypt_public_blocks(counters(1, 2), rounds=1), before, "single-key output after NULL key bits")

@@ -994,24 +994,25 @@ class FheContext(NoiseContext):
         of (nonce, P, aad) returns, with a tag of tag_len bytes.  Returns (FHE encryptions of the plaintext bits
         [len(data) − tag_len][8][big+1], an encrypted validity bit [big+1]: 1 exactly when the tag is genuine).  The
         plaintext comes back whatever the tag; acting on the validity bit is the caller's business."""
-        return self._aes_ccm([(nonce, data, tag_len, aad)], None)[0]
+        return self._aes_records(self.L.tac_aes_ccm_transcipher, _ccm_messages, [(nonce, data, tag_len, aad)], None)[0]
 
     def aes_ccm_transcipher_many(self, messages):
         """aes_ccm_transcipher for many senders in one call: messages = [(key_index, nonce, data, tag_len, aad)], each
         under key table entry key_index.  Returns one (plaintext bits, validity bit) pair per message."""
         messages = list(messages)
         k = _key_index([m[0] for m in messages], len(messages), self.n_keys)
-        return self._aes_ccm([m[1:] for m in messages], k)
+        return self._aes_records(self.L.tac_aes_ccm_transcipher, _ccm_messages, [m[1:] for m in messages], k)
 
-    def _aes_ccm(self, messages, key_index):
-        msgs, keep, sizes = _ccm_messages(messages)
+    def _aes_records(self, fn, build, messages, key_index):
+        """fn (tac_aes_ccm_transcipher / tac_aes_gcm_transcipher) over the records that build (_ccm_messages /
+        _gcm_messages) makes of messages; one (plaintext bits, validity bit) pair per record"""
+        msgs, keep, sizes = build(messages)
         if not sizes:
             return []
         L1 = self.params.big_lwe_size
         pt = np.empty((sum(sizes), 8, L1), dtype=np.uint64)
         valid = np.empty((len(sizes), L1), dtype=np.uint64)
-        self._check(self.L.tac_aes_ccm_transcipher(self.h, len(sizes), None if key_index is None else key_index.ctypes.data, msgs,
-                                                   pt.ctypes.data, valid.ctypes.data))
+        self._check(fn(self.h, len(sizes), None if key_index is None else key_index.ctypes.data, msgs, pt.ctypes.data, valid.ctypes.data))
         offs = np.cumsum([0] + sizes)
         return [(pt[offs[i]:offs[i + 1]], valid[i]) for i in range(len(sizes))]
 
@@ -1036,26 +1037,14 @@ class FheContext(NoiseContext):
         """Transciphering of one AES-GCM record under the resident key schedule and its GHASH key table: `data` = C ‖ T is
         what AES-GCM encryption of (iv, P, aad) returns.  Returns (FHE encryptions of the plaintext bits
         [len(data) − tag_len][8][big+1], an encrypted validity bit [big+1]: 1 exactly when the tag is genuine)."""
-        return self._aes_gcm([(iv, data, tag_len, aad)], None)[0]
+        return self._aes_records(self.L.tac_aes_gcm_transcipher, _gcm_messages, [(iv, data, tag_len, aad)], None)[0]
 
     def aes_gcm_transcipher_many(self, messages):
         """aes_gcm_transcipher for many senders in one call: messages = [(key_index, iv, data, tag_len, aad)], each under
         key table entry key_index.  Returns one (plaintext bits, validity bit) pair per record."""
         messages = list(messages)
         k = _key_index([m[0] for m in messages], len(messages), self.n_keys)
-        return self._aes_gcm([m[1:] for m in messages], k)
-
-    def _aes_gcm(self, messages, key_index):
-        msgs, keep, sizes = _gcm_messages(messages)
-        if not sizes:
-            return []
-        L1 = self.params.big_lwe_size
-        pt = np.empty((sum(sizes), 8, L1), dtype=np.uint64)
-        valid = np.empty((len(sizes), L1), dtype=np.uint64)
-        self._check(self.L.tac_aes_gcm_transcipher(self.h, len(sizes), None if key_index is None else key_index.ctypes.data, msgs,
-                                                   pt.ctypes.data, valid.ctypes.data))
-        offs = np.cumsum([0] + sizes)
-        return [(pt[offs[i]:offs[i + 1]], valid[i]) for i in range(len(sizes))]
+        return self._aes_records(self.L.tac_aes_gcm_transcipher, _gcm_messages, [m[1:] for m in messages], k)
 
     def gf128_mul(self, a, b):
         """encrypted products a·b in GF(2^128) (GCM's field and bit order): a, b [n][128][big+1] → [n][128][big+1], output

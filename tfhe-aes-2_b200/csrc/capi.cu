@@ -28,10 +28,33 @@ namespace {
 // last error of the calling thread (entry points may be used from many threads; a per-context string would race)
 thread_local std::string g_error;
 
+// device memory owned by the context: freed when the buffer is, or when ensure() replaces it by a larger one
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+    ~DevBuf() { if (p) cudaFree(p); }
     template <class T> T* as() const { return reinterpret_cast<T*>(p); }
+};
+
+// AES-GCM: the GHASH key table H^1..H^depth [K][depth][128][kN+1] of a key set, valid while its schedules are resident
+struct GcmTable { DevBuf buf; int depth = 0; bool valid = false; };
+
+// A set of resident AES-128 key schedules: the single schedule (n = 1) or the key table (n entries), each with its inverse
+// schedules and its GHASH key table.  w [n][44 words][4][8][kN+1]; dk, the equivalent inverse cipher's schedules, same
+// layout, valid while made from (or uploaded for) the resident w.  n = 0: absent.  Writing w sets n = 0 and marks dk and
+// the GHASH table stale first; n is set once w is complete.  The state errors name the calls that fix them.
+struct KeySet {
+    DevBuf w, dk;
+    int n = 0;
+    bool dk_valid = false;
+    GcmTable gcm;
+    const char *absent, *no_dk, *no_gcm;
+    KeySet(const char* absent, const char* no_dk, const char* no_gcm) : absent(absent), no_dk(no_dk), no_gcm(no_gcm) {}
 };
 
 struct Lut {
@@ -72,17 +95,14 @@ struct tac_ctx {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     // keys
-    cplx* bsk_f = nullptr;
-    uint64_t* ksk = nullptr;
-    uint64_t* pfpksk = nullptr;
-    uint64_t* ks_corr = nullptr;
-    uint64_t* pfks_corr = nullptr;
-    uint8_t* ks_planes = nullptr;        // byte planes of the KSK
-    uint8_t* pfks_planes = nullptr;      // byte-plane tiles of the PFPKSK for the tcgen05 GEMM (kernels_gemm_umma.cuh)
-    uint32_t* pfks_fix = nullptr;        // [0] = count, then uint2 (ct, k) entries
+    DevBuf bsk_f;                        // cplx
+    DevBuf ksk, pfpksk, ks_corr, pfks_corr;
+    DevBuf ks_planes;                    // byte planes of the KSK
+    DevBuf pfks_planes;                  // byte-plane tiles of the PFPKSK for the tcgen05 GEMM (kernels_gemm_umma.cuh)
+    DevBuf pfks_fix;                     // uint32: [0] = count, then uint2 (ct, k) entries
     bool keys_allocated = false, keys_valid = false;
     // tables
-    cplx* wT = nullptr;            // combined twist/twiddle table (ep_core.cuh)
+    DevBuf wT;                     // cplx: combined twist/twiddle table (ep_core.cuh)
     const ShapeOps* ops = nullptr; // kernels of this (N, k)
     // LUTs
     std::vector<Lut> luts;
@@ -90,27 +110,22 @@ struct tac_ctx {
     int aes_lut_inv32 = -1, aes_lut_inv8 = -1, aes_lut_key32 = -1;   // decryption: InvS·{14,11,13,9}, InvS, b·{14,11,13,9}
     int ccm_lut_zero8 = -1, ccm_lut_ones8 = -1, ccm_lut_ones2 = -1;   // AES-CCM tag check: byte == 0, 8 bits all 1, 2 bits all 1
     int gf_lut_mul = -1;                 // GF(2^128) product: 8 → 7 carry-less product of two 4-bit polynomials
-    // AES key schedule
-    uint64_t* key_sched = nullptr;
-    uint64_t* inv_key_sched = nullptr;   // equivalent inverse cipher's schedule dk, same layout [44 words][4][8][kN+1]
-    bool inv_key_sched_valid = false;    // dk belongs to the resident key_sched (cleared by tac_aes_set_key_schedule)
-    uint64_t* rc_rows = nullptr;     // trivial(RC[1..10]) as byte ciphertexts [10][8][kN+1], uploaded once
-    // AES under many keys: a table of n_keys schedules [n_keys][44 words][4][8][kN+1] and their inverse schedules, apart
-    // from the single schedule above (neither replaces the other)
-    DevBuf key_table, inv_key_table;
-    int n_keys = 0;                      // 0: no key table
-    bool inv_key_table_valid = false;    // inv_key_table belongs to the resident key_table
+    // AES keys: the single schedule and, for AES under many keys, a table of schedules; neither replaces the other
+    KeySet single{"no key schedule on the device (tac_aes_set_key_schedule)",
+                  "no inverse key schedule for the resident key schedule (tac_aes_inv_key_schedule or tac_aes_set_inv_key_schedule)",
+                  "no GHASH key table for the resident key schedule (tac_aes_gcm_hash_key)"};
+    KeySet table{"no key table on the device (tac_aes_key_table or tac_aes_set_key_table)",
+                 "no inverse key table for the resident key table (tac_aes_inv_key_table or tac_aes_set_inv_key_table)",
+                 "no GHASH key table for the resident key table (tac_aes_gcm_hash_key_table)"};
+    DevBuf rc_rows;                  // trivial(RC[1..10]) as byte ciphertexts [10][8][kN+1], uploaded once
     // workspace
     DevBuf ws_in, ws_out, ws_small, ws_ksdig, ws_pbs, ws_pfdig, ws_ggsw, ws_ggswf, ws_tree_a, ws_tree_b, ws_state, ws_muls, ws_misc;
     DevBuf ws_plan, ws_rep;          // public-block AES: uploaded plan tables / public bytes, compact S-box inputs
     // AES-CCM, apart from the buffers aes_blocks_dev reuses on every call: the public call's output (rows 0..n−1 are the
     // CBC-MAC chain state), the chain input / tag check, and the descriptors of all steps
     DevBuf ccm_pub, ccm_work, ccm_desc;
-    // AES-GCM: the GHASH key tables H^1..H^depth [K][depth][128][kN+1] of the single schedule and of the key table (valid
-    // while the schedule / key table they were made from is resident); the linear layer's descriptors, group sums and
-    // level outputs; the product's GGSW index table, box outputs and operands; a transciphering call's buffers
-    struct GcmTable { DevBuf buf; int depth = 0, n_keys = 0; bool valid = false; };
-    GcmTable gcm_h, gcm_h_keyed;
+    // AES-GCM: the linear layer's descriptors, group sums and level outputs; the product's GGSW index table, box outputs
+    // and operands; a transciphering call's buffers
     DevBuf lin_desc, lin_sum, lin_lvl, gf_idx, gf_box, gf_ops, gf_prod, gcm_pub, gcm_dy;
     int gf_idx_np = 0;                   // products per pass gf_idx was built for
     size_t max_cts = 16384;
@@ -147,11 +162,15 @@ int fail(tac_ctx*, int code, const std::string& msg) {
         if (rc__) return rc__; \
     } while (0)
 
-int ensure(tac_ctx* ctx, DevBuf& b, size_t bytes) {
+// room for `bytes` in b (contents not kept when it grows); `what` names the buffer in the error text
+int ensure(tac_ctx* ctx, DevBuf& b, size_t bytes, const char* what = "a device buffer") {
     if (b.cap >= bytes) return TAC_OK;
-    if (b.p) CU(cudaFree(b.p));
-    b.p = nullptr; b.cap = 0;
-    CU(cudaMalloc(&b.p, bytes));
+    b = DevBuf();
+    if (cudaMalloc(&b.p, bytes) != cudaSuccess) {
+        cudaGetLastError();          // clear the allocation error so that the next launch check does not report it
+        b.p = nullptr;
+        return fail(ctx, TAC_ERR_CUDA, std::string(what) + " (" + std::to_string(bytes >> 20) + " MiB) does not fit in device memory");
+    }
     b.cap = bytes;
     return TAC_OK;
 }
@@ -188,7 +207,7 @@ std::string unsupported_params(const TacParams& p) {
 }
 
 // ---------------------------------------------------------------------------------------------- launch wrappers
-KLaunch klaunch(tac_ctx* ctx) { return KLaunch{ctx->stream, ctx->wT, ctx->sm_count}; }
+KLaunch klaunch(tac_ctx* ctx) { return KLaunch{ctx->stream, ctx->wT.as<cplx>(), ctx->sm_count}; }
 int check_launch(tac_ctx* ctx, cudaError_t e, const char* what) {
     ctx->launches++;
     if (e == cudaErrorInvalidValue) return fail(ctx, TAC_ERR_ARG, std::string(what) + ": unsupported level count / shape for this parameter set");
@@ -219,7 +238,7 @@ int pbs(tac_ctx* ctx, const uint64_t* small, int nct, uint64_t* out, uint64_t al
     if (nct == 0) return TAC_OK;
     const TacParams& p = ctx->p;
     if (alpha == 0) alpha = 1ull << (63 - p.cbs_b * p.cbs_l);
-    return check_launch(ctx, ctx->ops->pbs(klaunch(ctx), p.pbs_l, small, nct, p.n, ctx->bsk_f, p.pbs_b, alpha, out), "pbs kernel");
+    return check_launch(ctx, ctx->ops->pbs(klaunch(ctx), p.pbs_l, small, nct, p.n, ctx->bsk_f.as<cplx>(), p.pbs_b, alpha, out), "pbs kernel");
 }
 
 // vertical packing of `nbox` boxes from Fourier GGSWs ([nbox][n_in][cbs_l][G][G][M]) → out [nbox][n_out][big+1]
@@ -279,34 +298,37 @@ int stage_ks(tac_ctx* ctx, const uint64_t* in, int nct, uint64_t* small) {
     const int W = p.n + 1, mpad = ((nct + UG_MT - 1) / UG_MT) * UG_MT;
     TRY(ensure(ctx, ctx->ws_ksdig, (size_t)nkb * 2 * mpad * 16));
     uint8_t* DA = ctx->ws_ksdig.as<uint8_t>();
+    uint32_t* fix = ctx->pfks_fix.as<uint32_t>();
     umma_digit_tiles_kernel<<<grid1d((size_t)mpad * nkb * 2, 256, ctx->sm_count), 256, 0, ctx->stream>>>(
-        in, nct, mpad, big + 1, p.ks_b, p.ks_l, Kd, nkb, 1, DA, ctx->pfks_fix, reinterpret_cast<uint2*>(ctx->pfks_fix + 2), 0);
+        in, nct, mpad, big + 1, p.ks_b, p.ks_l, Kd, nkb, 1, DA, fix, reinterpret_cast<uint2*>(fix + 2), 0);
     TRY(post_launch(ctx, "umma_digit_tiles_kernel(ks)"));
-    return gemm_umma<1>(ctx, DA, nct, ctx->ks_planes, W, 1, nkb, ctx->ks_corr, in + big, (size_t)big + 1, small);
+    return gemm_umma<1>(ctx, DA, nct, ctx->ks_planes.as<uint8_t>(), W, 1, nkb, ctx->ks_corr.as<uint64_t>(), in + big, (size_t)big + 1, small);
 }
 // PFKS with all k+1 keys on the tensor cores: in [nct][big+1] → ggsw_std [nct][G][G·N]
 int stage_pfks(tac_ctx* ctx, const uint64_t* in, int nct, uint64_t* ggsw) {
     const TacParams& p = ctx->p;
     const int big1 = ctx->big() + 1, Kd = big1 * p.pfks_l, nkb = (Kd + UG_KB - 1) / UG_KB;
     const int W = ctx->G() * p.N, mpad = ((nct + UG_MT - 1) / UG_MT) * UG_MT;
+    const uint64_t* pfpksk = ctx->pfpksk.as<uint64_t>();
+    uint32_t* fix = ctx->pfks_fix.as<uint32_t>();
     if (p.pfks_b > 16) {       // digits wider than 16 bits (params_sqrd_lvl_1: base 2^24): 64-bit integer-pipe GEMM
         TRY(ensure(ctx, ctx->ws_pfdig, (size_t)nct * Kd * 4));
         pfks_digits_kernel<<<grid1d((size_t)nct * big1, 256, ctx->sm_count), 256, 0, ctx->stream>>>(in, nct, big1, p.pfks_b, p.pfks_l, ctx->ws_pfdig.as<uint32_t>());
         TRY(post_launch(ctx, "pfks_digits_kernel"));
-        return gemm(ctx, ctx->ws_pfdig.as<uint32_t>(), nct, Kd, ctx->pfpksk, W, ctx->G(), ctx->pfks_corr, nullptr, 0, ggsw);
+        return gemm(ctx, ctx->ws_pfdig.as<uint32_t>(), nct, Kd, pfpksk, W, ctx->G(), ctx->pfks_corr.as<uint64_t>(), nullptr, 0, ggsw);
     }
     TRY(ensure(ctx, ctx->ws_pfdig, (size_t)2 * nkb * 2 * mpad * 16));
-    CU(cudaMemsetAsync(ctx->pfks_fix, 0, 4, ctx->stream));
+    CU(cudaMemsetAsync(fix, 0, 4, ctx->stream));
     uint8_t* DA = ctx->ws_pfdig.as<uint8_t>();
     umma_digit_tiles_kernel<<<grid1d((size_t)mpad * nkb * 2, 256, ctx->sm_count), 256, 0, ctx->stream>>>(
-        in, nct, mpad, big1, p.pfks_b, p.pfks_l, Kd, nkb, 0, DA, ctx->pfks_fix, reinterpret_cast<uint2*>(ctx->pfks_fix + 2), ctx->fix_cap);
+        in, nct, mpad, big1, p.pfks_b, p.pfks_l, Kd, nkb, 0, DA, fix, reinterpret_cast<uint2*>(fix + 2), ctx->fix_cap);
     TRY(post_launch(ctx, "umma_digit_tiles_kernel(pfks)"));
-    TRY(gemm_umma<2>(ctx, DA, nct, ctx->pfks_planes, W, ctx->G(), nkb, ctx->pfks_corr, nullptr, 0, ggsw));
-    pfks_fixup_kernel<<<64, 256, 0, ctx->stream>>>(ctx->pfks_fix, reinterpret_cast<const uint2*>(ctx->pfks_fix + 2), ctx->fix_cap, ctx->pfpksk, Kd, W, ctx->G(), ggsw);
+    TRY(gemm_umma<2>(ctx, DA, nct, ctx->pfks_planes.as<uint8_t>(), W, ctx->G(), nkb, ctx->pfks_corr.as<uint64_t>(), nullptr, 0, ggsw));
+    pfks_fixup_kernel<<<64, 256, 0, ctx->stream>>>(fix, reinterpret_cast<const uint2*>(fix + 2), ctx->fix_cap, pfpksk, Kd, W, ctx->G(), ggsw);
     TRY(post_launch(ctx, "pfks_fixup_kernel"));
     // more ties than the list holds (crafted / trivial inputs): this kernel re-derives them all; otherwise it returns at once
     pfks_fixup_scan_kernel<<<dim3((ctx->G() * W + 255) / 256, std::min(nct, 2 * ctx->sm_count)), 256, 0, ctx->stream>>>(
-        ctx->pfks_fix, ctx->fix_cap, in, nct, big1, p.pfks_b, p.pfks_l, ctx->pfpksk, Kd, W, ctx->G(), ggsw);
+        fix, ctx->fix_cap, in, nct, big1, p.pfks_b, p.pfks_l, pfpksk, Kd, W, ctx->G(), ggsw);
     return post_launch(ctx, "pfks_fixup_scan_kernel");
 }
 
@@ -548,59 +570,44 @@ int aes_blocks_dev(tac_ctx* ctx, AesDir dir, const uint64_t* keys, const int32_t
     return post_launch(ctx, "aes_final_round_kernel");
 }
 
-// host-buffer form of an AES _dev entry point: ciphertext input (ct_in) through ws_in, the output through ws_out;
-// dev_call(in_dev, out_dev) runs the _dev entry point
-template <class DevCall>
-int aes_blocks_host(tac_ctx* ctx, int n_blocks, bool ct_in, const uint64_t* in_host, uint64_t* out_host, DevCall dev_call) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
-    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
-    if (ct_in) TRY(ensure(ctx, ctx->ws_in, bytes));
-    TRY(ensure(ctx, ctx->ws_out, bytes));
-    if (ct_in) CU(cudaMemcpyAsync(ctx->ws_in.p, in_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    TRY(dev_call(ctx->ws_in.as<const uint64_t>(), ctx->ws_out.as<uint64_t>()));
-    CU(cudaMemcpyAsync(out_host, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return TAC_OK;
-}
-
-// dk present and made from (or uploaded for) the resident encryption schedule
-int inv_key_sched_check(tac_ctx* ctx) {
-    if (!ctx->inv_key_sched || !ctx->inv_key_sched_valid)
-        return fail(ctx, TAC_ERR_STATE, "no inverse key schedule for the resident key schedule (tac_aes_inv_key_schedule or tac_aes_set_inv_key_schedule)");
-    return TAC_OK;
-}
-
 size_t key_sched_bytes(const tac_ctx* ctx) { return (size_t)44 * 32 * (ctx->big() + 1) * 8; }
 
-// room for n_keys schedules in a key table (contents not kept when it grows)
-int alloc_key_table(tac_ctx* ctx, DevBuf& b, int n_keys) {
-    const size_t bytes = (size_t)n_keys * key_sched_bytes(ctx);
-    if (b.cap >= bytes) return TAC_OK;
-    if (b.p) CU(cudaFree(b.p));
-    b.p = nullptr; b.cap = 0;
-    if (cudaMalloc(&b.p, bytes) != cudaSuccess) {
-        cudaGetLastError();          // clear the allocation error so that the next launch check does not report it
-        b.p = nullptr;
-        return fail(ctx, TAC_ERR_CUDA, "a key table of " + std::to_string(n_keys) + " schedules (" + std::to_string(bytes >> 20) +
-                                           " MiB) does not fit in device memory");
-    }
-    b.cap = bytes;
+// The key set of a call, checked on the host before anything is enqueued: the single schedule, or (keyed) the key table
+// with an index in [0, n) for each of the n_items blocks or records.  Decrypting needs a valid dk, which the single set may
+// hold without its w (tac_aes_set_inv_key_schedule).
+int keys_for(tac_ctx* ctx, AesDir dir, bool keyed, const int32_t* key_idx, int n_items, KeySet** out) {
+    KeySet& ks = keyed ? ctx->table : ctx->single;
+    const bool inv = dir == AesDir::Inverse;
+    if (ks.n < 1 && (keyed || !inv)) return fail(ctx, TAC_ERR_STATE, ks.absent);
+    if (inv && !ks.dk_valid) return fail(ctx, TAC_ERR_STATE, ks.no_dk);
+    if (keyed && n_items > 0 && !key_idx) return fail(ctx, TAC_ERR_ARG, "NULL key index");
+    for (int b = 0; keyed && b < n_items; b++)
+        if (key_idx[b] < 0 || key_idx[b] >= ks.n)
+            return fail(ctx, TAC_ERR_ARG, "key index " + std::to_string(key_idx[b]) + " of block " + std::to_string(b) + " outside [0, " +
+                                              std::to_string(ks.n) + ")");
+    *out = &ks;
     return TAC_OK;
 }
 
-// the resident key table (and, decrypting, its inverse table) and a key index in [0, n_keys) for every block, checked on
-// the host before anything is enqueued
-int key_table_check(tac_ctx* ctx, AesDir dir, int n_blocks, const int32_t* key_idx) {
-    if (ctx->n_keys < 1) return fail(ctx, TAC_ERR_STATE, "no key table on the device (tac_aes_key_table or tac_aes_set_key_table)");
-    if (dir == AesDir::Inverse && !ctx->inv_key_table_valid)
-        return fail(ctx, TAC_ERR_STATE, "no inverse key table for the resident key table (tac_aes_inv_key_table or tac_aes_set_inv_key_table)");
-    if (n_blocks > 0 && !key_idx) return fail(ctx, TAC_ERR_ARG, "NULL key index");
-    for (int b = 0; b < n_blocks; b++)
-        if (key_idx[b] < 0 || key_idx[b] >= ctx->n_keys)
-            return fail(ctx, TAC_ERR_ARG, "key index " + std::to_string(key_idx[b]) + " of block " + std::to_string(b) + " outside [0, " +
-                                              std::to_string(ctx->n_keys) + ")");
+// Every AES block entry point: the keys of `dir` (keys_for), then aes_blocks_dev over ciphertexts `in`, or, with `in`
+// NULL, over public blocks_host.  host: `in` and `out` are host buffers, staged through ws_in and ws_out.
+int aes_call(tac_ctx* ctx, AesDir dir, bool keyed, const int32_t* key_idx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in,
+             const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out, bool host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    KeySet* ks;
+    TRY(keys_for(ctx, dir, keyed, key_idx, n_blocks, &ks));
+    const uint64_t* keys = (dir == AesDir::Forward ? ks->w : ks->dk).as<uint64_t>();
+    if (!host) return aes_blocks_dev(ctx, dir, keys, key_idx, n_blocks, rounds, in_noise_sq, in, blocks_host, xor_host, out);
+    if (n_blocks <= 0) return n_blocks == 0 ? TAC_OK : fail(ctx, TAC_ERR_ARG, "negative n_blocks");
+    const size_t bytes = (size_t)n_blocks * 128 * (ctx->big() + 1) * 8;
+    if (in) TRY(ensure(ctx, ctx->ws_in, bytes));
+    TRY(ensure(ctx, ctx->ws_out, bytes));
+    if (in) CU(cudaMemcpyAsync(ctx->ws_in.p, in, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    TRY(aes_blocks_dev(ctx, dir, keys, key_idx, n_blocks, rounds, in_noise_sq, in ? ctx->ws_in.as<uint64_t>() : nullptr, blocks_host, xor_host,
+                       ctx->ws_out.as<uint64_t>()));
+    CU(cudaMemcpyAsync(out, ctx->ws_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
     return TAC_OK;
 }
 
@@ -629,21 +636,21 @@ int key_expand(tac_ctx* ctx, int K, const uint64_t* key_bits_host, uint64_t* ek)
     CU(cudaMemcpy2DAsync(prev, word * 8, key_bits_host + 3 * word, 4 * word * 8, word * 8, (size_t)K, cudaMemcpyHostToDevice, ctx->stream));
     // trivial(RC) constants: body += encode_bit(1) on the set bits of RC[i/4], byte 0 (:154; Byte::trivial data_model.rs:35-43).
     // All ten rows are uploaded once per context, so the 40 steps below enqueue without a host synchronisation.
-    if (!ctx->rc_rows) {
+    if (!ctx->rc_rows.p) {
         static const uint8_t RC[11] = {0x00, 0x01, 0x02, 0x04, 0x08, 0x10, 0x20, 0x40, 0x80, 0x1B, 0x36};
         std::vector<uint64_t> rows((size_t)10 * byte, 0ull);
         for (int r = 1; r <= 10; r++)
             for (int bit = 0; bit < 8; bit++)
                 if (RC[r] & (0x80 >> bit)) rows[(size_t)(r - 1) * byte + (size_t)bit * L + (L - 1)] = tac_encode_bit(1);
-        CU(cudaMalloc(&ctx->rc_rows, rows.size() * 8));
-        CU(cudaMemcpy(ctx->rc_rows, rows.data(), rows.size() * 8, cudaMemcpyHostToDevice));
+        TRY(ensure(ctx, ctx->rc_rows, rows.size() * 8));
+        CU(cudaMemcpy(ctx->rc_rows.p, rows.data(), rows.size() * 8, cudaMemcpyHostToDevice));
     }
     const size_t total = (size_t)K * word;
     for (int i = 4; i < 44; i++) {
         const bool rot = i % 4 == 0;
         if (rot) TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut8], 4 * K, prev, sub));                                  // sub_word
         aes_key_step_kernel<<<grid1d(total, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ek, sched, i, rot ? sub : nullptr,
-                                                                                        ctx->rc_rows + (size_t)(i / 4 - 1) * byte, (int)L, total, acc);
+                                                                                        ctx->rc_rows.as<uint64_t>() + (size_t)(i / 4 - 1) * byte, (int)L, total, acc);
         TRY(post_launch(ctx, "aes_key_step_kernel"));
         TRY(wopbs_dev(ctx, ctx->luts[ctx->aes_lut1], 32 * K, acc, prev));                                          // boot_word → bootstrap_assign
         CU(cudaMemcpy2DAsync(ek + (size_t)i * word, sched * 8, prev, word * 8, word * 8, (size_t)K, cudaMemcpyDeviceToDevice, ctx->stream));
@@ -684,6 +691,62 @@ int inv_key_expand(tac_ctx* ctx, int K, const uint64_t* w, uint64_t* dk) {
     return TAC_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ key sets
+// w about to change: the set is absent, its dk and GHASH table stale, until the new w is complete
+void ks_reset(KeySet& ks) { ks.n = 0; ks.dk_valid = false; ks.gcm.valid = false; }
+
+// room for K schedules in w or dk (contents not kept when it grows; the single set's never grows, as K is 1)
+int ks_alloc(tac_ctx* ctx, DevBuf& b, int K) {
+    return ensure(ctx, b, (size_t)K * key_sched_bytes(ctx), ("a key set of " + std::to_string(K) + " schedules").c_str());
+}
+
+// K schedules [K][44 words][4][8][kN+1] from the host into w; w_host NULL: the caller fills w (tac_aes_key_schedule_buffer)
+int ks_set(tac_ctx* ctx, KeySet& ks, int K, const uint64_t* w_host) {
+    ks_reset(ks);
+    TRY(ks_alloc(ctx, ks.w, K));
+    if (w_host) {
+        CU(cudaMemcpyAsync(ks.w.p, w_host, (size_t)K * key_sched_bytes(ctx), cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+    }
+    ks.n = K;
+    return TAC_OK;
+}
+
+// w of K keys expanded on the device from their bits [K][128][kN+1] (key_expand); w_host: NULL or room for the schedules
+int ks_expand(tac_ctx* ctx, KeySet& ks, int K, const uint64_t* key_bits_host, uint64_t* w_host) {
+    TRY(key_schedule_noise_check(ctx));
+    ks_reset(ks);
+    TRY(ks_alloc(ctx, ks.w, K));
+    TRY(key_expand(ctx, K, key_bits_host, ks.w.as<uint64_t>()));
+    if (w_host) CU(cudaMemcpyAsync(w_host, ks.w.p, (size_t)K * key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ks.n = K;
+    return TAC_OK;
+}
+
+// dk of every schedule of the set, derived on the device (inv_key_expand); dk_host: NULL or room for them
+int ks_invert(tac_ctx* ctx, KeySet& ks, uint64_t* dk_host) {
+    if (ks.n < 1) return fail(ctx, TAC_ERR_STATE, ks.absent);
+    TRY(inv_key_schedule_noise_check(ctx));
+    ks.dk_valid = false;
+    TRY(ks_alloc(ctx, ks.dk, ks.n));
+    TRY(inv_key_expand(ctx, ks.n, ks.w.as<uint64_t>(), ks.dk.as<uint64_t>()));
+    if (dk_host) CU(cudaMemcpyAsync(dk_host, ks.dk.p, (size_t)ks.n * key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ks.dk_valid = true;
+    return TAC_OK;
+}
+
+// K inverse schedules from the host into dk
+int ks_set_inv(tac_ctx* ctx, KeySet& ks, int K, const uint64_t* dk_host) {
+    ks.dk_valid = false;
+    TRY(ks_alloc(ctx, ks.dk, K));
+    CU(cudaMemcpyAsync(ks.dk.p, dk_host, (size_t)K * key_sched_bytes(ctx), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    ks.dk_valid = true;
+    return TAC_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ AES-CCM
 // LUTs of the tag check, registered on the first AES-CCM call: 8 → 1 "byte is zero", 8 → 1 "all 8 bits set", 2 → 1 "both set"
 int ensure_ccm_luts(tac_ctx* ctx) {
@@ -697,26 +760,49 @@ int ensure_ccm_luts(tac_ctx* ctx) {
     return register_aes_lut(ctx, 2, 1, both, &ctx->ccm_lut_ones2);
 }
 
-// everything an AES-CCM call checks on the host before it enqueues anything; Σ p into *pt_bytes
-int ccm_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_bytes) {
+// The checks AES-CCM and AES-GCM make on the host before they enqueue anything: the records (shape: ccm_shape or
+// gcm_shape, bad_record the error text after "<what> <index>: "), Σ p into *pt_bytes, a middle round over chain inputs of
+// squared noise in_noise_sq, the keys (key_idx NULL: the single schedule) into *ks and the evaluation keys
+template <class Shape>
+int records_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, int (*shape)(const tac_ccm_msg&, Shape&),
+                  const char* what, const char* bad_record, int in_noise_sq, KeySet** ks, uint64_t* pt_bytes) {
     if (n_msgs < 0) return fail(ctx, TAC_ERR_ARG, "negative n_msgs");
     if (n_msgs > 0 && !msgs) return fail(ctx, TAC_ERR_ARG, "NULL messages");
     *pt_bytes = 0;
     for (int c = 0; c < n_msgs; c++) {
-        CcmShape s;
-        if (ccm_shape(msgs[c], s))
-            return fail(ctx, TAC_ERR_ARG, "AES-CCM message " + std::to_string(c) + ": need a nonce of 7..13 bytes, a tag length in {4, 6, …, 16}, "
-                                          "data_len >= tag_len, a payload below 2^(8q) bytes and no NULL pointer with a non-zero length");
+        Shape s;
+        if (shape(msgs[c], s)) return fail(ctx, TAC_ERR_ARG, std::string(what) + " " + std::to_string(c) + ": " + bad_record);
         *pt_bytes += s.p;
     }
-    TRY(aes_noise_check(ctx, 18, 10));           // a chain input X ⊕ P carries 18; a middle round 33
-    if (key_idx) {
-        TRY(key_table_check(ctx, AesDir::Forward, n_msgs, key_idx));
-    } else if (!ctx->key_sched) {
-        return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    }
+    TRY(aes_noise_check(ctx, in_noise_sq, 10));
+    TRY(keys_for(ctx, AesDir::Forward, key_idx != nullptr, key_idx, n_msgs, ks));
     if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
     return TAC_OK;
+}
+int outputs_check(tac_ctx* ctx, int n_msgs, uint64_t pt_bytes, const uint64_t* pt_out, const uint64_t* valid_out) {
+    if ((n_msgs > 0 && !valid_out) || (pt_bytes > 0 && !pt_out)) return fail(ctx, TAC_ERR_ARG, "NULL output");
+    return TAC_OK;
+}
+
+// every check of an AES-CCM call
+int ccm_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, const uint64_t* pt_out, const uint64_t* valid_out,
+              KeySet** ks, uint64_t* pt_bytes) {
+    TRY(records_check(ctx, n_msgs, key_idx, msgs, ccm_shape, "AES-CCM message",
+                      "need a nonce of 7..13 bytes, a tag length in {4, 6, …, 16}, data_len >= tag_len, a payload below 2^(8q) bytes and no "
+                      "NULL pointer with a non-zero length",
+                      18, ks, pt_bytes));           // a chain input X ⊕ P carries 18; a middle round 33
+    return outputs_check(ctx, n_msgs, *pt_bytes, pt_out, valid_out);
+}
+
+// The validity bits of n tags from their differences D [n][16][8][L] (1 exactly when D is all zero): byte == 0 over 16·n
+// bytes, all-8-set over 2·n groups, both-set over n pairs.  scratch: room for [n][16][L] + [n][2][L].
+int tag_validity(tac_ctx* ctx, int n, const uint64_t* diff, uint64_t* scratch, uint64_t* valid_out) {
+    const size_t L = (size_t)ctx->big() + 1;
+    uint64_t* zero = scratch;                                // [n][16][L]: byte b of D is zero
+    uint64_t* ones = zero + (size_t)n * 16 * L;              // [n][2][L]: bytes 0..7 / 8..15 all zero
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_zero8], 16 * n, diff, zero));
+    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones8], 2 * n, zero, ones));
+    return wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones2], n, ones, valid_out);
 }
 
 // AES-CCM transciphering of n messages (aes_ccm.h): one public-block AES call for B_0, A_0 and A_1..A_m of every message,
@@ -728,15 +814,15 @@ int ccm_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_ms
 // descriptors of all steps, the ranks and the tag lengths travel to the device in one upload into ccm_desc, since
 // aes_blocks_dev reuses ws_plan on every call.
 int aes_ccm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out, uint64_t* valid_out) {
-    uint64_t pt_bytes = 0;
-    TRY(ccm_check(ctx, n_msgs, key_idx, msgs, &pt_bytes));
-    if ((n_msgs > 0 && !valid_out) || (pt_bytes > 0 && !pt_out)) return fail(ctx, TAC_ERR_ARG, "NULL output");
+    KeySet* ks;
+    uint64_t pt_bytes;
+    TRY(ccm_check(ctx, n_msgs, key_idx, msgs, pt_out, valid_out, &ks, &pt_bytes));
     if (n_msgs == 0) return TAC_OK;
     TRY(ensure_ccm_luts(ctx));
     CcmPlan plan;
     ccm_plan_build(n_msgs, msgs, key_idx, plan);
     const int n = n_msgs;
-    const uint64_t* keys = key_idx ? ctx->key_table.as<uint64_t>() : ctx->key_sched;
+    const uint64_t* keys = ks->w.as<uint64_t>();
     const size_t L = (size_t)ctx->big() + 1, byte_words = 8 * L, blk = 16 * byte_words;
     const int64_t rows = (int64_t)(plan.pub_blocks.size() / 16);
     TRY(ensure(ctx, ctx->ccm_pub, (size_t)rows * blk * 8));
@@ -768,14 +854,10 @@ int aes_ccm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_
         d0 += (size_t)a;
     }
 
-    uint64_t* diff = work;                                   // [n][16][8][L]
-    uint64_t* zero = diff + (size_t)n * blk;                 // [n][16][L]: byte b of D is zero
-    uint64_t* ones = zero + (size_t)n * 16 * L;              // [n][2][L]: bytes 0..7 / 8..15 all zero
+    uint64_t* diff = work;                                   // [n][16][8][L], then tag_validity's scratch
     aes_ccm_tag_diff_kernel<<<grid1d((size_t)n * blk, 256, ctx->sm_count), 256, 0, ctx->stream>>>(pub, d_rank, d_tag_len, n, (int)L, (size_t)n * blk, diff);
     TRY(post_launch(ctx, "aes_ccm_tag_diff_kernel"));
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_zero8], 16 * n, diff, zero));
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones8], 2 * n, zero, ones));
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones2], n, ones, valid_out));
+    TRY(tag_validity(ctx, n, diff, diff + (size_t)n * blk, valid_out));
     // plaintext: the first p bytes of a message's A_1..A_m rows, contiguous, into its place in the caller's order
     for (int c = 0; c < n; c++)
         if (plan.shape[c].p)
@@ -964,62 +1046,37 @@ int gcm_hash_key_build(tac_ctx* ctx, const uint64_t* keys, const int32_t* key_id
     return TAC_OK;
 }
 
-// the GHASH key table of the single schedule (keyed false) or of the key table, built for `depth` powers
+// the GHASH key table of the single schedule or (keyed) of every key table entry, built for `depth` powers
 int gcm_hash_key(tac_ctx* ctx, bool keyed, int depth, uint64_t* out_host) {
     if (depth < 1 || depth > 1024 || (depth & (depth - 1))) return fail(ctx, TAC_ERR_ARG, "GHASH key depth must be a power of two in [1, 1024]");
     if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
-    if (keyed ? ctx->n_keys < 1 : !ctx->key_sched)
-        return fail(ctx, TAC_ERR_STATE, keyed ? "no key table on the device (tac_aes_key_table or tac_aes_set_key_table)"
-                                              : "no key schedule on the device (tac_aes_set_key_schedule)");
+    KeySet* ks;
+    TRY(keys_for(ctx, AesDir::Forward, keyed, nullptr, 0, &ks));
     TRY(aes_noise_check(ctx, 0, 10));
     if (depth > 1) TRY(gf_noise_check(ctx));
-    tac_ctx::GcmTable& t = keyed ? ctx->gcm_h_keyed : ctx->gcm_h;
-    const int K = keyed ? ctx->n_keys : 1;
+    GcmTable& t = ks->gcm;
+    const int K = ks->n;
     const size_t L = (size_t)ctx->big() + 1, bytes = (size_t)K * depth * 128 * L * 8;
     t.valid = false;
-    if (t.buf.cap < bytes) {
-        if (t.buf.p) CU(cudaFree(t.buf.p));
-        t.buf.p = nullptr; t.buf.cap = 0;
-        if (cudaMalloc(&t.buf.p, bytes) != cudaSuccess) {
-            cudaGetLastError();
-            return fail(ctx, TAC_ERR_CUDA, "a GHASH key table of " + std::to_string(K) + " keys × " + std::to_string(depth) + " powers (" +
-                                               std::to_string(bytes >> 20) + " MiB) does not fit in device memory");
-        }
-        t.buf.cap = bytes;
-    }
+    TRY(ensure(ctx, t.buf, bytes, ("a GHASH key table of " + std::to_string(K) + " keys × " + std::to_string(depth) + " powers").c_str()));
     std::vector<int32_t> kidx(K);
     for (int k = 0; k < K; k++) kidx[k] = k;
-    TRY(gcm_hash_key_build(ctx, keyed ? ctx->key_table.as<uint64_t>() : ctx->key_sched, keyed ? kidx.data() : nullptr, K, depth, t.buf.as<uint64_t>()));
+    TRY(gcm_hash_key_build(ctx, ks->w.as<uint64_t>(), keyed ? kidx.data() : nullptr, K, depth, t.buf.as<uint64_t>()));
     if (out_host) CU(cudaMemcpyAsync(out_host, t.buf.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
-    t.depth = depth; t.n_keys = K; t.valid = true;
+    t.depth = depth; t.valid = true;
     return TAC_OK;
 }
 
-// everything an AES-GCM call checks on the host before it enqueues anything; Σ p into *pt_bytes
-int gcm_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_bytes) {
-    if (n_msgs < 0) return fail(ctx, TAC_ERR_ARG, "negative n_msgs");
-    if (n_msgs > 0 && !msgs) return fail(ctx, TAC_ERR_ARG, "NULL messages");
-    *pt_bytes = 0;
-    for (int c = 0; c < n_msgs; c++) {
-        GcmShape s;
-        if (gcm_shape(msgs[c], s))
-            return fail(ctx, TAC_ERR_ARG, "AES-GCM record " + std::to_string(c) + ": need a 12-byte IV, a tag length in {4, 8, 12, 13, 14, 15, 16}, "
-                                          "data_len >= tag_len, a payload of at most 2^36 − 32 bytes, AAD below 2^61 bytes and no NULL pointer "
-                                          "with a non-zero length");
-        *pt_bytes += s.p;
-    }
-    TRY(aes_noise_check(ctx, 0, 10));
-    if (key_idx) {
-        TRY(key_table_check(ctx, AesDir::Forward, n_msgs, key_idx));
-    } else if (!ctx->key_sched) {
-        return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    }
-    if (!ctx->keys_valid) return fail(ctx, TAC_ERR_STATE, "evaluation keys not uploaded");
-    const tac_ctx::GcmTable& t = key_idx ? ctx->gcm_h_keyed : ctx->gcm_h;
-    if (!t.valid) return fail(ctx, TAC_ERR_STATE, key_idx ? "no GHASH key table for the resident key table (tac_aes_gcm_hash_key_table)"
-                                                          : "no GHASH key table for the resident key schedule (tac_aes_gcm_hash_key)");
-    return TAC_OK;
+// every check of an AES-GCM call
+int gcm_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, const uint64_t* pt_out, const uint64_t* valid_out,
+              KeySet** ks, uint64_t* pt_bytes) {
+    TRY(records_check(ctx, n_msgs, key_idx, msgs, gcm_shape, "AES-GCM record",
+                      "need a 12-byte IV, a tag length in {4, 8, 12, 13, 14, 15, 16}, data_len >= tag_len, a payload of at most 2^36 − 32 "
+                      "bytes, AAD below 2^61 bytes and no NULL pointer with a non-zero length",
+                      0, ks, pt_bytes));
+    if (!(*ks)->gcm.valid) return fail(ctx, TAC_ERR_STATE, (*ks)->no_gcm);
+    return outputs_check(ctx, n_msgs, *pt_bytes, pt_out, valid_out);
 }
 
 // AES-GCM transciphering of n records.  1. One public-block call over J0 of every record (rows 0..n−1, sorted order) and
@@ -1029,11 +1086,11 @@ int gcm_check(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_ms
 // (squared noise <= max) or, in a record's last step, the tag difference D = MSB_t(E(J0) ⊕ S) ⊕ T (bytes >= t trivial
 // zero).  3. CCM's three zero-test passes reduce D to the validity bit.
 int aes_gcm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out, uint64_t* valid_out) {
-    uint64_t pt_bytes = 0;
-    TRY(gcm_check(ctx, n_msgs, key_idx, msgs, &pt_bytes));
-    if ((n_msgs > 0 && !valid_out) || (pt_bytes > 0 && !pt_out)) return fail(ctx, TAC_ERR_ARG, "NULL output");
+    KeySet* ks;
+    uint64_t pt_bytes;
+    TRY(gcm_check(ctx, n_msgs, key_idx, msgs, pt_out, valid_out, &ks, &pt_bytes));
     if (n_msgs == 0) return TAC_OK;
-    const tac_ctx::GcmTable& tab = key_idx ? ctx->gcm_h_keyed : ctx->gcm_h;
+    const GcmTable& tab = ks->gcm;
     const int n = n_msgs, w = tab.depth, maxn = ctx->p.max_noise_sq;
     std::vector<GcmShape> sh(n);
     std::vector<int64_t> chunks(n);
@@ -1069,8 +1126,8 @@ int aes_gcm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_
     TRY(ensure(ctx, ctx->ccm_work, (size_t)n * 18 * L * 8));
     uint64_t* pub = ctx->gcm_pub.as<uint64_t>();
     uint64_t* dy = ctx->gcm_dy.as<uint64_t>();             // [n][128]: D in caller order, then [n][128]: Y in sorted order
-    TRY(aes_blocks_dev(ctx, AesDir::Forward, key_idx ? ctx->key_table.as<uint64_t>() : ctx->key_sched, key_idx ? kidx.data() : nullptr, (int)rows, 10, 0,
-                       nullptr, blocks.data(), xr.data(), pub));
+    TRY(aes_blocks_dev(ctx, AesDir::Forward, ks->w.as<uint64_t>(), key_idx ? kidx.data() : nullptr, (int)rows, 10, 0, nullptr, blocks.data(), xr.data(),
+                       pub));
     // GHASH steps
     std::vector<std::vector<uint8_t>> X(n);
     for (int c = 0; c < n; c++) {
@@ -1118,11 +1175,7 @@ int aes_gcm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_
         if (lin_plan_build(lrows, maxn, maxn, 3, plan)) return fail(ctx, TAC_ERR_NOISE, "GHASH: the sums do not fit max_noise_level_squared");
         TRY(lin_run(ctx, plan, {tab.buf.as<uint64_t>(), ctx->gf_prod.p ? ctx->gf_prod.as<uint64_t>() : pub, pub}, &orow, dy));
     }
-    uint64_t* zero = ctx->ccm_work.as<uint64_t>();          // [n][16][L]: byte b of D is zero
-    uint64_t* ones = zero + (size_t)n * 16 * L;              // [n][2][L]: bytes 0..7 / 8..15 all zero
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_zero8], 16 * n, dy, zero));
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones8], 2 * n, zero, ones));
-    TRY(wopbs_dev(ctx, ctx->luts[ctx->ccm_lut_ones2], n, ones, valid_out));
+    TRY(tag_validity(ctx, n, dy, ctx->ccm_work.as<uint64_t>(), valid_out));
     // plaintext: the first p bytes of a record's counter rows, contiguous, into its place in the caller's order
     uint64_t off = 0;
     for (int c = 0; c < n; c++) {
@@ -1130,6 +1183,28 @@ int aes_gcm_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_
             CU(cudaMemcpyAsync(pt_out + off * byte_words, pub + (size_t)pt_row[c] * blk, sh[c].p * byte_words * 8, cudaMemcpyDeviceToDevice, ctx->stream));
         off += sh[c].p;
     }
+    return TAC_OK;
+}
+
+// host form of tac_aes_{ccm,gcm}_transcipher: check (ccm_check / gcm_check) against the host outputs, dev
+// (aes_ccm_dev / aes_gcm_dev) into ws_out, then the plaintext and validity bits back
+using RecordCheck = int (*)(tac_ctx*, int, const int32_t*, const tac_ccm_msg*, const uint64_t*, const uint64_t*, KeySet**, uint64_t*);
+using RecordDev = int (*)(tac_ctx*, int, const int32_t*, const tac_ccm_msg*, uint64_t*, uint64_t*);
+int records_host(tac_ctx* ctx, RecordCheck check, RecordDev dev, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_host,
+                 uint64_t* valid_out_host) {
+    LOCK(ctx);
+    CU(cudaSetDevice(ctx->device));
+    KeySet* ks;
+    uint64_t pt_bytes;
+    TRY(check(ctx, n_msgs, key_idx, msgs, pt_out_host, valid_out_host, &ks, &pt_bytes));
+    if (n_msgs == 0) return TAC_OK;
+    const size_t L = (size_t)ctx->big() + 1, pt_words = (size_t)pt_bytes * 8 * L, valid_words = (size_t)n_msgs * L;
+    TRY(ensure(ctx, ctx->ws_out, (pt_words + valid_words) * 8));
+    uint64_t* pt = ctx->ws_out.as<uint64_t>();
+    TRY(dev(ctx, n_msgs, key_idx, msgs, pt, pt + pt_words));
+    if (pt_words) CU(cudaMemcpyAsync(pt_out_host, pt, pt_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(valid_out_host, pt + pt_words, valid_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
     return TAC_OK;
 }
 
@@ -1167,8 +1242,8 @@ tac_ctx* tac_ctx_create(const tac_params* pp, int device) {
     // combined twist/twiddle table in extended precision
     std::vector<cplx> w(tab_len(p.N));
     build_wT(p.N, w.data());
-    if (cudaMalloc(&ctx->wT, w.size() * sizeof(cplx)) != cudaSuccess) return bail("cudaMalloc(tables) failed");
-    cudaMemcpy(ctx->wT, w.data(), w.size() * sizeof(cplx), cudaMemcpyHostToDevice);
+    if (ensure(ctx, ctx->wT, w.size() * sizeof(cplx))) return bail("cudaMalloc(tables) failed");
+    cudaMemcpy(ctx->wT.p, w.data(), w.size() * sizeof(cplx), cudaMemcpyHostToDevice);
     return ctx;
 }
 
@@ -1176,19 +1251,10 @@ void tac_ctx_destroy(tac_ctx* ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
-    for (void* p : {(void*)ctx->bsk_f, (void*)ctx->ksk, (void*)ctx->pfpksk, (void*)ctx->ks_corr, (void*)ctx->pfks_corr, (void*)ctx->pfks_planes, (void*)ctx->ks_planes, (void*)ctx->pfks_fix, (void*)ctx->wT,
-                    (void*)ctx->key_sched, (void*)ctx->inv_key_sched, (void*)ctx->rc_rows})
-        if (p) cudaFree(p);
     for (auto& l : ctx->luts) cudaFree(l.dev);
-    for (DevBuf* b : {&ctx->ws_in, &ctx->ws_out, &ctx->ws_small, &ctx->ws_ksdig, &ctx->ws_pbs, &ctx->ws_pfdig, &ctx->ws_ggsw, &ctx->ws_ggswf,
-                      &ctx->ws_tree_a, &ctx->ws_tree_b, &ctx->ws_state, &ctx->ws_muls, &ctx->ws_misc, &ctx->ws_plan, &ctx->ws_rep,
-                      &ctx->key_table, &ctx->inv_key_table, &ctx->ccm_pub, &ctx->ccm_work, &ctx->ccm_desc, &ctx->gcm_h.buf,
-                      &ctx->gcm_h_keyed.buf, &ctx->lin_desc, &ctx->lin_sum, &ctx->lin_lvl, &ctx->gf_idx, &ctx->gf_box, &ctx->gf_ops,
-                      &ctx->gf_prod, &ctx->gcm_pub, &ctx->gcm_dy})
-        if (b->p) cudaFree(b->p);
     for (auto& r : ctx->prof_pool) for (auto& ev : r.ev) cudaEventDestroy(ev);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;             // the DevBufs free the rest
 }
 
 int tac_ctx_set_stream(tac_ctx* ctx, void* s) {
@@ -1247,19 +1313,17 @@ int tac_ctx_alloc_keys(tac_ctx* ctx) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (ctx->keys_allocated) return TAC_OK;
-    CU(cudaMalloc(&ctx->bsk_f, ctx->bsk_cplx() * sizeof(cplx)));
-    CU(cudaMalloc(&ctx->ksk, ctx->ksk_words() * 8));
-    CU(cudaMalloc(&ctx->pfpksk, ctx->pfpksk_words() * 8));
-    CU(cudaMalloc(&ctx->ks_corr, (size_t)(ctx->p.n + 1) * 8));
-    CU(cudaMalloc(&ctx->pfks_corr, (size_t)ctx->G() * ctx->G() * ctx->p.N * 8));
-    {
-        const int Kd = (ctx->big() + 1) * ctx->p.pfks_l, nkb = (Kd + UG_KB - 1) / UG_KB;
-        const int W = ctx->G() * ctx->p.N, tiles = (W + UG_NT - 1) / UG_NT;
-        CU(cudaMalloc(&ctx->pfks_planes, (size_t)ctx->G() * tiles * nkb * UG_B_BYTES));
-        CU(cudaMalloc(&ctx->pfks_fix, 8 + (size_t)kFixCap * 8));
-        const int Kd_ks = ctx->big() * ctx->p.ks_l, nkb_ks = (Kd_ks + UG_KB - 1) / UG_KB, tiles_ks = (ctx->p.n + 1 + UG_NT - 1) / UG_NT;
-        CU(cudaMalloc(&ctx->ks_planes, (size_t)tiles_ks * nkb_ks * UG_B_BYTES));
-    }
+    const int Kd = (ctx->big() + 1) * ctx->p.pfks_l, nkb = (Kd + UG_KB - 1) / UG_KB;
+    const int W = ctx->G() * ctx->p.N, tiles = (W + UG_NT - 1) / UG_NT;
+    const int Kd_ks = ctx->big() * ctx->p.ks_l, nkb_ks = (Kd_ks + UG_KB - 1) / UG_KB, tiles_ks = (ctx->p.n + 1 + UG_NT - 1) / UG_NT;
+    TRY(ensure(ctx, ctx->bsk_f, ctx->bsk_cplx() * sizeof(cplx), "the bootstrapping key"));
+    TRY(ensure(ctx, ctx->ksk, ctx->ksk_words() * 8, "the keyswitching key"));
+    TRY(ensure(ctx, ctx->pfpksk, ctx->pfpksk_words() * 8, "the private functional packing keyswitching keys"));
+    TRY(ensure(ctx, ctx->ks_corr, (size_t)(ctx->p.n + 1) * 8));
+    TRY(ensure(ctx, ctx->pfks_corr, (size_t)ctx->G() * ctx->G() * ctx->p.N * 8));
+    TRY(ensure(ctx, ctx->pfks_planes, (size_t)ctx->G() * tiles * nkb * UG_B_BYTES));
+    TRY(ensure(ctx, ctx->pfks_fix, 8 + (size_t)kFixCap * 8));
+    TRY(ensure(ctx, ctx->ks_planes, (size_t)tiles_ks * nkb_ks * UG_B_BYTES));
     ctx->keys_allocated = true;
     return TAC_OK;
 }
@@ -1267,9 +1331,9 @@ int tac_ctx_key_buffer(tac_ctx* ctx, int which, void** dev_ptr, size_t* bytes) {
     LOCK(ctx);
     if (!ctx->keys_allocated) return fail(ctx, TAC_ERR_STATE, "key buffers not allocated");
     switch (which) {
-        case 0: *dev_ptr = ctx->bsk_f; *bytes = ctx->bsk_cplx() * sizeof(cplx); return TAC_OK;
-        case 1: *dev_ptr = ctx->ksk; *bytes = ctx->ksk_words() * 8; return TAC_OK;
-        case 2: *dev_ptr = ctx->pfpksk; *bytes = ctx->pfpksk_words() * 8; return TAC_OK;
+        case 0: *dev_ptr = ctx->bsk_f.p; *bytes = ctx->bsk_cplx() * sizeof(cplx); return TAC_OK;
+        case 1: *dev_ptr = ctx->ksk.p; *bytes = ctx->ksk_words() * 8; return TAC_OK;
+        case 2: *dev_ptr = ctx->pfpksk.p; *bytes = ctx->pfpksk_words() * 8; return TAC_OK;
         default: return fail(ctx, TAC_ERR_ARG, "key buffer index");
     }
 }
@@ -1285,25 +1349,25 @@ int tac_ctx_keys_ready(tac_ctx* ctx) {
     std::vector<uint32_t> h(Kmax);
     std::fill(h.begin(), h.end(), 1u << (p.ks_b - 1));
     CU(cudaMemcpyAsync(ctx->ws_misc.p, h.data(), (size_t)Kd_ks * 4, cudaMemcpyHostToDevice, ctx->stream));
-    TRY(gemm(ctx, ctx->ws_misc.as<uint32_t>(), 1, Kd_ks, ctx->ksk, p.n + 1, 1, nullptr, nullptr, 0, ctx->ks_corr));
-    negate_kernel<<<grid1d(p.n + 1, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->ks_corr, (size_t)p.n + 1);
+    TRY(gemm(ctx, ctx->ws_misc.as<uint32_t>(), 1, Kd_ks, ctx->ksk.as<uint64_t>(), p.n + 1, 1, nullptr, nullptr, 0, ctx->ks_corr.as<uint64_t>()));
+    negate_kernel<<<grid1d(p.n + 1, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->ks_corr.as<uint64_t>(), (size_t)p.n + 1);
     TRY(post_launch(ctx, "negate_kernel"));
     CU(cudaStreamSynchronize(ctx->stream));
     std::fill(h.begin(), h.end(), 1u << (p.pfks_b - 1));
     CU(cudaMemcpyAsync(ctx->ws_misc.p, h.data(), (size_t)Kd_pf * 4, cudaMemcpyHostToDevice, ctx->stream));
     const size_t W = (size_t)ctx->G() * p.N;
-    TRY(gemm(ctx, ctx->ws_misc.as<uint32_t>(), 1, Kd_pf, ctx->pfpksk, (int)W, ctx->G(), nullptr, nullptr, 0, ctx->pfks_corr));
-    negate_kernel<<<grid1d(W * ctx->G(), 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->pfks_corr, W * ctx->G());
+    TRY(gemm(ctx, ctx->ws_misc.as<uint32_t>(), 1, Kd_pf, ctx->pfpksk.as<uint64_t>(), (int)W, ctx->G(), nullptr, nullptr, 0, ctx->pfks_corr.as<uint64_t>()));
+    negate_kernel<<<grid1d(W * ctx->G(), 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->pfks_corr.as<uint64_t>(), W * ctx->G());
     TRY(post_launch(ctx, "negate_kernel"));
     CU(cudaStreamSynchronize(ctx->stream));
     {   // byte-plane tiles of the PFPKSK and the KSK for the tcgen05 GEMM
         const int nkb = (Kd_pf + UG_KB - 1) / UG_KB, tiles = ((int)W + UG_NT - 1) / UG_NT;
         const size_t units = (size_t)ctx->G() * tiles * nkb * 2 * UG_NT;
-        umma_key_tiles_kernel<<<grid1d(units, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->pfpksk, ctx->G(), Kd_pf, (int)W, nkb, ctx->pfks_planes);
+        umma_key_tiles_kernel<<<grid1d(units, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->pfpksk.as<uint64_t>(), ctx->G(), Kd_pf, (int)W, nkb, ctx->pfks_planes.as<uint8_t>());
         TRY(post_launch(ctx, "umma_key_tiles_kernel(pfks)"));
         const int nkb_ks = (Kd_ks + UG_KB - 1) / UG_KB, tiles_ks = (p.n + 1 + UG_NT - 1) / UG_NT;
         const size_t units_ks = (size_t)tiles_ks * nkb_ks * 2 * UG_NT;
-        umma_key_tiles_kernel<<<grid1d(units_ks, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->ksk, 1, Kd_ks, p.n + 1, nkb_ks, ctx->ks_planes);
+        umma_key_tiles_kernel<<<grid1d(units_ks, 256, ctx->sm_count), 256, 0, ctx->stream>>>(ctx->ksk.as<uint64_t>(), 1, Kd_ks, p.n + 1, nkb_ks, ctx->ks_planes.as<uint8_t>());
         TRY(post_launch(ctx, "umma_key_tiles_kernel(ks)"));
         CU(cudaStreamSynchronize(ctx->stream));
     }
@@ -1314,8 +1378,8 @@ int tac_ctx_upload_keys(tac_ctx* ctx, const uint64_t* bsk_std, const uint64_t* k
     LOCK(ctx);
     TRY(tac_ctx_alloc_keys(ctx));
     const TacParams& p = ctx->p;
-    CU(cudaMemcpyAsync(ctx->ksk, ksk, ctx->ksk_words() * 8, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->pfpksk, pfpksk, ctx->pfpksk_words() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(ctx->ksk.p, ksk, ctx->ksk_words() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(ctx->pfpksk.p, pfpksk, ctx->pfpksk_words() * 8, cudaMemcpyHostToDevice, ctx->stream));
     // BSK: standard → Fourier on the device, in slices ([U] fft64/crypto/bootstrap.rs::fill_with_forward_fourier)
     const size_t polys = (size_t)p.n * p.pbs_l * ctx->G() * ctx->G();
     const size_t slice = 16384;
@@ -1323,7 +1387,7 @@ int tac_ctx_upload_keys(tac_ctx* ctx, const uint64_t* bsk_std, const uint64_t* k
     for (size_t q = 0; q < polys; q += slice) {
         const size_t cnt = std::min(slice, polys - q);
         CU(cudaMemcpyAsync(ctx->ws_misc.p, bsk_std + q * p.N, cnt * p.N * 8, cudaMemcpyHostToDevice, ctx->stream));
-        TRY(poly_fft(ctx, ctx->ws_misc.as<uint64_t>(), cnt, ctx->bsk_f + q * (p.N / 2)));
+        TRY(poly_fft(ctx, ctx->ws_misc.as<uint64_t>(), cnt, ctx->bsk_f.as<cplx>() + q * (p.N / 2)));
         CU(cudaStreamSynchronize(ctx->stream));
     }
     return tac_ctx_keys_ready(ctx);
@@ -1495,45 +1559,28 @@ int tac_lwe_add_batch(tac_ctx* ctx, uint64_t* a_host, const uint64_t* b_host, si
 int tac_aes_set_key_schedule(tac_ctx* ctx, const uint64_t* ks_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
-    const size_t bytes = (size_t)44 * 32 * (ctx->big() + 1) * 8;
-    if (!ctx->key_sched) CU(cudaMalloc(&ctx->key_sched, bytes));
-    ctx->inv_key_sched_valid = false;        // an inverse schedule belongs to the encryption schedule it was made from
-    ctx->gcm_h.valid = false;                // and so does a GHASH key table
-    if (ks_host) {
-        CU(cudaMemcpyAsync(ctx->key_sched, ks_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
-        CU(cudaStreamSynchronize(ctx->stream));
-    }
-    return TAC_OK;
+    return ks_set(ctx, ctx->single, 1, ks_host);
 }
 int tac_aes_key_schedule_buffer(tac_ctx* ctx, void** dev_ptr, size_t* bytes) {
     LOCK(ctx);
-    TRY(tac_aes_set_key_schedule(ctx, nullptr));
-    *dev_ptr = ctx->key_sched; *bytes = (size_t)44 * 32 * (ctx->big() + 1) * 8;
+    CU(cudaSetDevice(ctx->device));
+    TRY(ks_set(ctx, ctx->single, 1, nullptr));
+    *dev_ptr = ctx->single.w.p; *bytes = key_sched_bytes(ctx);
     return TAC_OK;
 }
 
 int tac_aes_encrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_dev, uint64_t* out_dev) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    return aes_blocks_dev(ctx, AesDir::Forward, ctx->key_sched, nullptr, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
+    return aes_call(ctx, AesDir::Forward, false, nullptr, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev, false);
 }
 int tac_aes_encrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host) {
-    return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
-        return tac_aes_encrypt_blocks_dev(ctx, n_blocks, rounds, in_noise_sq, in, out);
-    });
+    return aes_call(ctx, AesDir::Forward, false, nullptr, n_blocks, rounds, in_noise_sq, in_host, nullptr, nullptr, out_host, true);
 }
-
+// trivial input: no noise of its own
 int tac_aes_encrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    return aes_blocks_dev(ctx, AesDir::Forward, ctx->key_sched, nullptr, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);   // trivial input: no noise of its own
+    return aes_call(ctx, AesDir::Forward, false, nullptr, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev, false);
 }
 int tac_aes_encrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
-    return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
-        return tac_aes_encrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, out);
-    });
+    return aes_call(ctx, AesDir::Forward, false, nullptr, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_host, true);
 }
 
 // ------------------------------------------------------------------------------------ AES decryption (FIPS-197 §5.3.5)
@@ -1541,69 +1588,40 @@ int tac_aes_encrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const 
 // bootstrap per byte, so a middle round sums 4 outputs of squared noise 8 and one round key of level 1: 33, as in the
 // forward direction.  Round keys are read from dk only.
 int tac_aes_decrypt_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_dev, uint64_t* out_dev) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    TRY(inv_key_sched_check(ctx));
-    return aes_blocks_dev(ctx, AesDir::Inverse, ctx->inv_key_sched, nullptr, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
+    return aes_call(ctx, AesDir::Inverse, false, nullptr, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev, false);
 }
 int tac_aes_decrypt_blocks(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const uint64_t* in_host, uint64_t* out_host) {
-    return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
-        return tac_aes_decrypt_blocks_dev(ctx, n_blocks, rounds, in_noise_sq, in, out);
-    });
+    return aes_call(ctx, AesDir::Inverse, false, nullptr, n_blocks, rounds, in_noise_sq, in_host, nullptr, nullptr, out_host, true);
 }
 
 // decryption of PUBLIC ciphertext blocks (AES-ECB / AES-CBC transciphering): state0 = dk[40..43] + trivial(block), the
 // plan runs along the inverse dependence rule, xor_host (the previous ciphertext blocks for CBC) joins the final round
 int tac_aes_decrypt_public_blocks_dev(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_dev) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    TRY(inv_key_sched_check(ctx));
-    return aes_blocks_dev(ctx, AesDir::Inverse, ctx->inv_key_sched, nullptr, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);   // trivial input: no noise of its own
+    return aes_call(ctx, AesDir::Inverse, false, nullptr, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev, false);
 }
 int tac_aes_decrypt_public_blocks(tac_ctx* ctx, int n_blocks, int rounds, const uint8_t* blocks_host, const uint8_t* xor_host, uint64_t* out_host) {
-    return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
-        return tac_aes_decrypt_public_blocks_dev(ctx, n_blocks, rounds, blocks_host, xor_host, out);
-    });
+    return aes_call(ctx, AesDir::Inverse, false, nullptr, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_host, true);
 }
 
 // inverse key schedule on the device from the resident encryption schedule (inv_key_expand with one key)
 int tac_aes_inv_key_schedule(tac_ctx* ctx, uint64_t* out_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
-    if (!ctx->key_sched) return fail(ctx, TAC_ERR_STATE, "no key schedule on the device (tac_aes_set_key_schedule)");
-    TRY(inv_key_schedule_noise_check(ctx));
-    if (!ctx->inv_key_sched) CU(cudaMalloc(&ctx->inv_key_sched, key_sched_bytes(ctx)));
-    ctx->inv_key_sched_valid = false;
-    TRY(inv_key_expand(ctx, 1, ctx->key_sched, ctx->inv_key_sched));
-    if (out_host) CU(cudaMemcpyAsync(out_host, ctx->inv_key_sched, key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->inv_key_sched_valid = true;
-    return TAC_OK;
+    return ks_invert(ctx, ctx->single, out_host);
 }
 int tac_aes_set_inv_key_schedule(tac_ctx* ctx, const uint64_t* dk_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (!dk_host) return fail(ctx, TAC_ERR_ARG, "NULL inverse key schedule");
-    const size_t bytes = (size_t)44 * 32 * (ctx->big() + 1) * 8;
-    if (!ctx->inv_key_sched) CU(cudaMalloc(&ctx->inv_key_sched, bytes));
-    ctx->inv_key_sched_valid = false;
-    CU(cudaMemcpyAsync(ctx->inv_key_sched, dk_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->inv_key_sched_valid = true;
-    return TAC_OK;
+    return ks_set_inv(ctx, ctx->single, 1, dk_host);
 }
 
 // fhe_sbox_gal_mul_pbs::key_schedule (:134-164): key_expand with one key, into the single schedule
 int tac_aes_key_schedule(tac_ctx* ctx, const uint64_t* key_bits_host, uint64_t* out_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
-    TRY(key_schedule_noise_check(ctx));
-    TRY(ensure_aes_luts(ctx));
-    TRY(tac_aes_set_key_schedule(ctx, nullptr));
-    TRY(key_expand(ctx, 1, key_bits_host, ctx->key_sched));
-    if (out_host) CU(cudaMemcpyAsync(out_host, ctx->key_sched, key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return TAC_OK;
+    if (!key_bits_host) return fail(ctx, TAC_ERR_ARG, "NULL key bits");
+    return ks_expand(ctx, ctx->single, 1, key_bits_host, out_host);
 }
 
 // ------------------------------------------------------------------------------------------------ AES under many keys
@@ -1614,120 +1632,63 @@ int tac_aes_key_table(tac_ctx* ctx, int n_keys, const uint64_t* key_bits_host, u
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (n_keys < 1 || !key_bits_host) return fail(ctx, TAC_ERR_ARG, "need n_keys >= 1 and key bits");
-    TRY(key_schedule_noise_check(ctx));
-    ctx->n_keys = 0;
-    ctx->inv_key_table_valid = false;
-    ctx->gcm_h_keyed.valid = false;
-    TRY(alloc_key_table(ctx, ctx->key_table, n_keys));
-    TRY(key_expand(ctx, n_keys, key_bits_host, ctx->key_table.as<uint64_t>()));
-    if (key_scheds_host) CU(cudaMemcpyAsync(key_scheds_host, ctx->key_table.p, (size_t)n_keys * key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->n_keys = n_keys;
-    return TAC_OK;
+    return ks_expand(ctx, ctx->table, n_keys, key_bits_host, key_scheds_host);
 }
 int tac_aes_set_key_table(tac_ctx* ctx, int n_keys, const uint64_t* key_scheds_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
     if (n_keys < 1 || !key_scheds_host) return fail(ctx, TAC_ERR_ARG, "need n_keys >= 1 and key schedules");
-    ctx->n_keys = 0;
-    ctx->inv_key_table_valid = false;
-    ctx->gcm_h_keyed.valid = false;
-    TRY(alloc_key_table(ctx, ctx->key_table, n_keys));
-    CU(cudaMemcpyAsync(ctx->key_table.p, key_scheds_host, (size_t)n_keys * key_sched_bytes(ctx), cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->n_keys = n_keys;
-    return TAC_OK;
+    return ks_set(ctx, ctx->table, n_keys, key_scheds_host);
 }
 int tac_aes_inv_key_table(tac_ctx* ctx, uint64_t* inv_key_scheds_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
-    if (ctx->n_keys < 1) return fail(ctx, TAC_ERR_STATE, "no key table on the device (tac_aes_key_table or tac_aes_set_key_table)");
-    TRY(inv_key_schedule_noise_check(ctx));
-    ctx->inv_key_table_valid = false;
-    TRY(alloc_key_table(ctx, ctx->inv_key_table, ctx->n_keys));
-    TRY(inv_key_expand(ctx, ctx->n_keys, ctx->key_table.as<uint64_t>(), ctx->inv_key_table.as<uint64_t>()));
-    if (inv_key_scheds_host)
-        CU(cudaMemcpyAsync(inv_key_scheds_host, ctx->inv_key_table.p, (size_t)ctx->n_keys * key_sched_bytes(ctx), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->inv_key_table_valid = true;
-    return TAC_OK;
+    return ks_invert(ctx, ctx->table, inv_key_scheds_host);
 }
 int tac_aes_set_inv_key_table(tac_ctx* ctx, const uint64_t* inv_key_scheds_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
-    if (ctx->n_keys < 1) return fail(ctx, TAC_ERR_STATE, "no key table on the device (tac_aes_key_table or tac_aes_set_key_table)");
+    if (ctx->table.n < 1) return fail(ctx, TAC_ERR_STATE, ctx->table.absent);
     if (!inv_key_scheds_host) return fail(ctx, TAC_ERR_ARG, "NULL inverse key schedules");
-    ctx->inv_key_table_valid = false;
-    TRY(alloc_key_table(ctx, ctx->inv_key_table, ctx->n_keys));
-    CU(cudaMemcpyAsync(ctx->inv_key_table.p, inv_key_scheds_host, (size_t)ctx->n_keys * key_sched_bytes(ctx), cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    ctx->inv_key_table_valid = true;
-    return TAC_OK;
+    return ks_set_inv(ctx, ctx->table, ctx->table.n, inv_key_scheds_host);
 }
 
 int tac_aes_encrypt_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_dev,
                                      uint64_t* out_dev) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    TRY(key_table_check(ctx, AesDir::Forward, n_blocks, key_idx_host));
-    return aes_blocks_dev(ctx, AesDir::Forward, ctx->key_table.as<uint64_t>(), key_idx_host, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
+    return aes_call(ctx, AesDir::Forward, true, key_idx_host, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev, false);
 }
 int tac_aes_encrypt_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_host,
                                  uint64_t* out_host) {
-    LOCK(ctx);
-    TRY(key_table_check(ctx, AesDir::Forward, n_blocks, key_idx_host));
-    return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
-        return tac_aes_encrypt_blocks_keyed_dev(ctx, n_blocks, rounds, in_noise_sq, key_idx_host, in, out);
-    });
+    return aes_call(ctx, AesDir::Forward, true, key_idx_host, n_blocks, rounds, in_noise_sq, in_host, nullptr, nullptr, out_host, true);
 }
 int tac_aes_encrypt_public_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
                                             const uint8_t* xor_host, uint64_t* out_dev) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    TRY(key_table_check(ctx, AesDir::Forward, n_blocks, key_idx_host));
-    return aes_blocks_dev(ctx, AesDir::Forward, ctx->key_table.as<uint64_t>(), key_idx_host, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);
+    return aes_call(ctx, AesDir::Forward, true, key_idx_host, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev, false);
 }
 int tac_aes_encrypt_public_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
                                         const uint8_t* xor_host, uint64_t* out_host) {
-    LOCK(ctx);
-    TRY(key_table_check(ctx, AesDir::Forward, n_blocks, key_idx_host));
-    return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
-        return tac_aes_encrypt_public_blocks_keyed_dev(ctx, n_blocks, rounds, key_idx_host, blocks_host, xor_host, out);
-    });
+    return aes_call(ctx, AesDir::Forward, true, key_idx_host, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_host, true);
 }
 int tac_aes_decrypt_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_dev,
                                      uint64_t* out_dev) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    TRY(key_table_check(ctx, AesDir::Inverse, n_blocks, key_idx_host));
-    return aes_blocks_dev(ctx, AesDir::Inverse, ctx->inv_key_table.as<uint64_t>(), key_idx_host, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev);
+    return aes_call(ctx, AesDir::Inverse, true, key_idx_host, n_blocks, rounds, in_noise_sq, in_dev, nullptr, nullptr, out_dev, false);
 }
 int tac_aes_decrypt_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, int in_noise_sq, const int32_t* key_idx_host, const uint64_t* in_host,
                                  uint64_t* out_host) {
-    LOCK(ctx);
-    TRY(key_table_check(ctx, AesDir::Inverse, n_blocks, key_idx_host));
-    return aes_blocks_host(ctx, n_blocks, true, in_host, out_host, [&](const uint64_t* in, uint64_t* out) {
-        return tac_aes_decrypt_blocks_keyed_dev(ctx, n_blocks, rounds, in_noise_sq, key_idx_host, in, out);
-    });
+    return aes_call(ctx, AesDir::Inverse, true, key_idx_host, n_blocks, rounds, in_noise_sq, in_host, nullptr, nullptr, out_host, true);
 }
 int tac_aes_decrypt_public_blocks_keyed_dev(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
                                             const uint8_t* xor_host, uint64_t* out_dev) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    TRY(key_table_check(ctx, AesDir::Inverse, n_blocks, key_idx_host));
-    return aes_blocks_dev(ctx, AesDir::Inverse, ctx->inv_key_table.as<uint64_t>(), key_idx_host, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev);
+    return aes_call(ctx, AesDir::Inverse, true, key_idx_host, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_dev, false);
 }
 int tac_aes_decrypt_public_blocks_keyed(tac_ctx* ctx, int n_blocks, int rounds, const int32_t* key_idx_host, const uint8_t* blocks_host,
                                         const uint8_t* xor_host, uint64_t* out_host) {
-    LOCK(ctx);
-    TRY(key_table_check(ctx, AesDir::Inverse, n_blocks, key_idx_host));
-    return aes_blocks_host(ctx, n_blocks, false, nullptr, out_host, [&](const uint64_t*, uint64_t* out) {
-        return tac_aes_decrypt_public_blocks_keyed_dev(ctx, n_blocks, rounds, key_idx_host, blocks_host, xor_host, out);
-    });
+    return aes_call(ctx, AesDir::Inverse, true, key_idx_host, n_blocks, rounds, 0, nullptr, blocks_host, xor_host, out_host, true);
 }
 
-// ------------------------------------------------------------------------------------------------ AES-CCM transciphering
-// aes_ccm_dev under the single resident schedule (key_idx NULL) or the key table; the context lock is taken here only
+// ------------------------------------------------------------------------------------------------ AES-CCM / AES-GCM transciphering
+// key_idx NULL: every record under the single resident schedule, else record i under key table entry key_idx[i].  The
+// context lock is taken here only.
 int tac_aes_ccm_transcipher_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_dev,
                                 uint64_t* valid_out_dev) {
     LOCK(ctx);
@@ -1736,23 +1697,8 @@ int tac_aes_ccm_transcipher_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx
 }
 int tac_aes_ccm_transcipher(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_host,
                             uint64_t* valid_out_host) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    uint64_t pt_bytes = 0;
-    TRY(ccm_check(ctx, n_msgs, key_idx, msgs, &pt_bytes));
-    if ((n_msgs > 0 && !valid_out_host) || (pt_bytes > 0 && !pt_out_host)) return fail(ctx, TAC_ERR_ARG, "NULL output");
-    if (n_msgs == 0) return TAC_OK;
-    const size_t L = (size_t)ctx->big() + 1, pt_words = (size_t)pt_bytes * 8 * L, valid_words = (size_t)n_msgs * L;
-    TRY(ensure(ctx, ctx->ws_out, (pt_words + valid_words) * 8));
-    uint64_t* pt = ctx->ws_out.as<uint64_t>();
-    TRY(aes_ccm_dev(ctx, n_msgs, key_idx, msgs, pt, pt + pt_words));
-    if (pt_words) CU(cudaMemcpyAsync(pt_out_host, pt, pt_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaMemcpyAsync(valid_out_host, pt + pt_words, valid_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return TAC_OK;
+    return records_host(ctx, ccm_check, aes_ccm_dev, n_msgs, key_idx, msgs, pt_out_host, valid_out_host);
 }
-
-// ------------------------------------------------------------------------------------------------ AES-GCM transciphering
 int tac_aes_gcm_hash_key(tac_ctx* ctx, int depth, uint64_t* out_host) {
     LOCK(ctx);
     CU(cudaSetDevice(ctx->device));
@@ -1771,20 +1717,7 @@ int tac_aes_gcm_transcipher_dev(tac_ctx* ctx, int n_msgs, const int32_t* key_idx
 }
 int tac_aes_gcm_transcipher(tac_ctx* ctx, int n_msgs, const int32_t* key_idx, const tac_ccm_msg* msgs, uint64_t* pt_out_host,
                             uint64_t* valid_out_host) {
-    LOCK(ctx);
-    CU(cudaSetDevice(ctx->device));
-    uint64_t pt_bytes = 0;
-    TRY(gcm_check(ctx, n_msgs, key_idx, msgs, &pt_bytes));
-    if ((n_msgs > 0 && !valid_out_host) || (pt_bytes > 0 && !pt_out_host)) return fail(ctx, TAC_ERR_ARG, "NULL output");
-    if (n_msgs == 0) return TAC_OK;
-    const size_t L = (size_t)ctx->big() + 1, pt_words = (size_t)pt_bytes * 8 * L, valid_words = (size_t)n_msgs * L;
-    TRY(ensure(ctx, ctx->ws_out, (pt_words + valid_words) * 8));
-    uint64_t* pt = ctx->ws_out.as<uint64_t>();
-    TRY(aes_gcm_dev(ctx, n_msgs, key_idx, msgs, pt, pt + pt_words));
-    if (pt_words) CU(cudaMemcpyAsync(pt_out_host, pt, pt_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaMemcpyAsync(valid_out_host, pt + pt_words, valid_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    return TAC_OK;
+    return records_host(ctx, gcm_check, aes_gcm_dev, n_msgs, key_idx, msgs, pt_out_host, valid_out_host);
 }
 
 // ------------------------------------------------------------------------------------------------ single stages

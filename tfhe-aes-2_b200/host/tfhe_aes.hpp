@@ -439,27 +439,7 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
     };
     static std::vector<std::pair<std::vector<Byte>, BitCt>> ccm_transcipher(const Ctx& c, const std::vector<CcmRecord>& records,
                                                                              const std::vector<int32_t>& key_idx = {}) {
-        if (!key_idx.empty() && key_idx.size() != records.size()) throw std::invalid_argument("key_idx: one key index per record");
-        std::vector<tac_ccm_msg> msgs(records.size());
-        std::vector<size_t> off(records.size() + 1, 0);
-        for (size_t i = 0; i < records.size(); i++) {
-            const CcmRecord& r = records[i];
-            msgs[i] = tac_ccm_msg{r.nonce.data(), (int32_t)r.nonce.size(), r.tag_len, r.aad.data(), r.aad.size(), r.data.data(), r.data.size()};
-            off[i + 1] = off[i] + (r.data.size() >= (size_t)std::max(r.tag_len, 0) ? r.data.size() - r.tag_len : 0);
-        }
-        const size_t L = c.lwe_size();
-        std::vector<uint64_t> pt(off.back() * 8 * L), valid(records.size() * L);
-        c.check(tac_aes_ccm_transcipher(c.raw(), (int)records.size(), key_idx.empty() ? nullptr : key_idx.data(), msgs.data(), pt.data(), valid.data()));
-        auto bit = [&](const std::vector<uint64_t>& v, size_t idx, uint64_t noise) {
-            return BitCt::with_noise_level(std::vector<uint64_t>(v.begin() + idx * L, v.begin() + (idx + 1) * L), noise, c);
-        };
-        std::vector<std::pair<std::vector<Byte>, BitCt>> res;
-        for (size_t i = 0; i < records.size(); i++) {
-            std::vector<Byte> bytes(off[i + 1] - off[i]);
-            for (size_t b = 0; b < bytes.size(); b++) for (int j = 0; j < 8; j++) bytes[b][j] = bit(pt, (off[i] + b) * 8 + j, 8 + 1);
-            res.emplace_back(std::move(bytes), bit(valid, i, 2));
-        }
-        return res;
+        return transcipher_records(tac_aes_ccm_transcipher, c, records, key_idx);
     }
     // AES-GCM transciphering with the tag checked under FHE (NIST SP 800-38D, 96-bit IVs; the reference has none).  A record
     // is a CcmRecord with nonce = the 12-byte IV and data = C ‖ T.  Needs the GHASH key table of the schedule in use
@@ -468,6 +448,14 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
     static void gcm_hash_key_table(const Ctx& c, int depth = 8) { c.check(tac_aes_gcm_hash_key_table(c.raw(), depth, nullptr)); }
     static std::vector<std::pair<std::vector<Byte>, BitCt>> gcm_transcipher(const Ctx& c, const std::vector<CcmRecord>& records,
                                                                              const std::vector<int32_t>& key_idx = {}) {
+        return transcipher_records(tac_aes_gcm_transcipher, c, records, key_idx);
+    }
+
+private:
+    // fn (tac_aes_ccm_transcipher / tac_aes_gcm_transcipher) over the records
+    static std::vector<std::pair<std::vector<Byte>, BitCt>> transcipher_records(
+        int (*fn)(tac_ctx*, int, const int32_t*, const tac_ccm_msg*, uint64_t*, uint64_t*), const Ctx& c, const std::vector<CcmRecord>& records,
+        const std::vector<int32_t>& key_idx) {
         if (!key_idx.empty() && key_idx.size() != records.size()) throw std::invalid_argument("key_idx: one key index per record");
         std::vector<tac_ccm_msg> msgs(records.size());
         std::vector<size_t> off(records.size() + 1, 0);
@@ -478,7 +466,7 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
         }
         const size_t L = c.lwe_size();
         std::vector<uint64_t> pt(off.back() * 8 * L), valid(records.size() * L);
-        c.check(tac_aes_gcm_transcipher(c.raw(), (int)records.size(), key_idx.empty() ? nullptr : key_idx.data(), msgs.data(), pt.data(), valid.data()));
+        c.check(fn(c.raw(), (int)records.size(), key_idx.empty() ? nullptr : key_idx.data(), msgs.data(), pt.data(), valid.data()));
         auto bit = [&](const std::vector<uint64_t>& v, size_t idx, uint64_t noise) {
             return BitCt::with_noise_level(std::vector<uint64_t>(v.begin() + idx * L, v.begin() + (idx + 1) * L), noise, c);
         };
@@ -490,8 +478,6 @@ struct CudaWoppbs1BitSboxGalMulPbsAesEncrypt {
         }
         return res;
     }
-
-private:
     static std::vector<data_model::BlockT<Bit>> public_blocks_keyed(int (*fn)(tac_ctx*, int, int, const int32_t*, const uint8_t*, const uint8_t*, uint64_t*),
                                                                     const Ctx& c, const std::vector<int32_t>& key_idx,
                                                                     const std::vector<std::array<uint8_t, 16>>& blocks, int rounds,
